@@ -35,7 +35,10 @@ One JSON line is printed by rank 0:
   cpu_baseline  the CPU oracle port (C + OpenMP, all host threads) on a row sample
 --impl reference times the UNMODIFIED reference's em_step (staged copy oracle/_ref,
 see oracle/stage_ref.py) on one core.  --rows N replaces the workload by N
-undeduplicated rows per GPU (config-3 shard sizes).
+undeduplicated rows per GPU (config-3 shard sizes).  --dump-outputs DIR writes the
+log-proportions of the last timed step to DIR/lnprops.npy (bench_outputs/ in the tree is
+git-ignored for this); the workload and the start are seeded, so two builds run with the
+same arguments can be compared on it.
 """
 import argparse
 import json
@@ -81,7 +84,14 @@ def parse_args():
     ap.add_argument("--pageable-result", action="store_true",
                     help="e2e: leave the result in pageable memory (no pinned pool)")
     ap.add_argument("--cpu-rows", type=int, default=0, help="row sample of the CPU legs (0 = auto)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed EM iterations computed in their last step to "
+                         "DIR/<name>.npy, to compare two builds output for output (e.g. "
+                         "bench_outputs, which git ignores)")
+    opts = ap.parse_args()
+    if opts.dump_outputs and opts.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return opts
 
 
 MIXTURE5 = [("H1", 0.6), ("L3e", 0.25), ("U5a1", 0.1), ("M7", 0.04), ("D4a", 0.01)]
@@ -420,6 +430,11 @@ def run_b200(opts):
         wall = time.perf_counter() - t0
         launches = ctx.launch_count - l0
         dev_s = max_over_ranks(el.value / 1e3)
+        # what the last timed step handed back, read before profile() iterates on
+        # (mxb_em_iterate_fixed fails unless all opts.steps iterations ran)
+        if opts.dump_outputs and rank == 0:
+            lnprops = np.empty(h)
+            check(lib.mxb_em_get_lnprops(sess, 0, ptr(lnprops)))
         # per-kernel attribution (an event between the kernels of every iteration), rank-local
         kern = profile(sess, min(opts.steps, 100))
     cells_total = sum_over_ranks(float(n) * h)
@@ -685,6 +700,11 @@ def run_b200(opts):
                           "e2e": build_e2e},
                 "versions": {"numpy": np.__version__, "torch": torch.__version__}}
         print(json.dumps(line))
+        if opts.dump_outputs:
+            # the H log-proportions (float64) the last timed step produced, as
+            # mxb_em_get_lnprops hands them to a caller of the session
+            os.makedirs(opts.dump_outputs, exist_ok=True)
+            np.save(os.path.join(opts.dump_outputs, "lnprops.npy"), lnprops)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()

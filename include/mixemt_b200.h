@@ -231,7 +231,9 @@ int mxb_tile_plan(const int32_t *n_cls, int64_t n_batches, int64_t n_rows, int32
                   int32_t *seg_out, int64_t seg_cap, int32_t *n_cta, int32_t *n_seg,
                   int32_t *n_slots, int32_t *slot_bytes, int32_t *errors);
 
-/* Exactly n_iter iterations without convergence test or host sync (bench);
+/* Exactly n_iter iterations without convergence test or host sync (bench); MXB_ERR_RANGE
+ * when fewer ran (a row's mixture likelihood underflowed and the run stopped for the
+ * log-space step, which only mxb_em_iterate takes);
  * elapsed_ms (nullable) = device time between first and last launch,
  * pass_ms (nullable) = summed device time from the first pass kernel of an iteration to
  * its tail kernel (class sums + pass + gather for tiles; adds an event pair per iteration). */

@@ -872,6 +872,15 @@ int mxb_em_iterate_fixed(mxb_em *em, int64_t n_iter, float *elapsed_ms, float *p
         set_error("EM: a peer rank did not deliver its column sums in time");
         return MXB_ERR_CUDA;
     }
+    // a tail that set done (kDoneNeedsLogStep after a row-likelihood underflow) turned the
+    // remaining launches into no-ops: neither the time nor the proportions are those of n_iter
+    // iterations
+    if (em->host_state[0].done != 0 || em->host_state[0].iters != n_iter) {
+        set_error("mxb_em_iterate_fixed: stopped after %lld of %lld iterations (done = %d)",
+                  (long long)em->host_state[0].iters, (long long)n_iter,
+                  (int)em->host_state[0].done);
+        return MXB_ERR_RANGE;
+    }
     if (elapsed_ms) MXB_CUDA(cudaEventElapsedTime(elapsed_ms, e0, e1));
     if (pass_ms) {
         double total = 0.0;

@@ -177,49 +177,27 @@ def test_table_packing_fuzz_against_live_reference():
     sites (SURVEY F8), mutation counts past the 0.5 cap -- and signatures with repeated and
     unsorted positions and 'N' observations: the product's host tables (HapVarBaseMatrix.pack,
     parse_signatures) evaluated by the CPU oracle give the reference's build_em_matrix
-    (preprocess.py:177-198) bit for bit."""
+    (preprocess.py:177-198) bit for bit.  The reference's matrices are stored in
+    tests/golden/golden_live.npz (oracle/live_cases.py); where the reference is installed,
+    they are checked against it too."""
     import argparse
-    import types
-    from oracle import oracle_c, refload
-    if not refload.available():
-        pytest.skip("reference not mounted")
-    _, ref_pre, _ = refload.load()
-    rs = np.random.RandomState(1)
-    for it in range(60):
-        ref_len = rs.randint(30, 200)
-        refseq = "".join("ACGT"[i] for i in rs.randint(0, 4, size=ref_len))
-        n_pos = rs.randint(1, min(25, ref_len))
-        positions = np.sort(rs.choice(ref_len, size=n_pos, replace=False)).tolist()
-        variants = {}
-        for p in positions:
-            cnt = collections.Counter()
-            for _ in range(rs.randint(1, 4)):
-                cnt[rs.choice(list("ACGT"))] += int(rs.randint(1, 80))
-            variants[p] = cnt
-        hap_var = {}
-        for j in range(rs.randint(1, 12)):
-            vs = []
-            for _ in range(rs.randint(0, 8)):
-                p = int(rs.choice(positions)) if rs.rand() < 0.85 else int(rs.randint(ref_len))
-                v = "%s%d%s" % (refseq[p], p + 1, rs.choice(list("ACGTacgt")))
-                r = rs.rand()
-                v = ("(" + v + ")" if r < 0.15 else v + "!" if r < 0.3 else v + "!!" if r < 0.35
-                     else "(" + v + "!)" if r < 0.4 else v)
-                vs.append(v)
-            hap_var["h%d" % j] = vs
-        phylo = types.SimpleNamespace(variants=variants, hap_var=hap_var, refseq=refseq)
-        haps = sorted(hap_var)
-        reads = []
-        for _ in range(rs.randint(1, 10)):
-            ps = rs.choice(positions, size=rs.randint(1, n_pos + 1), replace=rs.rand() < 0.2)
-            reads.append(",".join("%d:%s" % (p, rs.choice(list("ACGTN"))) for p in ps))
-        want = ref_pre.build_em_matrix(refseq, phylo, reads, haps, argparse.Namespace(verbose=False))
+    from oracle import live_cases, oracle_c, refload
+    g = live_cases.load_golden()
+    ref_pre = refload.load()[1] if refload.available() else None
+    off = 0
+    for it, (refseq, phylo, haps, reads) in enumerate(live_cases.packing_cases()):
+        want = g["pack_mats"][off:off + len(reads) * len(haps)].reshape(len(reads), len(haps))
+        off += want.size
+        if ref_pre is not None:
+            live = ref_pre.build_em_matrix(refseq, phylo, reads, haps, argparse.Namespace(verbose=False))
+            assert np.array_equal(live, want), it
         tables = HapVarBaseMatrix(refseq, phylo, haps).pack()
         csr, err = parse_signatures(reads, tables)
         assert err is None
         got, counts = oracle_c.build_matrix(tables, csr)
         assert np.array_equal(got, want), it
         assert (counts >= 0).all() and (counts <= np.diff(csr.row_ptr)[:, None]).all()
+    assert off == g["pack_mats"].size
 
 
 @pytest.mark.parametrize("exotic", [None, "A0G", "A3é"])

@@ -1,12 +1,12 @@
 """Pins the CPU oracle (oracle/oracle_np.py, oracle/oracle.c) to the
 reference: against the golden vectors the unmodified reference produced
-(oracle/make_golden.py), and against the live reference when it is mounted."""
+(oracle/make_golden.py, oracle/live_cases.py), and against the live reference
+where it is installed."""
 import numpy as np
 import pytest
 
-from mixemt_b200 import synth
 from mixemt_b200.preprocess import HapVarBaseMatrix, parse_signatures
-from oracle import oracle_c, oracle_np, refload
+from oracle import live_cases, oracle_c, oracle_np, refload
 from conftest import load_golden, make_args
 
 
@@ -107,35 +107,38 @@ def test_run_em_build17_golden(phylo17):
         assert np.array_equal(np.argmax(mix, 1), g[tag + "_argmax"])
 
 
-@pytest.mark.skipif(not refload.available(), reason="reference not mounted on this box")
 def test_against_live_reference(phylo17):
-    """In the build container: the oracle against the reference itself."""
-    _, ref_pre, ref_em = refload.load()
+    """The oracles against the reference's build_em_matrix and run_em on 12 Build-17 reads
+    (tests/golden/golden_live.npz, oracle/live_cases.py); where the reference is installed,
+    the stored outputs against the reference itself."""
+    g = live_cases.load_golden()
     haps = sorted(phylo17.hap_var)
-    mix = synth.make_mixture(phylo17, phylo17.refseq, [("H1", 0.6), ("M7", 0.4)], 300, seed=9)
-    reads = mix.signatures[:12]
-    want = ref_pre.build_em_matrix(phylo17.refseq, phylo17, reads, haps, make_args())
+    reads, wts = str(g["b17_reads"]).split("\n"), g["b17_weights"]
+    want = g["b17_mat"]
+    if refload.available():
+        _, ref_pre, ref_em = refload.load()
+        assert (reads, wts.tolist()) == tuple(map(list, live_cases.build17_reads(phylo17)))
+        assert np.array_equal(ref_pre.build_em_matrix(phylo17.refseq, phylo17, reads, haps,
+                                                      make_args()), want)
     t = HapVarBaseMatrix(phylo17.refseq, phylo17, haps).pack()
     csr, _ = parse_signatures(reads, t)
     assert np.array_equal(oracle_c.build_matrix(t, csr)[0], want)
-    sub = want[:, ::11].copy()
-    np.random.seed(77)
-    p_ref, m_ref = ref_em.run_em(sub, mix.weights[:12], make_args(n_multi=2, max_iter=200))
-    inits = seeded_inits(77, 2, sub.shape[1])
-    p_np, m_np, _ = oracle_np.run_em(sub, mix.weights[:12], inits, 200, 1e-4)
-    p_c, m_c, _ = oracle_c.run_em(sub, mix.weights[:12], inits, 200, 1e-4)
+    sub = live_cases.build17_sub(want)
+    seed, n_multi, max_iter = (live_cases.RUN_EM_SEED, live_cases.RUN_EM_MULTI,
+                               live_cases.RUN_EM_MAX_ITER)
+    p_ref, m_ref = g["b17_props"], g["b17_mix"]
+    if refload.available():
+        np.random.seed(seed)
+        p_live, m_live = ref_em.run_em(sub, wts, make_args(n_multi=n_multi, max_iter=max_iter))
+        assert np.array_equal(p_live, p_ref) and np.array_equal(m_live, m_ref)
+    inits = seeded_inits(seed, n_multi, sub.shape[1])
+    p_np, m_np, _ = oracle_np.run_em(sub, wts, inits, max_iter, 1e-4)
+    p_c, m_c, _ = oracle_c.run_em(sub, wts, inits, max_iter, 1e-4)
     assert np.array_equal(p_np, p_ref) and np.array_equal(m_np, m_ref)
     assert np.abs(p_c - p_ref).max() < 1e-13 and np.abs(m_c - m_ref).max() < 1e-10
 
 
 # ---- consumers of the EM result (SURVEY.md 8f N2/N3) ---------------------------
-def _decode_assign(res, n):
-    out = np.full(n, -2, dtype=np.int32)
-    for name, rows in res.items():
-        out[sorted(rows)] = -1 if name == 'unassigned' else int(name[3:]) - 1
-    return out
-
-
 @pytest.mark.parametrize("seed", [71, 72])
 def test_consumers_golden(seed):
     g = load_golden("golden_consumers.npz")
@@ -149,57 +152,59 @@ def test_consumers_golden(seed):
     for tag, fold, cons in (("f2", 2.0, contribs), ("f1p2", 1.2, contribs[:2]),
                             ("single", 2.0, contribs[:1])):
         res = oracle_np.assign_read_indexes(cons, (props, mix), haps, len(mix), fold)
-        assert np.array_equal(_decode_assign(res, len(mix)), g["s%d_assign_%s" % (seed, tag)])
+        assert np.array_equal(live_cases.decode_assign(res, len(mix)), g["s%d_assign_%s" % (seed, tag)])
     red, new_haps = oracle_np.reduce_em_matrix(mix, haps, contribs)
     assert np.array_equal(red, g["s%d_reduced" % seed])
     assert [haps.index(x) for x in new_haps] == g["s%d_reduced_cols" % seed].tolist()
 
 
-@pytest.mark.skipif(not refload.available(), reason="reference not mounted")
 def test_consumers_live_reference():
-    refload.load()
-    from mixemt import assemble, preprocess as ref_pre
-    props, mix, wts = oracle_np.synthetic_em_result(99, n=150, h=40)
-    haps = ["hg%d" % j for j in range(40)]
-    ns = make_args(min_reads=25)
-    assert assemble._find_contribs_from_reads(mix, wts, ns) == \
-        oracle_np.find_contribs_from_reads(mix, wts, 25)
-    top = np.argsort(props)[::-1][:3].tolist()
-    contribs = [["hap%d" % (k + 1), haps[j], props[j]] for k, j in enumerate(top)]
-    ref = assemble.assign_read_indexes(contribs, (props, mix), haps, list(range(150)), 2.0)
-    got = oracle_np.assign_read_indexes(contribs, (props, mix), haps, 150, 2.0)
-    assert dict(ref) == got
-    a, b = ref_pre.reduce_em_matrix(mix, haps, contribs), oracle_np.reduce_em_matrix(mix, haps, contribs)
-    assert np.array_equal(a[0], b[0]) and a[1] == b[1]
+    """The consumers' restatements against the reference's assemble / reduce_em_matrix on a
+    150 x 40 stand-in (tests/golden/golden_live.npz); where the reference is installed, the
+    stored outputs against the reference itself."""
+    g = live_cases.load_golden()
+    props, mix, wts, haps, contribs = live_cases.consumers_case()
+    n, min_reads, fold = len(mix), live_cases.CONSUMERS_MIN_READS, live_cases.CONSUMERS_FOLD
+    want_red, want_cols = g["c_reduced"], [haps[j] for j in g["c_reduced_cols"].tolist()]
+    if refload.available():
+        refload.load()
+        from mixemt import assemble, preprocess as ref_pre
+        assert assemble._find_contribs_from_reads(mix, wts, make_args(min_reads=min_reads)) == \
+            g["c_contribs"].tolist()
+        ref = assemble.assign_read_indexes(contribs, (props, mix), haps, list(range(n)), fold)
+        assert np.array_equal(live_cases.decode_assign(ref, n), g["c_assign"])
+        a = ref_pre.reduce_em_matrix(mix, haps, contribs)
+        assert np.array_equal(a[0], want_red) and a[1] == want_cols
+    assert oracle_np.find_contribs_from_reads(mix, wts, min_reads) == g["c_contribs"].tolist()
+    got = oracle_np.assign_read_indexes(contribs, (props, mix), haps, n, fold)
+    assert np.array_equal(live_cases.decode_assign(got, n), g["c_assign"])
+    b = oracle_np.reduce_em_matrix(mix, haps, contribs)
+    assert np.array_equal(b[0], want_red) and b[1] == want_cols
 
 
-@pytest.mark.skipif(not refload.available(), reason="reference not mounted")
 def test_em_step_fuzz_against_live_reference():
     """The oracles' em_step against the reference's own (em.py:57-91, scipy logsumexp) on small
     random inputs with the edge values the domain has: -inf cells, ties among the row and
     column maxima, a row that fits no haplotype (NaN, like the reference), zero weights,
     components with zero proportion.  numpy restatement: bit-identical, NaN for NaN; C port:
-    the same non-finite pattern and within 1e-12."""
+    the same non-finite pattern and within 1e-12.  The reference's outputs are stored in
+    tests/golden/golden_live.npz; where the reference is installed, they are checked against
+    it too."""
     import warnings
-    _, _, ref_em = refload.load()
-    rs = np.random.RandomState(0)
+    g = live_cases.load_golden()
+    ref_em = refload.load()[2] if refload.available() else None
+    zo = po = 0
     with warnings.catch_warnings(), np.errstate(all="ignore"):
         warnings.simplefilter("ignore")
-        for it in range(200):
-            n, h = rs.randint(1, 14), rs.randint(1, 10)
-            mat = -rs.gamma(2.0, 4.0, size=(n, h))
-            mode = it % 5
-            if mode >= 1:
-                mat[rs.rand(n, h) < 0.2] = -np.inf
-            if mode >= 2:
-                mat = np.round(mat)
-            if mode == 3:
-                mat[rs.randint(n)] = -np.inf
-            wts = rs.randint(0 if mode >= 2 else 1, 50, size=n)
-            lp = np.log(rs.dirichlet([1.0] * h))
-            if mode == 4:
-                lp[rs.rand(h) < 0.3] = -np.inf
-            z_ref, p_ref = ref_em.em_step(mat, wts, lp, np.empty_like(mat))
+        for it, (mat, wts, lp) in enumerate(live_cases.em_step_cases()):
+            n, h = mat.shape
+            z_ref = g["step_z"][zo:zo + n * h].reshape(n, h)
+            p_ref = g["step_p"][po:po + h]
+            zo, po = zo + n * h, po + h
+            if ref_em is not None:
+                z_live, p_live = ref_em.em_step(mat, wts, lp, np.empty_like(mat))
+                assert np.array_equal(z_live, z_ref, equal_nan=True), it
+                assert np.array_equal(p_live, p_ref, equal_nan=True), it
             z_np, p_np = oracle_np.em_step(mat, wts, lp)
             assert np.array_equal(z_np, z_ref, equal_nan=True), it
             assert np.array_equal(p_np, p_ref, equal_nan=True), it
@@ -208,3 +213,4 @@ def test_em_step_fuzz_against_live_reference():
                 fin = np.isfinite(want)
                 assert np.array_equal(got[~fin], want[~fin], equal_nan=True), it
                 assert not fin.any() or np.abs(got[fin] - want[fin]).max() < 1e-12, it
+    assert (zo, po) == (g["step_z"].size, g["step_p"].size)

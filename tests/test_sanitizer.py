@@ -15,8 +15,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 @pytest.mark.parametrize("tool", ["memcheck", "racecheck", "synccheck"])
 def test_compute_sanitizer_clean(tool):
     exe = shutil.which("compute-sanitizer") or "/usr/local/cuda/bin/compute-sanitizer"
-    if not os.path.exists(exe):
-        pytest.skip("compute-sanitizer not installed")
+    if not os.access(exe, os.X_OK):
+        pytest.skip("compute-sanitizer not installed or not executable")
     res = subprocess.run([exe, "--tool", tool, "--print-limit", "5", sys.executable,
                           os.path.join(ROOT, "scripts", "sanitize.py")],
                          capture_output=True, text=True, timeout=900, cwd=ROOT)
