@@ -210,7 +210,9 @@ int mxb_em_destroy(mxb_em *em);
 /* Set the current log-proportions (em.py:123-124, host draws the Dirichlet). */
 int mxb_em_set_lnprops(mxb_em *em, const double *lnprops);
 /* Iterate em_step + converged (em.py:126-143) until sum|dprops| < tol or
- * max_iter.  iters_out = iterations run; converged_out = 1/0. */
+ * max_iter.  iters_out = iterations run; converged_out = 1/0.  An iteration in which a
+ * row's mixture likelihood underflows in linear space is redone in log space (em.py:80-89);
+ * in a sharded session all ranks redo it together, so the call stays collective. */
 int mxb_em_iterate(mxb_em *em, int64_t max_iter, double tol,
                    int64_t *iters_out, int32_t *converged_out);
 /* Bytes the kernels of one EM iteration read from HBM, and how the rows are stored:
@@ -233,7 +235,7 @@ int mxb_tile_plan(const int32_t *n_cls, int64_t n_batches, int64_t n_rows, int32
 
 /* Exactly n_iter iterations without convergence test or host sync (bench); MXB_ERR_RANGE
  * when fewer ran (a row's mixture likelihood underflowed and the run stopped for the
- * log-space step, which only mxb_em_iterate takes);
+ * log-space step, which only mxb_em_iterate and the one-call forms below take);
  * elapsed_ms (nullable) = device time between first and last launch,
  * pass_ms (nullable) = summed device time from the first pass kernel of an iteration to
  * its tail kernel (class sums + pass + gather for tiles; adds an event pair per iteration). */
@@ -254,7 +256,9 @@ int mxb_em_read_mix(mxb_em *em, mxb_matrix *dst, int mode, double sub_log);
 /* One-call forms with host buffers (what a reference-side FFI would bind). */
 /* em.run_em (em.py:94-165): init_lnprops[n_multi*n_cols] drawn by the host;
  * props_out[n_cols] linear scale; read_mix_out (nullable) N x H log scale;
- * iters_out[n_multi], converged_out[n_multi] (nullable). */
+ * iters_out[n_multi], converged_out[n_multi] (nullable).  Iterations whose row likelihoods
+ * underflow in linear space are redone in log space in every kind of session (one restart or
+ * two per pass, one GPU or row-sharded), as the reference computes them. */
 /* flags: MXB_EM_SHARDED = the rows are this rank's shard of a larger matrix
  * (column sums all-reduced over the ctx comm every iteration);
  * MXB_EM_RAW = skip the final averaging (em.py:158-163): props_out then holds

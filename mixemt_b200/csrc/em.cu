@@ -251,10 +251,11 @@ static int enqueue_iteration(mxb_em *em, cudaEvent_t pass_begin = nullptr,
         ctx->launches += 1;
         return MXB_OK;
     }
-    em_colreduce_kernel<<<(int)ceil_div(em->ld, 256), 256, 0, s>>>(em->partials, em->n_part,
-                                                                  em->ld, em->state, em->tsum);
+    em_colreduce_kernel<<<(int)ceil_div(em->ld + 1, 256), 256, 0, s>>>(em->partials, em->n_part,
+                                                                      em->ld, em->state, em->tsum);
     ctx->launches += 1;
-    if (em->sharded && ctx->world > 1) MXB_TRY(nccl_allreduce_sum_f64(ctx, em->tsum, em->ld));
+    // the column sums and the underflow flag behind them (tsum[ld])
+    if (em->sharded && ctx->world > 1) MXB_TRY(nccl_allreduce_sum_f64(ctx, em->tsum, em->ld + 1));
     em_update_kernel<<<1, kUpdThreads, 0, s>>>(em->tsum, em->n_cols, em->ld, em->lnp[0],
                                                em->lnp[1], em->pi[0], em->pi[1], em->state);
     ctx->launches += 1;
@@ -613,12 +614,13 @@ static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weigh
 #define STEP(call) do { if (e == cudaSuccess) e = (call); } while (0)
     const size_t ns = (size_t)em->n_slots;
     {   // everything else of the session in one block: [weights][coef][lnp x2][pi x2][partials]
-        // [tsum][props_in][state], each 256-byte aligned
+        // [tsum + underflow flag][props_in][state], each 256-byte aligned
         auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
         const size_t b_rows = up((size_t)em->n_rows * sizeof(double));
         const size_t b_vec = up(ns * row_bytes);
         const size_t b_part = up(ns * (size_t)em->n_part * row_bytes);
-        const size_t total = b_rows * (em->fast ? 1 : 2) + 4 * b_vec + b_part + up(row_bytes) +
+        const size_t total = b_rows * (em->fast ? 1 : 2) + 4 * b_vec + b_part +
+                             up(row_bytes + sizeof(double)) +
                              up((size_t)em->n_cols * sizeof(double)) + up(ns * sizeof(EmState));
         STEP(dev_alloc(ctx, (void **)&em->small, total));
         if (e == cudaSuccess) {
@@ -628,7 +630,7 @@ static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weigh
             for (int i = 0; i < 2; ++i) { em->lnp[i] = (double *)p; p += b_vec; }
             for (int i = 0; i < 2; ++i) { em->pi[i] = (double *)p; p += b_vec; }
             em->partials = (double *)p; p += b_part;
-            em->tsum = (double *)p; p += up(row_bytes);
+            em->tsum = (double *)p; p += up(row_bytes + sizeof(double));
             em->props_in = (double *)p; p += up((size_t)em->n_cols * sizeof(double));
             em->state = (EmState *)p;
         }
@@ -703,41 +705,72 @@ int mxb_em_pass_bytes(const mxb_em *em, int64_t *bytes_per_pass, int64_t *n_dens
     return MXB_OK;
 }
 
-// One iteration in log space on the session's current proportions (see em_logspace_*):
-// called when the tail flagged done = kDoneNeedsLogStep.  Leaves the control block as a normal
-// tail would (iters + 1, convergence / max_iter decision, buffers swapped).
-static int em_logspace_step(mxb_em *em, const EmState &seen) {
+// One iteration in log space on the proportions lnp[cur] of restart slot `slot` (see
+// em_logspace_*): called when the tail flagged done = kDoneNeedsLogStep.  Leaves the control
+// block as a normal tail would (iters + 1, convergence / max_iter decision, buffers swapped).
+// In a row-sharded session every rank calls it for the same iteration (the tails agree on
+// the flag): the row lse is local, the column reduction spans the ranks as scipy's
+// logsumexp forms it, global maxima first (all-reduce max), then the non-maximal sum s and
+// the weight m of the maximal terms per column (all-reduce sum), so every rank forms the
+// same ln pi' and takes the same decision.
+static int em_logspace_step(mxb_em *em, int cur, int slot = 0) {
     mxb_ctx *ctx = em->ctx;
     cudaStream_t s = ctx->stream;
-    const int64_t n = em->n_rows, h = em->n_cols;
+    const int64_t n = em->n_rows, h = em->n_cols, ld = em->ld;
+    const bool across = em->sharded && ctx->world > 1;
+    const int64_t n_sums = across ? 2 * h : h;      // [s][m] or the plain column sums
     constexpr int kRowBlocks = 64;
     auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
     const size_t b_lse = up((size_t)n * sizeof(double)), b_col = up((size_t)h * sizeof(double));
-    const size_t b_part = up((size_t)kRowBlocks * h * sizeof(double));
+    const size_t b_sum = up((size_t)n_sums * sizeof(double));
+    const size_t b_part = up((size_t)kRowBlocks * n_sums * sizeof(double));
     unsigned char *tmp = nullptr;
-    if (dev_alloc(ctx, (void **)&tmp, b_lse + 2 * b_col + b_part) != cudaSuccess) {
+    if (dev_alloc(ctx, (void **)&tmp, b_lse + b_col + b_sum + b_part) != cudaSuccess) {
         cudaGetLastError();
         set_error("EM log-space step: out of device memory");
         return MXB_ERR_NOMEM;
     }
     double *lse = (double *)tmp, *colmax = (double *)(tmp + b_lse);
-    double *colsum = (double *)(tmp + b_lse + b_col), *part = (double *)(tmp + b_lse + 2 * b_col);
-    const double *lnp = em->lnp[seen.cur];
+    double *colsum = (double *)(tmp + b_lse + b_col), *part = (double *)(tmp + b_lse + b_col + b_sum);
+    const double *lnp = em->lnp[cur] + slot * ld;
     const int col_blocks = (int)ceil_div(h, 256);
-    const int row_grid = (int)std::min<int64_t>(n, (int64_t)ctx->num_sms * 8);
-    em_logspace_rows_kernel<<<row_grid, 256, 0, s>>>(em->mat->data, n, h, lnp, lse);
-    em_logspace_cols_kernel<<<dim3(col_blocks, kRowBlocks), 256, 0, s>>>(
-        em->mat->data, n, h, lnp, lse, em->weights, nullptr, part);
+    const dim3 col_grid(col_blocks, kRowBlocks);
+    int rc = MXB_OK;
+    if (n > 0) {   // a rank of a row-sharded run may hold no rows
+        const int row_grid = (int)std::min<int64_t>(n, (int64_t)ctx->num_sms * 8);
+        em_logspace_rows_kernel<<<row_grid, 256, 0, s>>>(em->mat->data, n, h, lnp, lse);
+        ctx->launches += 1;
+    }
+    em_logspace_cols_kernel<<<col_grid, 256, 0, s>>>(em->mat->data, n, h, lnp, lse, em->weights,
+                                                     nullptr, part);
     em_logspace_colreduce_kernel<<<col_blocks, 256, 0, s>>>(part, kRowBlocks, h, 1, colmax);
-    em_logspace_cols_kernel<<<dim3(col_blocks, kRowBlocks), 256, 0, s>>>(
-        em->mat->data, n, h, lnp, lse, em->weights, colmax, part);
-    em_logspace_colreduce_kernel<<<col_blocks, 256, 0, s>>>(part, kRowBlocks, h, 0, colsum);
-    em_logspace_update_kernel<<<1, kUpdThreads, 0, s>>>(colmax, colsum, h, em->ld, em->lnp[0],
-                                                        em->lnp[1], em->pi[0], em->pi[1], em->state);
-    ctx->launches += 6;
+    ctx->launches += 2;
+    if (across) {
+        rc = nccl_allreduce_f64(ctx, colmax, h, 1);
+        if (rc == MXB_OK) {
+            em_logspace_cols_split_kernel<<<col_grid, 256, 0, s>>>(
+                em->mat->data, n, h, lnp, lse, em->weights, colmax, part);
+            em_logspace_colreduce_kernel<<<(int)ceil_div(n_sums, 256), 256, 0, s>>>(
+                part, kRowBlocks, n_sums, 0, colsum);
+            ctx->launches += 2;
+            rc = nccl_allreduce_sum_f64(ctx, colsum, n_sums);
+        }
+    } else {
+        em_logspace_cols_kernel<<<col_grid, 256, 0, s>>>(em->mat->data, n, h, lnp, lse,
+                                                         em->weights, colmax, part);
+        em_logspace_colreduce_kernel<<<col_blocks, 256, 0, s>>>(part, kRowBlocks, h, 0, colsum);
+        ctx->launches += 2;
+    }
+    if (rc == MXB_OK) {
+        em_logspace_update_kernel<<<1, kUpdThreads, 0, s>>>(
+            colmax, colsum, across ? colsum + h : nullptr, h, ld, em->lnp[0] + slot * ld,
+            em->lnp[1] + slot * ld, em->pi[0] + slot * ld, em->pi[1] + slot * ld, em->state + slot);
+        ctx->launches += 1;
+    }
     cudaError_t e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);
     dev_free(ctx, tmp);
+    if (rc != MXB_OK) return rc;
     if (e != cudaSuccess) {
         set_error("EM log-space step: %s", cudaGetErrorString(e));
         return MXB_ERR_CUDA;
@@ -808,7 +841,7 @@ int mxb_em_iterate(mxb_em *em, int64_t max_iter, double tol, int64_t *iters_out,
                 // that iteration in log space, go on from the state it leaves
                 MXB_CUDA(cudaStreamSynchronize(ctx->stream));
                 pending[0] = pending[1] = false;
-                MXB_TRY(em_logspace_step(em, em->host_state[wait_slot]));
+                MXB_TRY(em_logspace_step(em, em->host_state[wait_slot].cur));
                 ++log_steps;
                 MXB_CUDA(cudaMemcpyAsync(&em->host_state[wait_slot], em->state, sizeof(EmState),
                                          cudaMemcpyDeviceToHost, ctx->stream));
@@ -1141,6 +1174,15 @@ static int run_em_batched(mxb_em *em, const double *init_lnprops, int32_t n_mult
             for (int sl = 0; sl < em->n_slots && rc == MXB_OK; ++sl) {
                 const EmState st = em->host_state[other * kMaxSlots + sl];
                 if (slot_restart[sl] < 0 || poll_gen[other][sl] != slot_gen[sl] || !st.done) continue;
+                if (st.done == kDoneNeedsLogStep) {
+                    // a row's mixture likelihood underflowed in this slot's restart: redo that
+                    // iteration in log space on its slot and let the pair go on (the other
+                    // slot's restart kept iterating and is not touched).  The poll still in
+                    // flight was taken before the step: a new generation makes it skip the slot.
+                    rc = em_logspace_step(em, st.cur, sl);
+                    slot_gen[sl]++;
+                    continue;
+                }
                 const int32_t idx = slot_restart[sl];
                 if (st.bad) {
                     set_error("EM: the mixture likelihood of some rows underflowed to 0 in "

@@ -584,12 +584,15 @@ em_colacc_kernel(const double *__restrict__ lin, int64_t ld, int64_t n_rows,
     reinterpret_cast<double2 *>(partials + (size_t)blockIdx.x * ld)[c] = t;
 }
 
-// T_j = sum over CTAs of partials, fixed order.
+// T_j = sum over CTAs of partials, fixed order.  tsum[ld] carries the row-likelihood underflow
+// flag, so that a row-sharded run sums it over the ranks together with the column sums and
+// every rank takes the same decision in em_update_kernel.  Launch ceil_div(ld + 1, 256) CTAs.
 __global__ void __launch_bounds__(256)
 em_colreduce_kernel(const double *__restrict__ partials, int n_part, int64_t ld,
                     const EmState *__restrict__ st, double *__restrict__ tsum) {
     if (st->done) return;
     const int64_t j = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (j == ld) tsum[ld] = st->bad ? 1.0 : 0.0;
     if (j >= ld) return;
     double t = 0.0;
     for (int b = 0; b < n_part; ++b) t += partials[(size_t)b * ld + j];
@@ -604,7 +607,7 @@ em_update_kernel(const double *__restrict__ tsum, int64_t n_cols, int64_t ld,
                  double *__restrict__ pi0, double *__restrict__ pi1,
                  EmState *__restrict__ st) {
     if (st->done) return;
-    if (st->bad) {               // a row's mixture likelihood underflowed: see em_logspace_*
+    if (tsum[ld] != 0.0) {       // a row's mixture likelihood underflowed (on some rank): see em_logspace_*
         if (threadIdx.x == 0) st->done = kDoneNeedsLogStep;
         return;
     }
@@ -685,7 +688,13 @@ __device__ __forceinline__ double cluster_sum(double v, double *wsum, double *sl
 // `world` flags in its own block carry that number and adds the inbox rows in
 // rank order, so that every rank forms bit-identical totals and takes the same
 // convergence decision.  Two slots suffice: a rank can be at most one launch
-// ahead of a peer, because it needs that peer's flag to finish a launch.
+// ahead of a peer, because it needs that peer's flag to finish a launch.  A rank
+// whose pass flagged a row-likelihood underflow (st->bad) raises its flags with
+// kP2PBadBit set; every rank then sees it in the same launch, sets
+// done = kDoneNeedsLogStep instead of advancing, and the iteration is redone in log
+// space by all ranks together (em_logspace_step).  The sequence number advances as
+// in any other launch, so the mailboxes stay in step.
+constexpr unsigned long long kP2PBadBit = 1ull << 63;
 struct P2PArgs {
     int world, rank;
     unsigned char *block[kP2PMaxWorld];  // [r] = rank r's mailbox block (own block at [rank])
@@ -724,14 +733,14 @@ em_finish_kernel(const double *partials, int n_part, int64_t n_cols, int64_t ld,
         // A row's mixture likelihood underflowed in linear space: this iteration is redone in
         // log space by the host (em_logspace_* kernels), the queued launches become no-ops.
         // (st->bad was final before this launch began; the write below is seen by later
-        // launches only.)  Row-sharded runs keep reporting the condition as an error.
+        // launches only.)  Row-sharded runs first tell the other ranks (kP2PBadBit below).
         cooperative_groups::this_cluster().sync();
         if (blockIdx.x == 0 && threadIdx.x == 0) st->done = kDoneNeedsLogStep;
         return;
     }
     __shared__ double wsum[2][kFinThreads / 32];
     __shared__ double slots[2][kFinCtas];
-    __shared__ int s_timeout;
+    __shared__ int s_timeout, s_bad;
     const int cur = st->cur;
     const double *lnp_old = cur ? lnp1 : lnp0;
     const double *pi_old = cur ? pi1 : pi0;
@@ -779,7 +788,7 @@ em_finish_kernel(const double *partials, int n_part, int64_t n_cols, int64_t ld,
         const int W = pa.world;
         unsigned long long *my_flags = reinterpret_cast<unsigned long long *>(pa.block[pa.rank]);
         unsigned long long *my_seq = my_flags + 2 * kP2PMaxWorld;
-        if (threadIdx.x == 0) s_timeout = 0;
+        if (threadIdx.x == 0) { s_timeout = 0; s_bad = 0; }
         seq = *my_seq + 1;  // advanced by CTA 0 at the very end of this launch
         const int slot = (int)(seq & 1ull);
         if (owner) {
@@ -793,9 +802,15 @@ em_finish_kernel(const double *partials, int n_part, int64_t n_cols, int64_t ld,
         if (blockIdx.x == 0 && threadIdx.x < W) {
             const int r = threadIdx.x;
             unsigned long long *peer_flags = reinterpret_cast<unsigned long long *>(pa.block[r]);
-            st_release_sys(&peer_flags[slot * kP2PMaxWorld + pa.rank], seq);
+            st_release_sys(&peer_flags[slot * kP2PMaxWorld + pa.rank],
+                           seq | (st->bad ? kP2PBadBit : 0ull));
             const unsigned long long t0 = global_timer_ns();
-            while (ld_acquire_sys(&my_flags[slot * kP2PMaxWorld + r]) != seq) {
+            for (;;) {
+                const unsigned long long f = ld_acquire_sys(&my_flags[slot * kP2PMaxWorld + r]);
+                if ((f & ~kP2PBadBit) == seq) {
+                    if (f & kP2PBadBit) s_bad = 1;
+                    break;
+                }
                 if (global_timer_ns() - t0 > kP2PTimeoutNs) { s_timeout = 1; break; }
             }
         }
@@ -837,13 +852,17 @@ em_finish_kernel(const double *partials, int n_part, int64_t n_cols, int64_t ld,
     }
     const double delta = cluster_sum(dl, wsum[1], slots[1]);
     if (blockIdx.x == 0 && threadIdx.x == 0) {
-        st->delta = delta;
-        const long long it = st->iters + 1;
-        st->iters = it;
         if (kP2P) {
             unsigned long long *my_flags = reinterpret_cast<unsigned long long *>(pa.block[pa.rank]);
             my_flags[2 * kP2PMaxWorld] = seq;
         }
+        if (kP2P && !s_timeout && s_bad) {
+            st->done = kDoneNeedsLogStep;    // the proportions written above are discarded
+            return;
+        }
+        st->delta = delta;
+        const long long it = st->iters + 1;
+        st->iters = it;
         if (kP2P && s_timeout) st->done = 3;  // a peer never showed up
         else if (delta < st->tol) st->done = 1;
         else if (it >= st->max_iter) st->done = 2;
@@ -966,6 +985,34 @@ em_logspace_cols_kernel(const double *__restrict__ m, int64_t n_rows, int64_t n_
     part[(size_t)blockIdx.y * n_cols + j] = acc;
 }
 
+// Row-sharded form of the column sums: the maxima `colmax` are global (all-reduced over the
+// ranks), and scipy's logsumexp terms are kept apart as its formula needs them,
+// part[b][0][j] = s (sum of w_i exp(Z_ij - max) over the non-maximal terms) and
+// part[b][1][j] = m (sum of w_i over the maximal terms), so that the ranks' sums of s and m
+// can be added before ln pi'_j = log1p(s/m) + log(m) + max is formed.
+__global__ void __launch_bounds__(256)
+em_logspace_cols_split_kernel(const double *__restrict__ m, int64_t n_rows, int64_t n_cols,
+                              const double *__restrict__ lnp, const double *__restrict__ lse,
+                              const double *__restrict__ w, const double *__restrict__ colmax,
+                              double *__restrict__ part) {
+    const int64_t j = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (j >= n_cols) return;
+    const int64_t r0 = n_rows * blockIdx.y / gridDim.y, r1 = n_rows * (blockIdx.y + 1) / gridDim.y;
+    const double lp = lnp[j], cm = colmax[j];
+    double s = 0.0, cnt = 0.0;
+    if (cm > -INFINITY) {
+        for (int64_t r = r0; r < r1; ++r) {
+            const double wr = w[r];
+            if (wr == 0.0) continue;                   // scipy: a = -inf where b == 0
+            const double z = (m[r * n_cols + j] + lp) - lse[r];
+            if (z == cm) cnt += wr;
+            else s += wr * exp(z - cm);
+        }
+    }
+    part[(size_t)blockIdx.y * 2 * n_cols + j] = s;
+    part[(size_t)blockIdx.y * 2 * n_cols + n_cols + j] = cnt;
+}
+
 __global__ void __launch_bounds__(256)
 em_logspace_colreduce_kernel(const double *__restrict__ part, int n_part, int64_t n_cols,
                              int is_max, double *__restrict__ out) {
@@ -979,9 +1026,12 @@ em_logspace_colreduce_kernel(const double *__restrict__ part, int n_part, int64_
     out[j] = acc;
 }
 
-// ln pi' = colmax + log(colsum) - logsumexp(.), convergence test, control block (one CTA)
+// ln pi' = colmax + log(colsum) - logsumexp(.), convergence test, control block (one CTA).
+// With `colcnt` (row-sharded runs, em_logspace_cols_split_kernel) colsum holds scipy's s and
+// colcnt its m: ln pi' = log1p(s/m) + log(m) + colmax - logsumexp(.).
 __global__ void __launch_bounds__(kUpdThreads)
 em_logspace_update_kernel(const double *__restrict__ colmax, const double *__restrict__ colsum,
+                          const double *__restrict__ colcnt,
                           int64_t n_cols, int64_t ld, double *__restrict__ lnp0,
                           double *__restrict__ lnp1, double *__restrict__ pi0,
                           double *__restrict__ pi1, EmState *__restrict__ st) {
@@ -992,7 +1042,10 @@ em_logspace_update_kernel(const double *__restrict__ colmax, const double *__res
     double *pi_new = cur ? pi0 : pi1;
     double mx = -INFINITY;
     for (int64_t j = threadIdx.x; j < n_cols; j += kUpdThreads) {
-        const double v = colmax[j] > -INFINITY ? colmax[j] + log(colsum[j]) : -INFINITY;
+        double v = -INFINITY;
+        if (colmax[j] > -INFINITY)
+            v = colcnt ? log1p(colsum[j] / colcnt[j]) + log(colcnt[j]) + colmax[j]
+                       : colmax[j] + log(colsum[j]);
         lnp_new[j] = v;
         mx = fmax(mx, v);
     }
