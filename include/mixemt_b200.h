@@ -183,6 +183,13 @@ int mxb_matrix_gather_cols(mxb_ctx *ctx, const mxb_matrix *src, const int64_t *c
  * is column j; argmax_out (nullable) receives the row maxima positions. */
 int mxb_matrix_vote_count(mxb_ctx *ctx, const mxb_matrix *m, const int64_t *weights,
                           int64_t *votes_out, int64_t *argmax_out);
+/* assemble._find_contribs_from_reads (assemble.py:102-124) over a row shard whose first row
+ * is global row row0: votes_out[j] as mxb_matrix_vote_count; first_out[j] = smallest
+ * row0 + r whose first row maximum is column j, -1 when no row's maximum is j.  Two launches
+ * (row argmax, then integer-atomic votes and minima); only the 2 x n_cols results are copied
+ * back, so rows-mode ranks merge them with an O(H) all-reduce (consumers.py). */
+int mxb_matrix_vote_first(mxb_ctx *ctx, const mxb_matrix *m, const int64_t *weights,
+                          int64_t row0, int64_t *votes_out, int64_t *first_out);
 /* assemble.assign_read_indexes (assemble.py:267-334): per row the two contributor
  * columns with the highest read_mix[i][c] - con_lnprops[k]; assign_out[i] = k of the
  * best one when it leads the runner-up by at least ln_min_fold, else -1 (unassigned);

@@ -93,6 +93,7 @@ _PROTOS = {
     "mxb_matrix_destroy": (ctypes.c_int, [P]),
     "mxb_matrix_gather_cols": (ctypes.c_int, [P, P, P, c_i64, c_void_pp]),
     "mxb_matrix_vote_count": (ctypes.c_int, [P, P, P, P, P]),
+    "mxb_matrix_vote_first": (ctypes.c_int, [P, P, P, c_i64, P, P]),
     "mxb_assign_reads": (ctypes.c_int, [P, P, P, P, c_i32, c_dbl, P]),
     "mxb_matrix_download_rows": (ctypes.c_int, [P, P, c_i64, c_i64, P]),
     "mxb_matrix_upload_rows": (ctypes.c_int, [P, P, c_i64, c_i64, P]),

@@ -5,6 +5,7 @@
 //   mxb_matrix_gather_cols   preprocess.reduce_em_matrix   (preprocess.py:230-251)
 //   mxb_matrix_vote_count    assemble._find_contribs_from_reads (assemble.py:102-124),
 //                            stats.report_read_votes        (stats.py:34-46)
+//   mxb_matrix_vote_first    the same votes plus each column's first row, over a row shard
 //   mxb_assign_reads         assemble.assign_read_indexes   (assemble.py:267-334)
 //   mxb_matrix_{down,up}load_rows   row-range transfers for streaming .npy files
 //                            (bin/mixemt:214-245 dump_all / :168-211 load_prev)
@@ -28,13 +29,18 @@ gather_cols_kernel(const double *__restrict__ src, int64_t n_rows, int64_t src_c
     }
 }
 
-// votes[argmax[r]] += weights[r]  (integer atomics: order-independent)
+// votes[argmax[r]] += weights[r]; with first != nullptr also first[argmax[r]] = min(row0 + r).
+// Integer atomics: the result does not depend on the order the rows are visited in.
 __global__ void __launch_bounds__(256)
 vote_kernel(const int64_t *__restrict__ best, const int64_t *__restrict__ weights, int64_t n_rows,
-            unsigned long long *__restrict__ votes) {
+            unsigned long long *__restrict__ votes, unsigned long long *__restrict__ first,
+            int64_t row0) {
     for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n_rows;
-         r += (int64_t)gridDim.x * blockDim.x)
-        atomicAdd(&votes[best[r]], (unsigned long long)weights[r]);
+         r += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t j = best[r];
+        atomicAdd(&votes[j], (unsigned long long)weights[r]);
+        if (first) atomicMin(&first[j], (unsigned long long)(row0 + r));
+    }
 }
 
 // Per row: the two contributor columns with the highest read_mix - ln(props)
@@ -154,35 +160,50 @@ int mxb_matrix_gather_cols(mxb_ctx *ctx, const mxb_matrix *src, const int64_t *c
     return MXB_OK;
 }
 
-int mxb_matrix_vote_count(mxb_ctx *ctx, const mxb_matrix *m, const int64_t *weights,
-                          int64_t *votes_out, int64_t *argmax_out) {
+}  // extern "C"
+
+// Row argmax + weighted votes over m's rows; first_out (nullable) gets each column's smallest
+// row0 + r (-1: no row votes for it), argmax_out (nullable) the row maxima positions.
+static int vote_rows(mxb_ctx *ctx, const mxb_matrix *m, const int64_t *weights, int64_t row0,
+                     int64_t *votes_out, int64_t *first_out, int64_t *argmax_out,
+                     const char *what) {
     MXB_REQUIRE(ctx != nullptr && m != nullptr, "NULL argument");
     MXB_REQUIRE(m->n_cols > 0 || m->n_rows == 0, "vote count over empty rows");
     MXB_REQUIRE(votes_out != nullptr || m->n_cols == 0, "votes_out is NULL");
+    MXB_REQUIRE(row0 >= 0, "negative first row");
     for (int64_t j = 0; j < m->n_cols; ++j) votes_out[j] = 0;
+    if (first_out)
+        for (int64_t j = 0; j < m->n_cols; ++j) first_out[j] = -1;
     if (m->n_rows == 0) return MXB_OK;
     MXB_REQUIRE(weights != nullptr, "weights is NULL");
     MXB_CUDA(cudaSetDevice(ctx->device));
     int64_t *d_best = nullptr, *d_w = nullptr;
-    unsigned long long *d_votes = nullptr;
+    unsigned long long *d_votes = nullptr, *d_first = nullptr;
     cudaError_t e = cudaMalloc(&d_best, m->n_rows * sizeof(int64_t));
     if (e == cudaSuccess) e = cudaMalloc(&d_w, m->n_rows * sizeof(int64_t));
     if (e == cudaSuccess) e = cudaMalloc(&d_votes, m->n_cols * sizeof(unsigned long long));
+    if (e == cudaSuccess && first_out)
+        e = cudaMalloc(&d_first, m->n_cols * sizeof(unsigned long long));
     if (e == cudaSuccess)
         e = cudaMemcpyAsync(d_w, weights, m->n_rows * sizeof(int64_t), cudaMemcpyHostToDevice,
                             ctx->stream);
     if (e == cudaSuccess)
         e = cudaMemsetAsync(d_votes, 0, m->n_cols * sizeof(unsigned long long), ctx->stream);
+    if (e == cudaSuccess && d_first)      // all bits set: UINT64_MAX, no row yet (-1 as int64_t)
+        e = cudaMemsetAsync(d_first, 0xff, m->n_cols * sizeof(unsigned long long), ctx->stream);
     if (e == cudaSuccess) {
         const int blocks = (int)std::min<int64_t>(ceil_div(m->n_rows, 8), (int64_t)ctx->num_sms * 8);
         argmax_rows_kernel<<<blocks, 256, 0, ctx->stream>>>(m->data, m->n_rows, m->n_cols, d_best);
         vote_kernel<<<grid_for(ctx, m->n_rows, 256), 256, 0, ctx->stream>>>(d_best, d_w, m->n_rows,
-                                                                           d_votes);
+                                                                           d_votes, d_first, row0);
         ctx->launches += 2;
         e = cudaGetLastError();
     }
     if (e == cudaSuccess)
         e = cudaMemcpyAsync(votes_out, d_votes, m->n_cols * sizeof(int64_t),
+                            cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && d_first)
+        e = cudaMemcpyAsync(first_out, d_first, m->n_cols * sizeof(int64_t),
                             cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess && argmax_out)
         e = cudaMemcpyAsync(argmax_out, d_best, m->n_rows * sizeof(int64_t),
@@ -191,11 +212,25 @@ int mxb_matrix_vote_count(mxb_ctx *ctx, const mxb_matrix *m, const int64_t *weig
     cudaFree(d_best);
     cudaFree(d_w);
     cudaFree(d_votes);
+    cudaFree(d_first);
     if (e != cudaSuccess) {
-        set_error("mxb_matrix_vote_count: %s", cudaGetErrorString(e));
+        set_error("%s: %s", what, cudaGetErrorString(e));
         return MXB_ERR_CUDA;
     }
-    return MXB_OK;
+    return MXB_OK;     // an untouched first[j] (UINT64_MAX) reads back as int64_t -1
+}
+
+extern "C" {
+
+int mxb_matrix_vote_count(mxb_ctx *ctx, const mxb_matrix *m, const int64_t *weights,
+                          int64_t *votes_out, int64_t *argmax_out) {
+    return vote_rows(ctx, m, weights, 0, votes_out, nullptr, argmax_out, "mxb_matrix_vote_count");
+}
+
+int mxb_matrix_vote_first(mxb_ctx *ctx, const mxb_matrix *m, const int64_t *weights,
+                          int64_t row0, int64_t *votes_out, int64_t *first_out) {
+    MXB_REQUIRE(first_out != nullptr || m == nullptr || m->n_cols == 0, "first_out is NULL");
+    return vote_rows(ctx, m, weights, row0, votes_out, first_out, nullptr, "mxb_matrix_vote_first");
 }
 
 int mxb_assign_reads(mxb_ctx *ctx, const mxb_matrix *read_mix, const int64_t *con_cols,

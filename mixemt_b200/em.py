@@ -14,7 +14,8 @@ import numpy
 from . import _lib
 from ._lib import lib, check, ptr
 from . import sharding
-from .runtime import DeviceMatrix, get_context, lookup_resident, remember_resident, resident_mode
+from .runtime import (DeviceMatrix, RowShard, get_context, lookup_resident, remember_resident,
+                      resident_mode)
 
 
 def init_props(nhaps, alpha=1.0):
@@ -124,6 +125,9 @@ def run_em_device(dev_mat, weights, args, keep_device=False, want_host=True, ini
                                  ptr(iters), ptr(conv)))
         _report(verbose, 0, iters[:len(mine)], conv[:len(mine)])
     mix_dev = DeviceMatrix(ctx, mix_handle) if (need_dev and mix_handle.value) else None
+    if mix_dev is not None and shard == "rows" and ctx.world > 1:
+        # the kept read matrix holds this rank's rows: the consumers work on it as a shard
+        mix_dev.row_shard = dev_mat.row_shard or RowShard()
 
     if flags & _lib.MXB_EM_RAW:
         # restart fan-out: combine the per-rank partial results (em.py:145-163)

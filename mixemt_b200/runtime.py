@@ -102,12 +102,24 @@ def set_context(ctx):
     _default_ctx = ctx
 
 
+class RowShard(object):
+    """Marks a ``DeviceMatrix`` as this rank's contiguous slice of the rows of one
+    matrix split over the ranks (``args.b200_shard = "rows"``).  ``lo`` (the slice's
+    first global row) and ``n_total`` (rows of all slices) stay ``None`` until a
+    consumer needs them; it then computes them once with ``sharding.shard_offsets``."""
+
+    def __init__(self, lo=None, n_total=None):
+        self.lo, self.n_total = lo, n_total
+
+
 class DeviceMatrix(object):
-    """A row-major fp64 matrix resident in HBM (``mxb_matrix``)."""
+    """A row-major fp64 matrix resident in HBM (``mxb_matrix``).  ``row_shard`` is
+    ``None`` for a whole matrix, a :class:`RowShard` for a rows-mode shard."""
 
     def __init__(self, ctx, handle):
         self.ctx = ctx
         self.handle = handle
+        self.row_shard = None
         n, h = ctypes.c_int64(), ctypes.c_int64()
         check(lib.mxb_matrix_shape(handle, ctypes.byref(n), ctypes.byref(h)))
         self.shape = (n.value, h.value)

@@ -10,8 +10,35 @@ world_size-2 gloo group.
                  combines restarts (em.py:145-163): log-proportions are summed
                  and divided by n_multi, read matrices are folded with
                  logaddexp and shifted by -log(n_multi).
+* rows-mode consumers: each rank knows only its shard of the read matrix, so the
+                 votes of find_contribs_from_reads, the kept columns of
+                 reduce_em_matrix, global row indexes and .npy files are formed from
+                 O(H) all-reduces and the shards' offsets.
+
+The fp64 all-reduces carry integers exactly while they stay below 2**53.  A
+collective that may be the first one of a call carries an ``ok`` flag as an extra
+element: when any rank passes ``ok=False`` every rank raises ``RankFailed``, so no
+rank is left waiting in a later collective.
 """
+import io
+
 import numpy as np
+from numpy.lib import format as npy_format
+
+_EXACT = 2.0 ** 53
+
+
+class RankFailed(ValueError):
+    """A rank could not take part in a row-sharded call (raised on every rank)."""
+
+
+def _fail_flag(ok):
+    return 0.0 if ok else 1.0
+
+
+def _raise_if_failed(flag):
+    if flag:
+        raise RankFailed("a rank failed in a row-sharded call; see that rank's error")
 
 
 def row_shard(n_rows, rank, world):
@@ -61,3 +88,76 @@ def share_from_rank0(make, shape, rank, allreduce):
     else:
         arr = np.zeros(shape, dtype=np.float64)
     return allreduce(arr, "sum")
+
+
+def shard_offsets(n_local, rank, world, allreduce, ok=True):
+    """``(lo, n_total)`` of this rank's ``n_local`` rows, the shards laid end to end in
+    rank order: one sum all-reduce of the ``world`` shard sizes (arbitrary or empty
+    boundaries work) plus the ok flag."""
+    vec = np.zeros(world + 1)
+    vec[rank] = n_local
+    vec[world] = _fail_flag(ok)
+    vec = allreduce(vec, "sum")
+    _raise_if_failed(vec[world])
+    n_total = vec[:world].sum()
+    assert n_total < _EXACT, "row count not exact in fp64"
+    return int(vec[:rank].sum()), int(n_total)
+
+
+def merge_votes(votes, first, allreduce, ok=True):
+    """The ranks' ``(votes[H], first[H])`` of ``mxb_matrix_vote_first`` merged into
+    those of the whole matrix: votes summed, first rows (-1 = absent) reduced to
+    their minimum as the maximum of their negations."""
+    h = len(votes)
+    vec = np.empty(h + 1)
+    vec[:h] = votes
+    vec[h] = _fail_flag(ok)
+    vec = allreduce(vec, "sum")
+    _raise_if_failed(vec[h])
+    assert vec[:h].sum() < _EXACT, "total weight not exact in fp64"
+    first = np.asarray(first)
+    neg = np.ascontiguousarray(np.where(first >= 0, -first.astype(np.float64), -np.inf))
+    neg = allreduce(neg, "max")
+    with np.errstate(invalid="ignore"):
+        merged = np.where(np.isfinite(neg), -neg, -1.0)
+    return vec[:h].astype(np.int64), merged.astype(np.int64)
+
+
+def contrib_order(votes, first, min_reads):
+    """Column indexes of ``_find_contribs_from_reads`` (assemble.py:102-124): every column
+    that some row votes for (also with 0 votes, from rows of weight 0), ordered by its
+    first row like the reference's dict, then those with ``votes >= min_reads``."""
+    first = np.asarray(first)
+    seen = np.nonzero(first >= 0)[0]
+    order = seen[np.argsort(first[seen], kind="stable")]
+    return [int(j) for j in order if votes[j] >= min_reads]
+
+
+def agree(vector, allreduce, ok=True):
+    """True on every rank when all ranks hold the same integer vector: the lengths, then
+    the elements, compared as max == min (max all-reduces of ``v`` and ``-v``)."""
+    vec = np.asarray(vector, dtype=np.float64).reshape(-1)
+    assert vec.size == 0 or np.abs(vec).max() < _EXACT, "values not exact in fp64"
+    n = float(vec.size)
+    head = allreduce(np.array([_fail_flag(ok), n, -n]), "max")
+    _raise_if_failed(head[0])
+    if head[1] != -head[2]:
+        return False
+    both = allreduce(np.concatenate([vec, -vec]), "max")
+    return bool(np.array_equal(both[:vec.size], -both[vec.size:]))
+
+
+def barrier(allreduce, ok=True):
+    """All-reduce of one flag: returns once every rank got here, raises ``RankFailed``
+    on every rank when one of them passes ``ok=False``."""
+    _raise_if_failed(allreduce(np.array([_fail_flag(ok)]), "sum")[0])
+
+
+def npy_layout(n_total, h, lo=0):
+    """``(header, offset)``: the bytes ``numpy.save`` writes before the data of a C-ordered
+    float64 ``(n_total, h)`` array, and the file offset of row ``lo``."""
+    buf = io.BytesIO()
+    npy_format.write_array_header_1_0(buf, {"descr": "<f8", "fortran_order": False,
+                                            "shape": (int(n_total), int(h))})
+    header = buf.getvalue()
+    return header, len(header) + int(lo) * int(h) * 8
