@@ -216,10 +216,12 @@ int mxb_em_create(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
 int mxb_em_destroy(mxb_em *em);
 /* Set the current log-proportions (em.py:123-124, host draws the Dirichlet). */
 int mxb_em_set_lnprops(mxb_em *em, const double *lnprops);
-/* Iterate em_step + converged (em.py:126-143) until sum|dprops| < tol or
- * max_iter.  iters_out = iterations run; converged_out = 1/0.  An iteration in which a
- * row's mixture likelihood underflows in linear space is redone in log space (em.py:80-89);
- * in a sharded session all ranks redo it together, so the call stays collective. */
+/* Iterate em_step + converged (em.py:126-143) from the proportions mxb_em_set_lnprops set,
+ * until sum|dprops| < tol or max_iter (max_iter <= 0 runs no iteration).  iters_out =
+ * iterations run; converged_out = 1/0.  Driven by the same host loop as mxb_run_em's restarts.
+ * An iteration in which a row's mixture likelihood underflows in linear space is redone in log
+ * space (em.py:80-89); in a sharded session all ranks redo it together, so the call stays
+ * collective. */
 int mxb_em_iterate(mxb_em *em, int64_t max_iter, double tol,
                    int64_t *iters_out, int32_t *converged_out);
 /* Bytes the kernels of one EM iteration read from HBM, and how the rows are stored:
@@ -263,9 +265,11 @@ int mxb_em_read_mix(mxb_em *em, mxb_matrix *dst, int mode, double sub_log);
 /* One-call forms with host buffers (what a reference-side FFI would bind). */
 /* em.run_em (em.py:94-165): init_lnprops[n_multi*n_cols] drawn by the host;
  * props_out[n_cols] linear scale; read_mix_out (nullable) N x H log scale;
- * iters_out[n_multi], converged_out[n_multi] (nullable).  Iterations whose row likelihoods
- * underflow in linear space are redone in log space in every kind of session (one restart or
- * two per pass, one GPU or row-sharded), as the reference computes them. */
+ * iters_out[n_multi], converged_out[n_multi] (nullable).  One scheduler runs the restarts,
+ * one per pass or, over fp64 rows, two per pass (MXB_EM_NO_BATCH=1: one), and combines them in
+ * restart order as em.py:145-163 does; with max_iter <= 0 every restart hands back its init.
+ * Iterations whose row likelihoods underflow in linear space are redone in log space in every
+ * kind of session (one GPU or row-sharded), as the reference computes them. */
 /* flags: MXB_EM_SHARDED = the rows are this rank's shard of a larger matrix
  * (column sums all-reduced over the ctx comm every iteration);
  * MXB_EM_RAW = skip the final averaging (em.py:158-163): props_out then holds
@@ -290,7 +294,9 @@ int mxb_run_em_dev(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
  * ranks): m = logaddexp over ranks (in rank order) of m - sub_log, in place on every rank.
  * All-to-all of row shards (ncclSend/ncclRecv), local fold, shards broadcast back. */
 int mxb_matrix_fold_ranks(mxb_ctx *ctx, mxb_matrix *m, double sub_log);
-/* em.em_step (em.py:57-91): one E+M step, read_mix_out written in full. */
+/* em.em_step (em.py:57-91): one E+M step, read_mix_out written in full.  The same as
+ * mxb_run_em with MXB_EM_RAW, one restart, max_iter 1 and tol -1: new_props_out receives the
+ * new log-proportions, read_mix_out the read matrix of ln_props. */
 int mxb_em_step(mxb_ctx *ctx, const double *read_hap_mat, const double *weights,
                 const double *ln_props, int64_t n_rows, int64_t n_cols,
                 double *read_mix_out, double *new_props_out);

@@ -778,6 +778,114 @@ static int em_logspace_step(mxb_em *em, int cur, int slot = 0) {
     return MXB_OK;
 }
 
+}  // extern "C"
+
+namespace mxb {
+
+// The host side of every EM run that stops on convergence (mxb_em_iterate, run_em's restarts).
+// Iterations are enqueued in chunks ahead of the device for the restart slots that are live, and
+// the host polls the control blocks of all slots two chunks behind; a finished restart turns
+// the launches queued after it into early-exit no-ops.  No more iterations are enqueued than a
+// live restart may still run (max_iter minus those already enqueued for it), so a run of one
+// iteration launches one iteration's kernels.  Every decision depends only on the polled
+// control blocks and the arguments: in a row-sharded session the control blocks are identical
+// on every rank, so every rank enqueues the same launches (the NCCL tail and the peer-mailbox
+// sequence numbers rely on it).
+// An iteration flagged kDoneNeedsLogStep is redone in log space on its slot, and the run goes
+// on from the state the step leaves; the other slot's restart is not touched.  Polls taken
+// before a slot was redone or handed a new restart are ignored for that slot (generation
+// counters).  finish(slot, state, again) is called for every restart that converged or reached
+// max_iter; it sets `again` when it has put a new restart on the slot.
+template <typename Finish>
+static int em_poll_loop(mxb_em *em, int64_t max_iter, int n_live, Finish finish) {
+    mxb_ctx *ctx = em->ctx;
+    cudaStream_t s = ctx->stream;
+    constexpr int64_t kChunk = 16;
+    bool live[kMaxSlots] = {};
+    int gen[kMaxSlots] = {}, poll_gen[2][kMaxSlots] = {};
+    int64_t enq[kMaxSlots] = {}, poll_enq[2][kMaxSlots] = {};   // iterations enqueued per restart
+    bool pending[2] = {false, false};
+    for (int sl = 0; sl < n_live; ++sl) live[sl] = true;
+    auto room = [&]() {   // iterations the live restarts may still run
+        int64_t r = 0;
+        for (int sl = 0; sl < kMaxSlots; ++sl)
+            if (live[sl]) r = std::max(r, max_iter - enq[sl]);
+        return r;
+    };
+    for (int which = 0; n_live > 0; which ^= 1) {
+        const int64_t n = std::min(kChunk, room());
+        for (int64_t i = 0; i < n; ++i) MXB_TRY(enqueue_iteration(em));
+        for (int sl = 0; sl < kMaxSlots; ++sl) enq[sl] += n;
+        MXB_CUDA(cudaMemcpyAsync(em->host_state + which * kMaxSlots, em->state,
+                                 em->n_slots * sizeof(EmState), cudaMemcpyDeviceToHost, s));
+        MXB_CUDA(cudaEventRecord(em->poll_ev[which], s));
+        std::copy(gen, gen + kMaxSlots, poll_gen[which]);
+        std::copy(enq, enq + kMaxSlots, poll_enq[which]);
+        pending[which] = true;
+        // wait for the older poll, or for this one when nothing more can be enqueued
+        const int w = pending[which ^ 1] ? which ^ 1 : room() == 0 ? which : -1;
+        if (w < 0) continue;
+        MXB_CUDA(cudaEventSynchronize(em->poll_ev[w]));
+        pending[w] = false;
+        for (int sl = 0; sl < em->n_slots; ++sl) {
+            if (!live[sl] || poll_gen[w][sl] != gen[sl]) continue;
+            EmState &st = em->host_state[w * kMaxSlots + sl];
+            if (st.done == kDoneNeedsLogStep) {
+                MXB_TRY(em_logspace_step(em, st.cur, sl));   // returns with the stream drained
+                ++gen[sl];
+                MXB_CUDA(cudaMemcpyAsync(&st, em->state + sl, sizeof(EmState),
+                                         cudaMemcpyDeviceToHost, s));
+                MXB_CUDA(cudaStreamSynchronize(s));
+                enq[sl] = st.iters;
+            } else if (!st.done && poll_enq[w][sl] >= max_iter) {
+                // cannot happen: max_iter iterations always set done
+                set_error("EM: run did not terminate");
+                return MXB_ERR_CUDA;
+            }
+            if (!st.done) continue;
+            if (st.done == 3) {
+                set_error("EM: a peer rank did not deliver its column sums within %llu s",
+                          (unsigned long long)(kP2PTimeoutNs / 1000000000ull));
+                return MXB_ERR_CUDA;
+            }
+            if (st.bad) {
+                set_error("EM: the mixture likelihood of %d row group(s) underflowed to 0 "
+                          "(proportions left the fp64 range)", st.bad);
+                return MXB_ERR_RANGE;
+            }
+            bool again = false;
+            MXB_TRY(finish(sl, st, again));
+            if (again) {
+                ++gen[sl];
+                enq[sl] = 0;
+            } else {
+                live[sl] = false;
+                --n_live;
+            }
+        }
+    }
+    MXB_CUDA(cudaStreamSynchronize(s));
+    return MXB_OK;
+}
+
+// Read matrix of the log-proportions lnp (em.py:80-83) stored into dst (mode 0) or folded into
+// it with numpy.logaddexp (mode 1, em.py:156); sub_log is subtracted afterwards (em.py:161).
+static int launch_read_mix(mxb_em *em, const double *lnp, mxb_matrix *dst, int mode,
+                           double sub_log) {
+    if (em->n_rows == 0) return MXB_OK;   // a rank of a row-sharded run may hold no rows
+    mxb_ctx *ctx = em->ctx;
+    const int grid = (int)std::min<int64_t>(em->n_rows, (int64_t)ctx->num_sms * 8);
+    read_mix_kernel<<<grid, kMixThreads, 0, ctx->stream>>>(em->mat->data, em->n_rows, em->n_cols,
+                                                           lnp, dst->data, mode, sub_log);
+    ctx->launches++;
+    MXB_CUDA(cudaGetLastError());
+    return MXB_OK;
+}
+
+}  // namespace mxb
+
+extern "C" {
+
 int mxb_em_set_lnprops(mxb_em *em, const double *lnprops) {
     MXB_REQUIRE(em != nullptr && lnprops != nullptr, "NULL argument");
     mxb_ctx *ctx = em->ctx;
@@ -801,81 +909,15 @@ int mxb_em_iterate(mxb_em *em, int64_t max_iter, double tol, int64_t *iters_out,
     MXB_CUDA(cudaSetDevice(ctx->device));
     if (iters_out) *iters_out = 0;
     if (converged_out) *converged_out = 0;
-    if (max_iter <= 0) {  // em.py:126 loop body never runs; :141-143 hands back the init
-        em->zero_iter = true;
-        return MXB_OK;
-    }
-    em->zero_iter = false;
+    em->zero_iter = max_iter <= 0;
+    if (em->zero_iter) return MXB_OK;  // em.py:126 loop body never runs; :141-143 hands back the init
     // keep `cur` as set_lnprops left it (0), restart counters
     MXB_TRY(reset_state(em, max_iter, tol));
-
-    // Chunks of iterations are enqueued ahead of the host; a finished run turns
-    // the remaining launches into early-exit no-ops.  Two chunks in flight.
-    const int64_t kChunk = 16;
-    int64_t enqueued = 0;
-    int slot = 0;
-    bool pending[2] = {false, false};
-    EmState fin;
-    memset(&fin, 0, sizeof(fin));
-    bool finished = false;
-    int64_t log_steps = 0;
-    while (!finished) {
-        if (enqueued < max_iter) {
-            const int64_t n = std::min<int64_t>(kChunk, max_iter - enqueued);
-            for (int64_t i = 0; i < n; ++i) MXB_TRY(enqueue_iteration(em));
-            enqueued += n;
-        }
-        MXB_CUDA(cudaMemcpyAsync(&em->host_state[slot], em->state, sizeof(EmState),
-                                 cudaMemcpyDeviceToHost, ctx->stream));
-        MXB_CUDA(cudaEventRecord(em->poll_ev[slot], ctx->stream));
-        pending[slot] = true;
-        const int other = slot ^ 1;
-        // wait for the older chunk (or this one when nothing else can be queued)
-        const int wait_slot = pending[other] ? other : slot;
-        const bool must_wait = pending[other] || enqueued >= max_iter;
-        if (must_wait) {
-            MXB_CUDA(cudaEventSynchronize(em->poll_ev[wait_slot]));
-            pending[wait_slot] = false;
-            if (em->host_state[wait_slot].done == kDoneNeedsLogStep) {
-                // everything queued behind the flagged iteration was a no-op: drain, redo
-                // that iteration in log space, go on from the state it leaves
-                MXB_CUDA(cudaStreamSynchronize(ctx->stream));
-                pending[0] = pending[1] = false;
-                MXB_TRY(em_logspace_step(em, em->host_state[wait_slot].cur));
-                ++log_steps;
-                MXB_CUDA(cudaMemcpyAsync(&em->host_state[wait_slot], em->state, sizeof(EmState),
-                                         cudaMemcpyDeviceToHost, ctx->stream));
-                MXB_CUDA(cudaStreamSynchronize(ctx->stream));
-                enqueued = em->host_state[wait_slot].iters;
-                if (em->host_state[wait_slot].done) {
-                    fin = em->host_state[wait_slot];
-                    finished = true;
-                }
-            } else if (em->host_state[wait_slot].done) {
-                fin = em->host_state[wait_slot];
-                finished = true;
-            } else if (wait_slot == slot && enqueued >= max_iter) {
-                // cannot happen: max_iter iterations always set done
-                set_error("mxb_em_iterate: run did not terminate");
-                return MXB_ERR_CUDA;
-            }
-        }
-        slot = other;
-    }
-    MXB_CUDA(cudaStreamSynchronize(ctx->stream));
-    if (iters_out) *iters_out = fin.iters;
-    if (converged_out) *converged_out = (fin.done == 1);
-    if (fin.done == 3) {
-        set_error("EM: a peer rank did not deliver its column sums within %llu s",
-                  (unsigned long long)(kP2PTimeoutNs / 1000000000ull));
-        return MXB_ERR_CUDA;
-    }
-    if (fin.bad) {
-        set_error("EM: the mixture likelihood of %d row group(s) underflowed to 0 "
-                  "(proportions left the fp64 range)", fin.bad);
-        return MXB_ERR_RANGE;
-    }
-    return MXB_OK;
+    return em_poll_loop(em, max_iter, 1, [&](int, const EmState &st, bool &) {
+        if (iters_out) *iters_out = st.iters;
+        if (converged_out) *converged_out = (st.done == 1);
+        return MXB_OK;
+    });
 }
 
 int mxb_em_iterate_fixed(mxb_em *em, int64_t n_iter, float *elapsed_ms, float *pass_ms) {
@@ -1035,14 +1077,7 @@ int mxb_em_read_mix(mxb_em *em, mxb_matrix *dst, int mode, double sub_log) {
     EmState st;
     MXB_CUDA(cudaMemcpyAsync(&st, em->state, sizeof(st), cudaMemcpyDeviceToHost, ctx->stream));
     MXB_CUDA(cudaStreamSynchronize(ctx->stream));
-    if (em->n_rows == 0) return MXB_OK;
-    const int grid = (int)std::min<int64_t>(em->n_rows, (int64_t)ctx->num_sms * 8);
-    read_mix_kernel<<<grid, kMixThreads, 0, ctx->stream>>>(em->mat->data, em->n_rows, em->n_cols,
-                                                           em->lnp[st.cur], dst->data, mode,
-                                                           sub_log);
-    ctx->launches++;
-    MXB_CUDA(cudaGetLastError());
-    return MXB_OK;
+    return launch_read_mix(em, em->lnp[st.cur], dst, mode, sub_log);
 }
 
 int mxb_matrix_fold_ranks(mxb_ctx *ctx, mxb_matrix *m, double sub_log) {
@@ -1093,16 +1128,16 @@ int mxb_matrix_fold_ranks(mxb_ctx *ctx, mxb_matrix *m, double sub_log) {
 
 namespace mxb {
 
-// run_em's restart loop (em.py:117-156) on a two-slot session: two restarts iterate per
-// read of L; a slot whose restart has finished is handed the next one while the other
-// keeps going.  The host polls the control blocks two chunks behind the device, exactly
-// like mxb_em_iterate does for one restart.  Results are combined as the reference
-// combines them: final log-proportions summed in restart order (em.py:145-155), read
-// matrices folded with logaddexp in restart order (em.py:156): a restart that finishes before
-// an earlier one parks the proportions its read matrix is formed from until its turn.
-static int run_em_batched(mxb_em *em, const double *init_lnprops, int32_t n_multi,
-                          int64_t max_iter, double tol, bool raw, mxb_matrix *mix,
-                          double *props_out, int64_t *iters_out, int32_t *converged_out) {
+// run_em's restart loop (em.py:117-163) on a session with one or two restart slots: restart i
+// starts on the device from init_lnprops[i] as soon as a slot is free (two slots iterate two
+// restarts per read of L), and em_poll_loop drives all of them.  Results are combined as the
+// reference combines them: final log-proportions summed in restart order (em.py:145-155), then
+// averaged and exponentiated unless `raw` (em.py:158-163); read matrices folded with logaddexp
+// in restart order (em.py:156, :161).  A restart that finishes before an earlier one parks the
+// proportions its read matrix is formed from until its turn.
+static int run_restarts(mxb_em *em, const double *init_lnprops, int32_t n_multi, int64_t max_iter,
+                        double tol, bool raw, mxb_matrix *mix, StageTimer &tm, double *props_out,
+                        int64_t *iters_out, int32_t *converged_out) {
     mxb_ctx *ctx = em->ctx;
     cudaStream_t s = ctx->stream;
     const int64_t h = em->n_cols, ld = em->ld;
@@ -1130,107 +1165,61 @@ static int run_em_batched(mxb_em *em, const double *init_lnprops, int32_t n_mult
     }
     int rc = copy_h2d(ctx, d_inits, init_lnprops, vec_bytes);
 
+    int32_t next = 0, folded = 0;
     int slot_restart[kMaxSlots] = {-1, -1};
-    int slot_gen[kMaxSlots] = {0, 0};
-    int poll_gen[2][kMaxSlots] = {{0, 0}, {0, 0}};
-    int32_t next = 0, finished = 0, folded = 0;
     auto start_slot = [&](int sl) {
         const int32_t idx = next++;
         slot_restart[sl] = idx;
-        slot_gen[sl]++;
         em_set_props_kernel<<<(int)ceil_div(ld, 256), 256, 0, s>>>(
             d_inits + (size_t)idx * h, h, ld, em->lnp[0] + sl * ld, em->pi[0] + sl * ld,
             em->lnp[1] + sl * ld, em->pi[1] + sl * ld);
         em_reset_state_kernel<<<1, 1, 0, s>>>(em->state + sl, (long long)max_iter, tol);
         ctx->launches += 2;
     };
-    for (int sl = 0; sl < em->n_slots && rc == MXB_OK; ++sl)
-        if (next < n_multi) start_slot(sl);
-
-    const int64_t kChunk = 16;
-    bool pending[2] = {false, false};
-    int which = 0;
-    const int grid_mix = (int)std::min<int64_t>(em->n_rows, (int64_t)ctx->num_sms * 8);
-    while (rc == MXB_OK && finished < n_multi) {
-        for (int64_t i = 0; i < kChunk && rc == MXB_OK; ++i) rc = enqueue_iteration(em);
-        if (rc != MXB_OK) break;
-        if (cudaMemcpyAsync(&em->host_state[which * kMaxSlots], em->state,
-                            em->n_slots * sizeof(EmState), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
-            cudaEventRecord(em->poll_ev[which], s) != cudaSuccess) {
-            set_error("run_em: poll enqueue failed");
-            rc = MXB_ERR_CUDA;
-            break;
+    // fin, prev: the restart's final log-proportions and the ones before its last step
+    auto finish_restart = [&](int32_t idx, const double *fin, const double *prev,
+                              const EmState &st) -> int {
+        if (iters_out) iters_out[idx] = st.iters;
+        if (converged_out) converged_out[idx] = (st.done == 1);
+        MXB_CUDA(cudaMemcpyAsync(d_fin + (size_t)idx * h, fin, h * sizeof(double),
+                                 cudaMemcpyDeviceToDevice, s));
+        if (!mix) return MXB_OK;
+        // the read matrix comes from the proportions before the last step (SURVEY F5)
+        MXB_CUDA(cudaMemcpyAsync(d_prev + (size_t)idx * h, prev, h * sizeof(double),
+                                 cudaMemcpyDeviceToDevice, s));
+        done_restart[(size_t)idx] = 1;
+        if (!done_restart[(size_t)folded]) return MXB_OK;
+        tm.mark("iterate", kStageIterate);
+        for (; folded < n_multi && done_restart[(size_t)folded]; ++folded) {
+            const bool last = folded == n_multi - 1;
+            const double sub = (last && n_multi > 1 && !raw) ? log((double)n_multi) : 0.0;
+            MXB_TRY(launch_read_mix(em, d_prev + (size_t)folded * h, mix, folded == 0 ? 0 : 1, sub));
         }
-        for (int sl = 0; sl < kMaxSlots; ++sl) poll_gen[which][sl] = slot_gen[sl];
-        pending[which] = true;
-        const int other = which ^ 1;
-        if (pending[other]) {
-            if (cudaEventSynchronize(em->poll_ev[other]) != cudaSuccess) {
-                set_error("run_em: poll wait failed");
-                rc = MXB_ERR_CUDA;
-                break;
-            }
-            pending[other] = false;
-            for (int sl = 0; sl < em->n_slots && rc == MXB_OK; ++sl) {
-                const EmState st = em->host_state[other * kMaxSlots + sl];
-                if (slot_restart[sl] < 0 || poll_gen[other][sl] != slot_gen[sl] || !st.done) continue;
-                if (st.done == kDoneNeedsLogStep) {
-                    // a row's mixture likelihood underflowed in this slot's restart: redo that
-                    // iteration in log space on its slot and let the pair go on (the other
-                    // slot's restart kept iterating and is not touched).  The poll still in
-                    // flight was taken before the step: a new generation makes it skip the slot.
-                    rc = em_logspace_step(em, st.cur, sl);
-                    slot_gen[sl]++;
-                    continue;
-                }
-                const int32_t idx = slot_restart[sl];
-                if (st.bad) {
-                    set_error("EM: the mixture likelihood of some rows underflowed to 0 in "
-                              "restart %d (proportions left the fp64 range)", (int)idx);
-                    rc = MXB_ERR_RANGE;
-                    break;
-                }
-                if (iters_out) iters_out[idx] = st.iters;
-                if (converged_out) converged_out[idx] = (st.done == 1);
-                // lnp[cur] = proportions before the last step, lnp[1-cur] = after it
-                if (cudaMemcpyAsync(d_fin + (size_t)idx * h, em->lnp[1 - st.cur] + sl * ld,
-                                    h * sizeof(double), cudaMemcpyDeviceToDevice, s) != cudaSuccess) {
-                    set_error("run_em: result copy failed");
-                    rc = MXB_ERR_CUDA;
-                    break;
-                }
-                ++finished;
-                if (mix) {
-                    // the read matrix comes from the proportions before the last step (SURVEY
-                    // F5); the slot is reused, so they are kept until the restarts before this
-                    // one have been folded
-                    if (cudaMemcpyAsync(d_prev + (size_t)idx * h, em->lnp[st.cur] + sl * ld,
-                                        h * sizeof(double), cudaMemcpyDeviceToDevice, s) != cudaSuccess) {
-                        set_error("run_em: result copy failed");
-                        rc = MXB_ERR_CUDA;
-                        break;
-                    }
-                    done_restart[(size_t)idx] = 1;
-                    while (folded < n_multi && done_restart[(size_t)folded]) {
-                        const bool last = folded == n_multi - 1;
-                        const double sub = (last && n_multi > 1 && !raw) ? log((double)n_multi) : 0.0;
-                        read_mix_kernel<<<grid_mix, kMixThreads, 0, s>>>(
-                            em->mat->data, em->n_rows, em->n_cols, d_prev + (size_t)folded * h,
-                            mix->data, folded == 0 ? 0 : 1, sub);
-                        ctx->launches++;
-                        ++folded;
-                    }
-                }
-                slot_restart[sl] = -1;
-                if (next < n_multi) start_slot(sl);
-            }
-        }
-        which = other;
+        tm.mark("read_mix kernel", kStageReadMix);
+        return MXB_OK;
+    };
+    if (rc == MXB_OK && max_iter <= 0) {
+        // em.py:126's loop body never runs: every restart hands back its init (em.py:141-143)
+        const EmState none = {};
+        for (int32_t i = 0; i < n_multi && rc == MXB_OK; ++i)
+            rc = finish_restart(i, d_inits + (size_t)i * h, d_inits + (size_t)i * h, none);
+    } else if (rc == MXB_OK) {
+        int n_live = 0;
+        for (; n_live < em->n_slots && n_live < n_multi; ++n_live) start_slot(n_live);
+        rc = em_poll_loop(em, max_iter, n_live, [&](int sl, const EmState &st, bool &again) -> int {
+            // lnp[cur] = proportions before the last step, lnp[1-cur] = after it
+            MXB_TRY(finish_restart(slot_restart[sl], em->lnp[1 - st.cur] + sl * ld,
+                                   em->lnp[st.cur] + sl * ld, st));
+            again = next < n_multi;
+            if (again) start_slot(sl);
+            return MXB_OK;
+        });
     }
     if (cudaStreamSynchronize(s) != cudaSuccess && rc == MXB_OK) {
         set_error("run_em: stream sync failed: %s", cudaGetErrorString(cudaGetLastError()));
         rc = MXB_ERR_CUDA;
     }
+    tm.mark("iterate", kStageIterate);
     if (rc == MXB_OK) rc = copy_d2h(ctx, h_fin.data(), d_fin, vec_bytes);
     if (rc == MXB_OK) {
         for (int64_t j = 0; j < h; ++j) {
@@ -1265,7 +1254,6 @@ int mxb_run_em_dev(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
 
     mxb_em *em = nullptr;
     mxb_matrix *mix = nullptr;
-    std::vector<double> acc((size_t)h, 0.0), cur((size_t)h);
     StageTimer tm(ctx->stream);
     // the caller's result buffer is usually fresh pageable memory: fault its pages in
     // from background threads while the GPU iterates
@@ -1281,51 +1269,13 @@ int mxb_run_em_dev(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
     // process's mmap lock)
     if (rc == MXB_OK && read_mix_out)
         fault_mix.start(read_mix_out, (size_t)m->n_rows * (size_t)h * sizeof(double));
-    const bool batched = rc == MXB_OK && em->n_slots == 2;
-    if (batched) {
-        rc = run_em_batched(em, init_lnprops, n_multi, max_iter, tol, raw, mix, props_out,
-                            iters_out, converged_out);
-        tm.mark("iterate (two restarts per pass)", kStageIterate);
-    }
-    for (int32_t i = 0; rc == MXB_OK && !batched && i < n_multi; ++i) {
-        int64_t iters = 0;
-        int32_t conv = 0;
-        rc = mxb_em_set_lnprops(em, init_lnprops + (size_t)i * h);
-        if (rc == MXB_OK) rc = mxb_em_iterate(em, max_iter, tol, &iters, &conv);
-        tm.mark("iterate", kStageIterate);
-        if (iters_out) iters_out[i] = iters;
-        if (converged_out) converged_out[i] = conv;
-        if (rc == MXB_OK) rc = mxb_em_get_lnprops(em, 0, cur.data());
-        if (rc == MXB_OK) {
-            // em.py:145-155: first run stored, later runs added in place
-            if (i == 0) acc = cur;
-            else for (int64_t j = 0; j < h; ++j) acc[j] += cur[j];
-        }
-        if (rc == MXB_OK && want_mix) {
-            const bool last = (i == n_multi - 1);
-            const double sub = (last && n_multi > 1 && !raw) ? log((double)n_multi) : 0.0;
-            rc = mxb_em_read_mix(em, mix, i == 0 ? 0 : 1, sub);
-            tm.mark("read_mix kernel", kStageReadMix);
-        }
-    }
-    if (rc == MXB_OK) {
-        for (int64_t j = 0; j < h && !batched; ++j) {
-            double v = acc[j];
-            if (!raw) {
-                if (n_multi > 1) v /= (double)n_multi;  // em.py:158-160
-                v = exp(v);                             // em.py:163
-            }
-            props_out[j] = v;
-        }
-        if (read_mix_out) {
-            fault_mix.join();
-            rc = mxb_matrix_download(ctx, mix, read_mix_out);
-            tm.mark("download read_mix", kStageD2H);
-        }
-        else if (cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
-            set_error("mxb_run_em: stream sync failed");
-            rc = MXB_ERR_CUDA;
-        }
+    if (rc == MXB_OK)
+        rc = run_restarts(em, init_lnprops, n_multi, max_iter, tol, raw, mix, tm, props_out,
+                          iters_out, converged_out);
+    if (rc == MXB_OK && read_mix_out) {
+        fault_mix.join();
+        rc = mxb_matrix_download(ctx, mix, read_mix_out);
+        tm.mark("download read_mix", kStageD2H);
     }
     mxb_em_destroy(em);
     if (rc == MXB_OK && read_mix_dev) *read_mix_dev = mix;
@@ -1351,21 +1301,10 @@ int mxb_em_step(mxb_ctx *ctx, const double *read_hap_mat, const double *weights,
                 double *new_props_out) {
     MXB_REQUIRE(read_mix_out != nullptr && new_props_out != nullptr && ln_props != nullptr,
                 "NULL buffer");
-    mxb_matrix *m = nullptr, *mix = nullptr;
-    mxb_em *em = nullptr;
-    MXB_TRY(mxb_matrix_upload(ctx, read_hap_mat, n_rows, n_cols, &m));
-    int rc = mxb_em_create(ctx, m, weights, 0, &em);
-    if (rc == MXB_OK) rc = mxb_matrix_alloc(ctx, n_rows, n_cols, &mix);
-    if (rc == MXB_OK) rc = mxb_em_set_lnprops(em, ln_props);
-    // one iteration, never "converged": afterwards previous = ln_props, latest = new
-    if (rc == MXB_OK) rc = mxb_em_iterate(em, 1, -1.0, nullptr, nullptr);
-    if (rc == MXB_OK) rc = mxb_em_get_lnprops(em, 0, new_props_out);
-    if (rc == MXB_OK) rc = mxb_em_read_mix(em, mix, 0, 0.0);
-    if (rc == MXB_OK) rc = mxb_matrix_download(ctx, mix, read_mix_out);
-    mxb_em_destroy(em);
-    mxb_matrix_destroy(mix);
-    mxb_matrix_destroy(m);
-    return rc;
+    // one restart, one iteration that never converges (tol -1), not averaged: the result is
+    // its new log-proportions, the read matrix is stored from the previous ones (= ln_props)
+    return mxb_run_em(ctx, read_hap_mat, weights, n_rows, n_cols, ln_props, 1, 1, -1.0,
+                      MXB_EM_RAW, new_props_out, read_mix_out, nullptr, nullptr);
 }
 
 }  // extern "C"
