@@ -301,6 +301,34 @@ int mxb_em_step(mxb_ctx *ctx, const double *read_hap_mat, const double *weights,
                 const double *ln_props, int64_t n_rows, int64_t n_cols,
                 double *read_mix_out, double *new_props_out);
 
+/* ---- nonparametric bootstrap of the proportions (no counterpart in the reference) ----
+ * Replicate b draws W = sum(weights) fragments with replacement from the rows (row i carries
+ * weights[i] fragments; the weights must be finite non-negative integers with 1 <= W < 2^32,
+ * else MXB_ERR_VALUE): fragment f takes r = x0 | x1 << 32 of Philox4x32-10 with counter
+ * {f_lo, f_hi, b, 0} and key {seed_lo, seed_hi}, t = mulhi64(r, W), and the first row i whose
+ * inclusive prefix sum of the weights exceeds t.
+ * counts_out[k][i] = draws of row i by replicate boot0 + k (k < n_boot). */
+int mxb_boot_counts(mxb_ctx *ctx, const double *weights, int64_t n_rows, uint64_t seed,
+                    int64_t boot0, int64_t n_boot, uint32_t *counts_out);
+/* Replicates boot0 .. boot0 + n_boot - 1 of the fit start_lnprops (log-proportions, -inf for a
+ * zero): replicate b's row of lnprops_out is the final log-proportions of one run_em restart
+ * (em.py:117-143, with max_iter, tol, the swap back of em.py:141-143 and max_iter <= 0 handing
+ * back the start) on the matrix with replicate b's counts as weights, started from
+ * start_lnprops; iters_out / converged_out per replicate.  A replicate's result depends only on
+ * (m, weights, start_lnprops, seed, b, max_iter, tol).  Over class tiles several replicates
+ * iterate per launch; slots_out (nullable) = how many (chosen from the matrix by
+ * mxb_boot_slots' rule), 1 over fp64 rows. */
+int mxb_em_bootstrap(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
+                     const double *start_lnprops, int64_t boot0, int64_t n_boot, uint64_t seed,
+                     int64_t max_iter, double tol, double *lnprops_out, int64_t *iters_out,
+                     int32_t *converged_out, int32_t *slots_out);
+/* Replicate slots of a bootstrap session over class tiles with these batch class counts (as
+ * mxb_tile_plan takes them): the largest power of two R <= 16 whose tile plan for num_sms / R
+ * CTAs models at most R times the time of the plan for num_sms, with R * bytes_per_slot at
+ * most an eighth of free_bytes.  Host only, for the CPU tests. */
+int mxb_boot_slots(const int32_t *n_cls, int64_t n_batches, int64_t n_rows, int32_t num_sms,
+                   double bytes_per_slot, double free_bytes, int32_t *slots_out);
+
 #ifdef __cplusplus
 }
 #endif

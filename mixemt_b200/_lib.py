@@ -115,6 +115,11 @@ _PROTOS = {
     "mxb_run_em_dev": (ctypes.c_int, [P, P, P, P, c_i32, c_i64, c_dbl, c_i32, P, P,
                                       c_void_pp, P, P]),
     "mxb_em_step": (ctypes.c_int, [P, P, P, P, c_i64, c_i64, P, P]),
+    "mxb_boot_counts": (ctypes.c_int, [P, P, c_i64, ctypes.c_uint64, c_i64, c_i64, P]),
+    "mxb_em_bootstrap": (ctypes.c_int, [P, P, P, P, c_i64, c_i64, ctypes.c_uint64, c_i64, c_dbl,
+                                        P, P, P, ctypes.POINTER(c_i32)]),
+    "mxb_boot_slots": (ctypes.c_int, [P, c_i64, c_i64, c_i32, c_dbl, c_dbl,
+                                      ctypes.POINTER(c_i32)]),
 }
 
 EXPORTED_SYMBOLS = tuple(sorted(_PROTOS))

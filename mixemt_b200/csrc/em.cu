@@ -38,6 +38,7 @@
 #include <new>
 #include <vector>
 
+#include "bootstrap.cuh"
 #include "common.cuh"
 #include "em_kernels.cuh"
 #include "em_tiles.cuh"
@@ -95,6 +96,13 @@ struct mxb_em {
     int64_t tile_bytes_per_pass = 0;
     unsigned char *small = nullptr;  // one device block behind weights ... state (fewer driver calls)
     bool zero_iter = false;  // last iterate() ran no iteration
+    // Bootstrap session (run_bootstrap): n_slots replicates per launch, each with its own weight
+    // vector slot_w + s * n_rows; over class tiles the slots' Pi and U vectors lie
+    // tile_pi_stride and tile_u_stride doubles apart.
+    bool boot = false;
+    double *slot_w = nullptr;
+    unsigned char *boot_block = nullptr;
+    int64_t tile_pi_stride = 0, tile_u_stride = 0;
 };
 
 namespace mxb {
@@ -130,7 +138,7 @@ static pair_fn pick_pair(int nc) {
     return nullptr;
 }
 constexpr int kMaxPairNC = 6;   // 2 restarts x (pi + T) x NC double2 must fit 128 registers
-constexpr int kMaxSlots = 2;
+constexpr int kMaxSlots = kBootMaxSlots;
 
 // Launch with the programmatic-stream-serialization attribute (see pdl_wait): the kernel may
 // be scheduled before its predecessor in the stream has finished.  MXB_EM_NO_PDL=1 turns the
@@ -156,6 +164,48 @@ static cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, siz
     return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 
+// One iteration of every replicate slot of a bootstrap session over class tiles: the four
+// launches of a tiled iteration with the slot in blockIdx.y (z for the gather), all slots on
+// one plan of num_sms / n_slots CTAs.  A slot whose control block says done costs nothing.
+static int enqueue_tiles_slotted(mxb_em *em, cudaEvent_t *marks) {
+    mxb_ctx *ctx = em->ctx;
+    cudaStream_t s = ctx->stream;
+    const unsigned R = (unsigned)em->n_slots;
+    const int per = (int)ceil_div(em->n_cols, kTileThreads);
+    auto pi_fn = per <= 4 ? tile_pi_kernel<4, true> : per <= 8 ? tile_pi_kernel<8, true>
+                 : per <= 12 ? tile_pi_kernel<12, true> : tile_pi_kernel<16, true>;
+    MXB_CUDA(launch_pdl(pi_fn, dim3(std::min(em->n_batches, std::max(1, 2 * ctx->num_sms / (int)R)), R),
+                        dim3(kTileThreads), (size_t)em->ld * sizeof(double), s,
+                        (const unsigned short *)em->tile_perm, (const unsigned int *)em->tile_cword,
+                        em->tile_hs, (int)em->n_cols, (const TileDesc *)em->tile_desc,
+                        em->n_batches, (const double *)em->pi[0], (const double *)em->pi[1],
+                        (const EmState *)em->state, em->tile_pi, em->ld, em->tile_pi_stride));
+    if (marks) MXB_CUDA(cudaEventRecord(marks[0], s));
+    MXB_CUDA(launch_pdl(tile_pass_kernel<true>, dim3(em->tile_grid, R), dim3(kTilePassThreads),
+                        kTilePassSlotSmem, s, (const TileCta *)em->tile_ctas,
+                        (const TileSeg *)em->tile_segs, (const double *)em->tile_v,
+                        (const double *)em->tile_pi, em->state, em->tile_usum,
+                        em->tile_slot_bytes, em->tile_n_slots, (const double *)em->slot_w,
+                        em->n_rows, em->tile_pi_stride, em->tile_u_stride));
+    if (marks) MXB_CUDA(cudaEventRecord(marks[1], s));
+    g_plain_launch = true;   // as in the single-slot iteration (enqueue_iteration)
+    MXB_CUDA(launch_pdl(tile_gather_kernel<true>,
+                        dim3((unsigned)ceil_div(em->ld, kGatherThreads), em->tile_parts, R),
+                        dim3(kGatherThreads), 0, s, (const unsigned short *)em->tile_cmap,
+                        em->tile_hs, (int)em->n_cols, em->ld, (const int *)em->tile_ent_batch,
+                        (const int64_t *)em->tile_ent_off, em->tile_n_ent,
+                        (const double *)em->tile_usum, (const EmState *)em->state, em->partials,
+                        em->tile_u_stride));
+    if (marks) MXB_CUDA(cudaEventRecord(marks[2], s));
+    P2PArgs pa;
+    memset(&pa, 0, sizeof(pa));
+    MXB_CUDA(launch_pdl(em_finish_kernel<false>, dim3(kFinCtas, R), dim3(kFinThreads), 0, s,
+                        em->partials, em->n_part, em->n_cols, em->ld, em->lnp[0], em->lnp[1],
+                        em->pi[0], em->pi[1], em->state, pa));
+    ctx->launches += 4;
+    return MXB_OK;
+}
+
 // One EM iteration on em->ctx->stream (no host sync).
 // `marks` (optional, 3 events) are recorded after the class sums, after the pass and after the
 // gather of a tiled iteration (after the pass only for fp64 rows): per-kernel attribution.
@@ -164,6 +214,9 @@ static int enqueue_iteration(mxb_em *em, cudaEvent_t pass_begin = nullptr,
     mxb_ctx *ctx = em->ctx;
     cudaStream_t s = ctx->stream;
     if (pass_begin) MXB_CUDA(cudaEventRecord(pass_begin, s));
+    if (em->tiled && em->boot) return enqueue_tiles_slotted(em, marks);
+    // fp64 rows of a bootstrap session: one replicate at a time, with the slot's weights
+    const double *weights = em->slot_w ? em->slot_w : em->weights;
     if (em->n_slots == 2) {
         const size_t ps = (size_t)em->n_part * em->ld;
         {
@@ -192,37 +245,39 @@ static int enqueue_iteration(mxb_em *em, cudaEvent_t pass_begin = nullptr,
                                 (const unsigned short *)em->tile_perm,
                                 (const unsigned int *)em->tile_cword, em->tile_hs,
                                 (int)em->n_cols, (const TileDesc *)em->tile_desc, em->n_batches,
-                                (const double *)em->pi[0], (const double *)em->pi[1],
-                                (const EmState *)em->state, em->tile_pi));
+                                    (const double *)em->pi[0], (const double *)em->pi[1],
+                                (const EmState *)em->state, em->tile_pi, (int64_t)0, (int64_t)0));
         }
         if (marks) MXB_CUDA(cudaEventRecord(marks[0], s));
-        MXB_CUDA(launch_pdl(tile_pass_kernel, dim3(em->tile_grid), dim3(kTilePassThreads),
+        MXB_CUDA(launch_pdl(tile_pass_kernel<false>, dim3(em->tile_grid), dim3(kTilePassThreads),
                             kTilePassSmem, s, (const TileCta *)em->tile_ctas,
                             (const TileSeg *)em->tile_segs, (const double *)em->tile_v, (const double *)em->tile_pi, em->state,
-                            em->tile_usum, em->tile_slot_bytes, em->tile_n_slots));
+                            em->tile_usum, em->tile_slot_bytes, em->tile_n_slots,
+                            (const double *)nullptr, (int64_t)0, (int64_t)0, (int64_t)0));
         if (marks) MXB_CUDA(cudaEventRecord(marks[1], s));
         // The gather waits in plain stream order: launched early it would sit on the SMs the
         // first CTAs of the pass leave and keep them from nothing, but measured it costs 27 us
         // per iteration (B200, config 2), while the other three launches gain from the overlap.
         g_plain_launch = true;
-        MXB_CUDA(launch_pdl(tile_gather_kernel,
+        MXB_CUDA(launch_pdl(tile_gather_kernel<false>,
                             dim3((unsigned)ceil_div(em->ld, kGatherThreads), em->tile_parts),
                             dim3(kGatherThreads), 0, s, (const unsigned short *)em->tile_cmap,
                             em->tile_hs, (int)em->n_cols, em->ld, (const int *)em->tile_ent_batch,
                             (const int64_t *)em->tile_ent_off, em->tile_n_ent,
-                            (const double *)em->tile_usum, (const EmState *)em->state, em->partials));
+                            (const double *)em->tile_usum, (const EmState *)em->state, em->partials,
+                            (int64_t)0));
         if (marks) MXB_CUDA(cudaEventRecord(marks[2], s));
         ctx->launches += 3;
     } else if (em->fast) {
         MXB_CUDA(launch_pdl(pick_pass(em->nc), dim3(em->grid_fast), dim3(kPassThreads),
                             em->smem_bytes, s, (const unsigned char *)em->lin,
-                            (uint32_t)(em->ld * sizeof(double)), em->ld, em->n_rows, em->weights,
+                            (uint32_t)(em->ld * sizeof(double)), em->ld, em->n_rows, weights,
                             em->pi[0], em->pi[1], em->state, em->partials, em->n_stages));
         ctx->launches += 1;
     } else {
         const int rd_blocks = (int)std::max<int64_t>(
             1, std::min<int64_t>(ceil_div(em->n_rows, 8), (int64_t)ctx->num_sms * 8));
-        em_rowdot_kernel<<<rd_blocks, 256, 0, s>>>(em->lin, em->ld, em->n_rows, em->weights,
+        em_rowdot_kernel<<<rd_blocks, 256, 0, s>>>(em->lin, em->ld, em->n_rows, weights,
                                                    em->pi[0], em->pi[1], em->state, em->coef);
         dim3 grid(em->row_blocks, em->col_blocks);
         em_colacc_kernel<<<grid, 256, 0, s>>>(em->lin, em->ld, em->n_rows, em->coef, em->state,
@@ -311,6 +366,7 @@ int mxb_em_destroy(mxb_em *em) {
     dev_free(em->ctx, em->tile_vecs);
     dev_free(em->ctx, em->tile_v);
     dev_free(em->ctx, em->small);
+    dev_free(em->ctx, em->boot_block);
     for (int i = 0; i < 2; ++i)
         if (em->poll_ev[i]) cudaEventDestroy(em->poll_ev[i]);
     delete em;  // host_state points into the context's pinned scratch
@@ -431,6 +487,21 @@ static int em_pack_tiles(mxb_em *em) {
     if (!tile_ring(max_r_pad, slot_bytes, n_slots)) return give_up(false, "rows too long for the ring");
     TilePlanOut plan;
     tile_plan(desc, n, ctx->num_sms, slot_bytes, p_cells, plan);
+    int n_rep = 1;   // replicate slots of a bootstrap session (tile_plan.h: boot_slots)
+    if (em->boot && em->fused_tail) {
+        auto up8 = [](int64_t c) { return (double)(((size_t)c * 8 + 255) & ~(size_t)255); };
+        const int parts = std::max(1, std::min(32, (int)plan.ent_batch.size() / 8));
+        const double per_slot = up8(p_cells) + up8(p_cells + plan.extra_cells) +
+                                (double)parts * em->ld * 8 + (double)n * 8 + 4.0 * em->ld * 8 +
+                                sizeof(EmState);
+        size_t free_b = 0, total_b = 0;
+        if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { cudaGetLastError(); free_b = 0; }
+        n_rep = boot_slots(desc, n, ctx->num_sms, slot_bytes, p_cells, per_slot, (double)free_b);
+        if (n_rep > 1) {
+            plan = TilePlanOut();
+            tile_plan(desc, n, ctx->num_sms / n_rep, slot_bytes, p_cells, plan);
+        }
+    }
     const std::vector<TileCta> &ctas = plan.ctas;
     const std::vector<TileSeg> &segs = plan.segs;
     const std::vector<int> &ent_batch = plan.ent_batch;
@@ -477,12 +548,14 @@ static int em_pack_tiles(mxb_em *em) {
     const size_t b_seg = up((size_t)n_seg * sizeof(TileSeg));
     const size_t b_entb = up((size_t)n_ent * sizeof(int));
     const size_t b_ento = up((size_t)n_ent * sizeof(int64_t));
+    // [Pi x n_rep][U x n_rep][plan]
+    const size_t b_vecs = (size_t)n_rep * (b_pi + b_u);
     if (e == cudaSuccess)
-        e = dev_alloc(ctx, (void **)&vecs, b_pi + b_u + b_cta + b_seg + b_entb + b_ento);
+        e = dev_alloc(ctx, (void **)&vecs, b_vecs + b_cta + b_seg + b_entb + b_ento);
     if (e != cudaSuccess) { dev_free(ctx, vecs); return give_up(false, "tiles"); }
     double *pi_cls = reinterpret_cast<double *>(vecs);
-    double *u_sum = reinterpret_cast<double *>(vecs + b_pi);
-    unsigned char *tail = vecs + b_pi + b_u;
+    double *u_sum = reinterpret_cast<double *>(vecs + (size_t)n_rep * b_pi);
+    unsigned char *tail = vecs + b_vecs;
     TileCta *d_ctas = reinterpret_cast<TileCta *>(tail);
     TileSeg *d_segs = reinterpret_cast<TileSeg *>(tail + b_cta);
     int *d_entb = reinterpret_cast<int *>(tail + b_cta + b_seg);
@@ -496,7 +569,7 @@ static int em_pack_tiles(mxb_em *em) {
         e = cudaMemcpyAsync(d_entb, ent_batch.data(), (size_t)n_ent * sizeof(int), cudaMemcpyHostToDevice, ctx->stream);
     if (e == cudaSuccess)
         e = cudaMemcpyAsync(d_ento, ent_off.data(), (size_t)n_ent * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(vecs, 0, b_pi + b_u, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(vecs, 0, b_vecs, ctx->stream);
     if (e == cudaSuccess) e = cudaMemsetAsync(d_bad, 0, (size_t)nb * sizeof(int), ctx->stream);
     if (e == cudaSuccess) {
         tile_fill_kernel<<<std::min(nb, ctx->num_sms * 4), kTileThreads, 0, ctx->stream>>>(
@@ -509,11 +582,18 @@ static int em_pack_tiles(mxb_em *em) {
         e = cudaMemcpyAsync(bad.data(), d_bad, (size_t)nb * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     if (e == cudaSuccess)
-        e = cudaFuncSetAttribute((const void *)tile_pass_kernel,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTilePassSmem);
+        e = em->boot ? cudaFuncSetAttribute((const void *)tile_pass_kernel<true>,
+                                            cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                            (int)kTilePassSlotSmem)
+                     : cudaFuncSetAttribute((const void *)tile_pass_kernel<false>,
+                                            cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                            (int)kTilePassSmem);
     for (int v = 0; v < 4 && e == cudaSuccess; ++v) {
         const void *fn = v == 0 ? (const void *)tile_pi_kernel<4> : v == 1 ? (const void *)tile_pi_kernel<8>
                          : v == 2 ? (const void *)tile_pi_kernel<12> : (const void *)tile_pi_kernel<16>;
+        if (em->boot)
+            fn = v == 0 ? (const void *)tile_pi_kernel<4, true> : v == 1 ? (const void *)tile_pi_kernel<8, true>
+                 : v == 2 ? (const void *)tile_pi_kernel<12, true> : (const void *)tile_pi_kernel<16, true>;
         e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)(kTileMaxCols * sizeof(double)));
     }
@@ -546,14 +626,19 @@ static int em_pack_tiles(mxb_em *em) {
     em->tile_grid = n_cta;
     em->tile_parts = std::max(1, std::min(32, n_ent / 8));
     em->n_part = em->tile_parts;
+    em->tile_pi_stride = (int64_t)(b_pi / sizeof(double));
+    em->tile_u_stride = (int64_t)(b_u / sizeof(double));
+    if (em->boot) em->n_slots = n_rep;
     // what an iteration reads and writes: the tiles, perm + cmap (Pi), cmap (gather), the class
     // vectors (Pi written and read, U written and read)
     em->tile_bytes_per_pass = v_cells * 8 + 3 * (int64_t)nb * hs * 2 + 2 * (p_cells + u_cells) * 8;
     return rc;
 }
 
+static int em_alloc_boot_slots(mxb_em *em);
+
 static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weights, int sharded,
-                          int want_slots, mxb_em **out) {
+                          int want_slots, mxb_em **out, bool boot = false) {
     MXB_REQUIRE(ctx != nullptr && m != nullptr && out != nullptr, "NULL argument");
     // a rank of a row-sharded run may hold no rows at all (fewer signatures than GPUs)
     MXB_REQUIRE((m->n_rows > 0 || sharded) && m->n_cols > 0, "EM needs a non-empty matrix");
@@ -568,6 +653,7 @@ static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weigh
     em->n_cols = m->n_cols;
     em->ld = round_up(m->n_cols, kLdAlign);
     em->sharded = sharded != 0;
+    em->boot = boot;
 
     // launch geometry
     const size_t row_bytes = (size_t)em->ld * sizeof(double);
@@ -654,7 +740,14 @@ static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weigh
             mxb_em_destroy(em);
             return rc;
         }
-        if (em->tiled) em->n_slots = 1;   // restarts run one at a time over the tiles
+        if (em->tiled && !em->boot) em->n_slots = 1;   // restarts run one at a time over the tiles
+        if (em->boot) {
+            const int brc = em_alloc_boot_slots(em);
+            if (brc != MXB_OK) {
+                mxb_em_destroy(em);
+                return brc;
+            }
+        }
     }
     if (!em->tiled) STEP(dev_alloc(ctx, (void **)&em->lin, (size_t)em->n_rows * row_bytes));
     if (e == cudaSuccess && em->n_rows > 0 && !em->tiled) {
@@ -713,7 +806,7 @@ int mxb_em_pass_bytes(const mxb_em *em, int64_t *bytes_per_pass, int64_t *n_dens
 // logsumexp forms it, global maxima first (all-reduce max), then the non-maximal sum s and
 // the weight m of the maximal terms per column (all-reduce sum), so every rank forms the
 // same ln pi' and takes the same decision.
-static int em_logspace_step(mxb_em *em, int cur, int slot = 0) {
+static int em_logspace_step(mxb_em *em, int cur, int slot, const double *weights) {
     mxb_ctx *ctx = em->ctx;
     cudaStream_t s = ctx->stream;
     const int64_t n = em->n_rows, h = em->n_cols, ld = em->ld;
@@ -741,7 +834,7 @@ static int em_logspace_step(mxb_em *em, int cur, int slot = 0) {
         em_logspace_rows_kernel<<<row_grid, 256, 0, s>>>(em->mat->data, n, h, lnp, lse);
         ctx->launches += 1;
     }
-    em_logspace_cols_kernel<<<col_grid, 256, 0, s>>>(em->mat->data, n, h, lnp, lse, em->weights,
+    em_logspace_cols_kernel<<<col_grid, 256, 0, s>>>(em->mat->data, n, h, lnp, lse, weights,
                                                      nullptr, part);
     em_logspace_colreduce_kernel<<<col_blocks, 256, 0, s>>>(part, kRowBlocks, h, 1, colmax);
     ctx->launches += 2;
@@ -749,7 +842,7 @@ static int em_logspace_step(mxb_em *em, int cur, int slot = 0) {
         rc = nccl_allreduce_f64(ctx, colmax, h, 1);
         if (rc == MXB_OK) {
             em_logspace_cols_split_kernel<<<col_grid, 256, 0, s>>>(
-                em->mat->data, n, h, lnp, lse, em->weights, colmax, part);
+                em->mat->data, n, h, lnp, lse, weights, colmax, part);
             em_logspace_colreduce_kernel<<<(int)ceil_div(n_sums, 256), 256, 0, s>>>(
                 part, kRowBlocks, n_sums, 0, colsum);
             ctx->launches += 2;
@@ -757,7 +850,7 @@ static int em_logspace_step(mxb_em *em, int cur, int slot = 0) {
         }
     } else {
         em_logspace_cols_kernel<<<col_grid, 256, 0, s>>>(em->mat->data, n, h, lnp, lse,
-                                                         em->weights, colmax, part);
+                                                         weights, colmax, part);
         em_logspace_colreduce_kernel<<<col_blocks, 256, 0, s>>>(part, kRowBlocks, h, 0, colsum);
         ctx->launches += 2;
     }
@@ -792,7 +885,7 @@ namespace mxb {
 // on every rank, so every rank enqueues the same launches (the NCCL tail and the peer-mailbox
 // sequence numbers rely on it).
 // An iteration flagged kDoneNeedsLogStep is redone in log space on its slot, and the run goes
-// on from the state the step leaves; the other slot's restart is not touched.  Polls taken
+// on from the state the step leaves; the other slots' runs are not touched.  Polls taken
 // before a slot was redone or handed a new restart are ignored for that slot (generation
 // counters).  finish(slot, state, again) is called for every restart that converged or reached
 // max_iter; it sets `again` when it has put a new restart on the slot.
@@ -831,7 +924,9 @@ static int em_poll_loop(mxb_em *em, int64_t max_iter, int n_live, Finish finish)
             if (!live[sl] || poll_gen[w][sl] != gen[sl]) continue;
             EmState &st = em->host_state[w * kMaxSlots + sl];
             if (st.done == kDoneNeedsLogStep) {
-                MXB_TRY(em_logspace_step(em, st.cur, sl));   // returns with the stream drained
+                // (the slot's own weights in a bootstrap session)
+                const double *w = em->slot_w ? em->slot_w + sl * em->n_rows : em->weights;
+                MXB_TRY(em_logspace_step(em, st.cur, sl, w));   // returns with the stream drained
                 ++gen[sl];
                 MXB_CUDA(cudaMemcpyAsync(&st, em->state + sl, sizeof(EmState),
                                          cudaMemcpyDeviceToHost, s));
@@ -866,6 +961,18 @@ static int em_poll_loop(mxb_em *em, int64_t max_iter, int n_live, Finish finish)
     }
     MXB_CUDA(cudaStreamSynchronize(s));
     return MXB_OK;
+}
+
+// What a finished slot hands back (em.py:137-143): its final log-proportions are lnp[1 - cur],
+// the ones before its last step (the read matrix's, SURVEY F5) lnp[cur].
+struct SlotResult {
+    const double *fin, *prev;
+    int64_t iters;
+    int32_t converged;
+};
+static SlotResult slot_result(const mxb_em *em, int sl, const EmState &st) {
+    return {em->lnp[1 - st.cur] + sl * em->ld, em->lnp[st.cur] + sl * em->ld, st.iters,
+            st.done == 1 ? 1 : 0};
 }
 
 // Read matrix of the log-proportions lnp (em.py:80-83) stored into dst (mode 0) or folded into
@@ -1177,15 +1284,14 @@ static int run_restarts(mxb_em *em, const double *init_lnprops, int32_t n_multi,
         ctx->launches += 2;
     };
     // fin, prev: the restart's final log-proportions and the ones before its last step
-    auto finish_restart = [&](int32_t idx, const double *fin, const double *prev,
-                              const EmState &st) -> int {
-        if (iters_out) iters_out[idx] = st.iters;
-        if (converged_out) converged_out[idx] = (st.done == 1);
-        MXB_CUDA(cudaMemcpyAsync(d_fin + (size_t)idx * h, fin, h * sizeof(double),
+    auto finish_restart = [&](int32_t idx, const SlotResult &res) -> int {
+        if (iters_out) iters_out[idx] = res.iters;
+        if (converged_out) converged_out[idx] = res.converged;
+        MXB_CUDA(cudaMemcpyAsync(d_fin + (size_t)idx * h, res.fin, h * sizeof(double),
                                  cudaMemcpyDeviceToDevice, s));
         if (!mix) return MXB_OK;
         // the read matrix comes from the proportions before the last step (SURVEY F5)
-        MXB_CUDA(cudaMemcpyAsync(d_prev + (size_t)idx * h, prev, h * sizeof(double),
+        MXB_CUDA(cudaMemcpyAsync(d_prev + (size_t)idx * h, res.prev, h * sizeof(double),
                                  cudaMemcpyDeviceToDevice, s));
         done_restart[(size_t)idx] = 1;
         if (!done_restart[(size_t)folded]) return MXB_OK;
@@ -1200,16 +1306,13 @@ static int run_restarts(mxb_em *em, const double *init_lnprops, int32_t n_multi,
     };
     if (rc == MXB_OK && max_iter <= 0) {
         // em.py:126's loop body never runs: every restart hands back its init (em.py:141-143)
-        const EmState none = {};
         for (int32_t i = 0; i < n_multi && rc == MXB_OK; ++i)
-            rc = finish_restart(i, d_inits + (size_t)i * h, d_inits + (size_t)i * h, none);
+            rc = finish_restart(i, {d_inits + (size_t)i * h, d_inits + (size_t)i * h, 0, 0});
     } else if (rc == MXB_OK) {
         int n_live = 0;
         for (; n_live < em->n_slots && n_live < n_multi; ++n_live) start_slot(n_live);
         rc = em_poll_loop(em, max_iter, n_live, [&](int sl, const EmState &st, bool &again) -> int {
-            // lnp[cur] = proportions before the last step, lnp[1-cur] = after it
-            MXB_TRY(finish_restart(slot_restart[sl], em->lnp[1 - st.cur] + sl * ld,
-                                   em->lnp[st.cur] + sl * ld, st));
+            MXB_TRY(finish_restart(slot_restart[sl], slot_result(em, sl, st)));
             again = next < n_multi;
             if (again) start_slot(sl);
             return MXB_OK;
@@ -1236,9 +1339,201 @@ static int run_restarts(mxb_em *em, const double *init_lnprops, int32_t n_multi,
     return rc;
 }
 
+// The slot buffers of a bootstrap session, sized for its n_slots when it is created:
+// [weights ns x n][lnp 2 x ns x ld][pi 2 x ns x ld][partials ns x n_part x ld][state ns].  They
+// take the place of the single-slot buffers of the session's `small` block.
+static int em_alloc_boot_slots(mxb_em *em) {
+    mxb_ctx *ctx = em->ctx;
+    const int64_t n = em->n_rows, ld = em->ld;
+    const size_t ns = (size_t)em->n_slots;
+    auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t b_w = up(ns * n * sizeof(double)), b_vec = up(ns * ld * sizeof(double));
+    const size_t b_part = up(ns * (size_t)em->n_part * ld * sizeof(double));
+    const size_t b_st = up(ns * sizeof(EmState));
+    const size_t total_b = b_w + 4 * b_vec + b_part + b_st;
+    if (dev_alloc(ctx, (void **)&em->boot_block, total_b) != cudaSuccess) {
+        cudaGetLastError();
+        set_error("bootstrap: device allocation of %zu bytes failed", total_b);
+        return MXB_ERR_NOMEM;
+    }
+    unsigned char *p = em->boot_block;
+    em->slot_w = (double *)p; p += b_w;
+    for (int i = 0; i < 2; ++i) { em->lnp[i] = (double *)p; p += b_vec; }
+    for (int i = 0; i < 2; ++i) { em->pi[i] = (double *)p; p += b_vec; }
+    em->partials = (double *)p; p += b_part;
+    em->state = (EmState *)p;
+    return MXB_OK;
+}
+
+// Replicates whose results are kept on the device at a time: the output is downloaded in
+// windows of this many rows (at most 177 MB at H = 5408), whatever n_boot is.
+constexpr int64_t kBootOutRows = 4096;
+
+// The bootstrap (bootstrap.cu for the draw): replicates boot0 .. boot0 + n_boot - 1 are put on
+// the session's slots in order, each resampled on the device when its slot is handed it, started
+// from `start` and iterated by em_poll_loop as one restart of run_em on its counts; a finished
+// slot's final log-proportions go to row b - boot0 of the output and the slot takes the next
+// replicate of the window.  Over class tiles the slots iterate side by side
+// (enqueue_tiles_slotted), over fp64 rows one at a time.
+static int run_bootstrap(mxb_em *em, const double *start, const int64_t *d_cumw, uint64_t total,
+                         uint64_t seed, int64_t boot0, int64_t n_boot, int64_t max_iter,
+                         double tol, double *lnprops_out, int64_t *iters_out,
+                         int32_t *converged_out) {
+    mxb_ctx *ctx = em->ctx;
+    cudaStream_t s = ctx->stream;
+    const int64_t n = em->n_rows, h = em->n_cols, ld = em->ld;
+    const size_t ns = (size_t)em->n_slots;
+    const int64_t win = std::min(n_boot, kBootOutRows);
+    // [counts n][start h][results win x h]
+    auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    const size_t b_cnt = up((size_t)n * sizeof(uint32_t)), b_start = up((size_t)h * sizeof(double));
+    const size_t b_out = (size_t)win * h * sizeof(double);
+    unsigned char *work = nullptr;
+    if (dev_alloc(ctx, (void **)&work, b_cnt + b_start + b_out) != cudaSuccess) {
+        cudaGetLastError();
+        set_error("bootstrap: device allocation of %zu bytes failed", b_cnt + b_start + b_out);
+        return MXB_ERR_NOMEM;
+    }
+    uint32_t *counts = (uint32_t *)work;
+    double *d_start = (double *)(work + b_cnt);
+    double *d_out = (double *)(work + b_cnt + b_start);
+    int rc = MXB_OK;
+    if (cudaMemsetAsync(counts, 0, b_cnt, s) != cudaSuccess) {
+        set_error("bootstrap: %s", cudaGetErrorString(cudaGetLastError()));
+        rc = MXB_ERR_CUDA;
+    }
+    // slots that get no replicate (n_boot < n_slots) stay done: their CTAs exit at once
+    std::vector<EmState> idle(ns);
+    for (EmState &st : idle) {
+        memset(&st, 0, sizeof(st));
+        st.done = 1;
+    }
+    if (rc == MXB_OK) rc = copy_h2d(ctx, em->state, idle.data(), ns * sizeof(EmState));
+    if (rc == MXB_OK) rc = copy_h2d(ctx, d_start, start, (size_t)h * sizeof(double));
+
+    int64_t next = 0, w_end = 0;
+    int64_t slot_rep[kMaxSlots] = {};
+    auto start_slot = [&](int sl) -> int {
+        const int64_t k = next++;
+        slot_rep[sl] = k;
+        double *w = em->slot_w + sl * n;
+        MXB_TRY(boot_draw(ctx, d_cumw, n, total, seed, boot0 + k, 1, counts));
+        MXB_TRY(boot_take_counts(ctx, counts, n, w));
+        em_set_props_kernel<<<(int)ceil_div(ld, 256), 256, 0, s>>>(
+            d_start, h, ld, em->lnp[0] + sl * ld, em->pi[0] + sl * ld, em->lnp[1] + sl * ld,
+            em->pi[1] + sl * ld);
+        em_reset_state_kernel<<<1, 1, 0, s>>>(em->state + sl, (long long)max_iter, tol);
+        ctx->launches += 2;
+        MXB_CUDA(cudaGetLastError());
+        return MXB_OK;
+    };
+    for (int64_t w0 = 0; rc == MXB_OK && w0 < n_boot; w0 = w_end) {
+        w_end = std::min(n_boot, w0 + win);
+        int n_live = 0;
+        for (; rc == MXB_OK && n_live < em->n_slots && next < w_end; ++n_live) rc = start_slot(n_live);
+        if (rc == MXB_OK)
+            rc = em_poll_loop(em, max_iter, n_live, [&](int sl, const EmState &st, bool &again) -> int {
+                const SlotResult res = slot_result(em, sl, st);
+                const int64_t k = slot_rep[sl];
+                iters_out[k] = res.iters;
+                converged_out[k] = res.converged;
+                MXB_CUDA(cudaMemcpyAsync(d_out + (size_t)(k - w0) * h, res.fin,
+                                         h * sizeof(double), cudaMemcpyDeviceToDevice, s));
+                again = next < w_end;
+                if (again) MXB_TRY(start_slot(sl));
+                return MXB_OK;
+            });
+        if (rc == MXB_OK)
+            rc = copy_d2h(ctx, lnprops_out + (size_t)w0 * h, d_out,
+                          (size_t)(w_end - w0) * h * sizeof(double));
+    }
+    dev_free(ctx, work);
+    return rc;
+}
+
 }  // namespace mxb
 
 extern "C" {
+
+int mxb_boot_slots(const int32_t *n_cls, int64_t n_batches, int64_t n_rows, int32_t num_sms,
+                   double bytes_per_slot, double free_bytes, int32_t *slots_out) {
+    MXB_REQUIRE(n_cls != nullptr && slots_out != nullptr && n_batches > 0 &&
+                n_rows > (n_batches - 1) * kTileRows && n_rows <= n_batches * kTileRows &&
+                num_sms > 0, "bad arguments");
+    for (int64_t b = 0; b < n_batches; ++b)
+        MXB_REQUIRE(n_cls[b] >= 1 && n_cls[b] <= kTileMaxCols, "class counts must be in 1..8192");
+    std::vector<TileDesc> desc;
+    int64_t v_cells = 0, p_cells = 0;
+    int max_r_pad = 4;
+    tile_layout(n_cls, (int)n_batches, n_rows, desc, v_cells, p_cells, max_r_pad);
+    uint32_t slot_bytes = 0;
+    int n_slots = 0;
+    MXB_REQUIRE(tile_ring(max_r_pad, slot_bytes, n_slots), "rows too long for the ring");
+    *slots_out = boot_slots(desc, n_rows, num_sms, slot_bytes, p_cells, bytes_per_slot, free_bytes);
+    return MXB_OK;
+}
+
+int mxb_em_bootstrap(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
+                     const double *start_lnprops, int64_t boot0, int64_t n_boot, uint64_t seed,
+                     int64_t max_iter, double tol, double *lnprops_out, int64_t *iters_out,
+                     int32_t *converged_out, int32_t *slots_out) {
+    MXB_REQUIRE(ctx != nullptr && m != nullptr && weights != nullptr && start_lnprops != nullptr,
+                "NULL argument");
+    MXB_REQUIRE(lnprops_out != nullptr && iters_out != nullptr && converged_out != nullptr,
+                "NULL buffer");
+    const int64_t n = m->n_rows, h = m->n_cols;
+    if (n_boot < 1 || boot0 < 0 || boot0 + n_boot > (1ll << 32)) {
+        set_error("bootstrap: need n_boot >= 1 and replicate numbers in [0, 2^32)");
+        return MXB_ERR_VALUE;
+    }
+    double mass = 0.0;
+    for (int64_t j = 0; j < h; ++j) {
+        if (isnan(start_lnprops[j])) {
+            set_error("bootstrap: start log-proportion %lld is NaN", (long long)j);
+            return MXB_ERR_VALUE;
+        }
+        mass += exp(start_lnprops[j]);
+    }
+    if (!(mass > 0.0)) {
+        set_error("bootstrap: the start proportions sum to 0");
+        return MXB_ERR_VALUE;
+    }
+    std::vector<int64_t> cumw;
+    uint64_t total = 0;
+    MXB_TRY(boot_prefix(weights, n, cumw, total));
+    if (slots_out) *slots_out = 1;
+    if (max_iter <= 0) {
+        // em.py:126's loop body never runs: every replicate hands back the start (em.py:141-143)
+        for (int64_t k = 0; k < n_boot; ++k) {
+            memcpy(lnprops_out + k * h, start_lnprops, (size_t)h * sizeof(double));
+            iters_out[k] = 0;
+            converged_out[k] = 0;
+        }
+        return MXB_OK;
+    }
+    MXB_CUDA(cudaSetDevice(ctx->device));
+    mxb_em *em = nullptr;
+    MXB_TRY(em_create_impl(ctx, m, weights, 0, 1, &em, true));
+    int64_t *d_cumw = nullptr;
+    int rc = MXB_OK;
+    if (dev_alloc(ctx, (void **)&d_cumw, (size_t)n * sizeof(int64_t)) != cudaSuccess) {
+        cudaGetLastError();
+        set_error("bootstrap: device allocation failed");
+        rc = MXB_ERR_NOMEM;
+    }
+    if (rc == MXB_OK) rc = copy_h2d(ctx, d_cumw, cumw.data(), (size_t)n * sizeof(int64_t));
+    if (rc == MXB_OK && slots_out) *slots_out = em->n_slots;
+    if (rc == MXB_OK)
+        rc = run_bootstrap(em, start_lnprops, d_cumw, total, seed, boot0, n_boot, max_iter, tol,
+                           lnprops_out, iters_out, converged_out);
+    if (cudaStreamSynchronize(ctx->stream) != cudaSuccess && rc == MXB_OK) {
+        set_error("bootstrap: %s", cudaGetErrorString(cudaGetLastError()));
+        rc = MXB_ERR_CUDA;
+    }
+    dev_free(ctx, d_cumw);
+    mxb_em_destroy(em);
+    return rc;
+}
 
 int mxb_run_em_dev(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
                    const double *init_lnprops, int32_t n_multi, int64_t max_iter, double tol,

@@ -220,18 +220,27 @@ __device__ __forceinline__ SegItem seg_shfl_up(const SegItem &v, int off) {
     return o;
 }
 
-template <int PER>
+// kSlots (bootstrap sessions, em.cu: run_bootstrap): blockIdx.y is a replicate slot; its
+// proportions, control block and class sums lie pi_stride, one EmState and cls_stride further.
+template <int PER, bool kSlots = false>
 __global__ void __launch_bounds__(kTileThreads)
 tile_pi_kernel(const unsigned short *__restrict__ perm, const unsigned int *__restrict__ cword,
                int hs, int n_cols, const TileDesc *__restrict__ desc, int n_batches,
                const double *__restrict__ pi0, const double *__restrict__ pi1,
-               const EmState *__restrict__ st, double *__restrict__ pi_cls) {
+               const EmState *__restrict__ st, double *__restrict__ pi_cls,
+               int64_t pi_stride, int64_t cls_stride) {
     static_assert(PER % 4 == 0 && PER <= 16, "chunks are read as 8-byte words");
     extern __shared__ __align__(128) unsigned char tile_smem[];
     double *pi = reinterpret_cast<double *>(tile_smem);     // [n_cols]: the gathers below are
     // random 8-byte reads, cheaper from shared memory than through L1 tags
     pdl_wait();
     pdl_launch_dependents();
+    if (kSlots) {
+        st += blockIdx.y;
+        pi0 += blockIdx.y * pi_stride;
+        pi1 += blockIdx.y * pi_stride;
+        pi_cls += blockIdx.y * cls_stride;
+    }
     if (st->done) return;
     const double *__restrict__ pi_g = st->cur ? pi1 : pi0;
     __shared__ int s_flag[kTileWarps];
@@ -342,6 +351,12 @@ constexpr int kTileSlotBarrier0 = 10;
 constexpr size_t kTilePassSmem = kTileRingBytes + kTileScratchBytes +
                                  2 * kTileMaxSlots * sizeof(uint64_t) +
                                  2 * kTileWarps * sizeof(double) + 128;
+// the slotted pass (bootstrap) also stages the weights of two segments: [2][kTileRows] doubles
+// behind `red`
+constexpr size_t kTileWeightsOff = kTileRingBytes + kTileScratchBytes +
+                                   2 * kTileMaxSlots * sizeof(uint64_t) +
+                                   2 * kTileWarps * sizeof(double);
+constexpr size_t kTilePassSlotSmem = kTilePassSmem + 2 * kTileRows * sizeof(double);
 
 struct TileSeg {           // the rows of one batch inside one CTA's range
     int64_t v_off;         // its first row in V (doubles)
@@ -353,7 +368,8 @@ struct TileSeg {           // the rows of one batch inside one CTA's range
     int32_t n_rows;
     int32_t fit, n_copies; // rows per copy (the last one takes what is left), copies
     int32_t batch;
-    int32_t pad[3];
+    int32_t row0;          // global index of its first row (the weight of a bootstrap slot)
+    int32_t pad[2];
 };
 static_assert(sizeof(TileSeg) == 64, "one record per 64-byte line");
 
@@ -384,11 +400,19 @@ __device__ __forceinline__ void named_barrier(int id, int threads) {
 __device__ long long g_tile_trace[160 * kTileWarps * 8];
 #endif
 
+// kSlots: blockIdx.y is a bootstrap replicate slot (see tile_pi_kernel); the weight of a row is
+// the slot's (n_rows doubles per slot) instead of column n_cls of the tile.  The weights of a
+// segment are staged in shared memory (two buffers, segment si in buffer si & 1): the next
+// segment's are stored before the barrier of the end-of-batch exchange, after which nobody reads
+// the buffer they replace.
+template <bool kSlots = false>
 __global__ void __launch_bounds__(kTilePassThreads, 1)
 tile_pass_kernel(const TileCta *__restrict__ ctas, const TileSeg *__restrict__ segs,
                  const double *__restrict__ v,
                  const double *__restrict__ pi_cls, EmState *__restrict__ st,
-                 double *__restrict__ u_sum, uint32_t slot_bytes, int n_slots) {
+                 double *__restrict__ u_sum, uint32_t slot_bytes, int n_slots,
+                 const double *__restrict__ slot_w, int64_t n_rows, int64_t cls_stride,
+                 int64_t u_stride) {
     extern __shared__ __align__(128) unsigned char tile_smem[];
     double *scratch = reinterpret_cast<double *>(tile_smem + kTileRingBytes);
     uint64_t *full = reinterpret_cast<uint64_t *>(tile_smem + kTileRingBytes + kTileScratchBytes);
@@ -405,8 +429,17 @@ tile_pass_kernel(const TileCta *__restrict__ ctas, const TileSeg *__restrict__ s
     __syncthreads();
     pdl_wait();               // the class sums of this iteration are complete
     pdl_launch_dependents();
-    if (st->done) return;
+    // slot offsets are formed where a pointer is used, from the kernel parameters: registers are
+    // short, and the parameters can be read again at no register cost
+#define MXB_SLOT(stride) (kSlots ? (int64_t)blockIdx.y * (stride) : (int64_t)0)
+    if (st[MXB_SLOT(1)].done) return;
     const TileCta cta = ctas[blockIdx.x];
+    double *w_stage = reinterpret_cast<double *>(tile_smem + kTileWeightsOff);
+    if (kSlots) {
+        const TileSeg *s0 = segs + cta.seg0;
+        if (tid < s0->n_rows) w_stage[tid] = slot_w[MXB_SLOT(n_rows) + s0->row0 + tid];
+        __syncthreads();
+    }
     const uint32_t ring_u32 = smem_u32(tile_smem);
     const uint32_t full_u32 = smem_u32(full);
     const TileSeg *my_segs = segs + cta.seg0;
@@ -448,7 +481,7 @@ tile_pass_kernel(const TileCta *__restrict__ ctas, const TileSeg *__restrict__ s
     int L = 1 << sg.lg, idx = tid & (L - 1);
     int kl = min(K, max(0, (((sg.n_cls + 1) >> 1) - idx + L - 1) >> sg.lg));
     {
-        const double2 *pcls = reinterpret_cast<const double2 *>(pi_cls + sg.p_off) + idx;
+        const double2 *pcls = reinterpret_cast<const double2 *>(pi_cls + MXB_SLOT(cls_stride) + sg.p_off) + idx;
 #pragma unroll
         for (int k = 0; k < K; ++k) p[k] = k < kl ? pcls[k << sg.lg] : make_double2(0.0, 0.0);
     }
@@ -502,8 +535,16 @@ tile_pass_kernel(const TileCta *__restrict__ ctas, const TileSeg *__restrict__ s
                     for (int k = 0; k < K; ++k)
                         x[k] = lds_v2_f64(src + chunk0 + (uint32_t)min(k, k_last) * chunk_stride);
                     double wr;
-                    asm volatile("ld.shared.f64 %0, [%1];" : "=d"(wr) : "r"(src + (uint32_t)sg.n_cls * 8u) : "memory");
-                    if (!have) wr = 0.0;
+                    if (kSlots) {
+                        asm volatile("ld.shared.f64 %0, [%1];" : "=d"(wr)
+                                     : "r"(ring_u32 + (uint32_t)kTileWeightsOff +
+                                           (uint32_t)(((si & 1) * kTileRows + (have ? row : 0)) * 8))
+                                     : "memory");
+                        if (!have) wr = 0.0;
+                    } else {
+                        asm volatile("ld.shared.f64 %0, [%1];" : "=d"(wr) : "r"(src + (uint32_t)sg.n_cls * 8u) : "memory");
+                        if (!have) wr = 0.0;
+                    }
 #pragma unroll
                     for (int k = 0; k < K; k += 2) {
                         d0 = fma(x[k].x, p[k].x, d0);
@@ -591,7 +632,7 @@ tile_pass_kernel(const TileCta *__restrict__ ctas, const TileSeg *__restrict__ s
         idx = tid & (L - 1);
         kl = min(K, max(0, (((sg_next.n_cls + 1) >> 1) - idx + L - 1) >> sg_next.lg));
         if (si + 1 < cta.n_segs) {
-            const double2 *pcls = reinterpret_cast<const double2 *>(pi_cls + sg_next.p_off) + idx;
+            const double2 *pcls = reinterpret_cast<const double2 *>(pi_cls + MXB_SLOT(cls_stride) + sg_next.p_off) + idx;
 #pragma unroll
             for (int k = 0; k < K; ++k) p[k] = k < kl ? pcls[k << sg_next.lg] : make_double2(0.0, 0.0);
         }
@@ -619,10 +660,12 @@ tile_pass_kernel(const TileCta *__restrict__ ctas, const TileSeg *__restrict__ s
             for (int k = 0; k < K; ++k)
                 if (k < kl_cur) dst[k << lg] = u[k];
         }
+        if (kSlots && si + 1 < cta.n_segs && tid < sg_next.n_rows)
+            w_stage[((si + 1) & 1) * kTileRows + tid] = slot_w[MXB_SLOT(n_rows) + sg_next.row0 + tid];
         named_barrier(9, 32 * kTileConsumers);
         {
             const double2 *sc = sc_base;
-            double2 *out = reinterpret_cast<double2 *>(u_sum + sg.u_dst);
+            double2 *out = reinterpret_cast<double2 *>(u_sum + MXB_SLOT(u_stride) + sg.u_dst);
             for (int c = tid; c < chunks; c += 32 * kTileConsumers) {
                 double2 acc = sc[c];
                 for (int t = 1; t < n_slices; ++t) {
@@ -645,7 +688,8 @@ tile_pass_kernel(const TileCta *__restrict__ ctas, const TileSeg *__restrict__ s
         tr[5] = cta.n_segs; tr[6] = cta.n_copies; tr[7] = 1;
     }
 #endif
-    if (__any_sync(0xffffffffu, bad) && lane == 0) atomicAdd(&st->bad, 1);
+    if (__any_sync(0xffffffffu, bad) && lane == 0) atomicAdd(&st[MXB_SLOT(1)].bad, 1);
+#undef MXB_SLOT
 }
 
 // T_j = sum over batches of U_b[cmap_b[j]], batches in ascending order; the batches are split
@@ -654,13 +698,21 @@ tile_pass_kernel(const TileCta *__restrict__ ctas, const TileSeg *__restrict__ s
 constexpr int kGatherThreads = 256;
 constexpr int kGatherUnroll = 8;
 
+// kSlots: blockIdx.z is a bootstrap replicate slot (U vectors u_stride apart, partials of
+// gridDim.y ranges per slot).
+template <bool kSlots = false>
 __global__ void __launch_bounds__(kGatherThreads)
 tile_gather_kernel(const unsigned short *__restrict__ cmap, int hs, int n_cols, int64_t ld,
                    const int *__restrict__ ent_batch, const int64_t *__restrict__ ent_off,
                    int n_ent, const double *__restrict__ u_sum, const EmState *__restrict__ st,
-                   double *__restrict__ partials) {
+                   double *__restrict__ partials, int64_t u_stride) {
     pdl_wait();
     pdl_launch_dependents();
+    if (kSlots) {
+        st += blockIdx.z;
+        u_sum += blockIdx.z * u_stride;
+        partials += (size_t)blockIdx.z * gridDim.y * ld;
+    }
     if (st->done) return;
     const int j = blockIdx.x * kGatherThreads + threadIdx.x;
     if (j >= ld) return;

@@ -18,6 +18,7 @@ struct TilePlanOut {
     std::vector<int64_t> ent_off;
     int64_t extra_cells = 0;              // U vectors of the second, third.. segment of a batch
     int n_copy = 0;
+    double time = 0.0;                    // modelled time of the pass: its slowest CTA (cycles)
 };
 
 // Layout: threads per row, tile and class-vector offsets of every batch.
@@ -84,7 +85,10 @@ inline void tile_plan(const std::vector<TileDesc> &desc, int64_t n, int num_sms,
         auto close_cta = [&]() {
             if (warp_t > 0.0) {
                 ++used_ctas;
-                if (emit) out.ctas.push_back(cur);
+                if (emit) {
+                    out.ctas.push_back(cur);
+                    out.time = std::max(out.time, std::max(warp_t, mem_t));
+                }
             }
             cur.seg0 = (int)out.segs.size();
             cur.n_segs = cur.n_copies = 0;
@@ -132,6 +136,7 @@ inline void tile_plan(const std::vector<TileDesc> &desc, int64_t n, int num_sms,
                     sg.fit = fit;
                     sg.n_copies = (int)ceil_div(take, fit);
                     sg.v_off = d.v_off + (int64_t)r * d.r_pad;
+                    sg.row0 = d.row0 + r;
                     out.ent_batch.push_back(b);
                     out.ent_off.push_back(sg.u_dst);
                     cur.n_copies += sg.n_copies;
@@ -181,6 +186,29 @@ inline int tile_plan_check(const std::vector<TileDesc> &desc, const TilePlanOut 
     for (int b = 0; b < nb; ++b) if (rows_of[(size_t)b] != desc[(size_t)b].n_rows) ++errs;
     if (copies_sum != plan.n_copy || next_seg != (int)plan.segs.size()) ++errs;
     return errs;
+}
+
+// Replicate slots of a bootstrap session (em.cu: run_bootstrap): the pass of R slots runs on
+// num_sms / R CTAs per slot, all R in one wave on one plan.  R is the largest power of two up to
+// kBootMaxSlots whose plan models at most R times the time of the full-budget plan (R replicates
+// then cost no more than R iterations one after another; launch and tail costs, which the model
+// leaves out, only favour a larger R), and whose slot buffers (bytes_per_slot each) take at most
+// an eighth of the free device memory.  From the matrix alone: a replicate's arithmetic does not
+// depend on how many replicates are asked for.
+constexpr int kBootMaxSlots = 16;
+inline int boot_slots(const std::vector<TileDesc> &desc, int64_t n, int num_sms,
+                      uint32_t slot_bytes, int64_t p_cells, double bytes_per_slot,
+                      double free_bytes) {
+    TilePlanOut full;
+    tile_plan(desc, n, num_sms, slot_bytes, p_cells, full);
+    int best = 1;
+    for (int r = 2; r <= kBootMaxSlots && num_sms / r >= 1; r *= 2) {
+        if ((double)r * bytes_per_slot > free_bytes / 8) break;
+        TilePlanOut p;
+        tile_plan(desc, n, num_sms / r, slot_bytes, p_cells, p);
+        if (p.time <= r * full.time) best = r;
+    }
+    return best;
 }
 
 }  // namespace mxb

@@ -161,3 +161,21 @@ def npy_layout(n_total, h, lo=0):
                                             "shape": (int(n_total), int(h))})
     header = buf.getvalue()
     return header, len(header) + int(lo) * int(h) * 8
+
+
+def merge_bootstrap(lnprops, iters, conv, boot0, n_boot, allreduce):
+    """Bootstrap fan-out: this rank's replicates ``boot0 .. boot0 + len(lnprops) - 1`` (its
+    ``restart_shard`` block) placed into zero rows of the ``(n_boot, H)`` log-proportions and
+    the iteration counts and converged flags behind them, then one sum all-reduce.  Adding
+    zeros is exact (``-inf`` survives), so every rank gets what one rank running all
+    replicates computes."""
+    lnprops = np.asarray(lnprops, dtype=np.float64)   # (replicates of this rank, H)
+    h = lnprops.shape[1]
+    buf = np.zeros((n_boot, h + 2))
+    k = len(iters)
+    buf[boot0:boot0 + k, :h] = lnprops
+    buf[boot0:boot0 + k, h] = iters
+    buf[boot0:boot0 + k, h + 1] = conv
+    assert np.abs(buf[:, h]).max(initial=0) < _EXACT, "iteration counts not exact in fp64"
+    buf = allreduce(np.ascontiguousarray(buf), "sum")
+    return buf[:, :h], buf[:, h].astype(np.int64), buf[:, h + 1].astype(np.int32)
