@@ -627,8 +627,9 @@ em_update_kernel(const double *__restrict__ tsum, int64_t n_cols, int64_t ld,
         const double p = pi_old[j];
         const double t = tsum[j];
         double ln_new;
-        if (p >= 1e-290) ln_new = log(p * t / total);
-        else ln_new = lnp_old[j] + log(t / total);  // pi underflowed: stay in log space
+        // pi or pi * T underflows: stay in log space (see em_finish_kernel)
+        if (p >= 1e-290 && p * t >= 1e-290) ln_new = log(p * t / total);
+        else ln_new = lnp_old[j] + log(t / total);
         const double p_new = exp(ln_new);
         lnp_new[j] = ln_new;
         pi_new[j] = p_new;
@@ -835,14 +836,16 @@ em_finish_kernel(const double *partials, int n_part, int64_t n_cols, int64_t ld,
     double dl = 0.0;
     if (owner) {
         double2 ln_new = make_double2(-INFINITY, -INFINITY), p_new = make_double2(0.0, 0.0);
+        // pi underflowed, or pi * T did (a column far worse than the mixture in every row, whose
+        // decay factor T / total is tiny): stay in log space, else ln pi' would be -inf
         if (live_x) {
-            if (p.x >= 1e-290) ln_new.x = log(p.x * t.x / total);
-            else ln_new.x = lnp_old[2 * c] + log(t.x / total);  // pi underflowed: stay in log space
+            if (p.x >= 1e-290 && p.x * t.x >= 1e-290) ln_new.x = log(p.x * t.x / total);
+            else ln_new.x = lnp_old[2 * c] + log(t.x / total);
             p_new.x = exp(ln_new.x);
             dl += fabs(p_new.x - p.x);
         }
         if (live_y) {
-            if (p.y >= 1e-290) ln_new.y = log(p.y * t.y / total);
+            if (p.y >= 1e-290 && p.y * t.y >= 1e-290) ln_new.y = log(p.y * t.y / total);
             else ln_new.y = lnp_old[2 * c + 1] + log(t.y / total);
             p_new.y = exp(ln_new.y);
             dl += fabs(p_new.y - p.y);

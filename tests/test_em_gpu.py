@@ -239,6 +239,60 @@ def test_dying_components_stay_in_log_space():
     assert np.allclose(read_mix[fin], o_mix[fin], rtol=1e-9, atol=1e-9)
 
 
+@pytest.mark.parametrize("h,layout,gaps", [
+    (1100, "rows", (50.0, 200.0, 400.0)),
+    (5408, "tiles", (50.0, 200.0, 400.0)),
+    (3, "general", (50.0, 200.0)),
+    (9000, "general", (50.0, 200.0, 400.0)),
+])
+def test_fast_dying_components_stay_in_log_space(h, layout, gaps):
+    """Columns 50 to 400 log units below every row's best decay so fast that
+    pi * T underflows while pi is still above 1e-290: their log-proportions
+    must stay finite and track the reference as in
+    test_dying_components_stay_in_log_space (em_finish_kernel, em_update_kernel),
+    on class tiles, fp64 rows and the general path."""
+    import ctypes
+    import os
+    from mixemt_b200._lib import lib, check, ptr
+    rs = np.random.RandomState(3)
+    n = 64
+    if layout == "tiles":   # blocks of 64 identical columns: class tiles
+        mat = np.repeat(np.full((n, h // 64 + 1), -40.0), 64, axis=1)[:, :h].copy()
+    else:
+        mat = np.full((n, h), -40.0)
+    mat[np.arange(n), rs.randint(0, min(4, h), size=n)] = 0.0   # up to four live columns
+    dying = np.arange(h - len(gaps), h)
+    for j, g in zip(dying, gaps):
+        mat[:, j] = -g - rs.uniform(0.0, 5.0, size=n)
+    init = np.full(h, 1.0 / h)
+    init[dying] = 1e-3
+    inits = np.log(init).reshape(1, h)
+    max_iter = 40
+    ctx = get_context()
+    dev = DeviceMatrix.from_host(ctx, mat)
+    wts = np.ones(n)
+    if layout == "rows":     # the matrix compresses: keep fp64 rows on purpose
+        os.environ["MXB_EM_NO_PACK"] = "1"
+    try:
+        sess = ctypes.c_void_p()
+        check(lib.mxb_em_create(ctx.handle, dev.handle, ptr(wts), 0, ctypes.byref(sess)))
+        nbytes, flag = ctypes.c_int64(), ctypes.c_int64()
+        check(lib.mxb_em_pass_bytes(sess, ctypes.byref(nbytes), ctypes.byref(flag)))
+        lib.mxb_em_destroy(sess)
+        assert flag.value == (0 if layout == "tiles" else -1)
+        a = make_args(max_iter=max_iter, tolerance=0.0)
+        props, read_mix, info, _ = em.run_em_device(dev, wts, a, inits=inits)
+    finally:
+        os.environ.pop("MXB_EM_NO_PACK", None)
+        dev.free()
+    o_props, o_mix, _ = oracle_c.run_em(mat, wts, inits, max_iter, 0.0)
+    assert np.abs(props - o_props).max() < 1e-12
+    fin = np.isfinite(o_mix)
+    assert o_mix[fin].min() < -800.0                     # far below exp() underflow
+    assert np.allclose(read_mix[fin], o_mix[fin], rtol=1e-9, atol=1e-9)
+    assert close_mix(read_mix, o_mix)
+
+
 # ---- size-independent properties at scale ------------------------------------------
 def test_properties_config1_shape(phylo17):
     """Config-1 shape (10k fragments x 5408): proportions sum to 1, the true
