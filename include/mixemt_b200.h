@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define MXB_ABI_VERSION 1
+#define MXB_ABI_VERSION 2
 
 enum {
     MXB_OK = 0,
@@ -153,13 +153,18 @@ int mxb_phylo_destroy(mxb_phylo *phylo);
 /* ---- kernel 1: matrix build (replaces build_em_matrix, preprocess.py:177) --- */
 /* CSR rows -> fp64 N x H log-likelihood matrix.  out_host (nullable) receives
  * the matrix, match_host (nullable) the int32 per-cell match counts
- * (mismatches = K_i - matches), out_dev (nullable) keeps the matrix resident.
- * elapsed_ms (nullable) = device time of the build kernel alone. */
+ * (mismatches = K_i - matches), route_host (nullable) the path that finished
+ * each row: route_host[i] = path + 4 * (number of 32-column groups the class
+ * kernel walked with its per-group dense loop), path 0 = class kernel tier 1,
+ * 1 = tier 2, 2 = tier 2's dense row walk, 3 = dense kernel (H > 8192 or
+ * MXB_BUILD_DENSE=1).  Nothing is written to it when H == 0.  out_dev
+ * (nullable) keeps the matrix resident.  elapsed_ms (nullable) = device time
+ * of the build kernel alone. */
 int mxb_build_matrix(mxb_ctx *ctx, const mxb_phylo *phylo, int64_t n_rows,
                      const int64_t *row_ptr, const int32_t *pos_idx,
                      const uint8_t *base_code, double *out_host,
-                     int32_t *match_host, mxb_matrix **out_dev,
-                     float *elapsed_ms);
+                     int32_t *match_host, int32_t *route_host,
+                     mxb_matrix **out_dev, float *elapsed_ms);
 
 /* ---- device matrices ------------------------------------------------------- */
 int mxb_matrix_alloc(mxb_ctx *ctx, int64_t n_rows, int64_t n_cols, mxb_matrix **out);

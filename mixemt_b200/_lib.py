@@ -82,7 +82,7 @@ _PROTOS = {
     "mxb_sigset_destroy": (ctypes.c_int, [P]),
     "mxb_phylo_pack": (ctypes.c_int, [P, c_i32, c_i32, c_i32, P, P, P, P, P, P, c_void_pp]),
     "mxb_phylo_destroy": (ctypes.c_int, [P]),
-    "mxb_build_matrix": (ctypes.c_int, [P, P, c_i64, P, P, P, P, P, c_void_pp,
+    "mxb_build_matrix": (ctypes.c_int, [P, P, c_i64, P, P, P, P, P, P, c_void_pp,
                                         ctypes.POINTER(ctypes.c_float)]),
     "mxb_matrix_alloc": (ctypes.c_int, [P, c_i64, c_i64, c_void_pp]),
     "mxb_matrix_upload": (ctypes.c_int, [P, P, c_i64, c_i64, c_void_pp]),

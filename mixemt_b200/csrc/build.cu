@@ -63,6 +63,7 @@
 // observations) walks the dense bitset table cell by cell: build_dense_row /
 // the per-group dense loop, the same arithmetic as build_matrix_dense_kernel,
 // the plain kernel that is also used when H > 8192 (or MXB_BUILD_DENSE=1 is set).
+#include <algorithm>
 #include <new>
 #include <string.h>
 #include <vector>
@@ -345,6 +346,9 @@ __device__ __forceinline__ void run_chains(int first, int n_left, int lane, int 
 // Rows come from row_list[0 .. *n_list) when row_list != NULL, else 0 .. n_rows.
 // Rows that do not fit the pools are appended to overflow_list when there is
 // one (tier 1), else they take the dense path (tier 2).
+// route_out (nullable, zeroed by the host): route_out[row] = path + 4 * (groups walked by the
+// per-group dense loop), path 0 = tier 1, 1 = tier 2, 2 = build_dense_row (mxb_build_matrix).
+// Tier 1 writes only rows with dense groups, tier 2 every row it finishes.
 template <bool kCounts, class Tier, int kMaxGroups>
 __global__ void __launch_bounds__(Tier::kThreads, kCounts ? 1 : Tier::kMinBlocks)
 build_matrix_kernel(BuildTables tb, int64_t n_rows, const int32_t *__restrict__ row_list,
@@ -352,7 +356,8 @@ build_matrix_kernel(BuildTables tb, int64_t n_rows, const int32_t *__restrict__ 
                     int *__restrict__ overflow_count, int *__restrict__ work_counter,
                     const int64_t *__restrict__ row_ptr,
                     const int32_t *__restrict__ pos_idx, const uint8_t *__restrict__ base_code,
-                    double *__restrict__ out, int32_t *__restrict__ match_out) {
+                    double *__restrict__ out, int32_t *__restrict__ match_out,
+                    int32_t *__restrict__ route_out) {
     extern __shared__ __align__(16) unsigned char smem[];
     __shared__ int s_next[2];
     __shared__ int s_overflow;
@@ -361,6 +366,7 @@ build_matrix_kernel(BuildTables tb, int64_t n_rows, const int32_t *__restrict__ 
     __shared__ int s_nlist;
     using L = BuildSmem<Tier, kMaxGroups, kCounts>;
     constexpr int W = Tier::kObsWords;
+    constexpr bool kLastTier = W * 32 == kMaxObs;   // only the last tier has the staging room
     constexpr int kClassThreads = Tier::kThreads;
     constexpr int kClassWarps = kClassThreads / 32;
     constexpr int kWorkWarps = kClassWarps - 1;  // the last warp runs the prefix chain
@@ -624,17 +630,20 @@ build_matrix_kernel(BuildTables tb, int64_t n_rows, const int32_t *__restrict__ 
         if (too_long || s_overflow) {  // block-uniform: the row does not fit this tier's pools
             if (overflow_list) {
                 if (tid == 0) overflow_list[atomicAdd(overflow_count, 1)] = (int32_t)row;
-            } else if constexpr (W * 32 == kMaxObs) {  // only the last tier has the staging room
+            } else if constexpr (kLastTier) {
                 build_dense_row<kClassThreads>(tb.bits, tb.hitmiss, tb.n_planes, tb.n_words, n_hap,
                                                k0, k1, pos_idx, base_code, out_row, match_row,
                                                s_term, s_off);
+                if (route_out && tid == 0) route_out[row] = 2;
             }
             __syncthreads();  // the row's shared state is reused by the next row
             continue;
         }
 
+        if (kLastTier && route_out && tid == 0) route_out[row] = 1 + 4 * s_ndense;
         // groups with more than 32 deviating positions: walk the dense table, one warp each
         if (s_ndense > 0) {   // block-uniform
+            if (!kLastTier && route_out && tid == 0) route_out[row] = 4 * s_ndense;
 #pragma unroll 1
             for (int g = warp; g < n_groups; g += kClassWarps) {
                 if (s_gbase[g] != kDenseGroup) continue;
@@ -695,7 +704,7 @@ static cudaError_t launch_tier(mxb_ctx *ctx, const BuildTables &tb, int64_t n_ro
                                const int32_t *list_in, const int *n_in, int32_t *list_out,
                                int *n_out, int *work_counter, const int64_t *row_ptr,
                                const int32_t *pos_idx, const uint8_t *base_code, double *out,
-                               int32_t *match_out) {
+                               int32_t *match_out, int32_t *route_out) {
     constexpr size_t smem_bytes = BuildSmem<Tier, kMaxGroups, kCounts>::total;
     auto fn = build_matrix_kernel<kCounts, Tier, kMaxGroups>;
     cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -708,7 +717,7 @@ static cudaError_t launch_tier(mxb_ctx *ctx, const BuildTables &tb, int64_t n_ro
     const int grid = (int)std::min<int64_t>(n_rows, (int64_t)ctx->num_sms * per_sm);
     fn<<<grid, Tier::kThreads, smem_bytes, ctx->stream>>>(tb, n_rows, list_in, n_in, list_out,
                                                           n_out, work_counter, row_ptr, pos_idx,
-                                                          base_code, out, match_out);
+                                                          base_code, out, match_out, route_out);
     ctx->launches++;
     return cudaGetLastError();
 }
@@ -722,14 +731,14 @@ static cudaError_t launch_tier_groups(mxb_ctx *ctx, const BuildTables &tb, int64
                                       const int32_t *list_in, const int *n_in, int32_t *list_out,
                                       int *n_out, int *work_counter, const int64_t *row_ptr,
                                       const int32_t *pos_idx, const uint8_t *base_code, double *out,
-                                      int32_t *match_out) {
+                                      int32_t *match_out, int32_t *route_out) {
     if (tb.n_groups <= kGroupsSmall)
         return launch_tier<kCounts, Tier, kGroupsSmall>(ctx, tb, n_rows, list_in, n_in, list_out,
                                                         n_out, work_counter, row_ptr, pos_idx,
-                                                        base_code, out, match_out);
+                                                        base_code, out, match_out, route_out);
     return launch_tier<kCounts, Tier, kGroupsLarge>(ctx, tb, n_rows, list_in, n_in, list_out, n_out,
                                                     work_counter, row_ptr, pos_idx, base_code, out,
-                                                    match_out);
+                                                    match_out, route_out);
 }
 
 }  // namespace mxb
@@ -879,7 +888,7 @@ int mxb_phylo_destroy(mxb_phylo *ph) {
 int mxb_build_matrix(mxb_ctx *ctx, const mxb_phylo *ph, int64_t n_rows,
                      const int64_t *row_ptr, const int32_t *pos_idx,
                      const uint8_t *base_code, double *out_host, int32_t *match_host,
-                     mxb_matrix **out_dev, float *elapsed_ms) {
+                     int32_t *route_host, mxb_matrix **out_dev, float *elapsed_ms) {
     MXB_REQUIRE(ctx != nullptr && ph != nullptr, "NULL handle");
     MXB_REQUIRE(n_rows >= 0, "negative n_rows");
     MXB_REQUIRE(n_rows == 0 || row_ptr != nullptr, "row_ptr is NULL");
@@ -894,7 +903,7 @@ int mxb_build_matrix(mxb_ctx *ctx, const mxb_phylo *ph, int64_t n_rows,
     MXB_TRY(mxb_matrix_alloc(ctx, n_rows, ph->n_hap, &m));
     const size_t cells = (size_t)n_rows * (size_t)ph->n_hap;
     int64_t *d_row_ptr = nullptr;
-    int32_t *d_pos = nullptr, *d_match = nullptr, *d_overflow = nullptr;
+    int32_t *d_pos = nullptr, *d_match = nullptr, *d_overflow = nullptr, *d_route = nullptr;
     uint8_t *d_code = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     cudaError_t e = cudaSuccess;
@@ -934,6 +943,12 @@ int mxb_build_matrix(mxb_ctx *ctx, const mxb_phylo *ph, int64_t n_rows,
                 // of the two launches, [3..] = the deferred rows
                 STEP(cudaMalloc(&d_overflow, (n_rows + 3) * sizeof(int32_t)));
                 STEP(cudaMemsetAsync(d_overflow, 0, 3 * sizeof(int32_t), ctx->stream));
+                if (route_host) {   // rows tier 1 finishes without dense groups stay 0
+                    STEP(cudaMalloc(&d_route, n_rows * sizeof(int32_t)));
+                    STEP(cudaMemsetAsync(d_route, 0, n_rows * sizeof(int32_t), ctx->stream));
+                }
+            } else if (route_host) {
+                std::fill(route_host, route_host + n_rows, 3);
             }
             STEP(cudaEventRecord(ev0, ctx->stream));
             if (e == cudaSuccess && use_class) {
@@ -953,21 +968,23 @@ int mxb_build_matrix(mxb_ctx *ctx, const mxb_phylo *ph, int64_t n_rows,
                     e = counts ? launch_tier_groups<true, Tier1>(ctx, tb, n_rows, nullptr, nullptr,
                                                                  ov_list, ov_count, ov_count + 1,
                                                                  d_row_ptr, d_pos, d_code, m->data,
-                                                                 d_match)
+                                                                 d_match, d_route)
                                : launch_tier_groups<false, Tier1>(ctx, tb, n_rows, nullptr, nullptr,
                                                                   ov_list, ov_count, ov_count + 1,
                                                                   d_row_ptr, d_pos, d_code, m->data,
-                                                                  d_match);
+                                                                  d_match, d_route);
                 }
                 const int32_t *in2 = two_tiers ? ov_list : nullptr;
                 const int *n_in2 = two_tiers ? ov_count : nullptr;
                 if (e == cudaSuccess)
                     e = counts ? launch_tier_groups<true, Tier2>(ctx, tb, n_rows, in2, n_in2, nullptr,
                                                                  nullptr, ov_count + 2, d_row_ptr,
-                                                                 d_pos, d_code, m->data, d_match)
+                                                                 d_pos, d_code, m->data, d_match,
+                                                                 d_route)
                                : launch_tier_groups<false, Tier2>(ctx, tb, n_rows, in2, n_in2, nullptr,
                                                                   nullptr, ov_count + 2, d_row_ptr,
-                                                                  d_pos, d_code, m->data, d_match);
+                                                                  d_pos, d_code, m->data, d_match,
+                                                                  d_route);
                 ctx->launches--;  // counted once more below
             } else if (e == cudaSuccess) {
                 const int grid = (int)std::min<int64_t>(n_rows, (int64_t)ctx->num_sms * 4);
@@ -978,6 +995,9 @@ int mxb_build_matrix(mxb_ctx *ctx, const mxb_phylo *ph, int64_t n_rows,
             ctx->launches++;
             STEP(cudaGetLastError());
             STEP(cudaEventRecord(ev1, ctx->stream));
+            if (d_route)
+                STEP(cudaMemcpyAsync(route_host, d_route, n_rows * sizeof(int32_t),
+                                     cudaMemcpyDeviceToHost, ctx->stream));
         }
         // pageable results leave through the staged copy engine (api.cu)
         if (e == cudaSuccess && out_host) {
@@ -1005,6 +1025,7 @@ int mxb_build_matrix(mxb_ctx *ctx, const mxb_phylo *ph, int64_t n_rows,
     cudaFree(d_code);
     cudaFree(d_match);
     cudaFree(d_overflow);
+    cudaFree(d_route);
     if (rc != MXB_OK || !out_dev) mxb_matrix_destroy(m);
     else *out_dev = m;
     return rc;

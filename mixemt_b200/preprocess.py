@@ -253,9 +253,11 @@ def parse_signatures(reads, tables):
 
 
 def build_matrix_from_csr(tables, csr, ctx=None, want_host=True, want_counts=False,
-                          keep_device=False):
+                          keep_device=False, routes_out=None):
     """Run kernel 1 on packed inputs.  Returns ``(host_matrix|None,
-    match_counts|None, DeviceMatrix|None, kernel_ms)``."""
+    match_counts|None, DeviceMatrix|None, kernel_ms)``.  ``routes_out``: an int32
+    array of one entry per row, filled in place with the path that finished each row
+    (``mxb_build_matrix``'s ``route_host``)."""
     ctx = ctx or get_context()
     dev = tables.to_device(ctx)
     n, h = csr.n_rows, tables.n_hap
@@ -263,8 +265,10 @@ def build_matrix_from_csr(tables, csr, ctx=None, want_host=True, want_counts=Fal
     counts = np.empty((n, h), dtype=np.int32) if want_counts else None
     handle = ctypes.c_void_p()
     ms = ctypes.c_float(0.0)
+    if routes_out is not None and (routes_out.dtype != np.int32 or routes_out.shape != (n,)):
+        raise ValueError("routes_out must be an int32 array of %d entries" % n)
     check(lib.mxb_build_matrix(ctx.handle, dev.handle, n, ptr(csr.row_ptr), ptr(csr.pos_idx),
-                               ptr(csr.base_code), ptr(out), ptr(counts),
+                               ptr(csr.base_code), ptr(out), ptr(counts), ptr(routes_out),
                                ctypes.byref(handle) if keep_device else None,
                                ctypes.byref(ms)))
     dmat = DeviceMatrix(ctx, handle) if keep_device else None

@@ -30,8 +30,9 @@ def test_python_prototypes_cover_the_header():
     assert sorted(_lib.EXPORTED_SYMBOLS) == declared_symbols()
 
 
-def test_abi_version_and_error_string():
-    assert _lib.lib.mxb_abi_version() == 1
+def test_abi_version_2_and_error_string():
+    """Version 2: mxb_build_matrix takes route_host after match_host."""
+    assert _lib.lib.mxb_abi_version() == 2
     assert isinstance(_lib.last_error(), str)
 
 
