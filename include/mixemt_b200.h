@@ -214,8 +214,10 @@ int mxb_matrix_upload_rows(mxb_ctx *ctx, mxb_matrix *m, int64_t row0, int64_t n_
  * The session keeps L = exp(M - rowmax) either as class tiles (per 128-row batch the
  * bit-identical columns collapse into classes: exact, several times fewer bytes and FMAs;
  * needs rows in the reference's order, preprocess.py:219, to pay off) or, when the matrix does
- * not compress, as fp64 rows (see mxb_em_pass_bytes).  In a sharded session the call is
- * collective: every rank zeroes its peer mailboxes behind a barrier. */
+ * not compress, as fp64 rows (see mxb_em_pass_bytes).  What an iteration runs (the pass over
+ * tiles, fp64 rows or the general path, its restart slots and its tail) is decided once here
+ * (em.cu: decide_form).  In a sharded session the call is collective: every rank zeroes its
+ * peer mailboxes behind a barrier. */
 int mxb_em_create(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
                   int sharded, mxb_em **out);
 int mxb_em_destroy(mxb_em *em);
@@ -330,7 +332,8 @@ int mxb_em_bootstrap(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
 /* Replicate slots of a bootstrap session over class tiles with these batch class counts (as
  * mxb_tile_plan takes them): the largest power of two R <= 16 whose tile plan for num_sms / R
  * CTAs models at most R times the time of the plan for num_sms, with R * bytes_per_slot at
- * most an eighth of free_bytes.  Host only, for the CPU tests. */
+ * most an eighth of free_bytes (a session passes the bytes of one slot's buffers, em.cu:
+ * slot_block, plus its class vectors).  Host only, for the CPU tests. */
 int mxb_boot_slots(const int32_t *n_cls, int64_t n_batches, int64_t n_rows, int32_t num_sms,
                    double bytes_per_slot, double free_bytes, int32_t *slots_out);
 

@@ -303,7 +303,6 @@ struct BlockCache {
     size_t cached_bytes = 0;
     size_t limit = 0;
 };
-constexpr size_t kCacheMinBlock = (size_t)1 << 20;
 
 void *pinned_scratch(mxb_ctx *ctx) {
     if (!ctx->pinned && cudaHostAlloc(&ctx->pinned, kPinnedScratchBytes, cudaHostAllocDefault) != cudaSuccess) {

@@ -120,6 +120,7 @@ int copy_d2h(mxb_ctx *ctx, void *dst_host, const void *src_dev, size_t bytes);
 // matrix from any thread).
 constexpr size_t kPinnedScratchBytes = 4096;
 void *pinned_scratch(mxb_ctx *ctx);  // kPinnedScratchBytes of pinned host memory, NULL on failure
+constexpr size_t kCacheMinBlock = (size_t)1 << 20;   // smallest block the cache keeps
 cudaError_t dev_alloc(mxb_ctx *ctx, void **out, size_t bytes);
 void dev_free(mxb_ctx *ctx, void *ptr);
 void dev_cache_release(mxb_ctx *ctx);
@@ -143,5 +144,7 @@ extern double g_stage_ms[kNumStages];
 
 inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 inline int64_t round_up(int64_t a, int64_t b) { return ceil_div(a, b) * b; }
+// Byte size of one part of a device block whose parts each start 256-byte aligned.
+inline size_t align256(size_t bytes) { return (bytes + 255) & ~(size_t)255; }
 
 }  // namespace mxb

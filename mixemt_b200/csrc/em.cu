@@ -47,6 +47,15 @@
 
 using namespace mxb;
 
+namespace mxb {
+// What an iteration runs (decide_form): its pass over class tiles, over fp64 rows (streamed,
+// or streamed with two restarts per read of L) or the general path; its tail in one cluster
+// launch (em_finish_kernel), the same with the ranks' sums exchanged through peer memory, or
+// split (em_colreduce_kernel, NCCL all-reduce across ranks, em_update_kernel).
+enum class EmForm { kTiles, kRows, kRowPairs, kGeneral };
+enum class EmTail { kFused, kPeer, kSplit };
+}  // namespace mxb
+
 struct mxb_em {
     mxb_ctx *ctx = nullptr;
     const mxb_matrix *mat = nullptr;
@@ -64,21 +73,22 @@ struct mxb_em {
     EmState *host_state = nullptr;  // pinned, 2 slots
     cudaEvent_t poll_ev[2] = {nullptr, nullptr};
     int n_part = 0;
-    // fast path
-    bool fast = false;
+    // decide_form
+    EmForm form = EmForm::kGeneral;
+    EmTail tail = EmTail::kSplit;
+    // Restart slots: a batched session (run_em with n_multi > 1) iterates two restarts per read
+    // of L, a bootstrap session R replicates per iteration.  Slot s lives at lnp[b] + s*ld,
+    // pi[b] + s*ld, partials + s*n_part*ld, state + s (slot_block).
+    int n_slots = 1;
+    // streaming pass (n_stages > 0 when the rows fit its ring)
     int nc = 0;
     int n_stages = 0;
     size_t smem_bytes = 0;
     int grid_fast = 0;
     // general path
     int row_blocks = 0, col_blocks = 0;
-    bool fused_tail = false;  // colreduce + update in one cluster launch (em_finish_kernel)
-    // Restart slots: a batched session (run_em with n_multi > 1) iterates two restarts per
-    // read of L.  Slot s lives at lnp[b] + s*ld, pi[b] + s*ld, partials + s*n_part*ld, state + s.
-    int n_slots = 1;
-    // Class tiles (em_tiles.cuh): when `tiled` the pass reads `tile_v` instead of `lin`.
-    bool tiled = false;
-    int n_batches = 0, tile_hs = 0, tile_parts = 0, tile_grid = 0;
+    // Class tiles (em_tiles.cuh): form kTiles reads `tile_v` instead of `lin`.
+    int n_batches = 0, tile_hs = 0, tile_grid = 0;   // (the gather's blocks: n_part)
     unsigned char *tile_block = nullptr;   // [perm][cmap][cword][desc]
     unsigned char *tile_vecs = nullptr;    // [pi_cls][u_sum][ctas][segs][copies][gather entries]
     unsigned short *tile_perm = nullptr, *tile_cmap = nullptr;
@@ -94,23 +104,20 @@ struct mxb_em {
     double *tile_v = nullptr;
     int64_t tile_cells = 0;                // doubles in tile_v
     int64_t tile_bytes_per_pass = 0;
-    unsigned char *small = nullptr;  // one device block behind weights ... state (fewer driver calls)
+    unsigned char *small = nullptr;  // one device block behind weights ... props_in (fewer driver calls)
+    unsigned char *slots = nullptr;  // the slot block (slot_block)
     bool zero_iter = false;  // last iterate() ran no iteration
     // Bootstrap session (run_bootstrap): n_slots replicates per launch, each with its own weight
-    // vector slot_w + s * n_rows; over class tiles the slots' Pi and U vectors lie
-    // tile_pi_stride and tile_u_stride doubles apart.
+    // vector (slot_weights); over class tiles the slots' Pi and U vectors lie tile_pi_stride and
+    // tile_u_stride doubles apart.
     bool boot = false;
     double *slot_w = nullptr;
-    unsigned char *boot_block = nullptr;
     int64_t tile_pi_stride = 0, tile_u_stride = 0;
 };
 
 namespace mxb {
 
-typedef void (*pass_fn)(const unsigned char *, uint32_t, int64_t, int64_t, const double *,
-                        const double *, const double *, EmState *, double *, int);
-
-static pass_fn pick_pass(int nc) {
+static decltype(&em_pass_fast_kernel<1>) pick_pass(int nc) {
     switch (nc) {
         case 1: return em_pass_fast_kernel<1>;
         case 2: return em_pass_fast_kernel<2>;
@@ -123,10 +130,7 @@ static pass_fn pick_pass(int nc) {
     }
     return nullptr;
 }
-typedef void (*pair_fn)(const double *, int64_t, int64_t, const double *, const double *,
-                        const double *, const double *, const double *, EmState *, double *,
-                        double *, int);
-static pair_fn pick_pair(int nc) {
+static decltype(&em_pass_pair_kernel<1>) pick_pair(int nc) {
     switch (nc) {
         case 1: return em_pass_pair_kernel<1>;
         case 2: return em_pass_pair_kernel<2>;
@@ -164,117 +168,140 @@ static cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, siz
     return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 
-// One iteration of every replicate slot of a bootstrap session over class tiles: the four
-// launches of a tiled iteration with the slot in blockIdx.y (z for the gather), all slots on
-// one plan of num_sms / n_slots CTAs.  A slot whose control block says done costs nothing.
-static int enqueue_tiles_slotted(mxb_em *em, cudaEvent_t *marks) {
+// The weights slot `slot` iterates on: its resampled counts in a bootstrap session.
+static double *slot_weights(mxb_em *em, int slot) {
+    return em->boot ? em->slot_w + slot * em->n_rows : em->weights;
+}
+
+// The class-sum kernel of a tiled iteration for `per` = ceil(H / kTileThreads) columns a thread.
+template <bool kSlots>
+static auto pick_tile_pi(int64_t n_cols) {
+    const int per = (int)ceil_div(n_cols, kTileThreads);
+    return per <= 4 ? tile_pi_kernel<4, kSlots> : per <= 8 ? tile_pi_kernel<8, kSlots>
+           : per <= 12 ? tile_pi_kernel<12, kSlots> : tile_pi_kernel<16, kSlots>;
+}
+
+// The pass of a tiled iteration: class sums, pass and gather.  kSlots: the R replicate slots of
+// a bootstrap session side by side, the slot in blockIdx.y (z for the gather), all on one plan
+// of num_sms / R CTAs; a slot whose control block says done costs nothing.
+template <bool kSlots>
+static int enqueue_tile_pass(mxb_em *em, unsigned R, cudaEvent_t *marks) {
     mxb_ctx *ctx = em->ctx;
     cudaStream_t s = ctx->stream;
-    const unsigned R = (unsigned)em->n_slots;
-    const int per = (int)ceil_div(em->n_cols, kTileThreads);
-    auto pi_fn = per <= 4 ? tile_pi_kernel<4, true> : per <= 8 ? tile_pi_kernel<8, true>
-                 : per <= 12 ? tile_pi_kernel<12, true> : tile_pi_kernel<16, true>;
-    MXB_CUDA(launch_pdl(pi_fn, dim3(std::min(em->n_batches, std::max(1, 2 * ctx->num_sms / (int)R)), R),
+    const int64_t pi_stride = kSlots ? em->tile_pi_stride : 0;
+    const int64_t u_stride = kSlots ? em->tile_u_stride : 0;
+    MXB_CUDA(launch_pdl(pick_tile_pi<kSlots>(em->n_cols),
+                        dim3(std::min(em->n_batches, std::max(1, 2 * ctx->num_sms / (int)R)), R),
                         dim3(kTileThreads), (size_t)em->ld * sizeof(double), s,
                         (const unsigned short *)em->tile_perm, (const unsigned int *)em->tile_cword,
                         em->tile_hs, (int)em->n_cols, (const TileDesc *)em->tile_desc,
                         em->n_batches, (const double *)em->pi[0], (const double *)em->pi[1],
-                        (const EmState *)em->state, em->tile_pi, em->ld, em->tile_pi_stride));
+                        (const EmState *)em->state, em->tile_pi, kSlots ? em->ld : (int64_t)0,
+                        pi_stride));
     if (marks) MXB_CUDA(cudaEventRecord(marks[0], s));
-    MXB_CUDA(launch_pdl(tile_pass_kernel<true>, dim3(em->tile_grid, R), dim3(kTilePassThreads),
-                        kTilePassSlotSmem, s, (const TileCta *)em->tile_ctas,
+    MXB_CUDA(launch_pdl(tile_pass_kernel<kSlots>, dim3(em->tile_grid, R), dim3(kTilePassThreads),
+                        kSlots ? kTilePassSlotSmem : kTilePassSmem, s, (const TileCta *)em->tile_ctas,
                         (const TileSeg *)em->tile_segs, (const double *)em->tile_v,
                         (const double *)em->tile_pi, em->state, em->tile_usum,
-                        em->tile_slot_bytes, em->tile_n_slots, (const double *)em->slot_w,
-                        em->n_rows, em->tile_pi_stride, em->tile_u_stride));
+                        em->tile_slot_bytes, em->tile_n_slots,
+                        (const double *)(kSlots ? slot_weights(em, 0) : nullptr),
+                        kSlots ? em->n_rows : (int64_t)0, pi_stride, u_stride));
     if (marks) MXB_CUDA(cudaEventRecord(marks[1], s));
-    g_plain_launch = true;   // as in the single-slot iteration (enqueue_iteration)
-    MXB_CUDA(launch_pdl(tile_gather_kernel<true>,
-                        dim3((unsigned)ceil_div(em->ld, kGatherThreads), em->tile_parts, R),
+    // The gather waits in plain stream order: launched early it would sit on the SMs the
+    // first CTAs of the pass leave and keep them from nothing, but measured it costs 27 us
+    // per iteration (B200, config 2), while the other three launches gain from the overlap.
+    g_plain_launch = true;
+    MXB_CUDA(launch_pdl(tile_gather_kernel<kSlots>,
+                        dim3((unsigned)ceil_div(em->ld, kGatherThreads), em->n_part, R),
                         dim3(kGatherThreads), 0, s, (const unsigned short *)em->tile_cmap,
                         em->tile_hs, (int)em->n_cols, em->ld, (const int *)em->tile_ent_batch,
                         (const int64_t *)em->tile_ent_off, em->tile_n_ent,
                         (const double *)em->tile_usum, (const EmState *)em->state, em->partials,
-                        em->tile_u_stride));
+                        u_stride));
     if (marks) MXB_CUDA(cudaEventRecord(marks[2], s));
-    P2PArgs pa;
-    memset(&pa, 0, sizeof(pa));
-    MXB_CUDA(launch_pdl(em_finish_kernel<false>, dim3(kFinCtas, R), dim3(kFinThreads), 0, s,
-                        em->partials, em->n_part, em->n_cols, em->ld, em->lnp[0], em->lnp[1],
-                        em->pi[0], em->pi[1], em->state, pa));
-    ctx->launches += 4;
+    ctx->launches += 3;
     return MXB_OK;
 }
 
-// One EM iteration on em->ctx->stream (no host sync).
-// `marks` (optional, 3 events) are recorded after the class sums, after the pass and after the
-// gather of a tiled iteration (after the pass only for fp64 rows): per-kernel attribution.
+// Shared memory of the pass and of the class sums, set once per session.
+template <bool kSlots>
+static cudaError_t tile_pass_attrs(int64_t n_cols) {
+    cudaError_t e = cudaFuncSetAttribute((const void *)tile_pass_kernel<kSlots>,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)(kSlots ? kTilePassSlotSmem : kTilePassSmem));
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute((const void *)pick_tile_pi<kSlots>(n_cols),
+                                cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)(kTileMaxCols * sizeof(double)));
+}
+
+// Blocks of the gather over n_ent U vectors: the partial column sums the tail adds (n_part).
+static int tile_gather_parts(int n_ent) { return std::max(1, std::min(32, n_ent / 8)); }
+
+// The tail of an iteration of R slots (em->tail): column sums, M-step, control block.
+static int enqueue_tail(mxb_em *em, unsigned R) {
+    mxb_ctx *ctx = em->ctx;
+    cudaStream_t s = ctx->stream;
+    if (em->tail == EmTail::kSplit) {
+        em_colreduce_kernel<<<(int)ceil_div(em->ld + 1, 256), 256, 0, s>>>(
+            em->partials, em->n_part, em->ld, em->state, em->tsum);
+        ctx->launches += 1;
+        // the column sums and the underflow flag behind them (tsum[ld])
+        if (em->sharded && ctx->world > 1) MXB_TRY(nccl_allreduce_sum_f64(ctx, em->tsum, em->ld + 1));
+        em_update_kernel<<<1, kUpdThreads, 0, s>>>(em->tsum, em->n_cols, em->ld, em->lnp[0],
+                                                   em->lnp[1], em->pi[0], em->pi[1], em->state);
+        ctx->launches += 1;
+        MXB_CUDA(cudaGetLastError());
+        return MXB_OK;
+    }
+    P2PArgs pa;
+    memset(&pa, 0, sizeof(pa));
+    if (em->tail == EmTail::kPeer) {
+        pa.world = ctx->world;
+        pa.rank = ctx->rank;
+        for (int r = 0; r < ctx->world; ++r) pa.block[r] = ctx->p2p_block[r];
+    }
+    MXB_CUDA(launch_pdl(em->tail == EmTail::kPeer ? em_finish_kernel<true> : em_finish_kernel<false>,
+                        dim3(kFinCtas, R), dim3(kFinThreads), 0, s, em->partials, em->n_part,
+                        em->n_cols, em->ld, em->lnp[0], em->lnp[1], em->pi[0], em->pi[1],
+                        em->state, pa));
+    ctx->launches += 1;
+    return MXB_OK;
+}
+
+// One EM iteration on em->ctx->stream (no host sync): the pass of the session's form, then its
+// tail.  `marks` (optional, 3 events) are recorded after the class sums, after the pass and
+// after the gather of a tiled iteration (after the pass only for fp64 rows): per-kernel
+// attribution.
 static int enqueue_iteration(mxb_em *em, cudaEvent_t pass_begin = nullptr,
                              cudaEvent_t pass_end = nullptr, cudaEvent_t *marks = nullptr) {
     mxb_ctx *ctx = em->ctx;
     cudaStream_t s = ctx->stream;
-    if (pass_begin) MXB_CUDA(cudaEventRecord(pass_begin, s));
-    if (em->tiled && em->boot) return enqueue_tiles_slotted(em, marks);
+    const unsigned R = (unsigned)em->n_slots;
     // fp64 rows of a bootstrap session: one replicate at a time, with the slot's weights
-    const double *weights = em->slot_w ? em->slot_w : em->weights;
-    if (em->n_slots == 2) {
-        const size_t ps = (size_t)em->n_part * em->ld;
-        {
-            MXB_CUDA(launch_pdl(pick_pair(em->nc), dim3(em->grid_fast), dim3(kPassThreads),
-                                em->smem_bytes, s, em->lin, em->ld, em->n_rows, em->weights,
-                                em->pi[0], em->pi[1], em->pi[0] + em->ld, em->pi[1] + em->ld,
-                                em->state, em->partials, em->partials + ps, em->n_stages));
-            ctx->launches += 1;
-        }
-        if (pass_end) MXB_CUDA(cudaEventRecord(pass_end, s));
-        P2PArgs pa;
-        memset(&pa, 0, sizeof(pa));
-        MXB_CUDA(launch_pdl(em_finish_kernel<false>, dim3(kFinCtas, 2), dim3(kFinThreads), 0, s,
-                            em->partials, em->n_part, em->n_cols, em->ld, em->lnp[0], em->lnp[1],
-                            em->pi[0], em->pi[1], em->state, pa));
+    const double *weights = slot_weights(em, 0);
+    if (pass_begin) MXB_CUDA(cudaEventRecord(pass_begin, s));
+    switch (em->form) {
+    case EmForm::kTiles:
+        MXB_TRY(em->boot ? enqueue_tile_pass<true>(em, R, marks)
+                         : enqueue_tile_pass<false>(em, R, marks));
+        break;
+    case EmForm::kRowPairs:
+        MXB_CUDA(launch_pdl(pick_pair(em->nc), dim3(em->grid_fast), dim3(kPassThreads),
+                            em->smem_bytes, s, em->lin, em->ld, em->n_rows, em->weights,
+                            em->pi[0], em->pi[1], em->pi[0] + em->ld, em->pi[1] + em->ld,
+                            em->state, em->partials,
+                            em->partials + (size_t)em->n_part * em->ld, em->n_stages));
         ctx->launches += 1;
-        return MXB_OK;
-    }
-    if (em->tiled) {
-        {
-            const int per = (int)ceil_div(em->n_cols, kTileThreads);
-            auto pi_fn = per <= 4 ? tile_pi_kernel<4> : per <= 8 ? tile_pi_kernel<8>
-                         : per <= 12 ? tile_pi_kernel<12> : tile_pi_kernel<16>;
-            MXB_CUDA(launch_pdl(pi_fn, dim3(std::min(em->n_batches, 2 * ctx->num_sms)),
-                                dim3(kTileThreads), (size_t)em->ld * sizeof(double), s,
-                                (const unsigned short *)em->tile_perm,
-                                (const unsigned int *)em->tile_cword, em->tile_hs,
-                                (int)em->n_cols, (const TileDesc *)em->tile_desc, em->n_batches,
-                                    (const double *)em->pi[0], (const double *)em->pi[1],
-                                (const EmState *)em->state, em->tile_pi, (int64_t)0, (int64_t)0));
-        }
-        if (marks) MXB_CUDA(cudaEventRecord(marks[0], s));
-        MXB_CUDA(launch_pdl(tile_pass_kernel<false>, dim3(em->tile_grid), dim3(kTilePassThreads),
-                            kTilePassSmem, s, (const TileCta *)em->tile_ctas,
-                            (const TileSeg *)em->tile_segs, (const double *)em->tile_v, (const double *)em->tile_pi, em->state,
-                            em->tile_usum, em->tile_slot_bytes, em->tile_n_slots,
-                            (const double *)nullptr, (int64_t)0, (int64_t)0, (int64_t)0));
-        if (marks) MXB_CUDA(cudaEventRecord(marks[1], s));
-        // The gather waits in plain stream order: launched early it would sit on the SMs the
-        // first CTAs of the pass leave and keep them from nothing, but measured it costs 27 us
-        // per iteration (B200, config 2), while the other three launches gain from the overlap.
-        g_plain_launch = true;
-        MXB_CUDA(launch_pdl(tile_gather_kernel<false>,
-                            dim3((unsigned)ceil_div(em->ld, kGatherThreads), em->tile_parts),
-                            dim3(kGatherThreads), 0, s, (const unsigned short *)em->tile_cmap,
-                            em->tile_hs, (int)em->n_cols, em->ld, (const int *)em->tile_ent_batch,
-                            (const int64_t *)em->tile_ent_off, em->tile_n_ent,
-                            (const double *)em->tile_usum, (const EmState *)em->state, em->partials,
-                            (int64_t)0));
-        if (marks) MXB_CUDA(cudaEventRecord(marks[2], s));
-        ctx->launches += 3;
-    } else if (em->fast) {
+        break;
+    case EmForm::kRows:
         MXB_CUDA(launch_pdl(pick_pass(em->nc), dim3(em->grid_fast), dim3(kPassThreads),
                             em->smem_bytes, s, (const unsigned char *)em->lin,
                             (uint32_t)(em->ld * sizeof(double)), em->ld, em->n_rows, weights,
                             em->pi[0], em->pi[1], em->state, em->partials, em->n_stages));
         ctx->launches += 1;
-    } else {
+        break;
+    case EmForm::kGeneral: {
         const int rd_blocks = (int)std::max<int64_t>(
             1, std::min<int64_t>(ceil_div(em->n_rows, 8), (int64_t)ctx->num_sms * 8));
         em_rowdot_kernel<<<rd_blocks, 256, 0, s>>>(em->lin, em->ld, em->n_rows, weights,
@@ -283,39 +310,13 @@ static int enqueue_iteration(mxb_em *em, cudaEvent_t pass_begin = nullptr,
         em_colacc_kernel<<<grid, 256, 0, s>>>(em->lin, em->ld, em->n_rows, em->coef, em->state,
                                               em->partials);
         ctx->launches += 2;
+        break;
+    }
     }
     if (pass_end) MXB_CUDA(cudaEventRecord(pass_end, s));
-    if (marks && !em->tiled) {
+    if (marks && em->form != EmForm::kTiles)
         for (int i = 0; i < 3; ++i) MXB_CUDA(cudaEventRecord(marks[i], s));
-    }
-    if (em->fused_tail) {
-        P2PArgs pa;
-        memset(&pa, 0, sizeof(pa));
-        if (em->sharded && ctx->world > 1) {
-            pa.world = ctx->world;
-            pa.rank = ctx->rank;
-            for (int r = 0; r < ctx->world; ++r) pa.block[r] = ctx->p2p_block[r];
-            MXB_CUDA(launch_pdl(em_finish_kernel<true>, dim3(kFinCtas), dim3(kFinThreads), 0, s,
-                                em->partials, em->n_part, em->n_cols, em->ld, em->lnp[0],
-                                em->lnp[1], em->pi[0], em->pi[1], em->state, pa));
-        } else {
-            MXB_CUDA(launch_pdl(em_finish_kernel<false>, dim3(kFinCtas), dim3(kFinThreads), 0, s,
-                                em->partials, em->n_part, em->n_cols, em->ld, em->lnp[0],
-                                em->lnp[1], em->pi[0], em->pi[1], em->state, pa));
-        }
-        ctx->launches += 1;
-        return MXB_OK;
-    }
-    em_colreduce_kernel<<<(int)ceil_div(em->ld + 1, 256), 256, 0, s>>>(em->partials, em->n_part,
-                                                                      em->ld, em->state, em->tsum);
-    ctx->launches += 1;
-    // the column sums and the underflow flag behind them (tsum[ld])
-    if (em->sharded && ctx->world > 1) MXB_TRY(nccl_allreduce_sum_f64(ctx, em->tsum, em->ld + 1));
-    em_update_kernel<<<1, kUpdThreads, 0, s>>>(em->tsum, em->n_cols, em->ld, em->lnp[0],
-                                               em->lnp[1], em->pi[0], em->pi[1], em->state);
-    ctx->launches += 1;
-    MXB_CUDA(cudaGetLastError());
-    return MXB_OK;
+    return enqueue_tail(em, R);
 }
 
 // Wall-clock stage times of the one-call entry points: collected into g_stage_ms when
@@ -366,7 +367,7 @@ int mxb_em_destroy(mxb_em *em) {
     dev_free(em->ctx, em->tile_vecs);
     dev_free(em->ctx, em->tile_v);
     dev_free(em->ctx, em->small);
-    dev_free(em->ctx, em->boot_block);
+    dev_free(em->ctx, em->slots);
     for (int i = 0; i < 2; ++i)
         if (em->poll_ev[i]) cudaEventDestroy(em->poll_ev[i]);
     delete em;  // host_state points into the context's pinned scratch
@@ -387,11 +388,94 @@ __global__ void em_reset_state_kernel(EmState *st, long long max_iter, double to
     st->delta = 0.0;
 }
 
-// Class tiles of the session's matrix (em_tiles.cuh), built straight from M: no N x ld copy of
-// L is ever allocated when this succeeds.  Falls through (MXB_OK, em->tiled == false) when the
-// matrix does not compress to less than half of its fp64 rows, when memory is short, or when
-// a batch fails the exact class check; the caller then sets up the fp64 rows.
-// MXB_EM_NO_PACK=1 keeps the fp64 rows (cross-check).
+// The slot block of a session with R slots: [slot weights (bootstrap sessions) R x n_rows]
+// [lnp 2 x R x ld][pi 2 x R x ld][partials R x n_part x ld][control blocks R], each part
+// 256-byte aligned.  Returns its bytes, and with `base` points the session's slot buffers into
+// it; R = 1 gives the bytes of one slot.
+static size_t slot_block(mxb_em *em, int R, int n_part, unsigned char *base) {
+    const size_t ns = (size_t)R, row_bytes = (size_t)em->ld * sizeof(double);
+    const size_t b_w = em->boot ? align256(ns * em->n_rows * sizeof(double)) : 0;
+    const size_t b_vec = align256(ns * row_bytes);
+    const size_t b_part = align256(ns * n_part * row_bytes);
+    if (base) {
+        unsigned char *p = base;
+        if (em->boot) { em->slot_w = (double *)p; p += b_w; }
+        for (int i = 0; i < 2; ++i) { em->lnp[i] = (double *)p; p += b_vec; }
+        for (int i = 0; i < 2; ++i) { em->pi[i] = (double *)p; p += b_vec; }
+        em->partials = (double *)p; p += b_part;
+        em->state = (EmState *)p;
+    }
+    return b_w + 4 * b_vec + b_part + align256(ns * sizeof(EmState));
+}
+
+// Layout of the batches and ring of the pass for the class counts of n rows (tile_plan.h).
+struct TileShape {
+    std::vector<TileDesc> desc;
+    int64_t v_cells = 0, p_cells = 0;
+    uint32_t ring_bytes = 0;   // ring slots of the pass and their count (tile_ring)
+    int ring_slots = 0;
+    bool ring_ok = false;      // false: rows too long for the ring
+};
+static void tile_shape(const int32_t *n_cls, int nb, int64_t n, TileShape &t) {
+    int max_r_pad = 4;
+    tile_layout(n_cls, nb, n, t.desc, t.v_cells, t.p_cells, max_r_pad);
+    t.ring_ok = tile_ring(max_r_pad, t.ring_bytes, t.ring_slots);
+}
+// The same for class counts handed in from outside (mxb_tile_plan, mxb_boot_slots), checked
+// first; an error names the entry point `who`.
+static int tile_shape_checked(const char *who, const int32_t *n_cls, int64_t n_batches,
+                              int64_t n_rows, int32_t num_sms, TileShape &t) {
+    const char *bad = nullptr;
+    if (!(n_cls != nullptr && n_batches > 0 && n_rows > (n_batches - 1) * kTileRows &&
+          n_rows <= n_batches * kTileRows && num_sms > 0))
+        bad = "bad arguments";
+    for (int64_t b = 0; !bad && b < n_batches; ++b)
+        if (n_cls[b] < 1 || n_cls[b] > kTileMaxCols) bad = "class counts must be in 1..8192";
+    if (bad) {
+        set_error("%s: %s", who, bad);
+        return MXB_ERR_ARG;
+    }
+    tile_shape(n_cls, (int)n_batches, n_rows, t);
+    return MXB_OK;
+}
+
+// The session's form, slot count and tail (EmForm, EmTail, n_slots): decided here and nowhere
+// else.  `tiles`: the session iterates over class tiles (em_pack_tiles, once their class counts
+// are known; `plan` is their plan on all SMs).  A session whose tiles do not pay off is decided
+// again without them.
+static void decide_form(mxb_em *em, int want_slots, const TileShape *tiles = nullptr,
+                        const TilePlanOut *plan = nullptr) {
+    mxb_ctx *ctx = em->ctx;
+    const bool streams = em->n_stages > 0;
+    const bool across = em->sharded && ctx->world > 1;
+    const bool fused = streams && em->ld <= (int64_t)kFinCtas * kFinThreads &&
+                       (!across || ctx->p2p_ready) && getenv("MXB_EM_SPLIT_TAIL") == nullptr;
+    em->tail = !fused ? EmTail::kSplit : across ? EmTail::kPeer : EmTail::kFused;
+    em->n_slots = 1;
+    if (tiles) {
+        em->form = EmForm::kTiles;   // restarts run one at a time over the tiles
+        if (!em->boot) return;
+        // the slotted tile kernels exist for the fused tail only
+        em->tail = EmTail::kFused;
+        if (!fused) return;
+        const int parts = tile_gather_parts((int)plan->ent_batch.size());
+        const size_t vecs = align256((size_t)tiles->p_cells * sizeof(double)) +
+                            align256((size_t)(tiles->p_cells + plan->extra_cells) * sizeof(double));
+        size_t free_b = 0, total_b = 0;
+        if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { cudaGetLastError(); free_b = 0; }
+        em->n_slots = boot_slots(tiles->desc, em->n_rows, ctx->num_sms, tiles->ring_bytes,
+                                 tiles->p_cells, (double)(slot_block(em, 1, parts, nullptr) + vecs),
+                                 (double)free_b);
+    } else if (!streams) {
+        em->form = EmForm::kGeneral;
+    } else if (want_slots == 2 && fused && em->nc <= kMaxPairNC && !em->sharded) {
+        em->form = EmForm::kRowPairs;
+        em->n_slots = 2;
+    } else {
+        em->form = EmForm::kRows;
+    }
+}
+
 template <int ITEMS>
 static cudaError_t launch_tile_class(mxb_ctx *ctx, int grid, const unsigned long long *hash, int hs,
                                      int n_cols, int n_batches, unsigned short *perm,
@@ -407,23 +491,34 @@ static cudaError_t launch_tile_class(mxb_ctx *ctx, int grid, const unsigned long
                                                                         perm, cword, cmap, rep, n_cls);
     return cudaGetLastError();
 }
+// The class kernel for `items` = ceil(H / kTileThreads) columns a thread.
+static auto pick_tile_class(int64_t n_cols) {
+    const int items = (int)ceil_div(n_cols, kTileThreads);
+    return items <= 4 ? launch_tile_class<4> : items <= 8 ? launch_tile_class<8>
+           : items <= 12 ? launch_tile_class<12> : launch_tile_class<16>;
+}
 
-static int em_pack_tiles(mxb_em *em) {
+// Class tiles of the session's matrix (em_tiles.cuh), built straight from M: no N x ld copy of
+// L is ever allocated when this succeeds (`built`).  The session's form is decided once the
+// class counts are known (decide_form).  Falls through (MXB_OK, built == false) when the matrix
+// does not compress to less than half of its fp64 rows, when memory is short, or when a batch
+// fails the exact class check; the caller then decides the form without tiles and sets up the
+// fp64 rows.  MXB_EM_NO_PACK=1 keeps the fp64 rows (cross-check).
+static int em_pack_tiles(mxb_em *em, int want_slots, bool &built) {
     mxb_ctx *ctx = em->ctx;
-    if (!em->fast || em->n_rows == 0 || em->n_cols > kTileMaxCols ||
+    built = false;
+    if (em->n_stages == 0 || em->n_rows == 0 || em->n_cols > kTileMaxCols ||
         getenv("MXB_EM_NO_PACK"))
         return MXB_OK;
     const int64_t n = em->n_rows, h = em->n_cols;
     const int nb = (int)ceil_div(n, kTileRows);
     const int hs = (int)round_up(h, 8);
-    auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
-    const size_t b_map = up((size_t)nb * hs * sizeof(unsigned short));
+    const size_t b_map = align256((size_t)nb * hs * sizeof(unsigned short));
     unsigned char *tmp = nullptr, *block = nullptr;
     double *v = nullptr;
     // scratch: [hash][rep][n_cls][bad]
-    const size_t b_hash = up((size_t)nb * hs * sizeof(unsigned long long));
-    const size_t b_int = up((size_t)nb * sizeof(int));
-    int rc = MXB_OK;
+    const size_t b_hash = align256((size_t)nb * hs * sizeof(unsigned long long));
+    const size_t b_int = align256((size_t)nb * sizeof(int));
     cudaError_t e = dev_alloc(ctx, (void **)&tmp, b_hash + b_map + 2 * b_int);
     const bool verbose = getenv("MXB_TIMING") != nullptr;
     auto give_up = [&](bool hard, const char *what) {
@@ -446,8 +541,8 @@ static int em_pack_tiles(mxb_em *em) {
     int *d_bad = reinterpret_cast<int *>(tmp + b_hash + b_map + b_int);
     // persistent: [perm][cmap][desc]; the class vectors and the plan of the pass follow in a
     // second block once the class counts are known
-    const size_t b_desc = up((size_t)nb * sizeof(TileDesc));
-    const size_t b_cword = up((size_t)nb * kTileThreads * sizeof(unsigned int));
+    const size_t b_desc = align256((size_t)nb * sizeof(TileDesc));
+    const size_t b_cword = align256((size_t)nb * kTileThreads * sizeof(unsigned int));
     const size_t head_bytes = 2 * b_map + b_cword + b_desc;
     unsigned char *maps = nullptr;
     e = dev_alloc(ctx, (void **)&maps, head_bytes);
@@ -462,13 +557,8 @@ static int em_pack_tiles(mxb_em *em) {
     tile_hash_kernel<<<std::min(nb, ctx->num_sms * 4), kTileThreads, 0, ctx->stream>>>(
         em->mat->data, n, h, nb, hash, hs);
     e = cudaGetLastError();
-    if (e == cudaSuccess) {
-        const int items = (int)ceil_div(h, kTileThreads);
-        if (items <= 4) e = launch_tile_class<4>(ctx, grid, hash, hs, (int)h, nb, perm, cword, cmap, rep, d_ncls);
-        else if (items <= 8) e = launch_tile_class<8>(ctx, grid, hash, hs, (int)h, nb, perm, cword, cmap, rep, d_ncls);
-        else if (items <= 12) e = launch_tile_class<12>(ctx, grid, hash, hs, (int)h, nb, perm, cword, cmap, rep, d_ncls);
-        else e = launch_tile_class<16>(ctx, grid, hash, hs, (int)h, nb, perm, cword, cmap, rep, d_ncls);
-    }
+    if (e == cudaSuccess)
+        e = pick_tile_class(h)(ctx, grid, hash, hs, (int)h, nb, perm, cword, cmap, rep, d_ncls);
     ctx->launches += 2;
     std::vector<int> ncls((size_t)nb);
     if (e == cudaSuccess)
@@ -478,29 +568,20 @@ static int em_pack_tiles(mxb_em *em) {
     if (e != cudaSuccess) return give_up(true, "classes");
 
     // layout of the batches, ring geometry and plan of the pass (tile_plan.h)
-    std::vector<TileDesc> desc;
-    int64_t v_cells = 0, p_cells = 0;
-    int max_r_pad = 4;
-    tile_layout(ncls.data(), nb, n, desc, v_cells, p_cells, max_r_pad);
-    uint32_t slot_bytes = 0;
-    int n_slots = 0;
-    if (!tile_ring(max_r_pad, slot_bytes, n_slots)) return give_up(false, "rows too long for the ring");
+    TileShape shape;
+    tile_shape(ncls.data(), nb, n, shape);
+    if (!shape.ring_ok) return give_up(false, "rows too long for the ring");
+    const std::vector<TileDesc> &desc = shape.desc;
+    const int64_t v_cells = shape.v_cells, p_cells = shape.p_cells;
+    const uint32_t slot_bytes = shape.ring_bytes;
+    const int n_slots = shape.ring_slots;
     TilePlanOut plan;
     tile_plan(desc, n, ctx->num_sms, slot_bytes, p_cells, plan);
-    int n_rep = 1;   // replicate slots of a bootstrap session (tile_plan.h: boot_slots)
-    if (em->boot && em->fused_tail) {
-        auto up8 = [](int64_t c) { return (double)(((size_t)c * 8 + 255) & ~(size_t)255); };
-        const int parts = std::max(1, std::min(32, (int)plan.ent_batch.size() / 8));
-        const double per_slot = up8(p_cells) + up8(p_cells + plan.extra_cells) +
-                                (double)parts * em->ld * 8 + (double)n * 8 + 4.0 * em->ld * 8 +
-                                sizeof(EmState);
-        size_t free_b = 0, total_b = 0;
-        if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { cudaGetLastError(); free_b = 0; }
-        n_rep = boot_slots(desc, n, ctx->num_sms, slot_bytes, p_cells, per_slot, (double)free_b);
-        if (n_rep > 1) {
-            plan = TilePlanOut();
-            tile_plan(desc, n, ctx->num_sms / n_rep, slot_bytes, p_cells, plan);
-        }
+    decide_form(em, want_slots, &shape, &plan);
+    const int n_rep = em->n_slots;   // replicate slots of a bootstrap session
+    if (n_rep > 1) {
+        plan = TilePlanOut();
+        tile_plan(desc, n, ctx->num_sms / n_rep, slot_bytes, p_cells, plan);
     }
     const std::vector<TileCta> &ctas = plan.ctas;
     const std::vector<TileSeg> &segs = plan.segs;
@@ -542,12 +623,12 @@ static int em_pack_tiles(mxb_em *em) {
 
     e = dev_alloc(ctx, (void **)&v, (size_t)v_cells * sizeof(double));
     unsigned char *vecs = nullptr;
-    const size_t b_pi = up((size_t)p_cells * sizeof(double));
-    const size_t b_u = up((size_t)u_cells * sizeof(double));
-    const size_t b_cta = up((size_t)n_cta * sizeof(TileCta));
-    const size_t b_seg = up((size_t)n_seg * sizeof(TileSeg));
-    const size_t b_entb = up((size_t)n_ent * sizeof(int));
-    const size_t b_ento = up((size_t)n_ent * sizeof(int64_t));
+    const size_t b_pi = align256((size_t)p_cells * sizeof(double));
+    const size_t b_u = align256((size_t)u_cells * sizeof(double));
+    const size_t b_cta = align256((size_t)n_cta * sizeof(TileCta));
+    const size_t b_seg = align256((size_t)n_seg * sizeof(TileSeg));
+    const size_t b_entb = align256((size_t)n_ent * sizeof(int));
+    const size_t b_ento = align256((size_t)n_ent * sizeof(int64_t));
     // [Pi x n_rep][U x n_rep][plan]
     const size_t b_vecs = (size_t)n_rep * (b_pi + b_u);
     if (e == cudaSuccess)
@@ -581,29 +662,14 @@ static int em_pack_tiles(mxb_em *em) {
     if (e == cudaSuccess)
         e = cudaMemcpyAsync(bad.data(), d_bad, (size_t)nb * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e == cudaSuccess)
-        e = em->boot ? cudaFuncSetAttribute((const void *)tile_pass_kernel<true>,
-                                            cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                            (int)kTilePassSlotSmem)
-                     : cudaFuncSetAttribute((const void *)tile_pass_kernel<false>,
-                                            cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                            (int)kTilePassSmem);
-    for (int v = 0; v < 4 && e == cudaSuccess; ++v) {
-        const void *fn = v == 0 ? (const void *)tile_pi_kernel<4> : v == 1 ? (const void *)tile_pi_kernel<8>
-                         : v == 2 ? (const void *)tile_pi_kernel<12> : (const void *)tile_pi_kernel<16>;
-        if (em->boot)
-            fn = v == 0 ? (const void *)tile_pi_kernel<4, true> : v == 1 ? (const void *)tile_pi_kernel<8, true>
-                 : v == 2 ? (const void *)tile_pi_kernel<12, true> : (const void *)tile_pi_kernel<16, true>;
-        e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)(kTileMaxCols * sizeof(double)));
-    }
+    if (e == cudaSuccess) e = em->boot ? tile_pass_attrs<true>(h) : tile_pass_attrs<false>(h);
     if (e != cudaSuccess) { dev_free(ctx, vecs); return give_up(true, "fill"); }
     bool any_bad = false;
     for (int b = 0; b < nb; ++b) any_bad |= bad[(size_t)b] != 0;
     if (any_bad) { dev_free(ctx, vecs); return give_up(false, "hash collision"); }
 
     dev_free(ctx, tmp);
-    em->tiled = true;
+    built = true;
     em->n_batches = nb;
     em->tile_hs = hs;
     em->tile_block = maps;
@@ -624,18 +690,14 @@ static int em_pack_tiles(mxb_em *em) {
     em->tile_v = v;
     em->tile_cells = v_cells;
     em->tile_grid = n_cta;
-    em->tile_parts = std::max(1, std::min(32, n_ent / 8));
-    em->n_part = em->tile_parts;
+    em->n_part = tile_gather_parts(n_ent);
     em->tile_pi_stride = (int64_t)(b_pi / sizeof(double));
     em->tile_u_stride = (int64_t)(b_u / sizeof(double));
-    if (em->boot) em->n_slots = n_rep;
     // what an iteration reads and writes: the tiles, perm + cmap (Pi), cmap (gather), the class
     // vectors (Pi written and read, U written and read)
     em->tile_bytes_per_pass = v_cells * 8 + 3 * (int64_t)nb * hs * 2 + 2 * (p_cells + u_cells) * 8;
-    return rc;
+    return MXB_OK;
 }
-
-static int em_alloc_boot_slots(mxb_em *em);
 
 static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weights, int sharded,
                           int want_slots, mxb_em **out, bool boot = false) {
@@ -663,32 +725,14 @@ static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weigh
     if (!force_general && em->ld >= 1024 && em->nc <= kMaxNC && ctx->smem_optin > fixed) {
         int stages = (int)std::min<size_t>(8, (ctx->smem_optin - fixed) / row_bytes);
         if (stages >= kPassGroup + 1) {
-            em->fast = true;
             em->n_stages = stages;
             em->smem_bytes = (size_t)stages * row_bytes + fixed;
             em->grid_fast = (int)std::max<int64_t>(1, std::min<int64_t>(ctx->num_sms, em->n_rows));
+            em->n_part = em->grid_fast;
         }
     }
-    em->fused_tail = em->fast && em->ld <= (int64_t)kFinCtas * kFinThreads &&
-                     (!(em->sharded && ctx->world > 1) || ctx->p2p_ready) &&
-                     getenv("MXB_EM_SPLIT_TAIL") == nullptr;
-    if (want_slots == 2 && em->fast && em->fused_tail && em->nc <= kMaxPairNC && !em->sharded)
-        em->n_slots = 2;
-    if (em->fast) {
-        em->n_part = em->grid_fast;
-        cudaError_t e = cudaFuncSetAttribute((const void *)pick_pass(em->nc),
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             (int)em->smem_bytes);
-        if (e == cudaSuccess && em->n_slots == 2)
-            e = cudaFuncSetAttribute((const void *)pick_pair(em->nc),
-                                     cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)em->smem_bytes);
-        if (e != cudaSuccess) {
-            set_error("cudaFuncSetAttribute(smem=%zu): %s", em->smem_bytes, cudaGetErrorString(e));
-            delete em;
-            return MXB_ERR_CUDA;
-        }
-    } else {
+    const bool streams = em->n_stages > 0;
+    if (!streams) {
         em->col_blocks = (int)ceil_div(em->ld / 2, 256);
         int64_t rb = std::max<int64_t>(1, (int64_t)ctx->num_sms * 4 / em->col_blocks);
         rb = std::min<int64_t>(rb, ceil_div(em->n_rows, 16));
@@ -698,59 +742,55 @@ static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weigh
 
     cudaError_t e = cudaSuccess;
 #define STEP(call) do { if (e == cudaSuccess) e = (call); } while (0)
-    const size_t ns = (size_t)em->n_slots;
-    {   // everything else of the session in one block: [weights][coef][lnp x2][pi x2][partials]
-        // [tsum + underflow flag][props_in][state], each 256-byte aligned
-        auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
-        const size_t b_rows = up((size_t)em->n_rows * sizeof(double));
-        const size_t b_vec = up(ns * row_bytes);
-        const size_t b_part = up(ns * (size_t)em->n_part * row_bytes);
-        const size_t total = b_rows * (em->fast ? 1 : 2) + 4 * b_vec + b_part +
-                             up(row_bytes + sizeof(double)) +
-                             up((size_t)em->n_cols * sizeof(double)) + up(ns * sizeof(EmState));
-        STEP(dev_alloc(ctx, (void **)&em->small, total));
+    // both blocks >= kCacheMinBlock: reused from the block cache, no cudaMalloc/cudaFree per session
+    {   // the session-wide buffers in one block, each 256-byte aligned: [weights][coef (general
+        // path)][tsum + underflow flag][props_in]
+        const size_t b_rows = align256((size_t)em->n_rows * sizeof(double));
+        const size_t b_tsum = align256(row_bytes + sizeof(double));
+        const size_t total = b_rows * (streams ? 1 : 2) + b_tsum +
+                             align256((size_t)em->n_cols * sizeof(double));
+        STEP(dev_alloc(ctx, (void **)&em->small, std::max(total, kCacheMinBlock)));
         if (e == cudaSuccess) {
             unsigned char *p = em->small;
             em->weights = (double *)p; p += b_rows;
-            if (!em->fast) { em->coef = (double *)p; p += b_rows; }
-            for (int i = 0; i < 2; ++i) { em->lnp[i] = (double *)p; p += b_vec; }
-            for (int i = 0; i < 2; ++i) { em->pi[i] = (double *)p; p += b_vec; }
-            em->partials = (double *)p; p += b_part;
-            em->tsum = (double *)p; p += up(row_bytes + sizeof(double));
-            em->props_in = (double *)p; p += up((size_t)em->n_cols * sizeof(double));
-            em->state = (EmState *)p;
+            if (!streams) { em->coef = (double *)p; p += b_rows; }
+            em->tsum = (double *)p; p += b_tsum;
+            em->props_in = (double *)p;
         }
     }
     for (int i = 0; i < 2; ++i)
         STEP(cudaEventCreateWithFlags(&em->poll_ev[i], cudaEventDisableTiming));
-    STEP(cudaMemsetAsync(em->state, 0, ns * sizeof(EmState), ctx->stream));
     if (e == cudaSuccess) {
         static_assert(2 * kMaxSlots * sizeof(EmState) <= kPinnedScratchBytes, "pinned scratch");
         em->host_state = (EmState *)pinned_scratch(ctx);
         if (!em->host_state) e = cudaErrorMemoryAllocation;
     }
-    if (em->n_rows > 0)
+    if (em->n_rows > 0)   // (tile_fill_kernel reads them)
         STEP(cudaMemcpyAsync(em->weights, weights, em->n_rows * sizeof(double),
                              cudaMemcpyHostToDevice, ctx->stream));
     STEP(cudaStreamSynchronize(ctx->stream));
+    bool tiled = false;
     if (e == cudaSuccess) {
         // class tiles straight from M; only a matrix that does not compress gets fp64 rows of L
-        const int rc = em_pack_tiles(em);
+        const int rc = em_pack_tiles(em, want_slots, tiled);
         if (rc != MXB_OK) {
             mxb_em_destroy(em);
             return rc;
         }
-        if (em->tiled && !em->boot) em->n_slots = 1;   // restarts run one at a time over the tiles
-        if (em->boot) {
-            const int brc = em_alloc_boot_slots(em);
-            if (brc != MXB_OK) {
-                mxb_em_destroy(em);
-                return brc;
-            }
-        }
     }
-    if (!em->tiled) STEP(dev_alloc(ctx, (void **)&em->lin, (size_t)em->n_rows * row_bytes));
-    if (e == cudaSuccess && em->n_rows > 0 && !em->tiled) {
+    if (!tiled) decide_form(em, want_slots);
+    if (streams) STEP(cudaFuncSetAttribute((const void *)pick_pass(em->nc),
+                                           cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           (int)em->smem_bytes));
+    if (em->form == EmForm::kRowPairs)
+        STEP(cudaFuncSetAttribute((const void *)pick_pair(em->nc),
+                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)em->smem_bytes));
+    STEP(dev_alloc(ctx, (void **)&em->slots,
+                   std::max(slot_block(em, em->n_slots, em->n_part, nullptr), kCacheMinBlock)));
+    if (e == cudaSuccess) slot_block(em, em->n_slots, em->n_part, em->slots);
+    STEP(cudaMemsetAsync(em->state, 0, em->n_slots * sizeof(EmState), ctx->stream));
+    if (!tiled) STEP(dev_alloc(ctx, (void **)&em->lin, (size_t)em->n_rows * row_bytes));
+    if (e == cudaSuccess && em->n_rows > 0 && !tiled) {
         const int grid = (int)std::min<int64_t>(em->n_rows, (int64_t)ctx->num_sms * 8);
         to_linear_kernel<<<grid, 256, 0, ctx->stream>>>(m->data, em->n_rows, em->n_cols, em->ld,
                                                         em->lin);
@@ -765,12 +805,13 @@ static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weigh
         mxb_em_destroy(em);
         return e == cudaErrorMemoryAllocation ? MXB_ERR_NOMEM : MXB_ERR_CUDA;
     }
-    int rc = MXB_OK;
     // a sharded session starts from zeroed peer mailboxes on every rank (collective)
-    if (rc == MXB_OK && em->sharded && ctx->world > 1 && em->fused_tail) rc = p2p_resync(ctx);
-    if (rc != MXB_OK) {
-        mxb_em_destroy(em);
-        return rc;
+    if (em->tail == EmTail::kPeer) {
+        const int rc = p2p_resync(ctx);
+        if (rc != MXB_OK) {
+            mxb_em_destroy(em);
+            return rc;
+        }
     }
     *out = em;
     return MXB_OK;
@@ -788,7 +829,7 @@ int mxb_em_create(mxb_ctx *ctx, const mxb_matrix *m, const double *weights, int 
 int mxb_em_pass_bytes(const mxb_em *em, int64_t *bytes_per_pass, int64_t *n_dense_rows) {
     MXB_REQUIRE(em != nullptr, "NULL argument");
     const int64_t row_bytes = em->ld * (int64_t)sizeof(double);
-    if (bytes_per_pass && em->tiled) {
+    if (bytes_per_pass && em->form == EmForm::kTiles) {
         *bytes_per_pass = em->tile_bytes_per_pass;
         if (n_dense_rows) *n_dense_rows = 0;
         return MXB_OK;
@@ -813,10 +854,10 @@ static int em_logspace_step(mxb_em *em, int cur, int slot, const double *weights
     const bool across = em->sharded && ctx->world > 1;
     const int64_t n_sums = across ? 2 * h : h;      // [s][m] or the plain column sums
     constexpr int kRowBlocks = 64;
-    auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
-    const size_t b_lse = up((size_t)n * sizeof(double)), b_col = up((size_t)h * sizeof(double));
-    const size_t b_sum = up((size_t)n_sums * sizeof(double));
-    const size_t b_part = up((size_t)kRowBlocks * n_sums * sizeof(double));
+    const size_t b_lse = align256((size_t)n * sizeof(double));
+    const size_t b_col = align256((size_t)h * sizeof(double));
+    const size_t b_sum = align256((size_t)n_sums * sizeof(double));
+    const size_t b_part = align256((size_t)kRowBlocks * n_sums * sizeof(double));
     unsigned char *tmp = nullptr;
     if (dev_alloc(ctx, (void **)&tmp, b_lse + b_col + b_sum + b_part) != cudaSuccess) {
         cudaGetLastError();
@@ -924,9 +965,7 @@ static int em_poll_loop(mxb_em *em, int64_t max_iter, int n_live, Finish finish)
             if (!live[sl] || poll_gen[w][sl] != gen[sl]) continue;
             EmState &st = em->host_state[w * kMaxSlots + sl];
             if (st.done == kDoneNeedsLogStep) {
-                // (the slot's own weights in a bootstrap session)
-                const double *w = em->slot_w ? em->slot_w + sl * em->n_rows : em->weights;
-                MXB_TRY(em_logspace_step(em, st.cur, sl, w));   // returns with the stream drained
+                MXB_TRY(em_logspace_step(em, st.cur, sl, slot_weights(em, sl)));   // returns with the stream drained
                 ++gen[sl];
                 MXB_CUDA(cudaMemcpyAsync(&st, em->state + sl, sizeof(EmState),
                                          cudaMemcpyDeviceToHost, s));
@@ -1089,22 +1128,14 @@ extern "C" int mxb_debug_tile_trace(unsigned long long *out, size_t n_words) {
 int mxb_tile_plan(const int32_t *n_cls, int64_t n_batches, int64_t n_rows, int32_t num_sms,
                   int32_t *seg_out, int64_t seg_cap, int32_t *n_cta, int32_t *n_seg,
                   int32_t *n_slots_out, int32_t *slot_bytes_out, int32_t *errors) {
-    MXB_REQUIRE(n_cls != nullptr && n_batches > 0 && n_rows > (n_batches - 1) * kTileRows &&
-                n_rows <= n_batches * kTileRows && num_sms > 0, "bad arguments");
-    for (int64_t b = 0; b < n_batches; ++b)
-        MXB_REQUIRE(n_cls[b] >= 1 && n_cls[b] <= kTileMaxCols, "class counts must be in 1..8192");
-    std::vector<TileDesc> desc;
-    int64_t v_cells = 0, p_cells = 0;
-    int max_r_pad = 4;
-    tile_layout(n_cls, (int)n_batches, n_rows, desc, v_cells, p_cells, max_r_pad);
-    uint32_t slot_bytes = 0;
-    int n_slots = 0;
-    const bool ring_ok = tile_ring(max_r_pad, slot_bytes, n_slots);
-    if (n_slots_out) *n_slots_out = n_slots;
-    if (slot_bytes_out) *slot_bytes_out = (int32_t)slot_bytes;
-    MXB_REQUIRE(ring_ok, "rows too long for the ring");
+    TileShape t;
+    MXB_TRY(tile_shape_checked(__func__, n_cls, n_batches, n_rows, num_sms, t));
+    const std::vector<TileDesc> &desc = t.desc;
+    if (n_slots_out) *n_slots_out = t.ring_slots;
+    if (slot_bytes_out) *slot_bytes_out = (int32_t)t.ring_bytes;
+    MXB_REQUIRE(t.ring_ok, "rows too long for the ring");
     TilePlanOut plan;
-    tile_plan(desc, n_rows, num_sms, slot_bytes, p_cells, plan);
+    tile_plan(desc, n_rows, num_sms, t.ring_bytes, t.p_cells, plan);
     if (n_cta) *n_cta = (int32_t)plan.ctas.size();
     if (n_seg) *n_seg = (int32_t)plan.segs.size();
     if (errors) *errors = tile_plan_check(desc, plan);
@@ -1154,7 +1185,7 @@ int mxb_em_profile(mxb_em *em, int64_t n_iter, float *ms_out) {
     }
     for (auto &e : evs) cudaEventDestroy(e);
     // fp64 rows: the three marks coincide after the pass, so [0] holds the pass
-    if (!em->tiled) { tot[1] = tot[0]; tot[0] = 0.0; }
+    if (em->form != EmForm::kTiles) { tot[1] = tot[0]; tot[0] = 0.0; }
     for (int k = 0; k < 4; ++k) ms_out[k] = (float)(tot[k] / (double)n_iter);
     return MXB_OK;
 }
@@ -1339,32 +1370,6 @@ static int run_restarts(mxb_em *em, const double *init_lnprops, int32_t n_multi,
     return rc;
 }
 
-// The slot buffers of a bootstrap session, sized for its n_slots when it is created:
-// [weights ns x n][lnp 2 x ns x ld][pi 2 x ns x ld][partials ns x n_part x ld][state ns].  They
-// take the place of the single-slot buffers of the session's `small` block.
-static int em_alloc_boot_slots(mxb_em *em) {
-    mxb_ctx *ctx = em->ctx;
-    const int64_t n = em->n_rows, ld = em->ld;
-    const size_t ns = (size_t)em->n_slots;
-    auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
-    const size_t b_w = up(ns * n * sizeof(double)), b_vec = up(ns * ld * sizeof(double));
-    const size_t b_part = up(ns * (size_t)em->n_part * ld * sizeof(double));
-    const size_t b_st = up(ns * sizeof(EmState));
-    const size_t total_b = b_w + 4 * b_vec + b_part + b_st;
-    if (dev_alloc(ctx, (void **)&em->boot_block, total_b) != cudaSuccess) {
-        cudaGetLastError();
-        set_error("bootstrap: device allocation of %zu bytes failed", total_b);
-        return MXB_ERR_NOMEM;
-    }
-    unsigned char *p = em->boot_block;
-    em->slot_w = (double *)p; p += b_w;
-    for (int i = 0; i < 2; ++i) { em->lnp[i] = (double *)p; p += b_vec; }
-    for (int i = 0; i < 2; ++i) { em->pi[i] = (double *)p; p += b_vec; }
-    em->partials = (double *)p; p += b_part;
-    em->state = (EmState *)p;
-    return MXB_OK;
-}
-
 // Replicates whose results are kept on the device at a time: the output is downloaded in
 // windows of this many rows (at most 177 MB at H = 5408), whatever n_boot is.
 constexpr int64_t kBootOutRows = 4096;
@@ -1374,7 +1379,7 @@ constexpr int64_t kBootOutRows = 4096;
 // from `start` and iterated by em_poll_loop as one restart of run_em on its counts; a finished
 // slot's final log-proportions go to row b - boot0 of the output and the slot takes the next
 // replicate of the window.  Over class tiles the slots iterate side by side
-// (enqueue_tiles_slotted), over fp64 rows one at a time.
+// (enqueue_tile_pass<true>), over fp64 rows one at a time.
 static int run_bootstrap(mxb_em *em, const double *start, const int64_t *d_cumw, uint64_t total,
                          uint64_t seed, int64_t boot0, int64_t n_boot, int64_t max_iter,
                          double tol, double *lnprops_out, int64_t *iters_out,
@@ -1385,8 +1390,8 @@ static int run_bootstrap(mxb_em *em, const double *start, const int64_t *d_cumw,
     const size_t ns = (size_t)em->n_slots;
     const int64_t win = std::min(n_boot, kBootOutRows);
     // [counts n][start h][results win x h]
-    auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
-    const size_t b_cnt = up((size_t)n * sizeof(uint32_t)), b_start = up((size_t)h * sizeof(double));
+    const size_t b_cnt = align256((size_t)n * sizeof(uint32_t));
+    const size_t b_start = align256((size_t)h * sizeof(double));
     const size_t b_out = (size_t)win * h * sizeof(double);
     unsigned char *work = nullptr;
     if (dev_alloc(ctx, (void **)&work, b_cnt + b_start + b_out) != cudaSuccess) {
@@ -1416,7 +1421,7 @@ static int run_bootstrap(mxb_em *em, const double *start, const int64_t *d_cumw,
     auto start_slot = [&](int sl) -> int {
         const int64_t k = next++;
         slot_rep[sl] = k;
-        double *w = em->slot_w + sl * n;
+        double *w = slot_weights(em, sl);
         MXB_TRY(boot_draw(ctx, d_cumw, n, total, seed, boot0 + k, 1, counts));
         MXB_TRY(boot_take_counts(ctx, counts, n, w));
         em_set_props_kernel<<<(int)ceil_div(ld, 256), 256, 0, s>>>(
@@ -1457,19 +1462,12 @@ extern "C" {
 
 int mxb_boot_slots(const int32_t *n_cls, int64_t n_batches, int64_t n_rows, int32_t num_sms,
                    double bytes_per_slot, double free_bytes, int32_t *slots_out) {
-    MXB_REQUIRE(n_cls != nullptr && slots_out != nullptr && n_batches > 0 &&
-                n_rows > (n_batches - 1) * kTileRows && n_rows <= n_batches * kTileRows &&
-                num_sms > 0, "bad arguments");
-    for (int64_t b = 0; b < n_batches; ++b)
-        MXB_REQUIRE(n_cls[b] >= 1 && n_cls[b] <= kTileMaxCols, "class counts must be in 1..8192");
-    std::vector<TileDesc> desc;
-    int64_t v_cells = 0, p_cells = 0;
-    int max_r_pad = 4;
-    tile_layout(n_cls, (int)n_batches, n_rows, desc, v_cells, p_cells, max_r_pad);
-    uint32_t slot_bytes = 0;
-    int n_slots = 0;
-    MXB_REQUIRE(tile_ring(max_r_pad, slot_bytes, n_slots), "rows too long for the ring");
-    *slots_out = boot_slots(desc, n_rows, num_sms, slot_bytes, p_cells, bytes_per_slot, free_bytes);
+    MXB_REQUIRE(slots_out != nullptr, "bad arguments");
+    TileShape t;
+    MXB_TRY(tile_shape_checked(__func__, n_cls, n_batches, n_rows, num_sms, t));
+    MXB_REQUIRE(t.ring_ok, "rows too long for the ring");
+    *slots_out = boot_slots(t.desc, n_rows, num_sms, t.ring_bytes, t.p_cells, bytes_per_slot,
+                            free_bytes);
     return MXB_OK;
 }
 

@@ -599,6 +599,29 @@ em_colreduce_kernel(const double *__restrict__ partials, int n_part, int64_t ld,
     tsum[j] = t;
 }
 
+// ln pi'_j of the M-step (em.py:89) from pi_j, its column sum t and the normaliser total.
+// When pi or pi * T underflows (a column far worse than the mixture in every row, whose
+// decay factor T / total is tiny) it stays in log space, else ln pi' would be -inf.
+// lnp_old is read only then.
+__device__ __forceinline__ double mstep_lnp(double p, double t, double total,
+                                            const double *lnp_old) {
+    if (p >= 1e-290 && p * t >= 1e-290) return log(p * t / total);
+    return *lnp_old + log(t / total);
+}
+
+// Advances the control block after an iteration (em.py:39-54): one more iteration, then
+// converged, max_iter reached, a peer that timed out, or the proportion buffers swapped.
+__device__ __forceinline__ void advance_state(EmState *st, double delta, int cur,
+                                              bool timeout = false) {
+    st->delta = delta;
+    const long long it = st->iters + 1;
+    st->iters = it;
+    if (timeout) st->done = 3;
+    else if (delta < st->tol) st->done = 1;
+    else if (it >= st->max_iter) st->done = 2;
+    else st->cur = 1 - cur;
+}
+
 // M-step normalisation + convergence test (em.py:89 and :39-54), one CTA.
 constexpr int kUpdThreads = 1024;
 __global__ void __launch_bounds__(kUpdThreads)
@@ -625,25 +648,14 @@ em_update_kernel(const double *__restrict__ tsum, int64_t n_cols, int64_t ld,
     double dl = 0.0;
     for (int64_t j = threadIdx.x; j < n_cols; j += kUpdThreads) {
         const double p = pi_old[j];
-        const double t = tsum[j];
-        double ln_new;
-        // pi or pi * T underflows: stay in log space (see em_finish_kernel)
-        if (p >= 1e-290 && p * t >= 1e-290) ln_new = log(p * t / total);
-        else ln_new = lnp_old[j] + log(t / total);
+        const double ln_new = mstep_lnp(p, tsum[j], total, lnp_old + j);
         const double p_new = exp(ln_new);
         lnp_new[j] = ln_new;
         pi_new[j] = p_new;
         dl += fabs(p_new - p);
     }
     const double delta = block_sum<kUpdThreads>(dl, scratch);
-    if (threadIdx.x == 0) {
-        st->delta = delta;
-        const long long it = st->iters + 1;
-        st->iters = it;
-        if (delta < st->tol) st->done = 1;
-        else if (it >= st->max_iter) st->done = 2;
-        else st->cur = 1 - cur;
-    }
+    if (threadIdx.x == 0) advance_state(st, delta, cur);
 }
 
 // ---- fused tail of an iteration (fast path) ------------------------------------
@@ -836,17 +848,13 @@ em_finish_kernel(const double *partials, int n_part, int64_t n_cols, int64_t ld,
     double dl = 0.0;
     if (owner) {
         double2 ln_new = make_double2(-INFINITY, -INFINITY), p_new = make_double2(0.0, 0.0);
-        // pi underflowed, or pi * T did (a column far worse than the mixture in every row, whose
-        // decay factor T / total is tiny): stay in log space, else ln pi' would be -inf
         if (live_x) {
-            if (p.x >= 1e-290 && p.x * t.x >= 1e-290) ln_new.x = log(p.x * t.x / total);
-            else ln_new.x = lnp_old[2 * c] + log(t.x / total);
+            ln_new.x = mstep_lnp(p.x, t.x, total, lnp_old + 2 * c);
             p_new.x = exp(ln_new.x);
             dl += fabs(p_new.x - p.x);
         }
         if (live_y) {
-            if (p.y >= 1e-290 && p.y * t.y >= 1e-290) ln_new.y = log(p.y * t.y / total);
-            else ln_new.y = lnp_old[2 * c + 1] + log(t.y / total);
+            ln_new.y = mstep_lnp(p.y, t.y, total, lnp_old + 2 * c + 1);
             p_new.y = exp(ln_new.y);
             dl += fabs(p_new.y - p.y);
         }
@@ -863,13 +871,7 @@ em_finish_kernel(const double *partials, int n_part, int64_t n_cols, int64_t ld,
             st->done = kDoneNeedsLogStep;    // the proportions written above are discarded
             return;
         }
-        st->delta = delta;
-        const long long it = st->iters + 1;
-        st->iters = it;
-        if (kP2P && s_timeout) st->done = 3;  // a peer never showed up
-        else if (delta < st->tol) st->done = 1;
-        else if (it >= st->max_iter) st->done = 2;
-        else st->cur = 1 - cur;
+        advance_state(st, delta, cur, kP2P && s_timeout);   // timeout: a peer never showed up
     }
 }
 
@@ -1068,13 +1070,9 @@ em_logspace_update_kernel(const double *__restrict__ colmax, const double *__res
     }
     const double delta = block_sum<kUpdThreads>(dl, scratch);
     if (threadIdx.x == 0) {
-        st->delta = delta;
         st->bad = 0;
-        const long long it = st->iters + 1;
-        st->iters = it;
-        if (delta < st->tol) st->done = 1;
-        else if (it >= st->max_iter) st->done = 2;
-        else { st->done = 0; st->cur = 1 - cur; }
+        st->done = 0;
+        advance_state(st, delta, cur);
     }
 }
 

@@ -9,9 +9,13 @@ flags and the kernel launches the call issued (ctx.launch_count).  Cases: the to
 matrices with 1 and 3 restarts; the 2500 x 5408 noise matrix with 2 and 5 restarts, two per pass
 and one at a time (MXB_EM_NO_BATCH=1); starts whose row likelihoods underflow (one restart on
 fp64 rows and on class tiles, the "UFU" restarts two per pass and one at a time); max_iter 0
-and 1; sessions driven by mxb_em_iterate (mxb_em_get_lnprops and mxb_em_read_mix read back);
-em_step on the toy and the noise matrix.  The second form compares two such directories:
-every array and count must be equal; launch counts are printed side by side.
+and 1; the split tail (MXB_EM_SPLIT_TAIL=1) and the general path (MXB_EM_FORCE_GENERAL=1);
+sessions driven by mxb_em_iterate (mxb_em_get_lnprops and mxb_em_read_mix read back), by
+mxb_em_iterate_fixed (20 iterations) and by mxb_em_profile (launch count only: its times are
+not compared); em_step on the toy and the noise matrix; bootstraps on the Build-17 tiles with
+fewer replicates than slots and with more (refilled slots), over fp64 rows, and from a start
+whose row likelihoods underflow.  The second form compares two such directories: every array
+and every launch count must be equal; launch counts are printed side by side.
 """
 import argparse
 import glob
@@ -102,6 +106,19 @@ def _cases():
     for mat, it, tol in (("toy", 1000, 1e-6), ("noise", 90, 3e-3), ("under_fp64", 60, 1e-6),
                          ("under_tiles", 60, 1e-6), ("b17", 0, 1e-4), ("b17", 1, 1e-4)):
         c.append(("%s_session_iter%d" % (mat, it), mat, 1, it, tol, {}, "session"))
+    split, general = {"MXB_EM_SPLIT_TAIL": "1"}, {"MXB_EM_FORCE_GENERAL": "1"}
+    for mat, it, tol in (("b17", 400, 1e-5), ("noise", 90, 3e-3)):
+        for tag, env in (("split", split), ("general", general)):
+            for k in (1, 3):
+                c.append(("%s_%s_n%d" % (mat, tag, k), mat, k, it, tol, env, "run"))
+            c.append(("%s_%s_session" % (mat, tag), mat, 1, it, tol, env, "session"))
+    for kind in ("fixed", "profile"):
+        c.append(("b17_%s20" % kind, "b17", 1, 20, 0.0, {}, kind))
+        c.append(("b17_rows_%s20" % kind, "b17", 1, 20, 0.0, {"MXB_EM_NO_PACK": "1"}, kind))
+    c.append(("b17_boot1", "b17", 1, 400, 1e-5, {}, "boot"))
+    c.append(("b17_boot40", "b17", 40, 400, 1e-5, {}, "boot"))
+    c.append(("b17_rows_boot5", "b17", 5, 400, 1e-5, {"MXB_EM_NO_PACK": "1"}, "boot"))
+    c.append(("under_tiles_boot3", "under_tiles", 3, 60, 1e-6, {}, "boot"))
     c.append(("toy_em_step", "toy", 1, 1, 0.0, {}, "step"))
     c.append(("noise_em_step", "noise", 1, 1, 0.0, {}, "step"))
     return c
@@ -135,6 +152,45 @@ def _session(ctx, m, w, init, max_iter, tol):
     return props, mix, [it.value], [cv.value], launches
 
 
+def _fixed(ctx, m, w, init, n_iter, profile):
+    """mxb_em_iterate_fixed (or mxb_em_profile) for n_iter iterations on a session, then both
+    log-proportions (mxb_em_get_lnprops 0 and 1, concatenated)."""
+    import ctypes
+    from mixemt_b200._lib import check, lib, ptr
+    from mixemt_b200.runtime import DeviceMatrix
+    h = m.shape[1]
+    dev = DeviceMatrix.from_host(ctx, m)
+    sess = ctypes.c_void_p()
+    check(lib.mxb_em_create(ctx.handle, dev.handle, ptr(w), 0, ctypes.byref(sess)))
+    l0 = ctx.launch_count
+    check(lib.mxb_em_set_lnprops(sess, ptr(np.ascontiguousarray(init))))
+    if profile:
+        check(lib.mxb_em_profile(sess, n_iter, (ctypes.c_float * 4)()))
+    else:
+        check(lib.mxb_em_iterate_fixed(sess, n_iter, ctypes.byref(ctypes.c_float()), None))
+    launches = ctx.launch_count - l0
+    props = np.empty(2 * h)
+    check(lib.mxb_em_get_lnprops(sess, 0, ptr(props[:h])))
+    check(lib.mxb_em_get_lnprops(sess, 1, ptr(props[h:])))
+    lib.mxb_em_destroy(sess)
+    dev.free()
+    return props, np.zeros(0), [n_iter], [0], launches
+
+
+def _boot(ctx, m, w, start, n_boot, max_iter, tol):
+    """mxb_em_bootstrap of replicates 0 .. n_boot - 1 from `start` on seed 7: their final
+    log-proportions, iterations and converged flags; the slot count goes with the read matrix."""
+    from mixemt_b200 import bootstrap
+    from mixemt_b200.runtime import DeviceMatrix
+    dev = DeviceMatrix.from_host(ctx, m)
+    l0 = ctx.launch_count
+    lnp, iters, conv, slots = bootstrap._run(dev, w, np.ascontiguousarray(start), 0, n_boot, 7,
+                                             _args(max_iter=max_iter, tolerance=tol))
+    launches = ctx.launch_count - l0
+    dev.free()
+    return lnp, np.array([slots]), iters, conv, launches
+
+
 def run(out_dir):
     from mixemt_b200 import em
     from mixemt_b200.runtime import DeviceMatrix, get_context
@@ -148,6 +204,11 @@ def run(out_dir):
         try:
             if kind == "session":
                 props, mix, iters, conv, launches = _session(ctx, m, w, inits[0], it, tol)
+            elif kind in ("fixed", "profile"):
+                props, mix, iters, conv, launches = _fixed(ctx, m, w, inits[0], it,
+                                                           kind == "profile")
+            elif kind == "boot":
+                props, mix, iters, conv, launches = _boot(ctx, m, w, inits[0], k, it, tol)
             elif kind == "step":
                 mix = np.empty_like(m)
                 l0 = ctx.launch_count
@@ -184,7 +245,8 @@ def compare(a, b):
             bad += 1
             continue
         x, y = np.load(pa), np.load(pb)
-        diff = [f for f in ("props", "mix", "iters", "conv") if not np.array_equal(x[f], y[f])]
+        diff = [f for f in ("props", "mix", "iters", "conv", "launches")
+                if not np.array_equal(x[f], y[f])]
         bad += bool(diff)
         print("%-28s %-10s launches %6d %6d (%+d)" % (name, "DIFF " + ",".join(diff) if diff
                                                       else "equal", int(x["launches"]),

@@ -61,7 +61,8 @@ def steps17(build17):
 
 @pytest.fixture
 def layout_env(request):
-    old = {v: os.environ.pop(v, None) for v in ("MXB_EM_NO_PACK", "MXB_EM_NO_BATCH")}
+    old = {v: os.environ.pop(v, None) for v in ("MXB_EM_NO_PACK", "MXB_EM_NO_BATCH",
+                                                "MXB_EM_SPLIT_TAIL", "MXB_EM_FORCE_GENERAL")}
     os.environ.update(request.param)
     yield request.param
     for v, val in old.items():
@@ -70,7 +71,8 @@ def layout_env(request):
             os.environ[v] = val
 
 
-LAYOUTS = [{}, {"MXB_EM_NO_PACK": "1"}, {"MXB_EM_NO_PACK": "1", "MXB_EM_NO_BATCH": "1"}]
+LAYOUTS = [{}, {"MXB_EM_NO_PACK": "1"}, {"MXB_EM_NO_PACK": "1", "MXB_EM_NO_BATCH": "1"},
+           {"MXB_EM_NO_PACK": "1", "MXB_EM_SPLIT_TAIL": "1"}, {"MXB_EM_FORCE_GENERAL": "1"}]
 
 
 def _raw_run(dev, wts, init, max_iter, tol):
@@ -90,10 +92,12 @@ def _raw_run(dev, wts, init, max_iter, tol):
     return props, mix, int(iters[0]), int(conv[0])
 
 
-@pytest.mark.parametrize("layout_env", LAYOUTS, indirect=True, ids=["tiles", "rows", "rows1"])
+@pytest.mark.parametrize("layout_env", LAYOUTS, indirect=True,
+                         ids=["tiles", "rows", "rows1", "rows_split", "general"])
 def test_restarts_equal_independent_runs(build17, layout_env):
     """Three restarts in one call (one slot over class tiles, two slots over fp64 rows, one slot
-    with MXB_EM_NO_BATCH=1) against three single-restart calls combined in numpy."""
+    with MXB_EM_NO_BATCH=1, one slot over fp64 rows with the split tail, the general path)
+    against three single-restart calls combined in numpy."""
     mat, wts, inits, dev = build17
     a = make_args(n_multi=3, max_iter=400, tolerance=1e-5)
     props, mix, info, _ = em.run_em_device(dev, wts, a, inits=inits)
