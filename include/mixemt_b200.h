@@ -63,6 +63,10 @@ int mxb_ctx_synchronize(mxb_ctx *ctx);
  * up to MXB_CACHE_MB (default: a quarter of the device memory; 0 disables) -- cudaMalloc
  * and cudaFree of multi-GB blocks are slow and jittery.  mxb_ctx_trim hands them back. */
 int mxb_ctx_trim(mxb_ctx *ctx);
+/* Bytes of device memory this context has handed out and not yet freed (live), and bytes it
+ * keeps cached for reuse.  MXB_DEBUG_FAIL_ALLOC=k, read by mxb_ctx_create, makes the k-th
+ * device allocation of the new context fail as out of memory (error-path tests). */
+int mxb_ctx_mem_stats(const mxb_ctx *ctx, int64_t *live_bytes, int64_t *cached_bytes);
 /* Pinned host memory for matrix-sized results (no counterpart in the reference, which returns
  * numpy arrays: em.py:111, preprocess.py:183).  An N x H result that lives in one of these
  * blocks is downloaded by one DMA without staging copy or page faults.  Blocks are pooled

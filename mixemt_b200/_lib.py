@@ -60,6 +60,7 @@ _PROTOS = {
     "mxb_ctx_set_stream": (ctypes.c_int, [P, P]),
     "mxb_ctx_synchronize": (ctypes.c_int, [P]),
     "mxb_ctx_trim": (ctypes.c_int, [P]),
+    "mxb_ctx_mem_stats": (ctypes.c_int, [P, ctypes.POINTER(c_i64), ctypes.POINTER(c_i64)]),
     "mxb_ctx_launch_count": (c_i64, [P]),
     "mxb_host_alloc": (ctypes.c_int, [ctypes.c_size_t, ctypes.c_int, c_void_pp]),
     "mxb_host_free": (ctypes.c_int, [P]),

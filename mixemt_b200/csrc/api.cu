@@ -11,8 +11,6 @@
 #include <chrono>
 #include <new>
 #include <thread>
-#include <mutex>
-#include <unordered_map>
 #include <utility>
 #include <vector>
 
@@ -294,16 +292,8 @@ int copy_d2h(mxb_ctx *ctx, void *dst_host, const void *src_dev, size_t bytes) {
 }
 
 // ---------------------------------------------------------------------------
-// Cache of large device blocks (see common.cuh).
+// Device memory: the context's block pool (see common.cuh) and its owners.
 // ---------------------------------------------------------------------------
-struct BlockCache {
-    std::mutex mu;   // dev_free may run on whichever Python thread triggers a GC (ctypes drops the GIL)
-    std::unordered_map<void *, size_t> live;           // blocks handed out by dev_alloc
-    std::vector<std::pair<size_t, void *>> free_list;  // cached blocks
-    size_t cached_bytes = 0;
-    size_t limit = 0;
-};
-
 void *pinned_scratch(mxb_ctx *ctx) {
     if (!ctx->pinned && cudaHostAlloc(&ctx->pinned, kPinnedScratchBytes, cudaHostAllocDefault) != cudaSuccess) {
         cudaGetLastError();
@@ -312,96 +302,67 @@ void *pinned_scratch(mxb_ctx *ctx) {
     return ctx->pinned;
 }
 
-static std::mutex g_cache_create_mu;
-static BlockCache *cache_of(mxb_ctx *ctx) {
-    std::lock_guard<std::mutex> create_lock(g_cache_create_mu);
-    if (!ctx->block_cache) {
-        BlockCache *bc = new (std::nothrow) BlockCache();
-        if (!bc) return nullptr;
-        const char *env = getenv("MXB_CACHE_MB");
-        if (env) {
-            bc->limit = (size_t)atoll(env) << 20;
-        } else {
-            size_t free_b = 0, total_b = 0;
-            if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) bc->limit = total_b / 4;
-            else cudaGetLastError();
-        }
-        ctx->block_cache = bc;
-    }
-    return (BlockCache *)ctx->block_cache;
-}
-
-void dev_cache_release(mxb_ctx *ctx) {
-    BlockCache *bc = (BlockCache *)ctx->block_cache;
-    if (!bc) return;
-    std::lock_guard<std::mutex> lock(bc->mu);
-    for (auto &ent : bc->free_list) cudaFree(ent.second);
-    bc->free_list.clear();
-    bc->cached_bytes = 0;
-}
-
-cudaError_t dev_alloc(mxb_ctx *ctx, void **out, size_t bytes) {
-    *out = nullptr;
-    if (bytes == 0) return cudaSuccess;
-    BlockCache *bc = bytes >= kCacheMinBlock ? cache_of(ctx) : nullptr;
-    if (bc) {
-        std::lock_guard<std::mutex> lock(bc->mu);
-        // smallest cached block that fits without wasting more than 1/8
-        int best = -1;
-        for (int i = 0; i < (int)bc->free_list.size(); ++i) {
-            const size_t sz = bc->free_list[i].first;
-            if (sz >= bytes && sz - bytes <= bytes / 8 &&
-                (best < 0 || sz < bc->free_list[best].first))
-                best = i;
-        }
-        if (best >= 0) {
-            *out = bc->free_list[best].second;
-            bc->cached_bytes -= bc->free_list[best].first;
-            bc->live[*out] = bc->free_list[best].first;
-            bc->free_list.erase(bc->free_list.begin() + best);
-            return cudaSuccess;
-        }
-    }
-    cudaError_t e = cudaMalloc(out, bytes);
-    if (e == cudaErrorMemoryAllocation && ctx->block_cache) {
+void *cuda_block_new(size_t bytes) {
+    void *p = nullptr;
+    if (cudaMalloc(&p, bytes) != cudaSuccess) {
         cudaGetLastError();
-        dev_cache_release(ctx);
-        e = cudaMalloc(out, bytes);
+        return nullptr;
     }
-    if (e == cudaSuccess && bc) {
-        std::lock_guard<std::mutex> lock(bc->mu);
-        try { bc->live[*out] = bytes; } catch (...) {}
+    return p;
+}
+
+void cuda_block_delete(void *ptr) { cudaFree(ptr); }
+
+void *dev_alloc(mxb_ctx *ctx, size_t bytes) {
+    if (bytes == 0) return nullptr;
+    if (++ctx->n_allocs == ctx->fail_alloc_at) return nullptr;   // MXB_DEBUG_FAIL_ALLOC
+    void *p = ctx->pool.take(bytes);
+    if (!p) {   // the cached blocks may be what is missing
+        ctx->pool.trim();
+        p = ctx->pool.take(bytes);
     }
-    return e;
+    return p;
 }
 
 void dev_free(mxb_ctx *ctx, void *ptr) {
     if (!ptr) return;
-    BlockCache *bc = ctx ? (BlockCache *)ctx->block_cache : nullptr;
-    if (bc) {
-        size_t sz = 0;
-        {
-            std::lock_guard<std::mutex> lock(bc->mu);
-            auto it = bc->live.find(ptr);
-            if (it != bc->live.end()) {
-                sz = it->second;
-                bc->live.erase(it);
-            }
-        }
-        if (sz != 0) {
-            // the block may still be read by work queued on the context's stream
-            cudaStreamSynchronize(ctx->stream);
-            std::lock_guard<std::mutex> lock(bc->mu);
-            if (bc->cached_bytes + sz <= bc->limit) {
-                try {
-                    bc->free_list.emplace_back(sz, ptr);
-                    bc->cached_bytes += sz;
-                    return;
-                } catch (...) {}
-            }
-        }
+    // a block that is cached may still be read by work queued on the context's stream
+    ctx->pool.give(ptr, [ctx]() { cudaStreamSynchronize(ctx->stream); });
+}
+
+int DevBlock::alloc(mxb_ctx *ctx, size_t bytes, const char *who) {
+    reset();
+    ctx_ = ctx;
+    p_ = dev_alloc(ctx, bytes);
+    if (bytes && !p_) {
+        set_error("%s: out of device memory for %zu bytes", who, bytes);
+        return MXB_ERR_NOMEM;
     }
-    cudaFree(ptr);
+    return MXB_OK;
+}
+
+void DevBlock::reset() {
+    if (p_) dev_free(ctx_, p_);
+    p_ = nullptr;
+}
+
+int Events::create(size_t n, unsigned flags, const char *who) {
+    try {
+        ev_.reserve(ev_.size() + n);
+    } catch (const std::bad_alloc &) {
+        set_error("%s: out of host memory", who);
+        return MXB_ERR_NOMEM;
+    }
+    for (size_t i = 0; i < n; ++i) {
+        cudaEvent_t e = nullptr;
+        const cudaError_t err = cudaEventCreateWithFlags(&e, flags);
+        if (err != cudaSuccess) {
+            set_error("%s: cudaEventCreate: %s", who, cudaGetErrorString(err));
+            return MXB_ERR_CUDA;
+        }
+        ev_.push_back(e);
+    }
+    return MXB_OK;
 }
 
 // ---------------------------------------------------------------------------
@@ -415,26 +376,25 @@ void dev_free(mxb_ctx *ctx, void *ptr) {
 bool g_stage_on = false;
 double g_stage_ms[kNumStages] = {};
 
-struct HostPool {
-    std::mutex mu;
-    std::unordered_map<void *, size_t> live;
-    std::vector<std::pair<size_t, void *>> free_list;
-    size_t cached_bytes = 0;
-};
-static HostPool g_host_pool;
-
 static size_t host_pool_limit() {
-    static size_t limit = 0;
-    if (limit == 0) {
-        const char *env = getenv("MXB_PINNED_CACHE_MB");
-        if (env) {
-            limit = ((size_t)atoll(env) << 20) + 1;
-        } else {
-            const long pages = sysconf(_SC_PHYS_PAGES), psz = sysconf(_SC_PAGE_SIZE);
-            limit = pages > 0 && psz > 0 ? (size_t)pages * (size_t)psz / 4 : ((size_t)16 << 30);
-        }
-    }
-    return limit;
+    const char *env = getenv("MXB_PINNED_CACHE_MB");
+    if (env) return ((size_t)atoll(env) << 20) + 1;
+    const long pages = sysconf(_SC_PHYS_PAGES), psz = sysconf(_SC_PAGE_SIZE);
+    return pages > 0 && psz > 0 ? (size_t)pages * (size_t)psz / 4 : ((size_t)16 << 30);
+}
+
+static BlockPool &host_pool() {
+    static BlockPool pool(
+        [](size_t bytes) -> void * {
+            void *p = nullptr;
+            if (cudaHostAlloc(&p, bytes, cudaHostAllocPortable) != cudaSuccess) {
+                cudaGetLastError();
+                return nullptr;
+            }
+            return p;
+        },
+        [](void *p) { cudaFreeHost(p); }, 4, 0, host_pool_limit());
+    return pool;
 }
 
 struct PrefaultImpl {
@@ -490,8 +450,7 @@ static void p2p_teardown(mxb_ctx *ctx) {
         else cudaIpcCloseMemHandle(ctx->p2p_block[r]);
         ctx->p2p_block[r] = nullptr;
     }
-    if (ctx->p2p_vote) cudaFree(ctx->p2p_vote);
-    ctx->p2p_vote = nullptr;
+    ctx->p2p_vote.reset();
     ctx->p2p_ready = false;
 }
 
@@ -509,10 +468,11 @@ static int p2p_setup(mxb_ctx *ctx) {
     memset(handles, 0, sizeof(handles));
     int ok = cudaIpcGetMemHandle(&handles[ctx->rank], mine) == cudaSuccess;
     if (!ok) cudaGetLastError();
-    unsigned char *dh = nullptr;
-    double *vote = nullptr;
-    MXB_CUDA(cudaMalloc(&dh, sizeof(handles)));
-    MXB_CUDA(cudaMalloc(&vote, sizeof(double)));
+    DevBlock dh_block, vote_block;
+    MXB_TRY(dh_block.alloc(ctx, sizeof(handles), "mxb_comm_init"));
+    MXB_TRY(vote_block.alloc(ctx, sizeof(double), "mxb_comm_init"));
+    unsigned char *dh = dh_block.get();
+    double *vote = vote_block.get<double>();
     MXB_CUDA(cudaMemcpyAsync(dh, handles, sizeof(handles), cudaMemcpyHostToDevice, s));
     MXB_NCCL(g_nccl.allgather(dh + (size_t)ctx->rank * sizeof(cudaIpcMemHandle_t), dh,
                               sizeof(cudaIpcMemHandle_t), 1 /* ncclUint8 */, ctx->nccl_comm, s));
@@ -535,13 +495,11 @@ static int p2p_setup(mxb_ctx *ctx) {
     MXB_TRY(nccl_allreduce_f64(ctx, vote, 1, 0));
     MXB_CUDA(cudaMemcpyAsync(&v, vote, sizeof(v), cudaMemcpyDeviceToHost, s));
     MXB_CUDA(cudaStreamSynchronize(s));
-    cudaFree(dh);
     if (v != 0.0) {
-        cudaFree(vote);
         p2p_teardown(ctx);
         return MXB_OK;  // NCCL all-reduce path stays in use
     }
-    ctx->p2p_vote = vote;
+    ctx->p2p_vote = std::move(vote_block);
     ctx->p2p_ready = true;
     return MXB_OK;
 }
@@ -554,10 +512,11 @@ int p2p_resync(mxb_ctx *ctx) {
     if (!ctx->p2p_ready || ctx->world <= 1) return MXB_OK;
     cudaStream_t s = ctx->stream;
     MXB_CUDA(cudaStreamSynchronize(s));                 // my own tail launches are done
-    MXB_CUDA(cudaMemsetAsync(ctx->p2p_vote, 0, sizeof(double), s));
-    MXB_TRY(nccl_allreduce_f64(ctx, ctx->p2p_vote, 1, 0));   // ... and so are everybody else's
+    double *vote = ctx->p2p_vote.get<double>();
+    MXB_CUDA(cudaMemsetAsync(vote, 0, sizeof(double), s));
+    MXB_TRY(nccl_allreduce_f64(ctx, vote, 1, 0));   // ... and so are everybody else's
     MXB_CUDA(cudaMemsetAsync(ctx->p2p_block[ctx->rank], 0, kP2PInboxOffset, s));
-    MXB_TRY(nccl_allreduce_f64(ctx, ctx->p2p_vote, 1, 0));   // nobody stores before all are zeroed
+    MXB_TRY(nccl_allreduce_f64(ctx, vote, 1, 0));   // nobody stores before all are zeroed
     MXB_CUDA(cudaStreamSynchronize(s));
     return MXB_OK;
 }
@@ -600,6 +559,16 @@ int mxb_ctx_create(int device, mxb_ctx **out) {
     ctx->smem_optin = prop.sharedMemPerBlockOptin;
     MXB_CUDA(cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
     ctx->own_stream = true;
+    const char *env = getenv("MXB_CACHE_MB");
+    if (env) {
+        ctx->pool.set_limit((size_t)atoll(env) << 20);
+    } else {
+        size_t free_b = 0, total_b = 0;
+        if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) ctx->pool.set_limit(total_b / 4);
+        else cudaGetLastError();
+    }
+    env = getenv("MXB_DEBUG_FAIL_ALLOC");
+    ctx->fail_alloc_at = env ? atoll(env) : 0;
     *out = ctx;
     return MXB_OK;
 }
@@ -611,9 +580,7 @@ int mxb_ctx_destroy(mxb_ctx *ctx) {
     free_stage(ctx);
     if (ctx->pinned) cudaFreeHost(ctx->pinned);
     ctx->pinned = nullptr;
-    dev_cache_release(ctx);
-    delete (BlockCache *)ctx->block_cache;
-    ctx->block_cache = nullptr;
+    ctx->pool.trim();
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
     delete ctx;
     return MXB_OK;
@@ -641,60 +608,29 @@ int mxb_ctx_trim(mxb_ctx *ctx) {
     MXB_REQUIRE(ctx != nullptr, "ctx is NULL");
     MXB_CUDA(cudaSetDevice(ctx->device));
     MXB_CUDA(cudaStreamSynchronize(ctx->stream));
-    dev_cache_release(ctx);
+    ctx->pool.trim();
+    return MXB_OK;
+}
+
+int mxb_ctx_mem_stats(const mxb_ctx *ctx, int64_t *live_bytes, int64_t *cached_bytes) {
+    MXB_REQUIRE(ctx != nullptr, "ctx is NULL");
+    size_t live = 0, cached = 0;
+    ctx->pool.stats(&live, &cached);
+    if (live_bytes) *live_bytes = (int64_t)live;
+    if (cached_bytes) *cached_bytes = (int64_t)cached;
     return MXB_OK;
 }
 
 int mxb_host_alloc(size_t bytes, int only_if_cached, void **out) {
     MXB_REQUIRE(out != nullptr && bytes > 0, "bad argument");
-    *out = nullptr;
-    {
-        std::lock_guard<std::mutex> lock(g_host_pool.mu);
-        int best = -1;
-        for (int i = 0; i < (int)g_host_pool.free_list.size(); ++i) {
-            const size_t sz = g_host_pool.free_list[i].first;
-            if (sz >= bytes && sz - bytes <= bytes / 4 &&
-                (best < 0 || sz < g_host_pool.free_list[best].first))
-                best = i;
-        }
-        if (best >= 0) {
-            *out = g_host_pool.free_list[best].second;
-            g_host_pool.cached_bytes -= g_host_pool.free_list[best].first;
-            g_host_pool.live[*out] = g_host_pool.free_list[best].first;
-            g_host_pool.free_list.erase(g_host_pool.free_list.begin() + best);
-            return MXB_OK;
-        }
-    }
-    if (only_if_cached) return MXB_OK;   // *out stays NULL: the caller uses pageable memory
-    void *p = nullptr;
-    if (cudaHostAlloc(&p, bytes, cudaHostAllocPortable) != cudaSuccess) {
-        cudaGetLastError();
-        return MXB_OK;                   // not an error: pageable memory still works
-    }
-    std::lock_guard<std::mutex> lock(g_host_pool.mu);
-    try { g_host_pool.live[p] = bytes; } catch (...) { cudaFreeHost(p); return MXB_OK; }
-    *out = p;
+    // NULL when nothing fits or pinning fails: not an error, the caller uses pageable memory
+    *out = host_pool().take(bytes, only_if_cached != 0);
     return MXB_OK;
 }
 
 int mxb_host_free(void *ptr) {
     if (!ptr) return MXB_OK;
-    size_t sz = 0;
-    {
-        std::lock_guard<std::mutex> lock(g_host_pool.mu);
-        auto it = g_host_pool.live.find(ptr);
-        MXB_REQUIRE(it != g_host_pool.live.end(), "not a block of mxb_host_alloc");
-        sz = it->second;
-        g_host_pool.live.erase(it);
-        if (g_host_pool.cached_bytes + sz <= host_pool_limit()) {
-            try {
-                g_host_pool.free_list.emplace_back(sz, ptr);
-                g_host_pool.cached_bytes += sz;
-                return MXB_OK;
-            } catch (...) {}
-        }
-    }
-    cudaFreeHost(ptr);
+    MXB_REQUIRE(host_pool().give(ptr), "not a block of mxb_host_alloc");
     return MXB_OK;
 }
 
@@ -728,10 +664,7 @@ int mxb_stage_times(double *ms_out, int n) {
 }
 
 int mxb_host_trim(void) {
-    std::lock_guard<std::mutex> lock(g_host_pool.mu);
-    for (auto &ent : g_host_pool.free_list) cudaFreeHost(ent.second);
-    g_host_pool.free_list.clear();
-    g_host_pool.cached_bytes = 0;
+    host_pool().trim();
     return MXB_OK;
 }
 
@@ -781,19 +714,14 @@ int mxb_comm_allreduce_host(mxb_ctx *ctx, double *buf, int64_t n, int op_is_max)
     MXB_REQUIRE(ctx != nullptr && (buf != nullptr || n == 0) && n >= 0, "bad argument");
     if (!ctx->nccl_comm || ctx->world <= 1 || n == 0) return MXB_OK;
     MXB_CUDA(cudaSetDevice(ctx->device));
-    double *d = nullptr;
-    MXB_CUDA(cudaMalloc(&d, n * sizeof(double)));
-    int rc = MXB_OK;
-    if (cudaMemcpyAsync(d, buf, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess)
-        rc = MXB_ERR_CUDA;
-    if (rc == MXB_OK) rc = nccl_allreduce_f64(ctx, d, n, op_is_max);
-    if (rc == MXB_OK &&
-        cudaMemcpyAsync(buf, d, n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream) != cudaSuccess)
-        rc = MXB_ERR_CUDA;
-    if (cudaStreamSynchronize(ctx->stream) != cudaSuccess && rc == MXB_OK) rc = MXB_ERR_CUDA;
-    cudaFree(d);
-    if (rc == MXB_ERR_CUDA && g_error[0] == 0) set_error("allreduce_host: CUDA failure");
-    return rc;
+    DevBlock d_block;
+    MXB_TRY(d_block.alloc(ctx, n * sizeof(double), "mxb_comm_allreduce_host"));
+    double *d = d_block.get<double>();
+    MXB_CUDA(cudaMemcpyAsync(d, buf, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    MXB_TRY(nccl_allreduce_f64(ctx, d, n, op_is_max));
+    MXB_CUDA(cudaMemcpyAsync(buf, d, n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    MXB_CUDA(cudaStreamSynchronize(ctx->stream));
+    return MXB_OK;
 }
 
 // ---- matrices ---------------------------------------------------------------
@@ -808,16 +736,13 @@ int mxb_matrix_alloc(mxb_ctx *ctx, int64_t n_rows, int64_t n_cols, mxb_matrix **
     m->ctx = ctx;
     m->n_rows = n_rows;
     m->n_cols = n_cols;
-    size_t bytes = (size_t)n_rows * (size_t)n_cols * sizeof(double);
-    if (bytes) {
-        cudaError_t e = dev_alloc(ctx, (void **)&m->data, bytes);
-        if (e != cudaSuccess) {
-            set_error("cudaMalloc(%zu bytes) for %lld x %lld matrix: %s", bytes,
-                      (long long)n_rows, (long long)n_cols, cudaGetErrorString(e));
-            delete m;
-            return e == cudaErrorMemoryAllocation ? MXB_ERR_NOMEM : MXB_ERR_CUDA;
-        }
+    const int rc = m->mem.alloc(ctx, (size_t)n_rows * (size_t)n_cols * sizeof(double),
+                                "mxb_matrix_alloc");
+    if (rc != MXB_OK) {
+        delete m;
+        return rc;
     }
+    m->data = m->mem.get<double>();
     *out = m;
     return MXB_OK;
 }
@@ -862,11 +787,8 @@ void *mxb_matrix_data(const mxb_matrix *m) { return m ? (void *)m->data : nullpt
 
 int mxb_matrix_destroy(mxb_matrix *m) {
     if (!m) return MXB_OK;
-    if (m->data) {
-        cudaSetDevice(m->ctx->device);
-        dev_free(m->ctx, m->data);
-    }
-    delete m;
+    if (m->data) cudaSetDevice(m->ctx->device);
+    delete m;   // (gives its block back)
     return MXB_OK;
 }
 

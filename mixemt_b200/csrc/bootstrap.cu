@@ -114,23 +114,16 @@ extern "C" int mxb_boot_counts(mxb_ctx *ctx, const double *weights, int64_t n_ro
     uint64_t total = 0;
     MXB_TRY(boot_prefix(weights, n_rows, cumw, total));
     MXB_CUDA(cudaSetDevice(ctx->device));
-    const size_t b_cum = (size_t)n_rows * sizeof(int64_t);
     const size_t b_cnt = (size_t)n_boot * n_rows * sizeof(uint32_t);
-    unsigned char *buf = nullptr;
-    if (dev_alloc(ctx, (void **)&buf, b_cum + b_cnt) != cudaSuccess) {
-        cudaGetLastError();
-        set_error("mxb_boot_counts: device allocation of %zu bytes failed", b_cum + b_cnt);
-        return MXB_ERR_NOMEM;
-    }
-    int64_t *d_cum = (int64_t *)buf;
-    uint32_t *d_cnt = (uint32_t *)(buf + b_cum);
-    int rc = copy_h2d(ctx, d_cum, cumw.data(), b_cum);
-    if (rc == MXB_OK && cudaMemsetAsync(d_cnt, 0, b_cnt, ctx->stream) != cudaSuccess) {
-        set_error("mxb_boot_counts: %s", cudaGetErrorString(cudaGetLastError()));
-        rc = MXB_ERR_CUDA;
-    }
-    if (rc == MXB_OK) rc = boot_draw(ctx, d_cum, n_rows, total, seed, boot0, n_boot, d_cnt);
-    if (rc == MXB_OK) rc = copy_d2h(ctx, counts_out, d_cnt, b_cnt);
-    dev_free(ctx, buf);
-    return rc;
+    DevBlock buf;   // [prefix sums][counts]
+    int64_t *d_cum = nullptr;
+    uint32_t *d_cnt = nullptr;
+    MXB_TRY(buf.alloc_parts(ctx, "mxb_boot_counts", [&](Carve &c) {
+        d_cum = c.part<int64_t>(n_rows);
+        d_cnt = c.part<uint32_t>((size_t)n_boot * n_rows);
+    }));
+    MXB_TRY(copy_h2d(ctx, d_cum, cumw.data(), (size_t)n_rows * sizeof(int64_t)));
+    MXB_CUDA(cudaMemsetAsync(d_cnt, 0, b_cnt, ctx->stream));
+    MXB_TRY(boot_draw(ctx, d_cum, n_rows, total, seed, boot0, n_boot, d_cnt));
+    return copy_d2h(ctx, counts_out, d_cnt, b_cnt);
 }

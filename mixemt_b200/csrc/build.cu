@@ -64,6 +64,7 @@
 // the per-group dense loop, the same arithmetic as build_matrix_dense_kernel,
 // the plain kernel that is also used when H > 8192 (or MXB_BUILD_DENSE=1 is set).
 #include <algorithm>
+#include <memory>
 #include <new>
 #include <string.h>
 #include <vector>
@@ -831,7 +832,7 @@ int mxb_phylo_pack(mxb_ctx *ctx, int32_t n_pos, int32_t n_hap, int32_t n_sym,
         return MXB_ERR_NOMEM;
     }
     MXB_CUDA(cudaSetDevice(ctx->device));
-    mxb_phylo *ph = new (std::nothrow) mxb_phylo();
+    std::unique_ptr<mxb_phylo> ph(new (std::nothrow) mxb_phylo());
     if (!ph) { set_error("out of host memory"); return MXB_ERR_NOMEM; }
     ph->ctx = ctx;
     ph->n_pos = n_pos;
@@ -839,49 +840,37 @@ int mxb_phylo_pack(mxb_ctx *ctx, int32_t n_pos, int32_t n_hap, int32_t n_sym,
     ph->n_sym = n_sym;
     ph->n_words = n_words;
     ph->n_dev = (int64_t)dev_ent.size();
-    cudaError_t e = cudaSuccess;
     if (!bits.empty()) {
-        const size_t ent_bytes = std::max<size_t>(1, dev_ent.size()) * sizeof(uint2);
-        e = cudaMalloc(&ph->bits, bits.size() * sizeof(uint32_t));
-        if (e == cudaSuccess) e = cudaMalloc(&ph->hitmiss, hm.size() * sizeof(double2));
-        if (e == cudaSuccess) e = cudaMalloc(&ph->plane_base, std::max<size_t>(1, plane_base.size()));
-        if (e == cudaSuccess) e = cudaMalloc(&ph->dev_ptr, dev_ptr.size() * sizeof(int32_t));
-        if (e == cudaSuccess) e = cudaMalloc(&ph->dev_ent, ent_bytes);
-        if (e == cudaSuccess)
-            e = cudaMemcpyAsync(ph->bits, bits.data(), bits.size() * sizeof(uint32_t),
-                                cudaMemcpyHostToDevice, ctx->stream);
-        if (e == cudaSuccess)
-            e = cudaMemcpyAsync(ph->hitmiss, hm.data(), hm.size() * sizeof(double2),
-                                cudaMemcpyHostToDevice, ctx->stream);
-        if (e == cudaSuccess)
-            e = cudaMemcpyAsync(ph->plane_base, plane_base.data(), plane_base.size(),
-                                cudaMemcpyHostToDevice, ctx->stream);
-        if (e == cudaSuccess)
-            e = cudaMemcpyAsync(ph->dev_ptr, dev_ptr.data(), dev_ptr.size() * sizeof(int32_t),
-                                cudaMemcpyHostToDevice, ctx->stream);
-        if (e == cudaSuccess && !dev_ent.empty())
-            e = cudaMemcpyAsync(ph->dev_ent, dev_ent.data(), dev_ent.size() * sizeof(uint2),
-                                cudaMemcpyHostToDevice, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+        // [bits][hit, miss][plane baselines][deviation lists: offsets, entries]
+        MXB_TRY(ph->mem.alloc_parts(ctx, "mxb_phylo_pack", [&](Carve &c) {
+            ph->bits = c.part<uint32_t>(bits.size());
+            ph->hitmiss = c.part<double2>(hm.size());
+            ph->plane_base = c.part<uint8_t>(std::max<size_t>(1, plane_base.size()));
+            ph->dev_ptr = c.part<int32_t>(dev_ptr.size());
+            ph->dev_ent = c.part<uint2>(std::max<size_t>(1, dev_ent.size()));
+        }));
+        cudaStream_t s = ctx->stream;
+        MXB_CUDA(cudaMemcpyAsync(ph->bits, bits.data(), bits.size() * sizeof(uint32_t),
+                                 cudaMemcpyHostToDevice, s));
+        MXB_CUDA(cudaMemcpyAsync(ph->hitmiss, hm.data(), hm.size() * sizeof(double2),
+                                 cudaMemcpyHostToDevice, s));
+        MXB_CUDA(cudaMemcpyAsync(ph->plane_base, plane_base.data(), plane_base.size(),
+                                 cudaMemcpyHostToDevice, s));
+        MXB_CUDA(cudaMemcpyAsync(ph->dev_ptr, dev_ptr.data(), dev_ptr.size() * sizeof(int32_t),
+                                 cudaMemcpyHostToDevice, s));
+        if (!dev_ent.empty())
+            MXB_CUDA(cudaMemcpyAsync(ph->dev_ent, dev_ent.data(), dev_ent.size() * sizeof(uint2),
+                                     cudaMemcpyHostToDevice, s));
+        MXB_CUDA(cudaStreamSynchronize(s));
     }
-    if (e != cudaSuccess) {
-        set_error("mxb_phylo_pack: %s", cudaGetErrorString(e));
-        mxb_phylo_destroy(ph);
-        return MXB_ERR_CUDA;
-    }
-    *out = ph;
+    *out = ph.release();
     return MXB_OK;
 }
 
 int mxb_phylo_destroy(mxb_phylo *ph) {
     if (!ph) return MXB_OK;
     cudaSetDevice(ph->ctx->device);
-    if (ph->bits) cudaFree(ph->bits);
-    if (ph->hitmiss) cudaFree(ph->hitmiss);
-    if (ph->plane_base) cudaFree(ph->plane_base);
-    if (ph->dev_ptr) cudaFree(ph->dev_ptr);
-    if (ph->dev_ent) cudaFree(ph->dev_ent);
-    delete ph;
+    delete ph;   // (gives its tables back)
     return MXB_OK;
 }
 
@@ -899,136 +888,123 @@ int mxb_build_matrix(mxb_ctx *ctx, const mxb_phylo *ph, int64_t n_rows,
     MXB_REQUIRE(n_obs == 0 || (pos_idx && base_code), "NULL observation arrays");
     MXB_REQUIRE(n_obs == 0 || ph->n_pos > 0, "observations but no positions");
 
-    mxb_matrix *m = nullptr;
-    MXB_TRY(mxb_matrix_alloc(ctx, n_rows, ph->n_hap, &m));
+    mxb_matrix *mat = nullptr;
+    MXB_TRY(mxb_matrix_alloc(ctx, n_rows, ph->n_hap, &mat));
+    std::unique_ptr<mxb_matrix, decltype(&mxb_matrix_destroy)> m(mat, mxb_matrix_destroy);
     const size_t cells = (size_t)n_rows * (size_t)ph->n_hap;
-    int64_t *d_row_ptr = nullptr;
-    int32_t *d_pos = nullptr, *d_match = nullptr, *d_overflow = nullptr, *d_route = nullptr;
-    uint8_t *d_code = nullptr;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    cudaError_t e = cudaSuccess;
-    int rc = MXB_OK;
     Prefault fault_out, fault_match;  // first-touch the result pages while the GPU works
-#define STEP(call) do { if (e == cudaSuccess) e = (call); } while (0)
     if (cells) {
         if (out_host) fault_out.start(out_host, cells * sizeof(double));
         if (match_host) fault_match.start(match_host, cells * sizeof(int32_t));
-        STEP(cudaMalloc(&d_row_ptr, (n_rows + 1) * sizeof(int64_t)));
-        if (n_obs) {
-            STEP(cudaMalloc(&d_pos, n_obs * sizeof(int32_t)));
-            STEP(cudaMalloc(&d_code, n_obs * sizeof(uint8_t)));
-        }
-        if (match_host) STEP(cudaMalloc(&d_match, cells * sizeof(int32_t)));
-        STEP(cudaMemcpyAsync(d_row_ptr, row_ptr, (n_rows + 1) * sizeof(int64_t),
-                             cudaMemcpyHostToDevice, ctx->stream));
-        if (n_obs) {
-            STEP(cudaMemcpyAsync(d_pos, pos_idx, n_obs * sizeof(int32_t),
-                                 cudaMemcpyHostToDevice, ctx->stream));
-            STEP(cudaMemcpyAsync(d_code, base_code, n_obs * sizeof(uint8_t),
-                                 cudaMemcpyHostToDevice, ctx->stream));
-        }
-        STEP(cudaEventCreate(&ev0));
-        STEP(cudaEventCreate(&ev1));
-        if (e == cudaSuccess) {
-            // class kernel (two tiers) when its shared-memory layouts fit, else the dense kernel
-            const bool counts = d_match != nullptr;
-            const int n_groups = (int)ceil_div(ph->n_hap, 32);
-            const bool use_class = getenv("MXB_BUILD_DENSE") == nullptr &&
-                                   n_groups <= kGroupsLarge && n_rows < ((int64_t)1 << 31);
-            // MXB_BUILD_TIERS=2 skips tier 1 (cross-check of the large-pool launch)
-            const char *tiers_env = getenv("MXB_BUILD_TIERS");
-            const bool two_tiers = !(tiers_env && strcmp(tiers_env, "2") == 0);
-            if (use_class) {
-                // d_overflow[0] = number of rows deferred to tier 2, [1], [2] = the work counters
-                // of the two launches, [3..] = the deferred rows
-                STEP(cudaMalloc(&d_overflow, (n_rows + 3) * sizeof(int32_t)));
-                STEP(cudaMemsetAsync(d_overflow, 0, 3 * sizeof(int32_t), ctx->stream));
-                if (route_host) {   // rows tier 1 finishes without dense groups stay 0
-                    STEP(cudaMalloc(&d_route, n_rows * sizeof(int32_t)));
-                    STEP(cudaMemsetAsync(d_route, 0, n_rows * sizeof(int32_t), ctx->stream));
-                }
-            } else if (route_host) {
-                std::fill(route_host, route_host + n_rows, 3);
+        // class kernel (two tiers) when its shared-memory layouts fit, else the dense kernel
+        const bool counts = match_host != nullptr;
+        const int n_groups = (int)ceil_div(ph->n_hap, 32);
+        const bool use_class = getenv("MXB_BUILD_DENSE") == nullptr &&
+                               n_groups <= kGroupsLarge && n_rows < ((int64_t)1 << 31);
+        // MXB_BUILD_TIERS=2 skips tier 1 (cross-check of the large-pool launch)
+        const char *tiers_env = getenv("MXB_BUILD_TIERS");
+        const bool two_tiers = !(tiers_env && strcmp(tiers_env, "2") == 0);
+        // [row offsets][observations: positions, codes][match counts][class kernel: overflow,
+        // routes]; d_overflow[0] = number of rows deferred to tier 2, [1], [2] = the work counters
+        // of the two launches, [3..] = the deferred rows
+        DevBlock buf;
+        int64_t *d_row_ptr = nullptr;
+        int32_t *d_pos = nullptr, *d_match = nullptr, *d_overflow = nullptr, *d_route = nullptr;
+        uint8_t *d_code = nullptr;
+        MXB_TRY(buf.alloc_parts(ctx, "mxb_build_matrix", [&](Carve &c) {
+            d_row_ptr = c.part<int64_t>(n_rows + 1);
+            if (n_obs) {
+                d_pos = c.part<int32_t>(n_obs);
+                d_code = c.part<uint8_t>(n_obs);
             }
-            STEP(cudaEventRecord(ev0, ctx->stream));
-            if (e == cudaSuccess && use_class) {
-                BuildTables tb;
-                tb.bits = ph->bits;
-                tb.hitmiss = ph->hitmiss;
-                tb.plane_base = ph->plane_base;
-                tb.dev_ptr = ph->dev_ptr;
-                tb.dev_ent = ph->dev_ent;
-                tb.n_planes = ph->n_sym + 1;
-                tb.n_words = ph->n_words;
-                tb.n_hap = ph->n_hap;
-                tb.n_groups = n_groups;
-                int *ov_count = reinterpret_cast<int *>(d_overflow);
-                int32_t *ov_list = d_overflow + 3;
-                if (two_tiers) {
-                    e = counts ? launch_tier_groups<true, Tier1>(ctx, tb, n_rows, nullptr, nullptr,
-                                                                 ov_list, ov_count, ov_count + 1,
-                                                                 d_row_ptr, d_pos, d_code, m->data,
-                                                                 d_match, d_route)
-                               : launch_tier_groups<false, Tier1>(ctx, tb, n_rows, nullptr, nullptr,
-                                                                  ov_list, ov_count, ov_count + 1,
-                                                                  d_row_ptr, d_pos, d_code, m->data,
-                                                                  d_match, d_route);
-                }
-                const int32_t *in2 = two_tiers ? ov_list : nullptr;
-                const int *n_in2 = two_tiers ? ov_count : nullptr;
-                if (e == cudaSuccess)
-                    e = counts ? launch_tier_groups<true, Tier2>(ctx, tb, n_rows, in2, n_in2, nullptr,
-                                                                 nullptr, ov_count + 2, d_row_ptr,
-                                                                 d_pos, d_code, m->data, d_match,
-                                                                 d_route)
-                               : launch_tier_groups<false, Tier2>(ctx, tb, n_rows, in2, n_in2, nullptr,
-                                                                  nullptr, ov_count + 2, d_row_ptr,
-                                                                  d_pos, d_code, m->data, d_match,
-                                                                  d_route);
-                ctx->launches--;  // counted once more below
-            } else if (e == cudaSuccess) {
-                const int grid = (int)std::min<int64_t>(n_rows, (int64_t)ctx->num_sms * 4);
-                build_matrix_dense_kernel<<<grid, kBuildThreads, 0, ctx->stream>>>(
-                    ph->bits, ph->hitmiss, ph->n_sym + 1, ph->n_words, ph->n_hap, n_rows,
-                    d_row_ptr, d_pos, d_code, m->data, d_match);
-            }
-            ctx->launches++;
-            STEP(cudaGetLastError());
-            STEP(cudaEventRecord(ev1, ctx->stream));
-            if (d_route)
-                STEP(cudaMemcpyAsync(route_host, d_route, n_rows * sizeof(int32_t),
-                                     cudaMemcpyDeviceToHost, ctx->stream));
+            if (counts) d_match = c.part<int32_t>(cells);
+            if (use_class) d_overflow = c.part<int32_t>(n_rows + 3);
+            if (use_class && route_host) d_route = c.part<int32_t>(n_rows);
+        }));
+        Events ev;   // around the kernels
+        MXB_TRY(ev.create(2, cudaEventDefault, "mxb_build_matrix"));
+        cudaStream_t s = ctx->stream;
+        MXB_CUDA(cudaMemcpyAsync(d_row_ptr, row_ptr, (n_rows + 1) * sizeof(int64_t),
+                                 cudaMemcpyHostToDevice, s));
+        if (n_obs) {
+            MXB_CUDA(cudaMemcpyAsync(d_pos, pos_idx, n_obs * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+            MXB_CUDA(cudaMemcpyAsync(d_code, base_code, n_obs * sizeof(uint8_t), cudaMemcpyHostToDevice, s));
         }
+        if (use_class) {
+            MXB_CUDA(cudaMemsetAsync(d_overflow, 0, 3 * sizeof(int32_t), s));
+            // rows tier 1 finishes without dense groups stay 0
+            if (d_route) MXB_CUDA(cudaMemsetAsync(d_route, 0, n_rows * sizeof(int32_t), s));
+        } else if (route_host) {
+            std::fill(route_host, route_host + n_rows, 3);
+        }
+        MXB_CUDA(cudaEventRecord(ev[0], s));
+        if (use_class) {
+            BuildTables tb;
+            tb.bits = ph->bits;
+            tb.hitmiss = ph->hitmiss;
+            tb.plane_base = ph->plane_base;
+            tb.dev_ptr = ph->dev_ptr;
+            tb.dev_ent = ph->dev_ent;
+            tb.n_planes = ph->n_sym + 1;
+            tb.n_words = ph->n_words;
+            tb.n_hap = ph->n_hap;
+            tb.n_groups = n_groups;
+            int *ov_count = reinterpret_cast<int *>(d_overflow);
+            int32_t *ov_list = d_overflow + 3;
+            cudaError_t e = cudaSuccess;
+            if (two_tiers) {
+                e = counts ? launch_tier_groups<true, Tier1>(ctx, tb, n_rows, nullptr, nullptr,
+                                                             ov_list, ov_count, ov_count + 1,
+                                                             d_row_ptr, d_pos, d_code, m->data,
+                                                             d_match, d_route)
+                           : launch_tier_groups<false, Tier1>(ctx, tb, n_rows, nullptr, nullptr,
+                                                              ov_list, ov_count, ov_count + 1,
+                                                              d_row_ptr, d_pos, d_code, m->data,
+                                                              d_match, d_route);
+            }
+            const int32_t *in2 = two_tiers ? ov_list : nullptr;
+            const int *n_in2 = two_tiers ? ov_count : nullptr;
+            if (e == cudaSuccess)
+                e = counts ? launch_tier_groups<true, Tier2>(ctx, tb, n_rows, in2, n_in2, nullptr,
+                                                             nullptr, ov_count + 2, d_row_ptr,
+                                                             d_pos, d_code, m->data, d_match,
+                                                             d_route)
+                           : launch_tier_groups<false, Tier2>(ctx, tb, n_rows, in2, n_in2, nullptr,
+                                                              nullptr, ov_count + 2, d_row_ptr,
+                                                              d_pos, d_code, m->data, d_match,
+                                                              d_route);
+            if (e != cudaSuccess) {
+                cudaGetLastError();
+                set_error("mxb_build_matrix: %s", cudaGetErrorString(e));
+                return MXB_ERR_CUDA;
+            }
+            ctx->launches--;  // counted once more below
+        } else {
+            const int grid = (int)std::min<int64_t>(n_rows, (int64_t)ctx->num_sms * 4);
+            build_matrix_dense_kernel<<<grid, kBuildThreads, 0, s>>>(
+                ph->bits, ph->hitmiss, ph->n_sym + 1, ph->n_words, ph->n_hap, n_rows,
+                d_row_ptr, d_pos, d_code, m->data, d_match);
+        }
+        ctx->launches++;
+        MXB_CUDA(cudaGetLastError());
+        MXB_CUDA(cudaEventRecord(ev[1], s));
+        if (d_route)
+            MXB_CUDA(cudaMemcpyAsync(route_host, d_route, n_rows * sizeof(int32_t),
+                                     cudaMemcpyDeviceToHost, s));
         // pageable results leave through the staged copy engine (api.cu)
-        if (e == cudaSuccess && out_host) {
+        if (out_host) {
             fault_out.join();
-            rc = copy_d2h(ctx, out_host, m->data, cells * sizeof(double));
+            MXB_TRY(copy_d2h(ctx, out_host, m->data, cells * sizeof(double)));
         }
-        if (e == cudaSuccess && rc == MXB_OK && match_host) {
+        if (match_host) {
             fault_match.join();
-            rc = copy_d2h(ctx, match_host, d_match, cells * sizeof(int32_t));
+            MXB_TRY(copy_d2h(ctx, match_host, d_match, cells * sizeof(int32_t)));
         }
-        STEP(cudaStreamSynchronize(ctx->stream));
-        if (e == cudaSuccess && elapsed_ms) STEP(cudaEventElapsedTime(elapsed_ms, ev0, ev1));
+        MXB_CUDA(cudaStreamSynchronize(s));
+        if (elapsed_ms) MXB_CUDA(cudaEventElapsedTime(elapsed_ms, ev[0], ev[1]));
     }
-#undef STEP
-    fault_out.join();
-    fault_match.join();
-    if (e != cudaSuccess) {
-        set_error("mxb_build_matrix: %s", cudaGetErrorString(e));
-        rc = (e == cudaErrorMemoryAllocation) ? MXB_ERR_NOMEM : MXB_ERR_CUDA;
-    }
-    if (ev0) cudaEventDestroy(ev0);
-    if (ev1) cudaEventDestroy(ev1);
-    cudaFree(d_row_ptr);
-    cudaFree(d_pos);
-    cudaFree(d_code);
-    cudaFree(d_match);
-    cudaFree(d_overflow);
-    cudaFree(d_route);
-    if (rc != MXB_OK || !out_dev) mxb_matrix_destroy(m);
-    else *out_dev = m;
-    return rc;
+    if (out_dev) *out_dev = m.release();
+    return MXB_OK;
 }
 
 }  // extern "C"

@@ -12,6 +12,7 @@
 #include <math.h>
 
 #include <algorithm>
+#include <memory>
 
 #include "common.cuh"
 
@@ -133,30 +134,22 @@ int mxb_matrix_gather_cols(mxb_ctx *ctx, const mxb_matrix *src, const int64_t *c
         }
     }
     MXB_CUDA(cudaSetDevice(ctx->device));
-    mxb_matrix *dst = nullptr;
-    MXB_TRY(mxb_matrix_alloc(ctx, src->n_rows, n_out, &dst));
+    mxb_matrix *m = nullptr;
+    MXB_TRY(mxb_matrix_alloc(ctx, src->n_rows, n_out, &m));
+    std::unique_ptr<mxb_matrix, decltype(&mxb_matrix_destroy)> dst(m, mxb_matrix_destroy);
     const int64_t total = src->n_rows * n_out;
     if (total > 0) {
-        int64_t *d_cols = nullptr;
-        cudaError_t e = cudaMalloc(&d_cols, n_out * sizeof(int64_t));
-        if (e == cudaSuccess)
-            e = cudaMemcpyAsync(d_cols, cols, n_out * sizeof(int64_t), cudaMemcpyHostToDevice,
-                                ctx->stream);
-        if (e == cudaSuccess) {
-            gather_cols_kernel<<<grid_for(ctx, total, 256), 256, 0, ctx->stream>>>(
-                src->data, src->n_rows, src->n_cols, d_cols, n_out, dst->data);
-            ctx->launches++;
-            e = cudaGetLastError();
-        }
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-        cudaFree(d_cols);
-        if (e != cudaSuccess) {
-            set_error("mxb_matrix_gather_cols: %s", cudaGetErrorString(e));
-            mxb_matrix_destroy(dst);
-            return MXB_ERR_CUDA;
-        }
+        DevBlock d_cols;
+        MXB_TRY(d_cols.alloc(ctx, n_out * sizeof(int64_t), __func__));
+        MXB_CUDA(cudaMemcpyAsync(d_cols.get(), cols, n_out * sizeof(int64_t), cudaMemcpyHostToDevice,
+                                 ctx->stream));
+        gather_cols_kernel<<<grid_for(ctx, total, 256), 256, 0, ctx->stream>>>(
+            src->data, src->n_rows, src->n_cols, d_cols.get<int64_t>(), n_out, m->data);
+        ctx->launches++;
+        MXB_CUDA(cudaGetLastError());
+        MXB_CUDA(cudaStreamSynchronize(ctx->stream));
     }
-    *out = dst;
+    *out = dst.release();
     return MXB_OK;
 }
 
@@ -177,46 +170,34 @@ static int vote_rows(mxb_ctx *ctx, const mxb_matrix *m, const int64_t *weights, 
     if (m->n_rows == 0) return MXB_OK;
     MXB_REQUIRE(weights != nullptr, "weights is NULL");
     MXB_CUDA(cudaSetDevice(ctx->device));
+    DevBlock buf;   // [row maxima][weights][votes][first rows]
     int64_t *d_best = nullptr, *d_w = nullptr;
     unsigned long long *d_votes = nullptr, *d_first = nullptr;
-    cudaError_t e = cudaMalloc(&d_best, m->n_rows * sizeof(int64_t));
-    if (e == cudaSuccess) e = cudaMalloc(&d_w, m->n_rows * sizeof(int64_t));
-    if (e == cudaSuccess) e = cudaMalloc(&d_votes, m->n_cols * sizeof(unsigned long long));
-    if (e == cudaSuccess && first_out)
-        e = cudaMalloc(&d_first, m->n_cols * sizeof(unsigned long long));
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(d_w, weights, m->n_rows * sizeof(int64_t), cudaMemcpyHostToDevice,
-                            ctx->stream);
-    if (e == cudaSuccess)
-        e = cudaMemsetAsync(d_votes, 0, m->n_cols * sizeof(unsigned long long), ctx->stream);
-    if (e == cudaSuccess && d_first)      // all bits set: UINT64_MAX, no row yet (-1 as int64_t)
-        e = cudaMemsetAsync(d_first, 0xff, m->n_cols * sizeof(unsigned long long), ctx->stream);
-    if (e == cudaSuccess) {
-        const int blocks = (int)std::min<int64_t>(ceil_div(m->n_rows, 8), (int64_t)ctx->num_sms * 8);
-        argmax_rows_kernel<<<blocks, 256, 0, ctx->stream>>>(m->data, m->n_rows, m->n_cols, d_best);
-        vote_kernel<<<grid_for(ctx, m->n_rows, 256), 256, 0, ctx->stream>>>(d_best, d_w, m->n_rows,
-                                                                           d_votes, d_first, row0);
-        ctx->launches += 2;
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(votes_out, d_votes, m->n_cols * sizeof(int64_t),
-                            cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess && d_first)
-        e = cudaMemcpyAsync(first_out, d_first, m->n_cols * sizeof(int64_t),
-                            cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess && argmax_out)
-        e = cudaMemcpyAsync(argmax_out, d_best, m->n_rows * sizeof(int64_t),
-                            cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    cudaFree(d_best);
-    cudaFree(d_w);
-    cudaFree(d_votes);
-    cudaFree(d_first);
-    if (e != cudaSuccess) {
-        set_error("%s: %s", what, cudaGetErrorString(e));
-        return MXB_ERR_CUDA;
-    }
+    MXB_TRY(buf.alloc_parts(ctx, what, [&](Carve &c) {
+        d_best = c.part<int64_t>(m->n_rows);
+        d_w = c.part<int64_t>(m->n_rows);
+        d_votes = c.part<unsigned long long>(m->n_cols);
+        if (first_out) d_first = c.part<unsigned long long>(m->n_cols);
+    }));
+    cudaStream_t s = ctx->stream;
+    MXB_CUDA(cudaMemcpyAsync(d_w, weights, m->n_rows * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    MXB_CUDA(cudaMemsetAsync(d_votes, 0, m->n_cols * sizeof(unsigned long long), s));
+    if (d_first)      // all bits set: UINT64_MAX, no row yet (-1 as int64_t)
+        MXB_CUDA(cudaMemsetAsync(d_first, 0xff, m->n_cols * sizeof(unsigned long long), s));
+    const int blocks = (int)std::min<int64_t>(ceil_div(m->n_rows, 8), (int64_t)ctx->num_sms * 8);
+    argmax_rows_kernel<<<blocks, 256, 0, s>>>(m->data, m->n_rows, m->n_cols, d_best);
+    vote_kernel<<<grid_for(ctx, m->n_rows, 256), 256, 0, s>>>(d_best, d_w, m->n_rows, d_votes,
+                                                              d_first, row0);
+    ctx->launches += 2;
+    MXB_CUDA(cudaGetLastError());
+    MXB_CUDA(cudaMemcpyAsync(votes_out, d_votes, m->n_cols * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    if (d_first)
+        MXB_CUDA(cudaMemcpyAsync(first_out, d_first, m->n_cols * sizeof(int64_t),
+                                 cudaMemcpyDeviceToHost, s));
+    if (argmax_out)
+        MXB_CUDA(cudaMemcpyAsync(argmax_out, d_best, m->n_rows * sizeof(int64_t),
+                                 cudaMemcpyDeviceToHost, s));
+    MXB_CUDA(cudaStreamSynchronize(s));
     return MXB_OK;     // an untouched first[j] (UINT64_MAX) reads back as int64_t -1
 }
 
@@ -249,36 +230,25 @@ int mxb_assign_reads(mxb_ctx *ctx, const mxb_matrix *read_mix, const int64_t *co
     if (read_mix->n_rows == 0) return MXB_OK;
     MXB_REQUIRE(assign_out != nullptr, "assign_out is NULL");
     MXB_CUDA(cudaSetDevice(ctx->device));
+    DevBlock buf;   // [contributor columns][their log-proportions][assignments]
     int64_t *d_cols = nullptr;
     double *d_ln = nullptr;
     int32_t *d_out = nullptr;
-    cudaError_t e = cudaMalloc(&d_cols, n_con * sizeof(int64_t));
-    if (e == cudaSuccess) e = cudaMalloc(&d_ln, n_con * sizeof(double));
-    if (e == cudaSuccess) e = cudaMalloc(&d_out, read_mix->n_rows * sizeof(int32_t));
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(d_cols, con_cols, n_con * sizeof(int64_t), cudaMemcpyHostToDevice,
-                            ctx->stream);
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(d_ln, con_lnprops, n_con * sizeof(double), cudaMemcpyHostToDevice,
-                            ctx->stream);
-    if (e == cudaSuccess) {
-        assign_reads_kernel<<<grid_for(ctx, read_mix->n_rows, 256), 256, 0, ctx->stream>>>(
-            read_mix->data, read_mix->n_rows, read_mix->n_cols, d_cols, d_ln, n_con, ln_min_fold,
-            d_out);
-        ctx->launches++;
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(assign_out, d_out, read_mix->n_rows * sizeof(int32_t),
-                            cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    cudaFree(d_cols);
-    cudaFree(d_ln);
-    cudaFree(d_out);
-    if (e != cudaSuccess) {
-        set_error("mxb_assign_reads: %s", cudaGetErrorString(e));
-        return MXB_ERR_CUDA;
-    }
+    MXB_TRY(buf.alloc_parts(ctx, __func__, [&](Carve &c) {
+        d_cols = c.part<int64_t>(n_con);
+        d_ln = c.part<double>(n_con);
+        d_out = c.part<int32_t>(read_mix->n_rows);
+    }));
+    cudaStream_t s = ctx->stream;
+    MXB_CUDA(cudaMemcpyAsync(d_cols, con_cols, n_con * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    MXB_CUDA(cudaMemcpyAsync(d_ln, con_lnprops, n_con * sizeof(double), cudaMemcpyHostToDevice, s));
+    assign_reads_kernel<<<grid_for(ctx, read_mix->n_rows, 256), 256, 0, s>>>(
+        read_mix->data, read_mix->n_rows, read_mix->n_cols, d_cols, d_ln, n_con, ln_min_fold, d_out);
+    ctx->launches++;
+    MXB_CUDA(cudaGetLastError());
+    MXB_CUDA(cudaMemcpyAsync(assign_out, d_out, read_mix->n_rows * sizeof(int32_t),
+                             cudaMemcpyDeviceToHost, s));
+    MXB_CUDA(cudaStreamSynchronize(s));
     return MXB_OK;
 }
 
@@ -288,17 +258,15 @@ int mxb_matrix_argmax_rows(mxb_ctx *ctx, const mxb_matrix *m, int64_t *out_host)
     MXB_REQUIRE(out_host != nullptr, "out_host is NULL");
     MXB_REQUIRE(m->n_cols > 0, "argmax of empty rows");
     MXB_CUDA(cudaSetDevice(ctx->device));
-    int64_t *d = nullptr;
-    MXB_CUDA(cudaMalloc(&d, m->n_rows * sizeof(int64_t)));
+    DevBlock d;
+    MXB_TRY(d.alloc(ctx, m->n_rows * sizeof(int64_t), __func__));
     int blocks = (int)std::min<int64_t>(ceil_div(m->n_rows, 8), (int64_t)ctx->num_sms * 8);
-    argmax_rows_kernel<<<blocks, 256, 0, ctx->stream>>>(m->data, m->n_rows, m->n_cols, d);
+    argmax_rows_kernel<<<blocks, 256, 0, ctx->stream>>>(m->data, m->n_rows, m->n_cols, d.get<int64_t>());
     ctx->launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(out_host, d, m->n_rows * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    cudaFree(d);
-    if (e != cudaSuccess) { set_error("argmax_rows: %s", cudaGetErrorString(e)); return MXB_ERR_CUDA; }
+    MXB_CUDA(cudaGetLastError());
+    MXB_CUDA(cudaMemcpyAsync(out_host, d.get(), m->n_rows * sizeof(int64_t), cudaMemcpyDeviceToHost,
+                             ctx->stream));
+    MXB_CUDA(cudaStreamSynchronize(ctx->stream));
     return MXB_OK;
 }
 

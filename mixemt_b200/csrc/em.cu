@@ -35,6 +35,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <memory>
 #include <new>
 #include <vector>
 
@@ -61,7 +62,7 @@ struct mxb_em {
     const mxb_matrix *mat = nullptr;
     int64_t n_rows = 0, n_cols = 0, ld = 0;
     bool sharded = false;
-    double *lin = nullptr;        // [n_rows][ld]
+    DevBlock lin;                 // [n_rows][ld] doubles
     double *weights = nullptr;    // [n_rows]
     double *coef = nullptr;       // [n_rows] (general path)
     double *lnp[2] = {nullptr, nullptr};
@@ -71,7 +72,7 @@ struct mxb_em {
     double *props_in = nullptr;   // [n_cols] staging for set_lnprops
     EmState *state = nullptr;     // device
     EmState *host_state = nullptr;  // pinned, 2 slots
-    cudaEvent_t poll_ev[2] = {nullptr, nullptr};
+    Events poll_ev;               // 2
     int n_part = 0;
     // decide_form
     EmForm form = EmForm::kGeneral;
@@ -89,8 +90,8 @@ struct mxb_em {
     int row_blocks = 0, col_blocks = 0;
     // Class tiles (em_tiles.cuh): form kTiles reads `tile_v` instead of `lin`.
     int n_batches = 0, tile_hs = 0, tile_grid = 0;   // (the gather's blocks: n_part)
-    unsigned char *tile_block = nullptr;   // [perm][cmap][cword][desc]
-    unsigned char *tile_vecs = nullptr;    // [pi_cls][u_sum][ctas][segs][copies][gather entries]
+    DevBlock tile_block;   // [perm][cmap][cword][desc]
+    DevBlock tile_vecs;    // [pi_cls][u_sum][ctas][segs][gather entries]
     unsigned short *tile_perm = nullptr, *tile_cmap = nullptr;
     unsigned int *tile_cword = nullptr;
     TileDesc *tile_desc = nullptr;
@@ -101,11 +102,11 @@ struct mxb_em {
     int tile_n_ent = 0, tile_n_slots = 0;
     uint32_t tile_slot_bytes = 0;
     double *tile_pi = nullptr, *tile_usum = nullptr;
-    double *tile_v = nullptr;
+    DevBlock tile_v;                       // the tiles (doubles)
     int64_t tile_cells = 0;                // doubles in tile_v
     int64_t tile_bytes_per_pass = 0;
-    unsigned char *small = nullptr;  // one device block behind weights ... props_in (fewer driver calls)
-    unsigned char *slots = nullptr;  // the slot block (slot_block)
+    DevBlock small;   // one device block behind weights ... props_in (fewer driver calls)
+    DevBlock slots;   // the slot block (slot_block)
     bool zero_iter = false;  // last iterate() ran no iteration
     // Bootstrap session (run_bootstrap): n_slots replicates per launch, each with its own weight
     // vector (slot_weights); over class tiles the slots' Pi and U vectors lie tile_pi_stride and
@@ -201,7 +202,7 @@ static int enqueue_tile_pass(mxb_em *em, unsigned R, cudaEvent_t *marks) {
     if (marks) MXB_CUDA(cudaEventRecord(marks[0], s));
     MXB_CUDA(launch_pdl(tile_pass_kernel<kSlots>, dim3(em->tile_grid, R), dim3(kTilePassThreads),
                         kSlots ? kTilePassSlotSmem : kTilePassSmem, s, (const TileCta *)em->tile_ctas,
-                        (const TileSeg *)em->tile_segs, (const double *)em->tile_v,
+                        (const TileSeg *)em->tile_segs, em->tile_v.get<const double>(),
                         (const double *)em->tile_pi, em->state, em->tile_usum,
                         em->tile_slot_bytes, em->tile_n_slots,
                         (const double *)(kSlots ? slot_weights(em, 0) : nullptr),
@@ -288,7 +289,7 @@ static int enqueue_iteration(mxb_em *em, cudaEvent_t pass_begin = nullptr,
         break;
     case EmForm::kRowPairs:
         MXB_CUDA(launch_pdl(pick_pair(em->nc), dim3(em->grid_fast), dim3(kPassThreads),
-                            em->smem_bytes, s, em->lin, em->ld, em->n_rows, em->weights,
+                            em->smem_bytes, s, em->lin.get<const double>(), em->ld, em->n_rows, em->weights,
                             em->pi[0], em->pi[1], em->pi[0] + em->ld, em->pi[1] + em->ld,
                             em->state, em->partials,
                             em->partials + (size_t)em->n_part * em->ld, em->n_stages));
@@ -296,7 +297,7 @@ static int enqueue_iteration(mxb_em *em, cudaEvent_t pass_begin = nullptr,
         break;
     case EmForm::kRows:
         MXB_CUDA(launch_pdl(pick_pass(em->nc), dim3(em->grid_fast), dim3(kPassThreads),
-                            em->smem_bytes, s, (const unsigned char *)em->lin,
+                            em->smem_bytes, s, em->lin.get<const unsigned char>(),
                             (uint32_t)(em->ld * sizeof(double)), em->ld, em->n_rows, weights,
                             em->pi[0], em->pi[1], em->state, em->partials, em->n_stages));
         ctx->launches += 1;
@@ -304,10 +305,10 @@ static int enqueue_iteration(mxb_em *em, cudaEvent_t pass_begin = nullptr,
     case EmForm::kGeneral: {
         const int rd_blocks = (int)std::max<int64_t>(
             1, std::min<int64_t>(ceil_div(em->n_rows, 8), (int64_t)ctx->num_sms * 8));
-        em_rowdot_kernel<<<rd_blocks, 256, 0, s>>>(em->lin, em->ld, em->n_rows, weights,
+        em_rowdot_kernel<<<rd_blocks, 256, 0, s>>>(em->lin.get<double>(), em->ld, em->n_rows, weights,
                                                    em->pi[0], em->pi[1], em->state, em->coef);
         dim3 grid(em->row_blocks, em->col_blocks);
-        em_colacc_kernel<<<grid, 256, 0, s>>>(em->lin, em->ld, em->n_rows, em->coef, em->state,
+        em_colacc_kernel<<<grid, 256, 0, s>>>(em->lin.get<double>(), em->ld, em->n_rows, em->coef, em->state,
                                               em->partials);
         ctx->launches += 2;
         break;
@@ -362,15 +363,7 @@ int mxb_em_destroy(mxb_em *em) {
     if (!em) return MXB_OK;
     cudaSetDevice(em->ctx->device);
     cudaStreamSynchronize(em->ctx->stream);
-    dev_free(em->ctx, em->lin);
-    dev_free(em->ctx, em->tile_block);
-    dev_free(em->ctx, em->tile_vecs);
-    dev_free(em->ctx, em->tile_v);
-    dev_free(em->ctx, em->small);
-    dev_free(em->ctx, em->slots);
-    for (int i = 0; i < 2; ++i)
-        if (em->poll_ev[i]) cudaEventDestroy(em->poll_ev[i]);
-    delete em;  // host_state points into the context's pinned scratch
+    delete em;  // (its blocks and events go with it; host_state is the context's pinned scratch)
     return MXB_OK;
 }
 
@@ -389,23 +382,15 @@ __global__ void em_reset_state_kernel(EmState *st, long long max_iter, double to
 }
 
 // The slot block of a session with R slots: [slot weights (bootstrap sessions) R x n_rows]
-// [lnp 2 x R x ld][pi 2 x R x ld][partials R x n_part x ld][control blocks R], each part
-// 256-byte aligned.  Returns its bytes, and with `base` points the session's slot buffers into
-// it; R = 1 gives the bytes of one slot.
-static size_t slot_block(mxb_em *em, int R, int n_part, unsigned char *base) {
-    const size_t ns = (size_t)R, row_bytes = (size_t)em->ld * sizeof(double);
-    const size_t b_w = em->boot ? align256(ns * em->n_rows * sizeof(double)) : 0;
-    const size_t b_vec = align256(ns * row_bytes);
-    const size_t b_part = align256(ns * n_part * row_bytes);
-    if (base) {
-        unsigned char *p = base;
-        if (em->boot) { em->slot_w = (double *)p; p += b_w; }
-        for (int i = 0; i < 2; ++i) { em->lnp[i] = (double *)p; p += b_vec; }
-        for (int i = 0; i < 2; ++i) { em->pi[i] = (double *)p; p += b_vec; }
-        em->partials = (double *)p; p += b_part;
-        em->state = (EmState *)p;
-    }
-    return b_w + 4 * b_vec + b_part + align256(ns * sizeof(EmState));
+// [lnp 2 x R x ld][pi 2 x R x ld][partials R x n_part x ld][control blocks R], laid out on `c`
+// and the session's slot buffers pointed into it; R = 1 gives the bytes of one slot.
+static void slot_block(mxb_em *em, int R, int n_part, Carve &c) {
+    const size_t ns = (size_t)R, ld = (size_t)em->ld;
+    if (em->boot) em->slot_w = c.part<double>(ns * em->n_rows);
+    for (double *&p : em->lnp) p = c.part<double>(ns * ld);
+    for (double *&p : em->pi) p = c.part<double>(ns * ld);
+    em->partials = c.part<double>(ns * n_part * ld);
+    em->state = c.part<EmState>(ns);
 }
 
 // Layout of the batches and ring of the pass for the class counts of n rows (tile_plan.h).
@@ -458,13 +443,14 @@ static void decide_form(mxb_em *em, int want_slots, const TileShape *tiles = nul
         // the slotted tile kernels exist for the fused tail only
         em->tail = EmTail::kFused;
         if (!fused) return;
-        const int parts = tile_gather_parts((int)plan->ent_batch.size());
-        const size_t vecs = align256((size_t)tiles->p_cells * sizeof(double)) +
-                            align256((size_t)(tiles->p_cells + plan->extra_cells) * sizeof(double));
+        Carve one;   // one slot and its class vectors (Pi, U)
+        slot_block(em, 1, tile_gather_parts((int)plan->ent_batch.size()), one);
+        one.part<double>(tiles->p_cells);
+        one.part<double>(tiles->p_cells + plan->extra_cells);
         size_t free_b = 0, total_b = 0;
         if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { cudaGetLastError(); free_b = 0; }
         em->n_slots = boot_slots(tiles->desc, em->n_rows, ctx->num_sms, tiles->ring_bytes,
-                                 tiles->p_cells, (double)(slot_block(em, 1, parts, nullptr) + vecs),
+                                 tiles->p_cells, (double)one.bytes(),
                                  (double)free_b);
     } else if (!streams) {
         em->form = EmForm::kGeneral;
@@ -513,50 +499,46 @@ static int em_pack_tiles(mxb_em *em, int want_slots, bool &built) {
     const int64_t n = em->n_rows, h = em->n_cols;
     const int nb = (int)ceil_div(n, kTileRows);
     const int hs = (int)round_up(h, 8);
-    const size_t b_map = align256((size_t)nb * hs * sizeof(unsigned short));
-    unsigned char *tmp = nullptr, *block = nullptr;
-    double *v = nullptr;
-    // scratch: [hash][rep][n_cls][bad]
-    const size_t b_hash = align256((size_t)nb * hs * sizeof(unsigned long long));
-    const size_t b_int = align256((size_t)nb * sizeof(int));
-    cudaError_t e = dev_alloc(ctx, (void **)&tmp, b_hash + b_map + 2 * b_int);
     const bool verbose = getenv("MXB_TIMING") != nullptr;
-    auto give_up = [&](bool hard, const char *what) {
-        if (verbose)
-            fprintf(stderr, "[mxb tiles] not used: %s (%s)\n", what, cudaGetErrorString(e));
-        if (e != cudaSuccess) cudaGetLastError();
-        dev_free(ctx, tmp);
-        dev_free(ctx, block);
-        dev_free(ctx, v);
-        if (hard) {
-            set_error("em_pack_tiles (%s): %s", what, cudaGetErrorString(e));
-            return e == cudaErrorMemoryAllocation ? MXB_ERR_NOMEM : MXB_ERR_CUDA;
-        }
+    auto give_up = [&](const char *what) {
+        if (verbose) fprintf(stderr, "[mxb tiles] not used: %s\n", what);
         return MXB_OK;
     };
-    if (e != cudaSuccess) return give_up(false, "scratch");
-    unsigned long long *hash = reinterpret_cast<unsigned long long *>(tmp);
-    unsigned short *rep = reinterpret_cast<unsigned short *>(tmp + b_hash);
-    int *d_ncls = reinterpret_cast<int *>(tmp + b_hash + b_map);
-    int *d_bad = reinterpret_cast<int *>(tmp + b_hash + b_map + b_int);
-    // persistent: [perm][cmap][desc]; the class vectors and the plan of the pass follow in a
-    // second block once the class counts are known
-    const size_t b_desc = align256((size_t)nb * sizeof(TileDesc));
-    const size_t b_cword = align256((size_t)nb * kTileThreads * sizeof(unsigned int));
-    const size_t head_bytes = 2 * b_map + b_cword + b_desc;
-    unsigned char *maps = nullptr;
-    e = dev_alloc(ctx, (void **)&maps, head_bytes);
-    if (e != cudaSuccess) return give_up(false, "maps");
-    block = maps;
-    unsigned short *perm = reinterpret_cast<unsigned short *>(maps);
-    unsigned short *cmap = reinterpret_cast<unsigned short *>(maps + b_map);
-    unsigned int *cword = reinterpret_cast<unsigned int *>(maps + 2 * b_map);
-    TileDesc *d_desc = reinterpret_cast<TileDesc *>(maps + 2 * b_map + b_cword);
+    auto fail = [&](const char *what, cudaError_t e) {
+        cudaGetLastError();
+        set_error("em_pack_tiles (%s): %s", what, cudaGetErrorString(e));
+        return e == cudaErrorMemoryAllocation ? MXB_ERR_NOMEM : MXB_ERR_CUDA;
+    };
+    // scratch: [hash][rep][n_cls][bad]
+    DevBlock scratch;
+    unsigned long long *hash = nullptr;
+    unsigned short *rep = nullptr;
+    int *d_ncls = nullptr, *d_bad = nullptr;
+    if (scratch.alloc_parts(ctx, __func__, [&](Carve &c) {
+            hash = c.part<unsigned long long>((size_t)nb * hs);
+            rep = c.part<unsigned short>((size_t)nb * hs);
+            d_ncls = c.part<int>(nb);
+            d_bad = c.part<int>(nb);
+        }) != MXB_OK)
+        return give_up("scratch");
+    // persistent: [perm][cmap][cword][desc]; the class vectors and the plan of the pass follow in
+    // a second block once the class counts are known
+    DevBlock maps;
+    unsigned short *perm = nullptr, *cmap = nullptr;
+    unsigned int *cword = nullptr;
+    TileDesc *d_desc = nullptr;
+    if (maps.alloc_parts(ctx, __func__, [&](Carve &c) {
+            perm = c.part<unsigned short>((size_t)nb * hs);
+            cmap = c.part<unsigned short>((size_t)nb * hs);
+            cword = c.part<unsigned int>((size_t)nb * kTileThreads);
+            d_desc = c.part<TileDesc>(nb);
+        }) != MXB_OK)
+        return give_up("maps");
 
     const int grid = std::min(nb, ctx->num_sms * 2);
     tile_hash_kernel<<<std::min(nb, ctx->num_sms * 4), kTileThreads, 0, ctx->stream>>>(
         em->mat->data, n, h, nb, hash, hs);
-    e = cudaGetLastError();
+    cudaError_t e = cudaGetLastError();
     if (e == cudaSuccess)
         e = pick_tile_class(h)(ctx, grid, hash, hs, (int)h, nb, perm, cword, cmap, rep, d_ncls);
     ctx->launches += 2;
@@ -565,12 +547,12 @@ static int em_pack_tiles(mxb_em *em, int want_slots, bool &built) {
         e = cudaMemcpyAsync(ncls.data(), d_ncls, (size_t)nb * sizeof(int), cudaMemcpyDeviceToHost,
                             ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) return give_up(true, "classes");
+    if (e != cudaSuccess) return fail("classes", e);
 
     // layout of the batches, ring geometry and plan of the pass (tile_plan.h)
     TileShape shape;
     tile_shape(ncls.data(), nb, n, shape);
-    if (!shape.ring_ok) return give_up(false, "rows too long for the ring");
+    if (!shape.ring_ok) return give_up("rows too long for the ring");
     const std::vector<TileDesc> &desc = shape.desc;
     const int64_t v_cells = shape.v_cells, p_cells = shape.p_cells;
     const uint32_t slot_bytes = shape.ring_bytes;
@@ -619,28 +601,28 @@ static int em_pack_tiles(mxb_em *em, int want_slots, bool &built) {
                 (double)v_cells * 8 / 1e9, tile_bytes / 1e9, fp64_bytes / 1e9, n_cta, n_seg, n_copy,
                 n_slots, slot_bytes);
     }
-    if (tile_bytes > 0.5 * fp64_bytes) return give_up(false, "not worth it");
+    if (tile_bytes > 0.5 * fp64_bytes) return give_up("not worth it");
 
-    e = dev_alloc(ctx, (void **)&v, (size_t)v_cells * sizeof(double));
-    unsigned char *vecs = nullptr;
-    const size_t b_pi = align256((size_t)p_cells * sizeof(double));
-    const size_t b_u = align256((size_t)u_cells * sizeof(double));
-    const size_t b_cta = align256((size_t)n_cta * sizeof(TileCta));
-    const size_t b_seg = align256((size_t)n_seg * sizeof(TileSeg));
-    const size_t b_entb = align256((size_t)n_ent * sizeof(int));
-    const size_t b_ento = align256((size_t)n_ent * sizeof(int64_t));
     // [Pi x n_rep][U x n_rep][plan]
-    const size_t b_vecs = (size_t)n_rep * (b_pi + b_u);
-    if (e == cudaSuccess)
-        e = dev_alloc(ctx, (void **)&vecs, b_vecs + b_cta + b_seg + b_entb + b_ento);
-    if (e != cudaSuccess) { dev_free(ctx, vecs); return give_up(false, "tiles"); }
-    double *pi_cls = reinterpret_cast<double *>(vecs);
-    double *u_sum = reinterpret_cast<double *>(vecs + (size_t)n_rep * b_pi);
-    unsigned char *tail = vecs + b_vecs;
-    TileCta *d_ctas = reinterpret_cast<TileCta *>(tail);
-    TileSeg *d_segs = reinterpret_cast<TileSeg *>(tail + b_cta);
-    int *d_entb = reinterpret_cast<int *>(tail + b_cta + b_seg);
-    int64_t *d_ento = reinterpret_cast<int64_t *>(tail + b_cta + b_seg + b_entb);
+    DevBlock v, vecs;
+    double *pi_cls = nullptr, *u_sum = nullptr;
+    TileCta *d_ctas = nullptr;
+    TileSeg *d_segs = nullptr;
+    int *d_entb = nullptr;
+    int64_t *d_ento = nullptr;
+    int64_t pi_stride = 0, u_stride = 0;
+    size_t b_vecs = 0;
+    if (v.alloc(ctx, (size_t)v_cells * sizeof(double), __func__) != MXB_OK ||
+        vecs.alloc_parts(ctx, __func__, [&](Carve &c) {
+            pi_cls = c.parts<double>(p_cells, n_rep, &pi_stride);
+            u_sum = c.parts<double>(u_cells, n_rep, &u_stride);
+            b_vecs = c.bytes();
+            d_ctas = c.part<TileCta>(n_cta);
+            d_segs = c.part<TileSeg>(n_seg);
+            d_entb = c.part<int>(n_ent);
+            d_ento = c.part<int64_t>(n_ent);
+        }) != MXB_OK)
+        return give_up("tiles");
     e = cudaMemcpyAsync(d_desc, desc.data(), (size_t)nb * sizeof(TileDesc), cudaMemcpyHostToDevice, ctx->stream);
     if (e == cudaSuccess)
         e = cudaMemcpyAsync(d_ctas, ctas.data(), (size_t)n_cta * sizeof(TileCta), cudaMemcpyHostToDevice, ctx->stream);
@@ -650,11 +632,12 @@ static int em_pack_tiles(mxb_em *em, int want_slots, bool &built) {
         e = cudaMemcpyAsync(d_entb, ent_batch.data(), (size_t)n_ent * sizeof(int), cudaMemcpyHostToDevice, ctx->stream);
     if (e == cudaSuccess)
         e = cudaMemcpyAsync(d_ento, ent_off.data(), (size_t)n_ent * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(vecs, 0, b_vecs, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(pi_cls, 0, b_vecs, ctx->stream);
     if (e == cudaSuccess) e = cudaMemsetAsync(d_bad, 0, (size_t)nb * sizeof(int), ctx->stream);
     if (e == cudaSuccess) {
         tile_fill_kernel<<<std::min(nb, ctx->num_sms * 4), kTileThreads, 0, ctx->stream>>>(
-            em->mat->data, h, d_desc, nb, cmap, rep, hs, (const double *)em->weights, v, d_bad);
+            em->mat->data, h, d_desc, nb, cmap, rep, hs, (const double *)em->weights,
+            v.get<double>(), d_bad);
         ctx->launches += 1;
         e = cudaGetLastError();
     }
@@ -663,17 +646,16 @@ static int em_pack_tiles(mxb_em *em, int want_slots, bool &built) {
         e = cudaMemcpyAsync(bad.data(), d_bad, (size_t)nb * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     if (e == cudaSuccess) e = em->boot ? tile_pass_attrs<true>(h) : tile_pass_attrs<false>(h);
-    if (e != cudaSuccess) { dev_free(ctx, vecs); return give_up(true, "fill"); }
-    bool any_bad = false;
-    for (int b = 0; b < nb; ++b) any_bad |= bad[(size_t)b] != 0;
-    if (any_bad) { dev_free(ctx, vecs); return give_up(false, "hash collision"); }
+    if (e != cudaSuccess) return fail("fill", e);
+    for (int b = 0; b < nb; ++b)
+        if (bad[(size_t)b] != 0) return give_up("hash collision");
 
-    dev_free(ctx, tmp);
     built = true;
     em->n_batches = nb;
     em->tile_hs = hs;
-    em->tile_block = maps;
-    em->tile_vecs = vecs;
+    em->tile_block = std::move(maps);
+    em->tile_vecs = std::move(vecs);
+    em->tile_v = std::move(v);
     em->tile_perm = perm;
     em->tile_cmap = cmap;
     em->tile_cword = cword;
@@ -687,12 +669,11 @@ static int em_pack_tiles(mxb_em *em, int want_slots, bool &built) {
     em->tile_n_slots = n_slots;
     em->tile_usum = u_sum;
     em->tile_pi = pi_cls;
-    em->tile_v = v;
     em->tile_cells = v_cells;
     em->tile_grid = n_cta;
     em->n_part = tile_gather_parts(n_ent);
-    em->tile_pi_stride = (int64_t)(b_pi / sizeof(double));
-    em->tile_u_stride = (int64_t)(b_u / sizeof(double));
+    em->tile_pi_stride = pi_stride;
+    em->tile_u_stride = u_stride;
     // what an iteration reads and writes: the tiles, perm + cmap (Pi), cmap (gather), the class
     // vectors (Pi written and read, U written and read)
     em->tile_bytes_per_pass = v_cells * 8 + 3 * (int64_t)nb * hs * 2 + 2 * (p_cells + u_cells) * 8;
@@ -707,7 +688,7 @@ static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weigh
     MXB_REQUIRE(weights != nullptr || m->n_rows == 0, "weights is NULL");
     *out = nullptr;
     MXB_CUDA(cudaSetDevice(ctx->device));
-    mxb_em *em = new (std::nothrow) mxb_em();
+    std::unique_ptr<mxb_em> em(new (std::nothrow) mxb_em());
     if (!em) { set_error("out of host memory"); return MXB_ERR_NOMEM; }
     em->ctx = ctx;
     em->mat = m;
@@ -740,80 +721,55 @@ static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weigh
         em->n_part = em->row_blocks;
     }
 
-    cudaError_t e = cudaSuccess;
-#define STEP(call) do { if (e == cudaSuccess) e = (call); } while (0)
-    // both blocks >= kCacheMinBlock: reused from the block cache, no cudaMalloc/cudaFree per session
-    {   // the session-wide buffers in one block, each 256-byte aligned: [weights][coef (general
-        // path)][tsum + underflow flag][props_in]
-        const size_t b_rows = align256((size_t)em->n_rows * sizeof(double));
-        const size_t b_tsum = align256(row_bytes + sizeof(double));
-        const size_t total = b_rows * (streams ? 1 : 2) + b_tsum +
-                             align256((size_t)em->n_cols * sizeof(double));
-        STEP(dev_alloc(ctx, (void **)&em->small, std::max(total, kCacheMinBlock)));
-        if (e == cudaSuccess) {
-            unsigned char *p = em->small;
-            em->weights = (double *)p; p += b_rows;
-            if (!streams) { em->coef = (double *)p; p += b_rows; }
-            em->tsum = (double *)p; p += b_tsum;
-            em->props_in = (double *)p;
-        }
-    }
-    for (int i = 0; i < 2; ++i)
-        STEP(cudaEventCreateWithFlags(&em->poll_ev[i], cudaEventDisableTiming));
-    if (e == cudaSuccess) {
-        static_assert(2 * kMaxSlots * sizeof(EmState) <= kPinnedScratchBytes, "pinned scratch");
-        em->host_state = (EmState *)pinned_scratch(ctx);
-        if (!em->host_state) e = cudaErrorMemoryAllocation;
+    // both blocks >= kCacheMinBlock: reused from the pool's cache, no cudaMalloc/cudaFree per session
+    const char *who = "mxb_em_create";
+    // the session-wide buffers in one block: [weights][coef (general path)][tsum + underflow
+    // flag][props_in]
+    MXB_TRY(em->small.alloc_parts(ctx, who, [&](Carve &c) {
+        em->weights = c.part<double>(em->n_rows);
+        if (!streams) em->coef = c.part<double>(em->n_rows);
+        em->tsum = c.part<double>(em->ld + 1);
+        em->props_in = c.part<double>(em->n_cols);
+    }, kCacheMinBlock));
+    MXB_TRY(em->poll_ev.create(2, cudaEventDisableTiming, who));
+    static_assert(2 * kMaxSlots * sizeof(EmState) <= kPinnedScratchBytes, "pinned scratch");
+    em->host_state = (EmState *)pinned_scratch(ctx);
+    if (!em->host_state) {
+        set_error("%s: cannot pin %zu bytes of host memory", who, kPinnedScratchBytes);
+        return MXB_ERR_NOMEM;
     }
     if (em->n_rows > 0)   // (tile_fill_kernel reads them)
-        STEP(cudaMemcpyAsync(em->weights, weights, em->n_rows * sizeof(double),
-                             cudaMemcpyHostToDevice, ctx->stream));
-    STEP(cudaStreamSynchronize(ctx->stream));
+        MXB_CUDA(cudaMemcpyAsync(em->weights, weights, em->n_rows * sizeof(double),
+                                 cudaMemcpyHostToDevice, ctx->stream));
+    MXB_CUDA(cudaStreamSynchronize(ctx->stream));
+    // class tiles straight from M; only a matrix that does not compress gets fp64 rows of L
     bool tiled = false;
-    if (e == cudaSuccess) {
-        // class tiles straight from M; only a matrix that does not compress gets fp64 rows of L
-        const int rc = em_pack_tiles(em, want_slots, tiled);
-        if (rc != MXB_OK) {
-            mxb_em_destroy(em);
-            return rc;
-        }
-    }
-    if (!tiled) decide_form(em, want_slots);
-    if (streams) STEP(cudaFuncSetAttribute((const void *)pick_pass(em->nc),
-                                           cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           (int)em->smem_bytes));
+    MXB_TRY(em_pack_tiles(em.get(), want_slots, tiled));
+    if (!tiled) decide_form(em.get(), want_slots);
+    if (streams)
+        MXB_CUDA(cudaFuncSetAttribute((const void *)pick_pass(em->nc),
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)em->smem_bytes));
     if (em->form == EmForm::kRowPairs)
-        STEP(cudaFuncSetAttribute((const void *)pick_pair(em->nc),
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)em->smem_bytes));
-    STEP(dev_alloc(ctx, (void **)&em->slots,
-                   std::max(slot_block(em, em->n_slots, em->n_part, nullptr), kCacheMinBlock)));
-    if (e == cudaSuccess) slot_block(em, em->n_slots, em->n_part, em->slots);
-    STEP(cudaMemsetAsync(em->state, 0, em->n_slots * sizeof(EmState), ctx->stream));
-    if (!tiled) STEP(dev_alloc(ctx, (void **)&em->lin, (size_t)em->n_rows * row_bytes));
-    if (e == cudaSuccess && em->n_rows > 0 && !tiled) {
-        const int grid = (int)std::min<int64_t>(em->n_rows, (int64_t)ctx->num_sms * 8);
-        to_linear_kernel<<<grid, 256, 0, ctx->stream>>>(m->data, em->n_rows, em->n_cols, em->ld,
-                                                        em->lin);
-        ctx->launches++;
-        STEP(cudaGetLastError());
-    }
-    STEP(cudaStreamSynchronize(ctx->stream));
-#undef STEP
-    if (e != cudaSuccess) {
-        set_error("mxb_em_create (%lld x %lld): %s", (long long)em->n_rows,
-                  (long long)em->n_cols, cudaGetErrorString(e));
-        mxb_em_destroy(em);
-        return e == cudaErrorMemoryAllocation ? MXB_ERR_NOMEM : MXB_ERR_CUDA;
-    }
-    // a sharded session starts from zeroed peer mailboxes on every rank (collective)
-    if (em->tail == EmTail::kPeer) {
-        const int rc = p2p_resync(ctx);
-        if (rc != MXB_OK) {
-            mxb_em_destroy(em);
-            return rc;
+        MXB_CUDA(cudaFuncSetAttribute((const void *)pick_pair(em->nc),
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)em->smem_bytes));
+    MXB_TRY(em->slots.alloc_parts(ctx, who, [&](Carve &c) {
+        slot_block(em.get(), em->n_slots, em->n_part, c);
+    }, kCacheMinBlock));
+    MXB_CUDA(cudaMemsetAsync(em->state, 0, em->n_slots * sizeof(EmState), ctx->stream));
+    if (!tiled) {
+        MXB_TRY(em->lin.alloc(ctx, (size_t)em->n_rows * row_bytes, who));
+        if (em->n_rows > 0) {
+            const int grid = (int)std::min<int64_t>(em->n_rows, (int64_t)ctx->num_sms * 8);
+            to_linear_kernel<<<grid, 256, 0, ctx->stream>>>(m->data, em->n_rows, em->n_cols, em->ld,
+                                                            em->lin.get<double>());
+            ctx->launches++;
+            MXB_CUDA(cudaGetLastError());
         }
     }
-    *out = em;
+    MXB_CUDA(cudaStreamSynchronize(ctx->stream));
+    // a sharded session starts from zeroed peer mailboxes on every rank (collective)
+    if (em->tail == EmTail::kPeer) MXB_TRY(p2p_resync(ctx));
+    *out = em.release();
     return MXB_OK;
 }
 
@@ -854,22 +810,17 @@ static int em_logspace_step(mxb_em *em, int cur, int slot, const double *weights
     const bool across = em->sharded && ctx->world > 1;
     const int64_t n_sums = across ? 2 * h : h;      // [s][m] or the plain column sums
     constexpr int kRowBlocks = 64;
-    const size_t b_lse = align256((size_t)n * sizeof(double));
-    const size_t b_col = align256((size_t)h * sizeof(double));
-    const size_t b_sum = align256((size_t)n_sums * sizeof(double));
-    const size_t b_part = align256((size_t)kRowBlocks * n_sums * sizeof(double));
-    unsigned char *tmp = nullptr;
-    if (dev_alloc(ctx, (void **)&tmp, b_lse + b_col + b_sum + b_part) != cudaSuccess) {
-        cudaGetLastError();
-        set_error("EM log-space step: out of device memory");
-        return MXB_ERR_NOMEM;
-    }
-    double *lse = (double *)tmp, *colmax = (double *)(tmp + b_lse);
-    double *colsum = (double *)(tmp + b_lse + b_col), *part = (double *)(tmp + b_lse + b_col + b_sum);
+    DevBlock tmp;
+    double *lse = nullptr, *colmax = nullptr, *colsum = nullptr, *part = nullptr;
+    MXB_TRY(tmp.alloc_parts(ctx, "EM log-space step", [&](Carve &c) {
+        lse = c.part<double>(n);
+        colmax = c.part<double>(h);
+        colsum = c.part<double>(n_sums);
+        part = c.part<double>((size_t)kRowBlocks * n_sums);
+    }));
     const double *lnp = em->lnp[cur] + slot * ld;
     const int col_blocks = (int)ceil_div(h, 256);
     const dim3 col_grid(col_blocks, kRowBlocks);
-    int rc = MXB_OK;
     if (n > 0) {   // a rank of a row-sharded run may hold no rows
         const int row_grid = (int)std::min<int64_t>(n, (int64_t)ctx->num_sms * 8);
         em_logspace_rows_kernel<<<row_grid, 256, 0, s>>>(em->mat->data, n, h, lnp, lse);
@@ -880,35 +831,25 @@ static int em_logspace_step(mxb_em *em, int cur, int slot, const double *weights
     em_logspace_colreduce_kernel<<<col_blocks, 256, 0, s>>>(part, kRowBlocks, h, 1, colmax);
     ctx->launches += 2;
     if (across) {
-        rc = nccl_allreduce_f64(ctx, colmax, h, 1);
-        if (rc == MXB_OK) {
-            em_logspace_cols_split_kernel<<<col_grid, 256, 0, s>>>(
-                em->mat->data, n, h, lnp, lse, weights, colmax, part);
-            em_logspace_colreduce_kernel<<<(int)ceil_div(n_sums, 256), 256, 0, s>>>(
-                part, kRowBlocks, n_sums, 0, colsum);
-            ctx->launches += 2;
-            rc = nccl_allreduce_sum_f64(ctx, colsum, n_sums);
-        }
+        MXB_TRY(nccl_allreduce_f64(ctx, colmax, h, 1));
+        em_logspace_cols_split_kernel<<<col_grid, 256, 0, s>>>(
+            em->mat->data, n, h, lnp, lse, weights, colmax, part);
+        em_logspace_colreduce_kernel<<<(int)ceil_div(n_sums, 256), 256, 0, s>>>(
+            part, kRowBlocks, n_sums, 0, colsum);
+        ctx->launches += 2;
+        MXB_TRY(nccl_allreduce_sum_f64(ctx, colsum, n_sums));
     } else {
         em_logspace_cols_kernel<<<col_grid, 256, 0, s>>>(em->mat->data, n, h, lnp, lse,
                                                          weights, colmax, part);
         em_logspace_colreduce_kernel<<<col_blocks, 256, 0, s>>>(part, kRowBlocks, h, 0, colsum);
         ctx->launches += 2;
     }
-    if (rc == MXB_OK) {
-        em_logspace_update_kernel<<<1, kUpdThreads, 0, s>>>(
-            colmax, colsum, across ? colsum + h : nullptr, h, ld, em->lnp[0] + slot * ld,
-            em->lnp[1] + slot * ld, em->pi[0] + slot * ld, em->pi[1] + slot * ld, em->state + slot);
-        ctx->launches += 1;
-    }
-    cudaError_t e = cudaGetLastError();
-    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-    dev_free(ctx, tmp);
-    if (rc != MXB_OK) return rc;
-    if (e != cudaSuccess) {
-        set_error("EM log-space step: %s", cudaGetErrorString(e));
-        return MXB_ERR_CUDA;
-    }
+    em_logspace_update_kernel<<<1, kUpdThreads, 0, s>>>(
+        colmax, colsum, across ? colsum + h : nullptr, h, ld, em->lnp[0] + slot * ld,
+        em->lnp[1] + slot * ld, em->pi[0] + slot * ld, em->pi[1] + slot * ld, em->state + slot);
+    ctx->launches += 1;
+    MXB_CUDA(cudaGetLastError());
+    MXB_CUDA(cudaStreamSynchronize(s));
     return MXB_OK;
 }
 
@@ -1072,20 +1013,15 @@ int mxb_em_iterate_fixed(mxb_em *em, int64_t n_iter, float *elapsed_ms, float *p
     MXB_CUDA(cudaSetDevice(ctx->device));
     em->zero_iter = false;
     MXB_TRY(reset_state(em, (long long)1 << 60, -1.0));
-    std::vector<cudaEvent_t> evs;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    MXB_CUDA(cudaEventCreate(&e0));
-    MXB_CUDA(cudaEventCreate(&e1));
-    if (pass_ms) {
-        evs.resize((size_t)n_iter * 2);
-        for (auto &e : evs) MXB_CUDA(cudaEventCreate(&e));
-    }
-    MXB_CUDA(cudaEventRecord(e0, ctx->stream));
+    // [start][end] of the run, then [begin][end] of every pass (pass_ms)
+    Events evs;
+    MXB_TRY(evs.create(2 + (pass_ms ? 2 * (size_t)n_iter : 0), cudaEventDefault, __func__));
+    MXB_CUDA(cudaEventRecord(evs[0], ctx->stream));
     for (int64_t i = 0; i < n_iter; ++i) {
-        if (pass_ms) MXB_TRY(enqueue_iteration(em, evs[2 * i], evs[2 * i + 1]));
+        if (pass_ms) MXB_TRY(enqueue_iteration(em, evs[2 + 2 * i], evs[3 + 2 * i]));
         else MXB_TRY(enqueue_iteration(em));
     }
-    MXB_CUDA(cudaEventRecord(e1, ctx->stream));
+    MXB_CUDA(cudaEventRecord(evs[1], ctx->stream));
     MXB_CUDA(cudaMemcpyAsync(&em->host_state[0], em->state, sizeof(EmState),
                              cudaMemcpyDeviceToHost, ctx->stream));
     MXB_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -1102,19 +1038,16 @@ int mxb_em_iterate_fixed(mxb_em *em, int64_t n_iter, float *elapsed_ms, float *p
                   (int)em->host_state[0].done);
         return MXB_ERR_RANGE;
     }
-    if (elapsed_ms) MXB_CUDA(cudaEventElapsedTime(elapsed_ms, e0, e1));
+    if (elapsed_ms) MXB_CUDA(cudaEventElapsedTime(elapsed_ms, evs[0], evs[1]));
     if (pass_ms) {
         double total = 0.0;
         for (int64_t i = 0; i < n_iter; ++i) {
             float ms = 0.f;
-            MXB_CUDA(cudaEventElapsedTime(&ms, evs[2 * i], evs[2 * i + 1]));
+            MXB_CUDA(cudaEventElapsedTime(&ms, evs[2 + 2 * i], evs[3 + 2 * i]));
             total += ms;
         }
         *pass_ms = (float)total;
-        for (auto &e : evs) cudaEventDestroy(e);
     }
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
     return MXB_OK;
 }
 
@@ -1167,10 +1100,10 @@ int mxb_em_profile(mxb_em *em, int64_t n_iter, float *ms_out) {
     MXB_CUDA(cudaSetDevice(ctx->device));
     em->zero_iter = false;
     MXB_TRY(reset_state(em, (long long)1 << 60, -1.0));
-    std::vector<cudaEvent_t> evs((size_t)n_iter * 5);
-    for (auto &e : evs) MXB_CUDA(cudaEventCreate(&e));
+    Events evs;
+    MXB_TRY(evs.create((size_t)n_iter * 5, cudaEventDefault, __func__));
     for (int64_t i = 0; i < n_iter; ++i) {
-        cudaEvent_t *e = &evs[(size_t)i * 5];
+        cudaEvent_t *e = evs.data() + (size_t)i * 5;
         MXB_TRY(enqueue_iteration(em, e[0], nullptr, e + 1));
         MXB_CUDA(cudaEventRecord(e[4], ctx->stream));
     }
@@ -1183,7 +1116,6 @@ int mxb_em_profile(mxb_em *em, int64_t n_iter, float *ms_out) {
             tot[k] += ms;
         }
     }
-    for (auto &e : evs) cudaEventDestroy(e);
     // fp64 rows: the three marks coincide after the pass, so [0] holds the pass
     if (em->form != EmForm::kTiles) { tot[1] = tot[0]; tot[0] = 0.0; }
     for (int k = 0; k < 4; ++k) ms_out[k] = (float)(tot[k] / (double)n_iter);
@@ -1240,26 +1172,21 @@ int mxb_matrix_fold_ranks(mxb_ctx *ctx, mxb_matrix *m, double sub_log) {
     const int64_t lo = m->n_rows * me / W, hi = m->n_rows * (me + 1) / W;
     const int64_t max_rows = ceil_div(m->n_rows, W);
     const int64_t slot = max_rows * m->n_cols;
-    double *recv = nullptr;
-    if (dev_alloc(ctx, (void **)&recv, (size_t)W * (size_t)slot * sizeof(double)) != cudaSuccess) {
-        cudaGetLastError();
-        set_error("mxb_matrix_fold_ranks: no memory for the %d receive slots", W);
-        return MXB_ERR_NOMEM;
-    }
-    int rc = nccl_alltoall_rows(ctx, m->data, recv, m->n_rows, m->n_cols, slot);
-    if (rc == MXB_OK && hi > lo) {
+    DevBlock recv_block;   // the W receive slots
+    MXB_TRY(recv_block.alloc(ctx, (size_t)W * (size_t)slot * sizeof(double), __func__));
+    double *recv = recv_block.get<double>();
+    MXB_TRY(nccl_alltoall_rows(ctx, m->data, recv, m->n_rows, m->n_cols, slot));
+    if (hi > lo) {
         const int64_t cells = (hi - lo) * m->n_cols;
         const int grid = (int)std::min<int64_t>(ceil_div(cells, 256), (int64_t)ctx->num_sms * 16);
         fold_shards_kernel<<<grid, 256, 0, s>>>(m->data + lo * m->n_cols, recv, slot, cells, W, me,
                                                  sub_log);
         ctx->launches++;
-        if (cudaGetLastError() != cudaSuccess) rc = MXB_ERR_CUDA;
+        MXB_CUDA(cudaGetLastError());
     }
-    if (rc == MXB_OK) rc = nccl_allgather_rows(ctx, m->data, m->n_rows, m->n_cols);
-    if (cudaStreamSynchronize(s) != cudaSuccess && rc == MXB_OK) rc = MXB_ERR_CUDA;
-    dev_free(ctx, recv);
-    if (rc == MXB_ERR_CUDA && mxb_last_error()[0] == 0) set_error("mxb_matrix_fold_ranks: CUDA failure");
-    return rc;
+    MXB_TRY(nccl_allgather_rows(ctx, m->data, m->n_rows, m->n_cols));
+    MXB_CUDA(cudaStreamSynchronize(s));
+    return MXB_OK;
 }
 
 }  // extern "C"
@@ -1283,12 +1210,9 @@ static int run_restarts(mxb_em *em, const double *init_lnprops, int32_t n_multi,
     // the last step n_multi x h]; the finals are read back in one copy at the end (no pinned
     // host buffer, no blocking copy mid-run)
     const size_t vec_bytes = (size_t)n_multi * h * sizeof(double);
-    double *d_inits = nullptr;
-    if (dev_alloc(ctx, (void **)&d_inits, 3 * vec_bytes) != cudaSuccess) {
-        set_error("run_em: device allocation of %zu bytes failed", 3 * vec_bytes);
-        cudaGetLastError();
-        return MXB_ERR_NOMEM;
-    }
+    DevBlock vecs;
+    MXB_TRY(vecs.alloc(ctx, 3 * vec_bytes, "run_em"));
+    double *d_inits = vecs.get<double>();
     double *d_fin = d_inits + (size_t)n_multi * h;
     double *d_prev = d_fin + (size_t)n_multi * h;
     std::vector<double> h_fin;
@@ -1297,11 +1221,10 @@ static int run_restarts(mxb_em *em, const double *init_lnprops, int32_t n_multi,
         h_fin.resize((size_t)n_multi * h);
         done_restart.assign((size_t)n_multi, 0);
     } catch (const std::bad_alloc &) {
-        dev_free(ctx, d_inits);
         set_error("run_em: out of host memory");
         return MXB_ERR_NOMEM;
     }
-    int rc = copy_h2d(ctx, d_inits, init_lnprops, vec_bytes);
+    MXB_TRY(copy_h2d(ctx, d_inits, init_lnprops, vec_bytes));
 
     int32_t next = 0, folded = 0;
     int slot_restart[kMaxSlots] = {-1, -1};
@@ -1335,39 +1258,33 @@ static int run_restarts(mxb_em *em, const double *init_lnprops, int32_t n_multi,
         tm.mark("read_mix kernel", kStageReadMix);
         return MXB_OK;
     };
-    if (rc == MXB_OK && max_iter <= 0) {
+    if (max_iter <= 0) {
         // em.py:126's loop body never runs: every restart hands back its init (em.py:141-143)
-        for (int32_t i = 0; i < n_multi && rc == MXB_OK; ++i)
-            rc = finish_restart(i, {d_inits + (size_t)i * h, d_inits + (size_t)i * h, 0, 0});
-    } else if (rc == MXB_OK) {
+        for (int32_t i = 0; i < n_multi; ++i)
+            MXB_TRY(finish_restart(i, {d_inits + (size_t)i * h, d_inits + (size_t)i * h, 0, 0}));
+    } else {
         int n_live = 0;
         for (; n_live < em->n_slots && n_live < n_multi; ++n_live) start_slot(n_live);
-        rc = em_poll_loop(em, max_iter, n_live, [&](int sl, const EmState &st, bool &again) -> int {
+        MXB_TRY(em_poll_loop(em, max_iter, n_live, [&](int sl, const EmState &st, bool &again) -> int {
             MXB_TRY(finish_restart(slot_restart[sl], slot_result(em, sl, st)));
             again = next < n_multi;
             if (again) start_slot(sl);
             return MXB_OK;
-        });
+        }));
     }
-    if (cudaStreamSynchronize(s) != cudaSuccess && rc == MXB_OK) {
-        set_error("run_em: stream sync failed: %s", cudaGetErrorString(cudaGetLastError()));
-        rc = MXB_ERR_CUDA;
-    }
+    MXB_CUDA(cudaStreamSynchronize(s));
     tm.mark("iterate", kStageIterate);
-    if (rc == MXB_OK) rc = copy_d2h(ctx, h_fin.data(), d_fin, vec_bytes);
-    if (rc == MXB_OK) {
-        for (int64_t j = 0; j < h; ++j) {
-            double v = h_fin[j];
-            for (int32_t i = 1; i < n_multi; ++i) v += h_fin[(size_t)i * h + j];  // em.py:155
-            if (!raw) {
-                if (n_multi > 1) v /= (double)n_multi;  // em.py:158-160
-                v = exp(v);                             // em.py:163
-            }
-            props_out[j] = v;
+    MXB_TRY(copy_d2h(ctx, h_fin.data(), d_fin, vec_bytes));
+    for (int64_t j = 0; j < h; ++j) {
+        double v = h_fin[j];
+        for (int32_t i = 1; i < n_multi; ++i) v += h_fin[(size_t)i * h + j];  // em.py:155
+        if (!raw) {
+            if (n_multi > 1) v /= (double)n_multi;  // em.py:158-160
+            v = exp(v);                             // em.py:163
         }
+        props_out[j] = v;
     }
-    dev_free(ctx, d_inits);
-    return rc;
+    return MXB_OK;
 }
 
 // Replicates whose results are kept on the device at a time: the output is downloaded in
@@ -1390,31 +1307,23 @@ static int run_bootstrap(mxb_em *em, const double *start, const int64_t *d_cumw,
     const size_t ns = (size_t)em->n_slots;
     const int64_t win = std::min(n_boot, kBootOutRows);
     // [counts n][start h][results win x h]
-    const size_t b_cnt = align256((size_t)n * sizeof(uint32_t));
-    const size_t b_start = align256((size_t)h * sizeof(double));
-    const size_t b_out = (size_t)win * h * sizeof(double);
-    unsigned char *work = nullptr;
-    if (dev_alloc(ctx, (void **)&work, b_cnt + b_start + b_out) != cudaSuccess) {
-        cudaGetLastError();
-        set_error("bootstrap: device allocation of %zu bytes failed", b_cnt + b_start + b_out);
-        return MXB_ERR_NOMEM;
-    }
-    uint32_t *counts = (uint32_t *)work;
-    double *d_start = (double *)(work + b_cnt);
-    double *d_out = (double *)(work + b_cnt + b_start);
-    int rc = MXB_OK;
-    if (cudaMemsetAsync(counts, 0, b_cnt, s) != cudaSuccess) {
-        set_error("bootstrap: %s", cudaGetErrorString(cudaGetLastError()));
-        rc = MXB_ERR_CUDA;
-    }
+    DevBlock work;
+    uint32_t *counts = nullptr;
+    double *d_start = nullptr, *d_out = nullptr;
+    MXB_TRY(work.alloc_parts(ctx, "bootstrap", [&](Carve &c) {
+        counts = c.part<uint32_t>(n);
+        d_start = c.part<double>(h);
+        d_out = c.part<double>((size_t)win * h);
+    }));
+    MXB_CUDA(cudaMemsetAsync(counts, 0, (size_t)n * sizeof(uint32_t), s));
     // slots that get no replicate (n_boot < n_slots) stay done: their CTAs exit at once
     std::vector<EmState> idle(ns);
     for (EmState &st : idle) {
         memset(&st, 0, sizeof(st));
         st.done = 1;
     }
-    if (rc == MXB_OK) rc = copy_h2d(ctx, em->state, idle.data(), ns * sizeof(EmState));
-    if (rc == MXB_OK) rc = copy_h2d(ctx, d_start, start, (size_t)h * sizeof(double));
+    MXB_TRY(copy_h2d(ctx, em->state, idle.data(), ns * sizeof(EmState)));
+    MXB_TRY(copy_h2d(ctx, d_start, start, (size_t)h * sizeof(double)));
 
     int64_t next = 0, w_end = 0;
     int64_t slot_rep[kMaxSlots] = {};
@@ -1432,28 +1341,25 @@ static int run_bootstrap(mxb_em *em, const double *start, const int64_t *d_cumw,
         MXB_CUDA(cudaGetLastError());
         return MXB_OK;
     };
-    for (int64_t w0 = 0; rc == MXB_OK && w0 < n_boot; w0 = w_end) {
+    for (int64_t w0 = 0; w0 < n_boot; w0 = w_end) {
         w_end = std::min(n_boot, w0 + win);
         int n_live = 0;
-        for (; rc == MXB_OK && n_live < em->n_slots && next < w_end; ++n_live) rc = start_slot(n_live);
-        if (rc == MXB_OK)
-            rc = em_poll_loop(em, max_iter, n_live, [&](int sl, const EmState &st, bool &again) -> int {
+        for (; n_live < em->n_slots && next < w_end; ++n_live) MXB_TRY(start_slot(n_live));
+        MXB_TRY(em_poll_loop(em, max_iter, n_live, [&](int sl, const EmState &st, bool &again) -> int {
                 const SlotResult res = slot_result(em, sl, st);
                 const int64_t k = slot_rep[sl];
                 iters_out[k] = res.iters;
                 converged_out[k] = res.converged;
                 MXB_CUDA(cudaMemcpyAsync(d_out + (size_t)(k - w0) * h, res.fin,
                                          h * sizeof(double), cudaMemcpyDeviceToDevice, s));
-                again = next < w_end;
-                if (again) MXB_TRY(start_slot(sl));
-                return MXB_OK;
-            });
-        if (rc == MXB_OK)
-            rc = copy_d2h(ctx, lnprops_out + (size_t)w0 * h, d_out,
-                          (size_t)(w_end - w0) * h * sizeof(double));
+            again = next < w_end;
+            if (again) MXB_TRY(start_slot(sl));
+            return MXB_OK;
+        }));
+        MXB_TRY(copy_d2h(ctx, lnprops_out + (size_t)w0 * h, d_out,
+                         (size_t)(w_end - w0) * h * sizeof(double)));
     }
-    dev_free(ctx, work);
-    return rc;
+    return MXB_OK;
 }
 
 }  // namespace mxb
@@ -1512,25 +1418,16 @@ int mxb_em_bootstrap(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
     MXB_CUDA(cudaSetDevice(ctx->device));
     mxb_em *em = nullptr;
     MXB_TRY(em_create_impl(ctx, m, weights, 0, 1, &em, true));
-    int64_t *d_cumw = nullptr;
-    int rc = MXB_OK;
-    if (dev_alloc(ctx, (void **)&d_cumw, (size_t)n * sizeof(int64_t)) != cudaSuccess) {
-        cudaGetLastError();
-        set_error("bootstrap: device allocation failed");
-        rc = MXB_ERR_NOMEM;
-    }
-    if (rc == MXB_OK) rc = copy_h2d(ctx, d_cumw, cumw.data(), (size_t)n * sizeof(int64_t));
-    if (rc == MXB_OK && slots_out) *slots_out = em->n_slots;
-    if (rc == MXB_OK)
-        rc = run_bootstrap(em, start_lnprops, d_cumw, total, seed, boot0, n_boot, max_iter, tol,
-                           lnprops_out, iters_out, converged_out);
-    if (cudaStreamSynchronize(ctx->stream) != cudaSuccess && rc == MXB_OK) {
-        set_error("bootstrap: %s", cudaGetErrorString(cudaGetLastError()));
-        rc = MXB_ERR_CUDA;
-    }
-    dev_free(ctx, d_cumw);
-    mxb_em_destroy(em);
-    return rc;
+    std::unique_ptr<mxb_em, decltype(&mxb_em_destroy)> session(em, mxb_em_destroy);
+    DevBlock cumw_block;
+    MXB_TRY(cumw_block.alloc(ctx, (size_t)n * sizeof(int64_t), "bootstrap"));
+    int64_t *d_cumw = cumw_block.get<int64_t>();
+    MXB_TRY(copy_h2d(ctx, d_cumw, cumw.data(), (size_t)n * sizeof(int64_t)));
+    if (slots_out) *slots_out = em->n_slots;
+    MXB_TRY(run_bootstrap(em, start_lnprops, d_cumw, total, seed, boot0, n_boot, max_iter, tol,
+                          lnprops_out, iters_out, converged_out));
+    MXB_CUDA(cudaStreamSynchronize(ctx->stream));
+    return MXB_OK;
 }
 
 int mxb_run_em_dev(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
