@@ -924,7 +924,7 @@ static int em_poll_loop(mxb_em *em, int64_t max_iter, int n_live, Finish finish)
                 return MXB_ERR_CUDA;
             }
             if (st.bad) {
-                set_error("EM: the mixture likelihood of %d row group(s) underflowed to 0 "
+                set_error("EM: the mixture likelihood of %d row group(s) fell below 2^-960 or was NaN "
                           "(proportions left the fp64 range)", st.bad);
                 return MXB_ERR_RANGE;
             }

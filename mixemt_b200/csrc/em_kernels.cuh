@@ -22,13 +22,24 @@ struct EmState {
     int done;            // 0 running, 1 converged, 2 max_iter reached, 3 peer time-out,
                          // 4 the current iteration must be redone in log space
     int cur;             // index of the current (input) proportions buffer
-    int bad;             // rows whose mixture likelihood underflowed to 0
+    int bad;             // rows that cannot be carried in linear space (row_needs_logspace)
     int pad;
     long long iters;
     long long max_iter;
     double tol;
     double delta;
 };
+
+// The one rule that sends a row to the log-space step (em_logspace_*): a row whose mixture
+// likelihood t = sum_j L_ij pi_j lies below kRowLikelihoodMin, or is NaN, cannot be carried in
+// linear space.  The coefficient w / t overflows to +inf once t < w / DBL_MAX, which covers
+// every subnormal t and, with large weights, normal t too; the column sums then hold inf * L
+// and inf * 0 and every proportion becomes NaN.  Above 2^-960 the coefficient is at most
+// w * 2^960 and a column sum at most W * 2^960 (L <= 1), finite for any total weight W < 2^63;
+// subnormal products L_ij pi_j change t by at most H * 2^-1075 = H * 2^-115 of t, below an ulp
+// for any H < 2^62.
+constexpr double kRowLikelihoodMin = 0x1p-960;
+__device__ __forceinline__ bool row_needs_logspace(double t) { return !(t >= kRowLikelihoodMin); }
 
 constexpr int kPassThreads = 512;
 constexpr int kPassWarps = kPassThreads / 32;
@@ -309,7 +320,7 @@ em_pass_fast_kernel(const unsigned char *__restrict__ rows, uint32_t row_bytes, 
         double coef_mine = 0.0;
         if (w_mine != 0.0) {
             coef_mine = w_mine / t;
-            bad |= (t == 0.0);
+            bad |= row_needs_logspace(t);
         }
         const double coef0 = __shfl_sync(0xffffffffu, coef_mine, 0);
         const double coef1 = __shfl_sync(0xffffffffu, coef_mine, 16);
@@ -461,7 +472,7 @@ em_pass_pair_kernel(const double *__restrict__ lin, int64_t ld, int64_t n_rows,
         double coef_mine = 0.0;
         if (w_mine != 0.0) {
             coef_mine = w_mine / t;
-            bad |= (t == 0.0 && !mine_done);
+            bad |= (row_needs_logspace(t) && !mine_done);
         }
         const double c0a = __shfl_sync(0xffffffffu, coef_mine, 0);
         const double c0b = __shfl_sync(0xffffffffu, coef_mine, 8);
@@ -542,7 +553,7 @@ em_rowdot_kernel(const double *__restrict__ lin, int64_t ld, int64_t n_rows,
         if (lane == 0) {
             const double w = weights[r];
             double c = 0.0;
-            if (w != 0.0) { c = w / dot; bad |= (dot == 0.0); }
+            if (w != 0.0) { c = w / dot; bad |= row_needs_logspace(dot); }
             coef[r] = c;
         }
     }
@@ -630,7 +641,7 @@ em_update_kernel(const double *__restrict__ tsum, int64_t n_cols, int64_t ld,
                  double *__restrict__ pi0, double *__restrict__ pi1,
                  EmState *__restrict__ st) {
     if (st->done) return;
-    if (tsum[ld] != 0.0) {       // a row's mixture likelihood underflowed (on some rank): see em_logspace_*
+    if (tsum[ld] != 0.0) {       // a row needs the log-space step (on some rank): see em_logspace_*
         if (threadIdx.x == 0) st->done = kDoneNeedsLogStep;
         return;
     }
@@ -743,7 +754,7 @@ em_finish_kernel(const double *partials, int n_part, int64_t n_cols, int64_t ld,
     }
     if (st->done) return;  // same answer in every CTA: the block below is the only writer
     if (!kP2P && st->bad) {
-        // A row's mixture likelihood underflowed in linear space: this iteration is redone in
+        // A row's mixture likelihood is too small for linear space: this iteration is redone in
         // log space by the host (em_logspace_* kernels), the queued launches become no-ops.
         // (st->bad was final before this launch began; the write below is seen by later
         // launches only.)  Row-sharded runs first tell the other ranks (kP2PBadBit below).
@@ -945,10 +956,11 @@ read_mix_kernel(const double *__restrict__ m, int64_t n_rows, int64_t n_cols,
 }
 
 // ---- one EM iteration in log space (rescue path) -------------------------------------
-// The linear-space pass needs s_i = sum_j L_ij pi_j > 0.  When every haplotype that still
-// has mass explains a row more than ~700 log units worse than the row's best one, s_i
-// underflows although the reference's log-space arithmetic (em.py:80-89, max-shifted
-// logsumexp) stays finite.  The iteration is then redone exactly as the reference states it:
+// The linear-space pass needs s_i = sum_j L_ij pi_j >= kRowLikelihoodMin = 2^-960 (about
+// e^-665; row_needs_logspace), or w_i / s_i may overflow.  When every haplotype that still has
+// mass explains a row more than ~665 log units worse than the row's best one, s_i falls below
+// that although the reference's log-space arithmetic (em.py:80-89, max-shifted logsumexp)
+// stays finite.  The iteration is then redone exactly as the reference states it:
 //   Z_ij = M_ij + ln pi_j - lse_i,  ln pi'_j = lse_i(Z_ij + ln w_i) - lse_j(...)
 // in three sweeps over M (row lse; column maxima; column sums).  Rare and slow by design.
 __global__ void __launch_bounds__(256)

@@ -575,7 +575,7 @@ tile_pass_kernel(const TileCta *__restrict__ ctas, const TileSeg *__restrict__ s
                     double coef = 0.0;
                     if (wr != 0.0) {
                         coef = wr / dot;
-                        bad |= (dot == 0.0);
+                        bad |= row_needs_logspace(dot);
                     }
 #pragma unroll
                     for (int k = 0; k < K; ++k) {

@@ -2,14 +2,15 @@
 test_logspace_rescue_gpu.py):
 
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 \
-        --master-addr 127.0.0.1 --master-port 29519 tests/logspace_shards_check.py
+        --master-addr 127.0.0.1 --master-port 29519 tests/logspace_shards_check.py [level]
 
 For fp64 rows and for class tiles, every rank runs run_em on its row shard of a matrix whose
 rows underflow in linear space at the first iteration; all ranks redo that iteration in log
 space together.  Proportions and iteration counts must equal the CPU oracle on the whole
 matrix, and all ranks must hand back the same bits.  A following run that never underflows
 must succeed too (the peer mailboxes are still in step).  Rank 0 reports the time of one
-rescued iteration next to one plain iteration of the same session.
+rescued iteration next to one plain iteration of the same session.  The optional argument is
+ln pi_0 of the underflowing start (default -760, exactly 0 in fp64; -730 makes t subnormal).
 """
 import ctypes
 import os
@@ -23,9 +24,9 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 
-def underflowing_case(layout):
+def underflowing_case(layout, level=-760.0):
     """Rows whose mass sits ~800 log units below their best haplotype, which starts with a
-    proportion of e^-760 (0 in fp64): s_i = sum_j L_ij pi_j underflows to 0."""
+    proportion of e^level (e^-760 is 0 in fp64): s_i = sum_j L_ij pi_j is about e^level."""
     rs = np.random.RandomState(5)
     if layout == "fp64":
         n, h = 300, 1100
@@ -37,7 +38,7 @@ def underflowing_case(layout):
     mat[: n // 4, 1:] -= 800.0
     wts = rs.randint(1, 5, size=n).astype(np.float64)
     bad = np.full(h, -np.log(h - 1.0))
-    bad[0] = -760.0
+    bad[0] = level
     good = np.full(h, -np.log(float(h)))
     return mat, wts, bad.reshape(1, h), good.reshape(1, h)
 
@@ -51,6 +52,7 @@ def main():
     from mixemt_b200.runtime import DeviceMatrix, get_context
     from oracle import oracle_c
 
+    level = float(sys.argv[1]) if len(sys.argv) > 1 else -760.0
     local = int(os.environ["LOCAL_RANK"])
     torch.cuda.set_device(local)
     dist.init_process_group("nccl", device_id=torch.device("cuda", local))
@@ -60,7 +62,7 @@ def main():
 
     report = []
     for layout in ("fp64", "tiles"):
-        mat, wts, bad, good = underflowing_case(layout)
+        mat, wts, bad, good = underflowing_case(layout, level)
         n, h = mat.shape
         lo, hi = sharding.row_shard(n, rank, world)
         shard = DeviceMatrix.from_host(ctx, mat[lo:hi])
@@ -113,8 +115,8 @@ def main():
     if rank == 0:
         how = "p2p" if lib.mxb_comm_p2p_enabled(ctx.handle) else "nccl"
         name = torch.cuda.get_device_name(local)
-        print("LOGSPACE_SHARDS_OK world=%d exchange=%s device=%s | %s"
-              % (world, how, name, " | ".join(report)))
+        print("LOGSPACE_SHARDS_OK world=%d exchange=%s level=%g device=%s | %s"
+              % (world, how, level, name, " | ".join(report)))
     dist.destroy_process_group()
 
 
