@@ -341,6 +341,27 @@ int mxb_em_bootstrap(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
 int mxb_boot_slots(const int32_t *n_cls, int64_t n_batches, int64_t n_rows, int32_t num_sms,
                    double bytes_per_slot, double free_bytes, int32_t *slots_out);
 
+/* ---- log-likelihood of a fit and constrained refits (no counterpart in the reference) ----
+ * out[k] = sum_i weights[i] * logsumexp_j(M_ij + lnprops[k][j]) for the n_vec log-proportion
+ * vectors lnprops (n_vec x H, host; not renormalised here).  -inf cells and -inf log-proportions
+ * add nothing, a row without a finite term gives -inf, a row of weight 0 adds exactly 0.  Up to
+ * 16 vectors share one read of m; a vector's result is the same bits whichever vectors share the
+ * call.  A row that would underflow in linear space (the EM's 2^-960 rule) is redone in log
+ * space.  MXB_ERR_VALUE for a NaN log-proportion.  On a row shard the result covers the shard's
+ * rows (the caller adds the ranks' values). */
+int mxb_matrix_loglik(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
+                      const double *lnprops, int64_t n_vec, double *out);
+/* n_starts refits of the same matrix and weights: row k of lnprops_out (n_starts x H) is the
+ * final log-proportions of one run_em restart from starts[k] (log-proportions, -inf for a zero,
+ * which stays zero), as mxb_run_em_dev with MXB_EM_RAW and n_multi 1 returns them, with
+ * iters_out[k] and converged_out[k]; max_iter <= 0 hands back the starts.  Over class tiles
+ * several refits iterate per launch (slots_out, nullable: how many; mxb_boot_slots' rule), over
+ * fp64 rows one at a time.  MXB_ERR_VALUE before any launch for a NaN in a start or a start
+ * whose proportions sum to 0. */
+int mxb_em_refit(mxb_ctx *ctx, const mxb_matrix *m, const double *weights, const double *starts,
+                 int64_t n_starts, int64_t max_iter, double tol, double *lnprops_out,
+                 int64_t *iters_out, int32_t *converged_out, int32_t *slots_out);
+
 #ifdef __cplusplus
 }
 #endif

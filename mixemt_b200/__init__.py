@@ -14,6 +14,7 @@ from . import _lib  # noqa: F401  (loads libmixemt_b200.so or raises)
 from . import consumers, em, preprocess, runtime  # noqa: F401
 from .em import run_em, em_step, init_props, converged  # noqa: F401
 from .bootstrap import bootstrap_props, BootstrapResult  # noqa: F401
+from .likelihood import log_likelihood, contributor_lrt, LRTResult  # noqa: F401
 from .preprocess import build_em_matrix, HapVarBaseMatrix  # noqa: F401
 
 __version__ = "0.1.0"

@@ -121,6 +121,9 @@ _PROTOS = {
                                         P, P, P, ctypes.POINTER(c_i32)]),
     "mxb_boot_slots": (ctypes.c_int, [P, c_i64, c_i64, c_i32, c_dbl, c_dbl,
                                       ctypes.POINTER(c_i32)]),
+    "mxb_matrix_loglik": (ctypes.c_int, [P, P, P, P, c_i64, P]),
+    "mxb_em_refit": (ctypes.c_int, [P, P, P, P, c_i64, c_i64, c_dbl, P, P, P,
+                                    ctypes.POINTER(c_i32)]),
 }
 
 EXPORTED_SYMBOLS = tuple(sorted(_PROTOS))

@@ -51,6 +51,16 @@ def _validate(weights, props, n_rows, n_cols, n_boot):
     total = w.sum()
     if not 1 <= total < 2.0 ** 32:
         raise ValueError("bootstrap weights must sum to at least 1 and less than 2^32")
+    start = start_from_props(props, n_cols)
+    if int(n_boot) < 1:
+        raise ValueError("n_boot must be at least 1")
+    return w, start
+
+
+def start_from_props(props, n_cols):
+    """The log-proportions a refit of the fit ``props`` starts from: ``log(props) -
+    log(sum(props))`` (-inf for a zero); ``ValueError`` for a wrong length, NaN or a sum that is
+    not positive."""
     p = numpy.asarray(props, dtype=numpy.float64).reshape(-1)
     if p.shape[0] != n_cols:
         raise ValueError("props has %d entries for %d haplogroups" % (p.shape[0], n_cols))
@@ -58,11 +68,9 @@ def _validate(weights, props, n_rows, n_cols, n_boot):
         raise ValueError("props holds NaN")
     if not p.sum() > 0:
         raise ValueError("props must have a positive sum")
-    if int(n_boot) < 1:
-        raise ValueError("n_boot must be at least 1")
     with numpy.errstate(divide="ignore"):
         start = numpy.log(p) - numpy.log(p.sum())
-    return w, numpy.ascontiguousarray(start)
+    return numpy.ascontiguousarray(start)
 
 
 def _run(dev, w, start, boot0, n_boot, seed, args):

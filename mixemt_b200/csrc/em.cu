@@ -78,7 +78,7 @@ struct mxb_em {
     EmForm form = EmForm::kGeneral;
     EmTail tail = EmTail::kSplit;
     // Restart slots: a batched session (run_em with n_multi > 1) iterates two restarts per read
-    // of L, a bootstrap session R replicates per iteration.  Slot s lives at lnp[b] + s*ld,
+    // of L, a slotted session R restarts per iteration.  Slot s lives at lnp[b] + s*ld,
     // pi[b] + s*ld, partials + s*n_part*ld, state + s (slot_block).
     int n_slots = 1;
     // streaming pass (n_stages > 0 when the rows fit its ring)
@@ -108,10 +108,11 @@ struct mxb_em {
     DevBlock small;   // one device block behind weights ... props_in (fewer driver calls)
     DevBlock slots;   // the slot block (slot_block)
     bool zero_iter = false;  // last iterate() ran no iteration
-    // Bootstrap session (run_bootstrap): n_slots replicates per launch, each with its own weight
-    // vector (slot_weights); over class tiles the slots' Pi and U vectors lie tile_pi_stride and
-    // tile_u_stride doubles apart.
-    bool boot = false;
+    // Slotted session (run_slots): n_slots restarts per launch, side by side over class tiles.
+    // A bootstrap session gives every slot its own weight vector (own_weights: slot_w, the
+    // resampled counts); the slots of a refit session share `weights`.  Over class tiles the
+    // slots' Pi and U vectors lie tile_pi_stride and tile_u_stride doubles apart.
+    bool slotted = false, own_weights = false;
     double *slot_w = nullptr;
     int64_t tile_pi_stride = 0, tile_u_stride = 0;
 };
@@ -171,7 +172,7 @@ static cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, siz
 
 // The weights slot `slot` iterates on: its resampled counts in a bootstrap session.
 static double *slot_weights(mxb_em *em, int slot) {
-    return em->boot ? em->slot_w + slot * em->n_rows : em->weights;
+    return em->own_weights ? em->slot_w + slot * em->n_rows : em->weights;
 }
 
 // The class-sum kernel of a tiled iteration for `per` = ceil(H / kTileThreads) columns a thread.
@@ -182,9 +183,10 @@ static auto pick_tile_pi(int64_t n_cols) {
            : per <= 12 ? tile_pi_kernel<12, kSlots> : tile_pi_kernel<16, kSlots>;
 }
 
-// The pass of a tiled iteration: class sums, pass and gather.  kSlots: the R replicate slots of
-// a bootstrap session side by side, the slot in blockIdx.y (z for the gather), all on one plan
-// of num_sms / R CTAs; a slot whose control block says done costs nothing.
+// The pass of a tiled iteration: class sums, pass and gather.  kSlots: the R slots of a slotted
+// session side by side (weights n_rows apart, or shared), the slot in blockIdx.y (z for the
+// gather), all on one plan of num_sms / R CTAs; a slot whose control block says done costs
+// nothing.
 template <bool kSlots>
 static int enqueue_tile_pass(mxb_em *em, unsigned R, cudaEvent_t *marks) {
     mxb_ctx *ctx = em->ctx;
@@ -206,7 +208,7 @@ static int enqueue_tile_pass(mxb_em *em, unsigned R, cudaEvent_t *marks) {
                         (const double *)em->tile_pi, em->state, em->tile_usum,
                         em->tile_slot_bytes, em->tile_n_slots,
                         (const double *)(kSlots ? slot_weights(em, 0) : nullptr),
-                        kSlots ? em->n_rows : (int64_t)0, pi_stride, u_stride));
+                        em->own_weights ? em->n_rows : (int64_t)0, pi_stride, u_stride));
     if (marks) MXB_CUDA(cudaEventRecord(marks[1], s));
     // The gather waits in plain stream order: launched early it would sit on the SMs the
     // first CTAs of the pass leave and keep them from nothing, but measured it costs 27 us
@@ -279,12 +281,12 @@ static int enqueue_iteration(mxb_em *em, cudaEvent_t pass_begin = nullptr,
     mxb_ctx *ctx = em->ctx;
     cudaStream_t s = ctx->stream;
     const unsigned R = (unsigned)em->n_slots;
-    // fp64 rows of a bootstrap session: one replicate at a time, with the slot's weights
+    // fp64 rows of a slotted session: one restart at a time, with the slot's weights
     const double *weights = slot_weights(em, 0);
     if (pass_begin) MXB_CUDA(cudaEventRecord(pass_begin, s));
     switch (em->form) {
     case EmForm::kTiles:
-        MXB_TRY(em->boot ? enqueue_tile_pass<true>(em, R, marks)
+        MXB_TRY(em->slotted ? enqueue_tile_pass<true>(em, R, marks)
                          : enqueue_tile_pass<false>(em, R, marks));
         break;
     case EmForm::kRowPairs:
@@ -381,12 +383,12 @@ __global__ void em_reset_state_kernel(EmState *st, long long max_iter, double to
     st->delta = 0.0;
 }
 
-// The slot block of a session with R slots: [slot weights (bootstrap sessions) R x n_rows]
+// The slot block of a session with R slots: [slot weights (own_weights) R x n_rows]
 // [lnp 2 x R x ld][pi 2 x R x ld][partials R x n_part x ld][control blocks R], laid out on `c`
 // and the session's slot buffers pointed into it; R = 1 gives the bytes of one slot.
 static void slot_block(mxb_em *em, int R, int n_part, Carve &c) {
     const size_t ns = (size_t)R, ld = (size_t)em->ld;
-    if (em->boot) em->slot_w = c.part<double>(ns * em->n_rows);
+    if (em->own_weights) em->slot_w = c.part<double>(ns * em->n_rows);
     for (double *&p : em->lnp) p = c.part<double>(ns * ld);
     for (double *&p : em->pi) p = c.part<double>(ns * ld);
     em->partials = c.part<double>(ns * n_part * ld);
@@ -439,7 +441,7 @@ static void decide_form(mxb_em *em, int want_slots, const TileShape *tiles = nul
     em->n_slots = 1;
     if (tiles) {
         em->form = EmForm::kTiles;   // restarts run one at a time over the tiles
-        if (!em->boot) return;
+        if (!em->slotted) return;
         // the slotted tile kernels exist for the fused tail only
         em->tail = EmTail::kFused;
         if (!fused) return;
@@ -560,7 +562,7 @@ static int em_pack_tiles(mxb_em *em, int want_slots, bool &built) {
     TilePlanOut plan;
     tile_plan(desc, n, ctx->num_sms, slot_bytes, p_cells, plan);
     decide_form(em, want_slots, &shape, &plan);
-    const int n_rep = em->n_slots;   // replicate slots of a bootstrap session
+    const int n_rep = em->n_slots;   // the slots of a slotted session
     if (n_rep > 1) {
         plan = TilePlanOut();
         tile_plan(desc, n, ctx->num_sms / n_rep, slot_bytes, p_cells, plan);
@@ -645,7 +647,7 @@ static int em_pack_tiles(mxb_em *em, int want_slots, bool &built) {
     if (e == cudaSuccess)
         e = cudaMemcpyAsync(bad.data(), d_bad, (size_t)nb * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e == cudaSuccess) e = em->boot ? tile_pass_attrs<true>(h) : tile_pass_attrs<false>(h);
+    if (e == cudaSuccess) e = em->slotted ? tile_pass_attrs<true>(h) : tile_pass_attrs<false>(h);
     if (e != cudaSuccess) return fail("fill", e);
     for (int b = 0; b < nb; ++b)
         if (bad[(size_t)b] != 0) return give_up("hash collision");
@@ -681,7 +683,8 @@ static int em_pack_tiles(mxb_em *em, int want_slots, bool &built) {
 }
 
 static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weights, int sharded,
-                          int want_slots, mxb_em **out, bool boot = false) {
+                          int want_slots, mxb_em **out, bool slotted = false,
+                          bool own_weights = false) {
     MXB_REQUIRE(ctx != nullptr && m != nullptr && out != nullptr, "NULL argument");
     // a rank of a row-sharded run may hold no rows at all (fewer signatures than GPUs)
     MXB_REQUIRE((m->n_rows > 0 || sharded) && m->n_cols > 0, "EM needs a non-empty matrix");
@@ -696,7 +699,8 @@ static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weigh
     em->n_cols = m->n_cols;
     em->ld = round_up(m->n_cols, kLdAlign);
     em->sharded = sharded != 0;
-    em->boot = boot;
+    em->slotted = slotted;
+    em->own_weights = own_weights;
 
     // launch geometry
     const size_t row_bytes = (size_t)em->ld * sizeof(double);
@@ -1287,67 +1291,59 @@ static int run_restarts(mxb_em *em, const double *init_lnprops, int32_t n_multi,
     return MXB_OK;
 }
 
-// Replicates whose results are kept on the device at a time: the output is downloaded in
-// windows of this many rows (at most 177 MB at H = 5408), whatever n_boot is.
+// Tasks whose results are kept on the device at a time: the output is downloaded in windows of
+// this many rows (at most 177 MB at H = 5408), whatever the number of tasks.
 constexpr int64_t kBootOutRows = 4096;
 
-// The bootstrap (bootstrap.cu for the draw): replicates boot0 .. boot0 + n_boot - 1 are put on
-// the session's slots in order, each resampled on the device when its slot is handed it, started
-// from `start` and iterated by em_poll_loop as one restart of run_em on its counts; a finished
-// slot's final log-proportions go to row b - boot0 of the output and the slot takes the next
-// replicate of the window.  Over class tiles the slots iterate side by side
-// (enqueue_tile_pass<true>), over fp64 rows one at a time.
-static int run_bootstrap(mxb_em *em, const double *start, const int64_t *d_cumw, uint64_t total,
-                         uint64_t seed, int64_t boot0, int64_t n_boot, int64_t max_iter,
-                         double tol, double *lnprops_out, int64_t *iters_out,
-                         int32_t *converged_out) {
+// The driver of a slotted session (bootstrap replicates, constrained refits): tasks
+// 0 .. n_tasks - 1 are put on the session's slots in order.  When a slot is handed task k,
+// set_up(slot, k, start) does what the task needs first and names the device log-proportions it
+// starts from; the slot then runs one run_em restart from there under em_poll_loop.  A finished
+// slot's final log-proportions go to row k of the output and the slot takes the next task of the
+// window.  Over class tiles the slots iterate side by side (enqueue_tile_pass<true>), over fp64
+// rows one at a time.
+template <typename SetUp>
+static int run_slots(mxb_em *em, int64_t n_tasks, int64_t max_iter, double tol,
+                     double *lnprops_out, int64_t *iters_out, int32_t *converged_out,
+                     SetUp set_up) {
     mxb_ctx *ctx = em->ctx;
     cudaStream_t s = ctx->stream;
-    const int64_t n = em->n_rows, h = em->n_cols, ld = em->ld;
+    const int64_t h = em->n_cols, ld = em->ld;
     const size_t ns = (size_t)em->n_slots;
-    const int64_t win = std::min(n_boot, kBootOutRows);
-    // [counts n][start h][results win x h]
-    DevBlock work;
-    uint32_t *counts = nullptr;
-    double *d_start = nullptr, *d_out = nullptr;
-    MXB_TRY(work.alloc_parts(ctx, "bootstrap", [&](Carve &c) {
-        counts = c.part<uint32_t>(n);
-        d_start = c.part<double>(h);
-        d_out = c.part<double>((size_t)win * h);
-    }));
-    MXB_CUDA(cudaMemsetAsync(counts, 0, (size_t)n * sizeof(uint32_t), s));
-    // slots that get no replicate (n_boot < n_slots) stay done: their CTAs exit at once
+    const int64_t win = std::min(n_tasks, kBootOutRows);
+    DevBlock out_block;   // [results win x h]
+    MXB_TRY(out_block.alloc(ctx, (size_t)win * h * sizeof(double), "slotted EM"));
+    double *d_out = out_block.get<double>();
+    // slots that get no task (n_tasks < n_slots) stay done: their CTAs exit at once
     std::vector<EmState> idle(ns);
     for (EmState &st : idle) {
         memset(&st, 0, sizeof(st));
         st.done = 1;
     }
     MXB_TRY(copy_h2d(ctx, em->state, idle.data(), ns * sizeof(EmState)));
-    MXB_TRY(copy_h2d(ctx, d_start, start, (size_t)h * sizeof(double)));
 
     int64_t next = 0, w_end = 0;
-    int64_t slot_rep[kMaxSlots] = {};
+    int64_t slot_task[kMaxSlots] = {};
     auto start_slot = [&](int sl) -> int {
         const int64_t k = next++;
-        slot_rep[sl] = k;
-        double *w = slot_weights(em, sl);
-        MXB_TRY(boot_draw(ctx, d_cumw, n, total, seed, boot0 + k, 1, counts));
-        MXB_TRY(boot_take_counts(ctx, counts, n, w));
+        slot_task[sl] = k;
+        const double *start = nullptr;
+        MXB_TRY(set_up(sl, k, start));
         em_set_props_kernel<<<(int)ceil_div(ld, 256), 256, 0, s>>>(
-            d_start, h, ld, em->lnp[0] + sl * ld, em->pi[0] + sl * ld, em->lnp[1] + sl * ld,
+            start, h, ld, em->lnp[0] + sl * ld, em->pi[0] + sl * ld, em->lnp[1] + sl * ld,
             em->pi[1] + sl * ld);
         em_reset_state_kernel<<<1, 1, 0, s>>>(em->state + sl, (long long)max_iter, tol);
         ctx->launches += 2;
         MXB_CUDA(cudaGetLastError());
         return MXB_OK;
     };
-    for (int64_t w0 = 0; w0 < n_boot; w0 = w_end) {
-        w_end = std::min(n_boot, w0 + win);
+    for (int64_t w0 = 0; w0 < n_tasks; w0 = w_end) {
+        w_end = std::min(n_tasks, w0 + win);
         int n_live = 0;
         for (; n_live < em->n_slots && next < w_end; ++n_live) MXB_TRY(start_slot(n_live));
         MXB_TRY(em_poll_loop(em, max_iter, n_live, [&](int sl, const EmState &st, bool &again) -> int {
                 const SlotResult res = slot_result(em, sl, st);
-                const int64_t k = slot_rep[sl];
+                const int64_t k = slot_task[sl];
                 iters_out[k] = res.iters;
                 converged_out[k] = res.converged;
                 MXB_CUDA(cudaMemcpyAsync(d_out + (size_t)(k - w0) * h, res.fin,
@@ -1358,6 +1354,53 @@ static int run_bootstrap(mxb_em *em, const double *start, const int64_t *d_cumw,
         }));
         MXB_TRY(copy_d2h(ctx, lnprops_out + (size_t)w0 * h, d_out,
                          (size_t)(w_end - w0) * h * sizeof(double)));
+    }
+    return MXB_OK;
+}
+
+// The bootstrap (bootstrap.cu for the draw): task k is replicate boot0 + k, resampled on the
+// device into its slot's weights when the slot is handed it and started from `start`.
+static int run_bootstrap(mxb_em *em, const double *start, const int64_t *d_cumw, uint64_t total,
+                         uint64_t seed, int64_t boot0, int64_t n_boot, int64_t max_iter,
+                         double tol, double *lnprops_out, int64_t *iters_out,
+                         int32_t *converged_out) {
+    mxb_ctx *ctx = em->ctx;
+    const int64_t n = em->n_rows, h = em->n_cols;
+    DevBlock work;   // [counts n][start h]
+    uint32_t *counts = nullptr;
+    double *d_start = nullptr;
+    MXB_TRY(work.alloc_parts(ctx, "bootstrap", [&](Carve &c) {
+        counts = c.part<uint32_t>(n);
+        d_start = c.part<double>(h);
+    }));
+    MXB_CUDA(cudaMemsetAsync(counts, 0, (size_t)n * sizeof(uint32_t), ctx->stream));
+    MXB_TRY(copy_h2d(ctx, d_start, start, (size_t)h * sizeof(double)));
+    return run_slots(em, n_boot, max_iter, tol, lnprops_out, iters_out, converged_out,
+                     [&](int sl, int64_t k, const double *&from) -> int {
+        MXB_TRY(boot_draw(ctx, d_cumw, n, total, seed, boot0 + k, 1, counts));
+        MXB_TRY(boot_take_counts(ctx, counts, n, slot_weights(em, sl)));
+        from = d_start;
+        return MXB_OK;
+    });
+}
+
+// Start log-proportions (K x H, host): no NaN, and proportions that sum to more than 0; an error
+// names the entry point `who` and the vector.
+static int check_starts(const char *who, const double *starts, int64_t n_vec, int64_t h) {
+    for (int64_t k = 0; k < n_vec; ++k) {
+        double mass = 0.0;
+        for (int64_t j = 0; j < h; ++j) {
+            if (isnan(starts[k * h + j])) {
+                set_error("%s: start log-proportion %lld of vector %lld is NaN", who,
+                          (long long)j, (long long)k);
+                return MXB_ERR_VALUE;
+            }
+            mass += exp(starts[k * h + j]);
+        }
+        if (!(mass > 0.0)) {
+            set_error("%s: the start proportions of vector %lld sum to 0", who, (long long)k);
+            return MXB_ERR_VALUE;
+        }
     }
     return MXB_OK;
 }
@@ -1390,18 +1433,7 @@ int mxb_em_bootstrap(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
         set_error("bootstrap: need n_boot >= 1 and replicate numbers in [0, 2^32)");
         return MXB_ERR_VALUE;
     }
-    double mass = 0.0;
-    for (int64_t j = 0; j < h; ++j) {
-        if (isnan(start_lnprops[j])) {
-            set_error("bootstrap: start log-proportion %lld is NaN", (long long)j);
-            return MXB_ERR_VALUE;
-        }
-        mass += exp(start_lnprops[j]);
-    }
-    if (!(mass > 0.0)) {
-        set_error("bootstrap: the start proportions sum to 0");
-        return MXB_ERR_VALUE;
-    }
+    MXB_TRY(check_starts("bootstrap", start_lnprops, 1, h));
     std::vector<int64_t> cumw;
     uint64_t total = 0;
     MXB_TRY(boot_prefix(weights, n, cumw, total));
@@ -1417,7 +1449,7 @@ int mxb_em_bootstrap(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
     }
     MXB_CUDA(cudaSetDevice(ctx->device));
     mxb_em *em = nullptr;
-    MXB_TRY(em_create_impl(ctx, m, weights, 0, 1, &em, true));
+    MXB_TRY(em_create_impl(ctx, m, weights, 0, 1, &em, true, true));
     std::unique_ptr<mxb_em, decltype(&mxb_em_destroy)> session(em, mxb_em_destroy);
     DevBlock cumw_block;
     MXB_TRY(cumw_block.alloc(ctx, (size_t)n * sizeof(int64_t), "bootstrap"));
@@ -1426,6 +1458,44 @@ int mxb_em_bootstrap(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
     if (slots_out) *slots_out = em->n_slots;
     MXB_TRY(run_bootstrap(em, start_lnprops, d_cumw, total, seed, boot0, n_boot, max_iter, tol,
                           lnprops_out, iters_out, converged_out));
+    MXB_CUDA(cudaStreamSynchronize(ctx->stream));
+    return MXB_OK;
+}
+
+int mxb_em_refit(mxb_ctx *ctx, const mxb_matrix *m, const double *weights, const double *starts,
+                 int64_t n_starts, int64_t max_iter, double tol, double *lnprops_out,
+                 int64_t *iters_out, int32_t *converged_out, int32_t *slots_out) {
+    MXB_REQUIRE(ctx != nullptr && m != nullptr && weights != nullptr && starts != nullptr,
+                "NULL argument");
+    MXB_REQUIRE(lnprops_out != nullptr && iters_out != nullptr && converged_out != nullptr,
+                "NULL buffer");
+    MXB_REQUIRE(n_starts >= 1, "need at least one start");
+    const int64_t h = m->n_cols;
+    MXB_TRY(check_starts("refit", starts, n_starts, h));
+    if (slots_out) *slots_out = 1;
+    if (max_iter <= 0) {
+        // em.py:126's loop body never runs: every refit hands back its start (em.py:141-143)
+        memcpy(lnprops_out, starts, (size_t)(n_starts * h) * sizeof(double));
+        for (int64_t k = 0; k < n_starts; ++k) {
+            iters_out[k] = 0;
+            converged_out[k] = 0;
+        }
+        return MXB_OK;
+    }
+    MXB_CUDA(cudaSetDevice(ctx->device));
+    mxb_em *em = nullptr;
+    MXB_TRY(em_create_impl(ctx, m, weights, 0, 1, &em, true, false));
+    std::unique_ptr<mxb_em, decltype(&mxb_em_destroy)> session(em, mxb_em_destroy);
+    DevBlock starts_block;
+    MXB_TRY(starts_block.alloc(ctx, (size_t)(n_starts * h) * sizeof(double), "refit"));
+    const double *d_starts = starts_block.get<double>();
+    MXB_TRY(copy_h2d(ctx, starts_block.get(), starts, (size_t)(n_starts * h) * sizeof(double)));
+    if (slots_out) *slots_out = em->n_slots;
+    MXB_TRY(run_slots(em, n_starts, max_iter, tol, lnprops_out, iters_out, converged_out,
+                      [&](int, int64_t k, const double *&from) -> int {
+        from = d_starts + k * h;
+        return MXB_OK;
+    }));
     MXB_CUDA(cudaStreamSynchronize(ctx->stream));
     return MXB_OK;
 }

@@ -5,6 +5,8 @@
 #include <cooperative_groups.h>
 
 #include "common.cuh"
+#include "block_reduce.cuh"
+#include "row_likelihood.cuh"
 #define MXB_DYN_SHARED extern __shared__
 
 #include <math.h>
@@ -29,17 +31,6 @@ struct EmState {
     double tol;
     double delta;
 };
-
-// The one rule that sends a row to the log-space step (em_logspace_*): a row whose mixture
-// likelihood t = sum_j L_ij pi_j lies below kRowLikelihoodMin, or is NaN, cannot be carried in
-// linear space.  The coefficient w / t overflows to +inf once t < w / DBL_MAX, which covers
-// every subnormal t and, with large weights, normal t too; the column sums then hold inf * L
-// and inf * 0 and every proportion becomes NaN.  Above 2^-960 the coefficient is at most
-// w * 2^960 and a column sum at most W * 2^960 (L <= 1), finite for any total weight W < 2^63;
-// subnormal products L_ij pi_j change t by at most H * 2^-1075 = H * 2^-115 of t, below an ulp
-// for any H < 2^62.
-constexpr double kRowLikelihoodMin = 0x1p-960;
-__device__ __forceinline__ bool row_needs_logspace(double t) { return !(t >= kRowLikelihoodMin); }
 
 constexpr int kPassThreads = 512;
 constexpr int kPassWarps = kPassThreads / 32;
@@ -124,43 +115,6 @@ __device__ __forceinline__ double2 lds_v2_f64(uint32_t addr) {
     double2 v;
     asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(addr) : "memory");
     return v;
-}
-
-__device__ __forceinline__ double warp_sum(double v) {
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
-    return v;
-}
-__device__ __forceinline__ double warp_max(double v) {
-#pragma unroll
-    for (int off = 16; off > 0; off >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, off));
-    return v;
-}
-
-// Block-wide deterministic reductions (every thread gets the result).
-template <int kThreads>
-__device__ __forceinline__ double block_sum(double v, double *scratch /*[kThreads/32]*/) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    v = warp_sum(v);
-    __syncthreads();  // scratch free
-    if (lane == 0) scratch[warp] = v;
-    __syncthreads();
-    double t = 0.0;
-#pragma unroll
-    for (int i = 0; i < kThreads / 32; ++i) t += scratch[i];
-    return t;
-}
-template <int kThreads>
-__device__ __forceinline__ double block_max(double v, double *scratch) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    v = warp_max(v);
-    __syncthreads();
-    if (lane == 0) scratch[warp] = v;
-    __syncthreads();
-    double t = scratch[0];
-#pragma unroll
-    for (int i = 1; i < kThreads / 32; ++i) t = fmax(t, scratch[i]);
-    return t;
 }
 
 // ---- M -> L ------------------------------------------------------------------

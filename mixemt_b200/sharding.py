@@ -179,3 +179,15 @@ def merge_bootstrap(lnprops, iters, conv, boot0, n_boot, allreduce):
     assert np.abs(buf[:, h]).max(initial=0) < _EXACT, "iteration counts not exact in fp64"
     buf = allreduce(np.ascontiguousarray(buf), "sum")
     return buf[:, :h], buf[:, h].astype(np.int64), buf[:, h + 1].astype(np.int32)
+
+
+def sum_ranks(values, allreduce, ok=True):
+    """The ranks' vectors of per-shard sums (a row-sharded log-likelihood) added up: one sum
+    all-reduce that carries the ok flag; every rank gets the same total."""
+    values = np.asarray(values, dtype=np.float64).reshape(-1)
+    vec = np.empty(values.size + 1)
+    vec[:-1] = values
+    vec[-1] = _fail_flag(ok)
+    vec = allreduce(vec, "sum")
+    _raise_if_failed(vec[-1])
+    return vec[:-1].copy()
