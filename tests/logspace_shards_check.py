@@ -24,9 +24,10 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 
-def underflowing_case(layout, level=-760.0):
+def underflowing_case(layout, level=-760.0, bad_rows=None):
     """Rows whose mass sits ~800 log units below their best haplotype, which starts with a
-    proportion of e^level (e^-760 is 0 in fp64): s_i = sum_j L_ij pi_j is about e^level."""
+    proportion of e^level (e^-760 is 0 in fp64): s_i = sum_j L_ij pi_j is about e^level.
+    bad_rows(n) gives those rows (default the first quarter)."""
     rs = np.random.RandomState(5)
     if layout == "fp64":
         n, h = 300, 1100
@@ -35,7 +36,7 @@ def underflowing_case(layout, level=-760.0):
         n, h = 1280, 5408
         mat = np.repeat(-rs.gamma(2.0, 3.0, size=(n, h // 64 + 1)), 64, axis=1)[:, :h].copy()
     mat[:, 0] = 0.0
-    mat[: n // 4, 1:] -= 800.0
+    mat[slice(0, n // 4) if bad_rows is None else bad_rows(n), 1:] -= 800.0
     wts = rs.randint(1, 5, size=n).astype(np.float64)
     bad = np.full(h, -np.log(h - 1.0))
     bad[0] = level

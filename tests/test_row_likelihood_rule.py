@@ -11,7 +11,7 @@ from tile_cases import ld_iterate
 from window_cases import (LEVELS, LN_THETA, MODES, SCALES, THETA, model_iterate, rule_new,
                           rule_old, window_case)
 
-LN_TOL = 1e-12       # test_tile_kernels_gpu.LN_TOL
+LN_TOL = 1e-12       # rank_cases.LN_TOL
 K = 3
 
 _TRAJ = {}

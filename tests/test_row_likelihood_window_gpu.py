@@ -1,7 +1,7 @@
 """Rows whose mixture likelihood t = sum_j L_ij pi_j is tiny but not zero (window_cases: e^-760
 to e^-600, entered through pi, through L or through a product of two normal factors, weights
 scaled by 1, 1e3 and 1e6) in every EM pass, against the long-double reference
-(tile_cases.ld_iterate / ld_read_mix) with the tolerances of test_tile_kernels_gpu.py.  A row
+(tile_cases.ld_iterate / ld_read_mix) with the tolerances of rank_cases.py.  A row
 with t < 2^-960 (csrc/em_kernels.cuh: row_needs_logspace) is redone in log space; above it the
 linear-space pass must stay finite and accurate.  The flag probe pins the boundary from both
 sides."""
@@ -18,7 +18,7 @@ from oracle import oracle_c
 from bootstrap_oracle import boot_counts
 from conftest import make_args
 from test_logspace_rescue_gpu import _layout_and_underflow
-from test_tile_kernels_gpu import Session, assert_ln_close, assert_mix_close
+from rank_cases import Session, assert_ln_close, assert_mix_close
 from tile_cases import ld_iterate, ld_read_mix
 from window_cases import LN_THETA, MODES, SCALES, levels_of, plain_start, window_case
 

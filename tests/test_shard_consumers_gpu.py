@@ -23,6 +23,18 @@ pytestmark = pytest.mark.gpu
 
 SEEDS = (71, 72)
 MIN_READS = (1, 60, 400)
+TINY = (73, 5)      # seed and rows of a matrix with fewer rows than the widest world
+
+
+def datasets():
+    """(key, props, read matrix, weights, top columns): the golden seeds, and a matrix of
+    TINY[1] rows whose expected results come from the oracle alone."""
+    g = load_golden("golden_consumers.npz")
+    out = [(seed,) + oracle_np.synthetic_em_result(seed) + (g["s%d_top" % seed].tolist(),)
+           for seed in SEEDS]
+    props, mix, wts = oracle_np.synthetic_em_result(TINY[0], n=TINY[1])
+    out.append(("tiny", props, mix, wts, np.argsort(props)[::-1][:3].tolist()))
+    return out
 
 
 def free_port():
@@ -50,10 +62,8 @@ def decode_assign(res, n):
 
 def _synthetic(rank, world, ctx, tmp):
     from mixemt_b200.runtime import DeviceMatrix, RowShard
-    g = load_golden("golden_consumers.npz")
     res = {}
-    for seed in SEEDS:
-        props, mix, wts = oracle_np.synthetic_em_result(seed)
+    for seed, props, mix, wts, top in datasets():
         haps = ["hg%d" % j for j in range(mix.shape[1])]
         lo, hi = sharding.row_shard(len(mix), rank, world)
         dev = DeviceMatrix.from_host(ctx, mix[lo:hi])
@@ -65,7 +75,6 @@ def _synthetic(rank, world, ctx, tmp):
         r["offsets"] = (dev.row_shard.lo, dev.row_shard.n_total)
         r["contribs_host"] = consumers.find_contribs_from_reads(
             mix[lo:hi], wts[lo:hi], make_args(min_reads=60), sharded=True)
-        top = g["s%d_top" % seed].tolist()
         contribs = [["hap%d" % (k + 1), haps[j], props[j]] for k, j in enumerate(top)]
         r["assign"] = {}
         for tag, fold, cons in (("f2", 2.0, contribs), ("f1p2", 1.2, contribs[:2]),
@@ -80,7 +89,7 @@ def _synthetic(rank, world, ctx, tmp):
         red_host, _ = consumers.reduce_em_matrix(mix[lo:hi], haps, contribs, sharded=True)
         r["reduced_host"] = red_host
         consumers._CHUNK_BYTES = 8 * mix.shape[1] * 7      # 7-row chunks: ragged writes
-        path = consumers.save_npy(dev, os.path.join(tmp, "s%d" % seed))
+        path = consumers.save_npy(dev, os.path.join(tmp, "s%s" % seed))
         back = consumers.load_npy(path, sharded=True)
         r["loaded"] = back.to_host()
         r["loaded_offsets"] = (back.row_shard.lo, back.row_shard.n_total)
@@ -184,18 +193,29 @@ def run_ranks(job, world, tmp, timeout=300):
     return res
 
 
-@pytest.mark.parametrize("world", [2, 3])
+@pytest.mark.parametrize("world", [2, 3, 8])
 def test_sharded_consumers_match_reference(world, tmp_path):
+    """Also on a matrix of 5 rows: at world 8 three ranks hold none."""
     res = run_ranks("synthetic", world, tmp_path)
     g = load_golden("golden_consumers.npz")
-    for seed in SEEDS:
-        props, mix, wts = oracle_np.synthetic_em_result(seed)
+    for seed, props, mix, wts, top in datasets():
         haps = ["hg%d" % j for j in range(mix.shape[1])]
-        want = [g["s%d_contribs_r%d" % (seed, m)].tolist() for m in MIN_READS]
-        assert want == [oracle_np.find_contribs_from_reads(mix, wts, m) for m in MIN_READS]
+        contribs = [["hap%d" % (k + 1), haps[j], props[j]] for k, j in enumerate(top)]
+        want = [oracle_np.find_contribs_from_reads(mix, wts, m) for m in MIN_READS]
+        reduced, new_haps = oracle_np.reduce_em_matrix(mix, haps, contribs)
+        cols = [haps.index(x) for x in new_haps]
+        assign = {tag: decode_assign(oracle_np.assign_read_indexes(cons, (props, mix), haps,
+                                                                   len(mix), fold), len(mix))
+                  for tag, fold, cons in (("f2", 2.0, contribs), ("f1p2", 1.2, contribs[:2]),
+                                          ("single", 2.0, contribs[:1]))}
+        if seed != "tiny":    # the oracle agrees with the reference's outputs
+            assert want == [g["s%d_contribs_r%d" % (seed, m)].tolist() for m in MIN_READS]
+            assert cols == g["s%d_reduced_cols" % seed].tolist()
+            assert np.array_equal(reduced, g["s%d_reduced" % seed])
+            for tag in assign:
+                assert np.array_equal(assign[tag], g["s%d_assign_%s" % (seed, tag)])
         ref = tmp_path / "ref.npy"
         np.save(str(ref), mix)
-        cols = g["s%d_reduced_cols" % seed].tolist()
         for rank in range(world):
             r = res[rank][seed]
             lo, hi = r["lo"], r["hi"]
@@ -204,8 +224,8 @@ def test_sharded_consumers_match_reference(world, tmp_path):
             assert r["offsets"] == (lo, len(mix)) == r["loaded_offsets"]
             assert [haps.index(x) for x in r["new_haps"]] == cols
             assert r["reduced_marked"]
-            assert np.array_equal(r["reduced"], g["s%d_reduced" % seed][lo:hi])
-            assert np.array_equal(r["reduced_host"], g["s%d_reduced" % seed][lo:hi])
+            assert np.array_equal(r["reduced"], reduced[lo:hi])
+            assert np.array_equal(r["reduced_host"], reduced[lo:hi])
             assert np.array_equal(r["loaded"], mix[lo:hi])
         for tag in ("f2", "f1p2", "single"):
             union = {}
@@ -213,7 +233,7 @@ def test_sharded_consumers_match_reference(world, tmp_path):
                 for name, rows in res[rank][seed]["assign"][tag].items():
                     assert not set(rows) & set(union.get(name, ()))
                     union.setdefault(name, []).extend(rows)
-            assert np.array_equal(decode_assign(union, len(mix)), g["s%d_assign_%s" % (seed, tag)])
+            assert np.array_equal(decode_assign(union, len(mix)), assign[tag])
         path = res[0][seed]["path"]
         assert open(path, "rb").read() == open(str(ref), "rb").read()   # byte-identical
 

@@ -7,7 +7,6 @@ finish run; a dying column (200 log units below every row's best) crosses the wi
 pi * T underflows while pi does not.  The same matrices run over fp64 rows, two restarts per
 pass, and as bootstrap replicates; tiny and ragged row counts; and a matrix with a constructed
 hash collision falls back to fp64 rows."""
-import ctypes
 import os
 
 import numpy as np
@@ -19,49 +18,14 @@ from mixemt_b200.runtime import DeviceMatrix, get_context
 from oracle import oracle_c
 from bootstrap_oracle import boot_counts
 from conftest import make_args
+from rank_cases import Session, assert_ln_close, assert_mix_close, start_lnprops
 from test_tile_plan import ROWS
 from tile_cases import (CASES, case_matrix, class_matrix, colliding_column, ld_iterate,
                         ld_read_mix, predicted_pass_bytes)
 
 pytestmark = pytest.mark.gpu
 
-LN_TOL = 1e-12
-MIX_TOL = 1e-11
 SEED = 91
-
-
-def assert_ln_close(got, want, tol=LN_TOL):
-    got = np.asarray(got, dtype=np.float64)
-    want = np.asarray(want, dtype=np.longdouble)
-    assert np.array_equal(np.isneginf(got), np.isneginf(want)), \
-        np.flatnonzero(np.isneginf(got) != np.isneginf(want))[:10]
-    fin = np.isfinite(want)
-    assert np.isfinite(got[fin]).all()
-    if fin.any():
-        err = np.abs(got[fin] - want[fin]) / np.maximum(1.0, np.abs(want[fin]))
-        assert float(err.max()) <= tol, (float(err.max()), np.flatnonzero(fin)[np.argmax(err)])
-
-
-def assert_mix_close(got, want, tol=MIX_TOL):
-    want = np.asarray(want, dtype=np.longdouble)
-    assert np.array_equal(np.isneginf(got), np.isneginf(want))
-    fin = np.isfinite(want)
-    assert float(np.abs(got[fin] - want[fin]).max()) <= tol
-
-
-def start_lnprops(h, seed, dying=None):
-    """A Dirichlet draw with columns at 1e-200, 1e-295 and 0 (the dying column at 1e-3)."""
-    rs = np.random.RandomState(seed)
-    p = rs.dirichlet([1.0] * h)
-    cols = rs.permutation(h)
-    q = max(1, h // 16)
-    p[cols[:q]] = 1e-200
-    p[cols[q:2 * q]] = 1e-295
-    p[cols[2 * q:3 * q]] = 0.0
-    if dying is not None:
-        p[dying] = 1e-3
-    with np.errstate(divide="ignore"):
-        return np.log(p)
 
 
 @pytest.fixture
@@ -77,42 +41,6 @@ def env():
         os.environ.pop(k, None)
         if v is not None:
             os.environ[k] = v
-
-
-class Session:
-    def __init__(self, dev, w):
-        self.dev, self.w = dev, np.ascontiguousarray(w, dtype=np.float64)
-        self.h = ctypes.c_void_p()
-        check(lib.mxb_em_create(dev.ctx.handle, dev.handle, ptr(self.w), 0, ctypes.byref(self.h)))
-
-    def pass_bytes(self):
-        nbytes, layout = ctypes.c_int64(), ctypes.c_int64()
-        check(lib.mxb_em_pass_bytes(self.h, ctypes.byref(nbytes), ctypes.byref(layout)))
-        return layout.value, nbytes.value
-
-    def iterate(self, lnp, k):
-        """k iterations from lnp without a convergence test: (latest, previous, read matrix)."""
-        n, h = self.dev.shape
-        start = np.ascontiguousarray(lnp, dtype=np.float64)
-        check(lib.mxb_em_set_lnprops(self.h, ptr(start)))
-        it, cv = ctypes.c_int64(), ctypes.c_int32()
-        check(lib.mxb_em_iterate(self.h, k, -1.0, ctypes.byref(it), ctypes.byref(cv)))
-        assert (it.value, cv.value) == (k, 0)
-        latest, prev = np.empty(h), np.empty(h)
-        check(lib.mxb_em_get_lnprops(self.h, 0, ptr(latest)))
-        check(lib.mxb_em_get_lnprops(self.h, 1, ptr(prev)))
-        mh = ctypes.c_void_p()
-        check(lib.mxb_matrix_alloc(self.dev.ctx.handle, n, h, ctypes.byref(mh)))
-        mix_dev = DeviceMatrix(self.dev.ctx, mh)
-        try:
-            check(lib.mxb_em_read_mix(self.h, mix_dev.handle, 0, 0.0))
-            mix = mix_dev.to_host()
-        finally:
-            mix_dev.free()
-        return latest, prev, mix
-
-    def close(self):
-        lib.mxb_em_destroy(self.h)
 
 
 def check_session(dev, mat, w, lnp, traj, ks, want_layout, want_bytes=None):
