@@ -7,7 +7,7 @@ replicates' proportions gives percentile intervals.  The draw is counter-based
 (Philox4x32-10, csrc/bootstrap.cu), so replicate ``b`` depends only on the matrix,
 the weights, the start, the seed, ``b``, ``max_iter`` and ``tolerance``.  The refits
 run on the GPU, several replicates per launch over class tiles (csrc/em.cu:
-run_bootstrap).
+mxb_em_bootstrap).
 """
 import ctypes
 import sys
@@ -16,7 +16,7 @@ import numpy
 
 from . import _lib, sharding
 from ._lib import lib, check, ptr
-from .runtime import DeviceMatrix, get_context, lookup_resident
+from .runtime import OnDevice, get_context, matrix_shape
 
 
 class BootstrapResult:
@@ -87,6 +87,24 @@ def _run(dev, w, start, boot0, n_boot, seed, args):
     return lnp[:n_boot], iters[:n_boot], conv[:n_boot], slots.value
 
 
+def _deal_tasks(ctx, shard, n_tasks, run_block):
+    """Slotted tasks ``0 .. n_tasks - 1`` (bootstrap replicates, constrained refits):
+    ``run_block(k0, k)`` runs tasks ``k0 .. k0 + k - 1`` on this GPU and returns ``(lnprops,
+    iterations, converged, slots)``.  With ``shard == "restarts"`` in a world of more than one
+    rank the tasks are dealt to the ranks in contiguous blocks (``sharding.restart_shard``) and
+    every rank returns the results of all of them (``sharding.merge_bootstrap``); otherwise this
+    process runs them all."""
+    if shard == "restarts":
+        ctx.init_comm_from_torch()
+    if shard != "restarts" or ctx.world == 1:
+        return run_block(0, n_tasks)
+    mine = sharding.restart_shard(n_tasks, ctx.rank, ctx.world)
+    k0 = mine[0] if mine else 0
+    lnp, iters, conv, slots = run_block(k0, len(mine))
+    lnp, iters, conv = sharding.merge_bootstrap(lnp, iters, conv, k0, n_tasks, ctx.allreduce_host)
+    return lnp, iters, conv, slots
+
+
 def bootstrap_props(read_hap_mat, weights, args, props, n_boot=100, seed=None):
     """Bootstrap the fit ``props`` (what ``run_em`` returned for ``read_hap_mat`` and
     ``weights``): ``n_boot`` replicates, each one ``run_em`` restart (``args.max_iter``,
@@ -100,49 +118,24 @@ def bootstrap_props(read_hap_mat, weights, args, props, n_boot=100, seed=None):
     shard = getattr(args, "b200_shard", None)
     if shard == "rows":
         raise ValueError("a row-sharded bootstrap is not supported; use b200_shard='restarts'")
-    dev = None
-    if isinstance(read_hap_mat, DeviceMatrix):
-        dev = read_hap_mat
-        n, h = dev.shape
-    else:
-        if isinstance(read_hap_mat, numpy.ndarray):
-            dev = lookup_resident(read_hap_mat)
-        mat = read_hap_mat if dev is not None else _lib.as_f64(read_hap_mat)
-        if mat.ndim != 2:
-            raise ValueError("read_hap_mat must be 2-dimensional")
-        n, h = mat.shape
+    n, h = matrix_shape(read_hap_mat)
     n_boot = int(n_boot)
     w, start = _validate(weights, props, n, h, n_boot)
     if seed is not None and not 0 <= int(seed) < 2 ** 64:
         raise ValueError("seed must lie in [0, 2^64)")
 
     ctx = get_context()
-    fan_out = False
-    if shard == "restarts":
-        ctx.init_comm_from_torch()
-        fan_out = ctx.world > 1
     if seed is None:
         draw = lambda: numpy.array([numpy.random.randint(0, 2 ** 53, dtype=numpy.int64)])
-        if fan_out:
-            seed = int(sharding.share_from_rank0(draw, (1,), ctx.rank, ctx.allreduce_host)[0])
+        if shard == "restarts" and ctx.init_comm_from_torch().world > 1:
+            # every rank resamples with rank 0's seed
+            seed = sharding.share_from_rank0(draw, (1,), ctx.rank, ctx.allreduce_host)[0]
         else:
-            seed = int(draw()[0])
+            seed = draw()[0]
     seed = int(seed)
-    owned = dev is None
-    if owned:
-        dev = DeviceMatrix.from_host(ctx, mat)
-    try:
-        if fan_out:
-            mine = sharding.restart_shard(n_boot, ctx.rank, ctx.world)
-            boot0 = mine[0] if mine else 0
-            lnp, iters, conv, slots = _run(dev, w, start, boot0, len(mine), seed, args)
-            lnp, iters, conv = sharding.merge_bootstrap(lnp, iters, conv, boot0, n_boot,
-                                                        ctx.allreduce_host)
-        else:
-            lnp, iters, conv, slots = _run(dev, w, start, 0, n_boot, seed, args)
-    finally:
-        if owned:
-            dev.free()
+    with OnDevice(read_hap_mat, ctx) as dev:
+        lnp, iters, conv, slots = _deal_tasks(
+            ctx, shard, n_boot, lambda k0, k: _run(dev, w, start, k0, k, seed, args))
     if getattr(args, "verbose", False):
         sys.stderr.write("Bootstrap: %d replicates (seed %d), %d per launch, iterations mean "
                          "%.1f, %d converged\n" % (n_boot, seed, slots, iters.mean(),

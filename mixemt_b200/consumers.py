@@ -26,37 +26,10 @@ import ctypes
 
 import numpy
 
-from . import _lib
 from . import sharding
 from ._lib import lib, check, ptr
-from .runtime import (DeviceMatrix, RowShard, get_context, lookup_resident, remember_resident,
-                      resident_mode)
-
-
-class _OnDevice(object):
-    """Context manager: a DeviceMatrix view of ``mat``, freed on exit if it was
-    uploaded just for this call."""
-
-    def __init__(self, mat, ctx=None):
-        self.owned = False
-        if isinstance(mat, DeviceMatrix):
-            self.dev = mat
-            return
-        dev = lookup_resident(mat) if isinstance(mat, numpy.ndarray) else None
-        if dev is None:
-            arr = _lib.as_f64(mat)
-            if arr.ndim != 2:
-                raise ValueError("expected a 2-dimensional matrix")
-            dev = DeviceMatrix.from_host(ctx or get_context(), arr)
-            self.owned = True
-        self.dev = dev
-
-    def __enter__(self):
-        return self.dev
-
-    def __exit__(self, *exc):
-        if self.owned:
-            self.dev.free()
+from .runtime import (DeviceMatrix, OnDevice, RowShard, get_context, lookup_resident,
+                      remember_resident, resident_mode)
 
 
 def _shard_mark(mat, sharded):
@@ -123,12 +96,12 @@ def reduce_em_matrix(em_mat, haplogroups, contrib_props, sharded=False):
     was_resident = isinstance(em_mat, numpy.ndarray) and lookup_resident(em_mat) is not None
     mark, ctx = _shard_mark(em_mat, sharded)
     if mark is None:
-        with _OnDevice(em_mat) as dev:
+        with OnDevice(em_mat) as dev:
             small = gather_columns(dev, indexes)
     else:
         small, err = None, None
         try:
-            with _OnDevice(em_mat, ctx) as dev:
+            with OnDevice(em_mat, ctx) as dev:
                 small = gather_columns(dev, indexes)
             small.row_shard = mark
         except Exception as exc:      # local failure: reported through the agreement
@@ -152,7 +125,7 @@ def reduce_em_matrix(em_mat, haplogroups, contrib_props, sharded=False):
 def vote_count(read_hap_mat, wts):
     """``(votes[H], argmax[N])``: weighted votes per haplogroup column from the
     row maxima (first maximum, like ``numpy.argmax(read_hap_mat, 1)``)."""
-    with _OnDevice(read_hap_mat) as dev:
+    with OnDevice(read_hap_mat) as dev:
         n, h = dev.shape
         weights = _weights_for(wts, n)
         votes = numpy.zeros(h, dtype=numpy.int64)
@@ -173,7 +146,7 @@ def vote_first(read_hap_mat, wts, row0=0):
     """``(votes[H], first[H])``: the votes of :func:`vote_count` and, per column, the
     smallest ``row0 + r`` whose first row maximum it is (-1: none).  Only these 2H
     numbers come back from the device."""
-    with _OnDevice(read_hap_mat) as dev:
+    with OnDevice(read_hap_mat) as dev:
         n, h = dev.shape
         weights = _weights_for(wts, n)
         votes = numpy.zeros(h, dtype=numpy.int64)
@@ -215,7 +188,7 @@ def find_contribs_from_reads(read_hap_mat, wts, args, sharded=False):
 
 def read_votes(read_hap_mat):
     """``numpy.argmax(read_hap_mat, 1)`` of stats.report_read_votes (stats.py:39)."""
-    with _OnDevice(read_hap_mat) as dev:
+    with OnDevice(read_hap_mat) as dev:
         return dev.argmax_rows()
 
 
@@ -225,7 +198,7 @@ def assign_rows(read_hap_mat, props, con_indexes, min_fold):
     cols = numpy.ascontiguousarray(con_indexes, dtype=numpy.int64)
     log_props = numpy.log(numpy.asarray(props, dtype=numpy.float64))   # assemble.py:300
     con_ln = numpy.ascontiguousarray(log_props[cols])
-    with _OnDevice(read_hap_mat) as dev:
+    with OnDevice(read_hap_mat) as dev:
         out = numpy.empty(dev.shape[0], dtype=numpy.int32)
         check(lib.mxb_assign_reads(dev.ctx.handle, dev.handle, ptr(cols), ptr(con_ln), len(cols),
                                    float(numpy.log(min_fold)), ptr(out)))
@@ -293,7 +266,7 @@ def save_npy(mat, path, sharded=False):
     On a row shard every rank passes the same path on one node's filesystem and
     the file holds the whole matrix: rank 0 writes the header and sizes the file,
     then each rank writes its rows at their offset (two barriers)."""
-    with _OnDevice(mat) as dev:
+    with OnDevice(mat) as dev:
         n, h = dev.shape
         if not str(path).endswith(".npy"):
             path = str(path) + ".npy"          # numpy.save appends the suffix

@@ -1,5 +1,5 @@
 // Resampling of the nonparametric bootstrap (bootstrap.cu): the fragments a replicate draws,
-// as counts per signature row.  The EM side of a bootstrap lives in em.cu (run_bootstrap).
+// as counts per signature row.  The EM side of a bootstrap lives in em.cu (mxb_em_bootstrap).
 #pragma once
 
 #include <stdint.h>

@@ -55,6 +55,10 @@ namespace mxb {
 // split (em_colreduce_kernel, NCCL all-reduce across ranks, em_update_kernel).
 enum class EmForm { kTiles, kRows, kRowPairs, kGeneral };
 enum class EmTail { kFused, kPeer, kSplit };
+// What a session is created for: run_em's restarts (and mxb_em_create's sessions), or a slotted
+// session of constrained refits (the slots share one weight vector) or of bootstrap replicates
+// (every slot iterates on its own resampled counts).
+enum class EmKind { kRestarts, kRefit, kBootstrap };
 }  // namespace mxb
 
 struct mxb_em {
@@ -108,10 +112,10 @@ struct mxb_em {
     DevBlock small;   // one device block behind weights ... props_in (fewer driver calls)
     DevBlock slots;   // the slot block (slot_block)
     bool zero_iter = false;  // last iterate() ran no iteration
-    // Slotted session (run_slots): n_slots restarts per launch, side by side over class tiles.
-    // A bootstrap session gives every slot its own weight vector (own_weights: slot_w, the
-    // resampled counts); the slots of a refit session share `weights`.  Over class tiles the
-    // slots' Pi and U vectors lie tile_pi_stride and tile_u_stride doubles apart.
+    // Slotted session (EmKind::kRefit, kBootstrap): n_slots restarts per launch, side by side
+    // over class tiles.  A bootstrap session gives every slot its own weight vector (own_weights:
+    // slot_w, the resampled counts); the slots of a refit session share `weights`.  Over class
+    // tiles the slots' Pi and U vectors lie tile_pi_stride and tile_u_stride doubles apart.
     bool slotted = false, own_weights = false;
     double *slot_w = nullptr;
     int64_t tile_pi_stride = 0, tile_u_stride = 0;
@@ -683,8 +687,7 @@ static int em_pack_tiles(mxb_em *em, int want_slots, bool &built) {
 }
 
 static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weights, int sharded,
-                          int want_slots, mxb_em **out, bool slotted = false,
-                          bool own_weights = false) {
+                          int want_slots, EmKind kind, mxb_em **out) {
     MXB_REQUIRE(ctx != nullptr && m != nullptr && out != nullptr, "NULL argument");
     // a rank of a row-sharded run may hold no rows at all (fewer signatures than GPUs)
     MXB_REQUIRE((m->n_rows > 0 || sharded) && m->n_cols > 0, "EM needs a non-empty matrix");
@@ -699,8 +702,8 @@ static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weigh
     em->n_cols = m->n_cols;
     em->ld = round_up(m->n_cols, kLdAlign);
     em->sharded = sharded != 0;
-    em->slotted = slotted;
-    em->own_weights = own_weights;
+    em->slotted = kind != EmKind::kRestarts;
+    em->own_weights = kind == EmKind::kBootstrap;
 
     // launch geometry
     const size_t row_bytes = (size_t)em->ld * sizeof(double);
@@ -783,7 +786,7 @@ extern "C" {
 
 int mxb_em_create(mxb_ctx *ctx, const mxb_matrix *m, const double *weights, int sharded,
                   mxb_em **out) {
-    return em_create_impl(ctx, m, weights, sharded, 1, out);
+    return em_create_impl(ctx, m, weights, sharded, 1, EmKind::kRestarts, out);
 }
 
 int mxb_em_pass_bytes(const mxb_em *em, int64_t *bytes_per_pass, int64_t *n_dense_rows) {
@@ -861,7 +864,7 @@ static int em_logspace_step(mxb_em *em, int cur, int slot, const double *weights
 
 namespace mxb {
 
-// The host side of every EM run that stops on convergence (mxb_em_iterate, run_em's restarts).
+// The host side of every EM run that stops on convergence (mxb_em_iterate, run_tasks).
 // Iterations are enqueued in chunks ahead of the device for the restart slots that are live, and
 // the host polls the control blocks of all slots two chunks behind; a finished restart turns
 // the launches queued after it into early-exit no-ops.  No more iterations are enqueued than a
@@ -1197,133 +1200,51 @@ int mxb_matrix_fold_ranks(mxb_ctx *ctx, mxb_matrix *m, double sub_log) {
 
 namespace mxb {
 
-// run_em's restart loop (em.py:117-163) on a session with one or two restart slots: restart i
-// starts on the device from init_lnprops[i] as soon as a slot is free (two slots iterate two
-// restarts per read of L), and em_poll_loop drives all of them.  Results are combined as the
-// reference combines them: final log-proportions summed in restart order (em.py:145-155), then
-// averaged and exponentiated unless `raw` (em.py:158-163); read matrices folded with logaddexp
-// in restart order (em.py:156, :161).  A restart that finishes before an earlier one parks the
-// proportions its read matrix is formed from until its turn.
-static int run_restarts(mxb_em *em, const double *init_lnprops, int32_t n_multi, int64_t max_iter,
-                        double tol, bool raw, mxb_matrix *mix, StageTimer &tm, double *props_out,
-                        int64_t *iters_out, int32_t *converged_out) {
-    mxb_ctx *ctx = em->ctx;
-    cudaStream_t s = ctx->stream;
-    const int64_t h = em->n_cols, ld = em->ld;
-    // device: [inits n_multi x h][final log-proportions n_multi x h][the proportions before
-    // the last step n_multi x h]; the finals are read back in one copy at the end (no pinned
-    // host buffer, no blocking copy mid-run)
-    const size_t vec_bytes = (size_t)n_multi * h * sizeof(double);
-    DevBlock vecs;
-    MXB_TRY(vecs.alloc(ctx, 3 * vec_bytes, "run_em"));
-    double *d_inits = vecs.get<double>();
-    double *d_fin = d_inits + (size_t)n_multi * h;
-    double *d_prev = d_fin + (size_t)n_multi * h;
-    std::vector<double> h_fin;
-    std::vector<char> done_restart;       // finished, read matrix not folded yet (or folded)
-    try {
-        h_fin.resize((size_t)n_multi * h);
-        done_restart.assign((size_t)n_multi, 0);
-    } catch (const std::bad_alloc &) {
-        set_error("run_em: out of host memory");
-        return MXB_ERR_NOMEM;
-    }
-    MXB_TRY(copy_h2d(ctx, d_inits, init_lnprops, vec_bytes));
+// Tasks whose final log-proportions are kept on the device at a time: they are downloaded in
+// windows of this many rows (at most 177 MB at H = 5408), whatever the number of tasks.
+constexpr int64_t kOutRows = 4096;
 
-    int32_t next = 0, folded = 0;
-    int slot_restart[kMaxSlots] = {-1, -1};
-    auto start_slot = [&](int sl) {
-        const int32_t idx = next++;
-        slot_restart[sl] = idx;
-        em_set_props_kernel<<<(int)ceil_div(ld, 256), 256, 0, s>>>(
-            d_inits + (size_t)idx * h, h, ld, em->lnp[0] + sl * ld, em->pi[0] + sl * ld,
-            em->lnp[1] + sl * ld, em->pi[1] + sl * ld);
-        em_reset_state_kernel<<<1, 1, 0, s>>>(em->state + sl, (long long)max_iter, tol);
-        ctx->launches += 2;
-    };
-    // fin, prev: the restart's final log-proportions and the ones before its last step
-    auto finish_restart = [&](int32_t idx, const SlotResult &res) -> int {
-        if (iters_out) iters_out[idx] = res.iters;
-        if (converged_out) converged_out[idx] = res.converged;
-        MXB_CUDA(cudaMemcpyAsync(d_fin + (size_t)idx * h, res.fin, h * sizeof(double),
-                                 cudaMemcpyDeviceToDevice, s));
-        if (!mix) return MXB_OK;
-        // the read matrix comes from the proportions before the last step (SURVEY F5)
-        MXB_CUDA(cudaMemcpyAsync(d_prev + (size_t)idx * h, res.prev, h * sizeof(double),
-                                 cudaMemcpyDeviceToDevice, s));
-        done_restart[(size_t)idx] = 1;
-        if (!done_restart[(size_t)folded]) return MXB_OK;
-        tm.mark("iterate", kStageIterate);
-        for (; folded < n_multi && done_restart[(size_t)folded]; ++folded) {
-            const bool last = folded == n_multi - 1;
-            const double sub = (last && n_multi > 1 && !raw) ? log((double)n_multi) : 0.0;
-            MXB_TRY(launch_read_mix(em, d_prev + (size_t)folded * h, mix, folded == 0 ? 0 : 1, sub));
-        }
-        tm.mark("read_mix kernel", kStageReadMix);
-        return MXB_OK;
-    };
-    if (max_iter <= 0) {
-        // em.py:126's loop body never runs: every restart hands back its init (em.py:141-143)
-        for (int32_t i = 0; i < n_multi; ++i)
-            MXB_TRY(finish_restart(i, {d_inits + (size_t)i * h, d_inits + (size_t)i * h, 0, 0}));
-    } else {
-        int n_live = 0;
-        for (; n_live < em->n_slots && n_live < n_multi; ++n_live) start_slot(n_live);
-        MXB_TRY(em_poll_loop(em, max_iter, n_live, [&](int sl, const EmState &st, bool &again) -> int {
-            MXB_TRY(finish_restart(slot_restart[sl], slot_result(em, sl, st)));
-            again = next < n_multi;
-            if (again) start_slot(sl);
-            return MXB_OK;
-        }));
-    }
-    MXB_CUDA(cudaStreamSynchronize(s));
-    tm.mark("iterate", kStageIterate);
-    MXB_TRY(copy_d2h(ctx, h_fin.data(), d_fin, vec_bytes));
-    for (int64_t j = 0; j < h; ++j) {
-        double v = h_fin[j];
-        for (int32_t i = 1; i < n_multi; ++i) v += h_fin[(size_t)i * h + j];  // em.py:155
-        if (!raw) {
-            if (n_multi > 1) v /= (double)n_multi;  // em.py:158-160
-            v = exp(v);                             // em.py:163
-        }
-        props_out[j] = v;
-    }
-    return MXB_OK;
-}
-
-// Tasks whose results are kept on the device at a time: the output is downloaded in windows of
-// this many rows (at most 177 MB at H = 5408), whatever the number of tasks.
-constexpr int64_t kBootOutRows = 4096;
-
-// The driver of a slotted session (bootstrap replicates, constrained refits): tasks
-// 0 .. n_tasks - 1 are put on the session's slots in order.  When a slot is handed task k,
-// set_up(slot, k, start) does what the task needs first and names the device log-proportions it
-// starts from; the slot then runs one run_em restart from there under em_poll_loop.  A finished
-// slot's final log-proportions go to row k of the output and the slot takes the next task of the
-// window.  Over class tiles the slots iterate side by side (enqueue_tile_pass<true>), over fp64
-// rows one at a time.
-template <typename SetUp>
-static int run_slots(mxb_em *em, int64_t n_tasks, int64_t max_iter, double tol,
+// The driver of every run of restarts on a session's slots (run_em's restarts, bootstrap
+// replicates, constrained refits): tasks 0 .. n_tasks - 1 are put on the slots in order.  When a
+// slot is handed task k, set_up(slot, k, start) does what the task needs first and names the
+// device log-proportions it starts from; the slot then runs one run_em restart from there
+// (em.py:117-143) under em_poll_loop.  A finished task's iterations and converged flag go to
+// iters_out[k] and converged_out[k] (either may be NULL), its final log-proportions to row k of
+// lnprops_out (host; downloaded one window of kOutRows tasks at a time), and finish(k, result)
+// is called.  With max_iter <= 0 em.py:126's loop body never runs: every task hands back its
+// start (em.py:141-143) and nothing is launched on the slots.  Over class tiles the slots of a
+// slotted session iterate side by side (enqueue_tile_pass<true>), over fp64 rows one at a time;
+// the two slots of a run_em session iterate two restarts per read of L.
+template <typename SetUp, typename Finish>
+static int run_tasks(mxb_em *em, int64_t n_tasks, int64_t max_iter, double tol,
                      double *lnprops_out, int64_t *iters_out, int32_t *converged_out,
-                     SetUp set_up) {
+                     SetUp set_up, Finish finish) {
     mxb_ctx *ctx = em->ctx;
     cudaStream_t s = ctx->stream;
     const int64_t h = em->n_cols, ld = em->ld;
-    const size_t ns = (size_t)em->n_slots;
-    const int64_t win = std::min(n_tasks, kBootOutRows);
-    DevBlock out_block;   // [results win x h]
-    MXB_TRY(out_block.alloc(ctx, (size_t)win * h * sizeof(double), "slotted EM"));
+    const int64_t win = std::min(n_tasks, kOutRows);
+    DevBlock out_block;   // [final log-proportions win x h]
+    MXB_TRY(out_block.alloc(ctx, (size_t)win * h * sizeof(double), "EM tasks"));
     double *d_out = out_block.get<double>();
-    // slots that get no task (n_tasks < n_slots) stay done: their CTAs exit at once
-    std::vector<EmState> idle(ns);
-    for (EmState &st : idle) {
-        memset(&st, 0, sizeof(st));
-        st.done = 1;
+    if (max_iter > 0 && n_tasks < em->n_slots) {
+        // slots that get no task stay done: their CTAs exit at once
+        std::vector<EmState> idle((size_t)(em->n_slots - n_tasks));
+        for (EmState &st : idle) {
+            memset(&st, 0, sizeof(st));
+            st.done = 1;
+        }
+        MXB_TRY(copy_h2d(ctx, em->state + n_tasks, idle.data(), idle.size() * sizeof(EmState)));
     }
-    MXB_TRY(copy_h2d(ctx, em->state, idle.data(), ns * sizeof(EmState)));
 
-    int64_t next = 0, w_end = 0;
+    int64_t next = 0, w0 = 0, w_end = 0;
     int64_t slot_task[kMaxSlots] = {};
+    auto task_done = [&](int64_t k, const SlotResult &res) -> int {
+        if (iters_out) iters_out[k] = res.iters;
+        if (converged_out) converged_out[k] = res.converged;
+        MXB_CUDA(cudaMemcpyAsync(d_out + (size_t)(k - w0) * h, res.fin, h * sizeof(double),
+                                 cudaMemcpyDeviceToDevice, s));
+        return finish(k, res);
+    };
     auto start_slot = [&](int sl) -> int {
         const int64_t k = next++;
         slot_task[sl] = k;
@@ -1337,51 +1258,91 @@ static int run_slots(mxb_em *em, int64_t n_tasks, int64_t max_iter, double tol,
         MXB_CUDA(cudaGetLastError());
         return MXB_OK;
     };
-    for (int64_t w0 = 0; w0 < n_tasks; w0 = w_end) {
+    for (; w0 < n_tasks; w0 = w_end) {
         w_end = std::min(n_tasks, w0 + win);
-        int n_live = 0;
-        for (; n_live < em->n_slots && next < w_end; ++n_live) MXB_TRY(start_slot(n_live));
-        MXB_TRY(em_poll_loop(em, max_iter, n_live, [&](int sl, const EmState &st, bool &again) -> int {
-                const SlotResult res = slot_result(em, sl, st);
-                const int64_t k = slot_task[sl];
-                iters_out[k] = res.iters;
-                converged_out[k] = res.converged;
-                MXB_CUDA(cudaMemcpyAsync(d_out + (size_t)(k - w0) * h, res.fin,
-                                         h * sizeof(double), cudaMemcpyDeviceToDevice, s));
-            again = next < w_end;
-            if (again) MXB_TRY(start_slot(sl));
-            return MXB_OK;
-        }));
+        if (max_iter <= 0) {
+            for (; next < w_end; ++next) {
+                const double *start = nullptr;
+                MXB_TRY(set_up(0, next, start));
+                MXB_TRY(task_done(next, {start, start, 0, 0}));
+            }
+        } else {
+            int n_live = 0;
+            for (; n_live < em->n_slots && next < w_end; ++n_live) MXB_TRY(start_slot(n_live));
+            MXB_TRY(em_poll_loop(em, max_iter, n_live, [&](int sl, const EmState &st,
+                                                           bool &again) -> int {
+                MXB_TRY(task_done(slot_task[sl], slot_result(em, sl, st)));
+                again = next < w_end;
+                if (again) MXB_TRY(start_slot(sl));
+                return MXB_OK;
+            }));
+        }
         MXB_TRY(copy_d2h(ctx, lnprops_out + (size_t)w0 * h, d_out,
                          (size_t)(w_end - w0) * h * sizeof(double)));
     }
     return MXB_OK;
 }
 
-// The bootstrap (bootstrap.cu for the draw): task k is replicate boot0 + k, resampled on the
-// device into its slot's weights when the slot is handed it and started from `start`.
-static int run_bootstrap(mxb_em *em, const double *start, const int64_t *d_cumw, uint64_t total,
-                         uint64_t seed, int64_t boot0, int64_t n_boot, int64_t max_iter,
-                         double tol, double *lnprops_out, int64_t *iters_out,
-                         int32_t *converged_out) {
+// run_em (em.py:117-163) on a session with one or two restart slots: restart i starts from
+// init_lnprops[i] (run_tasks).  Results are combined as the reference combines them: final
+// log-proportions summed in restart order (em.py:145-155), then averaged and exponentiated
+// unless `raw` (em.py:158-163); read matrices folded with logaddexp in restart order (em.py:156,
+// :161).  A restart that finishes before an earlier one parks the proportions its read matrix
+// is formed from until its turn.
+static int run_em_session(mxb_em *em, const double *init_lnprops, int32_t n_multi,
+                          int64_t max_iter, double tol, bool raw, mxb_matrix *mix, StageTimer &tm,
+                          double *props_out, int64_t *iters_out, int32_t *converged_out) {
     mxb_ctx *ctx = em->ctx;
-    const int64_t n = em->n_rows, h = em->n_cols;
-    DevBlock work;   // [counts n][start h]
-    uint32_t *counts = nullptr;
-    double *d_start = nullptr;
-    MXB_TRY(work.alloc_parts(ctx, "bootstrap", [&](Carve &c) {
-        counts = c.part<uint32_t>(n);
-        d_start = c.part<double>(h);
-    }));
-    MXB_CUDA(cudaMemsetAsync(counts, 0, (size_t)n * sizeof(uint32_t), ctx->stream));
-    MXB_TRY(copy_h2d(ctx, d_start, start, (size_t)h * sizeof(double)));
-    return run_slots(em, n_boot, max_iter, tol, lnprops_out, iters_out, converged_out,
-                     [&](int sl, int64_t k, const double *&from) -> int {
-        MXB_TRY(boot_draw(ctx, d_cumw, n, total, seed, boot0 + k, 1, counts));
-        MXB_TRY(boot_take_counts(ctx, counts, n, slot_weights(em, sl)));
-        from = d_start;
+    const int64_t h = em->n_cols;
+    // device: [inits n_multi x h][the proportions before the last step n_multi x h]
+    const size_t vec_bytes = (size_t)n_multi * h * sizeof(double);
+    DevBlock vecs;
+    MXB_TRY(vecs.alloc(ctx, 2 * vec_bytes, "run_em"));
+    double *d_inits = vecs.get<double>();
+    double *d_prev = d_inits + (size_t)n_multi * h;
+    std::vector<double> h_fin;            // final log-proportions, restart by restart
+    std::vector<char> done_restart;       // finished, read matrix not folded yet (or folded)
+    try {
+        h_fin.resize((size_t)n_multi * h);
+        done_restart.assign((size_t)n_multi, 0);
+    } catch (const std::bad_alloc &) {
+        set_error("run_em: out of host memory");
+        return MXB_ERR_NOMEM;
+    }
+    MXB_TRY(copy_h2d(ctx, d_inits, init_lnprops, vec_bytes));
+
+    int32_t folded = 0;
+    MXB_TRY(run_tasks(em, n_multi, max_iter, tol, h_fin.data(), iters_out, converged_out,
+                      [&](int, int64_t i, const double *&start) -> int {
+        start = d_inits + (size_t)i * h;
         return MXB_OK;
-    });
+    }, [&](int64_t i, const SlotResult &res) -> int {
+        if (!mix) return MXB_OK;
+        // the read matrix comes from the proportions before the last step (SURVEY F5)
+        MXB_CUDA(cudaMemcpyAsync(d_prev + (size_t)i * h, res.prev, h * sizeof(double),
+                                 cudaMemcpyDeviceToDevice, ctx->stream));
+        done_restart[(size_t)i] = 1;
+        if (!done_restart[(size_t)folded]) return MXB_OK;
+        tm.mark("iterate", kStageIterate);
+        for (; folded < n_multi && done_restart[(size_t)folded]; ++folded) {
+            const bool last = folded == n_multi - 1;
+            const double sub = (last && n_multi > 1 && !raw) ? log((double)n_multi) : 0.0;
+            MXB_TRY(launch_read_mix(em, d_prev + (size_t)folded * h, mix, folded == 0 ? 0 : 1, sub));
+        }
+        tm.mark("read_mix kernel", kStageReadMix);
+        return MXB_OK;
+    }));
+    tm.mark("iterate", kStageIterate);
+    for (int64_t j = 0; j < h; ++j) {
+        double v = h_fin[j];
+        for (int32_t i = 1; i < n_multi; ++i) v += h_fin[(size_t)i * h + j];  // em.py:155
+        if (!raw) {
+            if (n_multi > 1) v /= (double)n_multi;  // em.py:158-160
+            v = exp(v);                             // em.py:163
+        }
+        props_out[j] = v;
+    }
+    return MXB_OK;
 }
 
 // Start log-proportions (K x H, host): no NaN, and proportions that sum to more than 0; an error
@@ -1402,6 +1363,46 @@ static int check_starts(const char *who, const double *starts, int64_t n_vec, in
             return MXB_ERR_VALUE;
         }
     }
+    return MXB_OK;
+}
+
+// The body of the slotted entry points (mxb_em_bootstrap, mxb_em_refit) once their arguments
+// are checked: n_tasks tasks on a session of `kind`, task k started from the host vector
+// starts + k * stride (stride 0: one start for all) after prepare(em, slot, k) has done what
+// else it needs.  With max_iter <= 0 em.py:126's loop body never runs: no session is created,
+// nothing is launched, and every task hands back its start (em.py:141-143).
+template <typename Prepare>
+static int run_slotted(mxb_ctx *ctx, const mxb_matrix *m, const double *weights, EmKind kind,
+                       const double *starts, int64_t stride, int64_t n_tasks, int64_t max_iter,
+                       double tol, double *lnprops_out, int64_t *iters_out,
+                       int32_t *converged_out, int32_t *slots_out, Prepare prepare) {
+    const int64_t h = m->n_cols;
+    if (slots_out) *slots_out = 1;
+    if (max_iter <= 0) {
+        for (int64_t k = 0; k < n_tasks; ++k) {
+            memcpy(lnprops_out + k * h, starts + k * stride, (size_t)h * sizeof(double));
+            iters_out[k] = 0;
+            converged_out[k] = 0;
+        }
+        return MXB_OK;
+    }
+    MXB_CUDA(cudaSetDevice(ctx->device));
+    mxb_em *em = nullptr;
+    MXB_TRY(em_create_impl(ctx, m, weights, 0, 1, kind, &em));
+    std::unique_ptr<mxb_em, decltype(&mxb_em_destroy)> session(em, mxb_em_destroy);
+    const size_t start_bytes = (size_t)(stride ? n_tasks : 1) * h * sizeof(double);
+    DevBlock starts_block;
+    MXB_TRY(starts_block.alloc(ctx, start_bytes, "slotted EM"));
+    const double *d_starts = starts_block.get<double>();
+    MXB_TRY(copy_h2d(ctx, starts_block.get(), starts, start_bytes));
+    if (slots_out) *slots_out = em->n_slots;
+    MXB_TRY(run_tasks(em, n_tasks, max_iter, tol, lnprops_out, iters_out, converged_out,
+                      [&](int sl, int64_t k, const double *&start) -> int {
+        MXB_TRY(prepare(em, sl, k));
+        start = d_starts + k * stride;
+        return MXB_OK;
+    }, [](int64_t, const SlotResult &) { return MXB_OK; }));
+    MXB_CUDA(cudaStreamSynchronize(ctx->stream));
     return MXB_OK;
 }
 
@@ -1437,29 +1438,25 @@ int mxb_em_bootstrap(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
     std::vector<int64_t> cumw;
     uint64_t total = 0;
     MXB_TRY(boot_prefix(weights, n, cumw, total));
-    if (slots_out) *slots_out = 1;
-    if (max_iter <= 0) {
-        // em.py:126's loop body never runs: every replicate hands back the start (em.py:141-143)
-        for (int64_t k = 0; k < n_boot; ++k) {
-            memcpy(lnprops_out + k * h, start_lnprops, (size_t)h * sizeof(double));
-            iters_out[k] = 0;
-            converged_out[k] = 0;
+    DevBlock work;   // [prefix sums n][counts n]
+    int64_t *d_cumw = nullptr;
+    uint32_t *counts = nullptr;
+    // task k is replicate boot0 + k (bootstrap.cu for the draw), resampled on the device into
+    // its slot's weights; all start from start_lnprops
+    return run_slotted(ctx, m, weights, EmKind::kBootstrap, start_lnprops, 0, n_boot, max_iter,
+                       tol, lnprops_out, iters_out, converged_out, slots_out,
+                       [&](mxb_em *em, int sl, int64_t k) -> int {
+        if (k == 0) {   // the first replicate takes the prefix sums to the device
+            MXB_TRY(work.alloc_parts(ctx, "bootstrap", [&](Carve &c) {
+                d_cumw = c.part<int64_t>(n);
+                counts = c.part<uint32_t>(n);
+            }));
+            MXB_TRY(copy_h2d(ctx, d_cumw, cumw.data(), (size_t)n * sizeof(int64_t)));
+            MXB_CUDA(cudaMemsetAsync(counts, 0, (size_t)n * sizeof(uint32_t), ctx->stream));
         }
-        return MXB_OK;
-    }
-    MXB_CUDA(cudaSetDevice(ctx->device));
-    mxb_em *em = nullptr;
-    MXB_TRY(em_create_impl(ctx, m, weights, 0, 1, &em, true, true));
-    std::unique_ptr<mxb_em, decltype(&mxb_em_destroy)> session(em, mxb_em_destroy);
-    DevBlock cumw_block;
-    MXB_TRY(cumw_block.alloc(ctx, (size_t)n * sizeof(int64_t), "bootstrap"));
-    int64_t *d_cumw = cumw_block.get<int64_t>();
-    MXB_TRY(copy_h2d(ctx, d_cumw, cumw.data(), (size_t)n * sizeof(int64_t)));
-    if (slots_out) *slots_out = em->n_slots;
-    MXB_TRY(run_bootstrap(em, start_lnprops, d_cumw, total, seed, boot0, n_boot, max_iter, tol,
-                          lnprops_out, iters_out, converged_out));
-    MXB_CUDA(cudaStreamSynchronize(ctx->stream));
-    return MXB_OK;
+        MXB_TRY(boot_draw(ctx, d_cumw, n, total, seed, boot0 + k, 1, counts));
+        return boot_take_counts(ctx, counts, n, slot_weights(em, sl));
+    });
 }
 
 int mxb_em_refit(mxb_ctx *ctx, const mxb_matrix *m, const double *weights, const double *starts,
@@ -1470,34 +1467,11 @@ int mxb_em_refit(mxb_ctx *ctx, const mxb_matrix *m, const double *weights, const
     MXB_REQUIRE(lnprops_out != nullptr && iters_out != nullptr && converged_out != nullptr,
                 "NULL buffer");
     MXB_REQUIRE(n_starts >= 1, "need at least one start");
-    const int64_t h = m->n_cols;
-    MXB_TRY(check_starts("refit", starts, n_starts, h));
-    if (slots_out) *slots_out = 1;
-    if (max_iter <= 0) {
-        // em.py:126's loop body never runs: every refit hands back its start (em.py:141-143)
-        memcpy(lnprops_out, starts, (size_t)(n_starts * h) * sizeof(double));
-        for (int64_t k = 0; k < n_starts; ++k) {
-            iters_out[k] = 0;
-            converged_out[k] = 0;
-        }
-        return MXB_OK;
-    }
-    MXB_CUDA(cudaSetDevice(ctx->device));
-    mxb_em *em = nullptr;
-    MXB_TRY(em_create_impl(ctx, m, weights, 0, 1, &em, true, false));
-    std::unique_ptr<mxb_em, decltype(&mxb_em_destroy)> session(em, mxb_em_destroy);
-    DevBlock starts_block;
-    MXB_TRY(starts_block.alloc(ctx, (size_t)(n_starts * h) * sizeof(double), "refit"));
-    const double *d_starts = starts_block.get<double>();
-    MXB_TRY(copy_h2d(ctx, starts_block.get(), starts, (size_t)(n_starts * h) * sizeof(double)));
-    if (slots_out) *slots_out = em->n_slots;
-    MXB_TRY(run_slots(em, n_starts, max_iter, tol, lnprops_out, iters_out, converged_out,
-                      [&](int, int64_t k, const double *&from) -> int {
-        from = d_starts + k * h;
-        return MXB_OK;
-    }));
-    MXB_CUDA(cudaStreamSynchronize(ctx->stream));
-    return MXB_OK;
+    MXB_TRY(check_starts("refit", starts, n_starts, m->n_cols));
+    // refit k starts from starts[k]
+    return run_slotted(ctx, m, weights, EmKind::kRefit, starts, m->n_cols, n_starts, max_iter,
+                       tol, lnprops_out, iters_out, converged_out, slots_out,
+                       [](mxb_em *, int, int64_t) { return MXB_OK; });
 }
 
 int mxb_run_em_dev(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
@@ -1521,7 +1495,7 @@ int mxb_run_em_dev(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
     const bool sharded = (flags & MXB_EM_SHARDED) != 0;
     const int want_slots = (n_multi >= 2 && max_iter > 0 && !sharded &&
                             getenv("MXB_EM_NO_BATCH") == nullptr) ? 2 : 1;
-    int rc = em_create_impl(ctx, m, weights, sharded, want_slots, &em);
+    int rc = em_create_impl(ctx, m, weights, sharded, want_slots, EmKind::kRestarts, &em);
     tm.mark("em_create (tiles or fp64 rows)", kStageSetup);
     if (rc == MXB_OK && want_mix) rc = mxb_matrix_alloc(ctx, m->n_rows, h, &mix);
     tm.mark("alloc read_mix", kStageSetup);
@@ -1530,8 +1504,8 @@ int mxb_run_em_dev(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
     if (rc == MXB_OK && read_mix_out)
         fault_mix.start(read_mix_out, (size_t)m->n_rows * (size_t)h * sizeof(double));
     if (rc == MXB_OK)
-        rc = run_restarts(em, init_lnprops, n_multi, max_iter, tol, raw, mix, tm, props_out,
-                          iters_out, converged_out);
+        rc = run_em_session(em, init_lnprops, n_multi, max_iter, tol, raw, mix, tm, props_out,
+                            iters_out, converged_out);
     if (rc == MXB_OK && read_mix_out) {
         fault_mix.join();
         rc = mxb_matrix_download(ctx, mix, read_mix_out);

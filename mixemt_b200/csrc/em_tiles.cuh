@@ -220,7 +220,7 @@ __device__ __forceinline__ SegItem seg_shfl_up(const SegItem &v, int off) {
     return o;
 }
 
-// kSlots (bootstrap sessions, em.cu: run_bootstrap): blockIdx.y is a replicate slot; its
+// kSlots (slotted sessions, em.cu: run_tasks): blockIdx.y is a replicate slot; its
 // proportions, control block and class sums lie pi_stride, one EmState and cls_stride further.
 template <int PER, bool kSlots = false>
 __global__ void __launch_bounds__(kTileThreads)

@@ -188,7 +188,7 @@ inline int tile_plan_check(const std::vector<TileDesc> &desc, const TilePlanOut 
     return errs;
 }
 
-// Replicate slots of a bootstrap session (em.cu: run_bootstrap): the pass of R slots runs on
+// Replicate slots of a slotted session (em.cu: run_tasks): the pass of R slots runs on
 // num_sms / R CTAs per slot, all R in one wave on one plan.  R is the largest power of two up to
 // kBootMaxSlots whose plan models at most R times the time of the full-budget plan (R replicates
 // then cost no more than R iterations one after another; launch and tail costs, which the model

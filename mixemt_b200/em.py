@@ -14,8 +14,8 @@ import numpy
 from . import _lib
 from ._lib import lib, check, ptr
 from . import sharding
-from .runtime import (DeviceMatrix, RowShard, get_context, lookup_resident, remember_resident,
-                      resident_mode)
+from .runtime import (DeviceMatrix, OnDevice, RowShard, get_context, matrix_shape,
+                      remember_resident, resident_mode)
 
 
 def init_props(nhaps, alpha=1.0):
@@ -159,24 +159,10 @@ def run_em(read_hap_mat, weights, args):
     Inputs are not modified.
     """
     ctx = get_context()
-    dev = None
-    owned = False
-    if isinstance(read_hap_mat, DeviceMatrix):
-        dev = read_hap_mat
-    elif isinstance(read_hap_mat, numpy.ndarray):
-        dev = lookup_resident(read_hap_mat)
-    if dev is None:
-        mat = _lib.as_f64(read_hap_mat)
-        if mat.ndim != 2:
-            raise ValueError("read_hap_mat must be 2-dimensional")
-        dev = DeviceMatrix.from_host(ctx, mat)
-        owned = True
+    matrix_shape(read_hap_mat)
     keep = resident_mode(args)
-    try:
+    with OnDevice(read_hap_mat, ctx) as dev:
         props, read_mix, _, mix_dev = run_em_device(dev, weights, args, keep_device=keep)
-    finally:
-        if owned:
-            dev.free()
     if keep and mix_dev is not None and read_mix is not None:
         # opt-in residency: the consumers in mixemt_b200.consumers find the HBM copy of
         # the result through the (read-only) host array, see runtime.remember_resident

@@ -24,18 +24,9 @@ import numpy
 
 from . import _lib, sharding
 from ._lib import lib, check, ptr
-from .bootstrap import start_from_props
-from .consumers import _OnDevice, _collective, _shard_mark
-from .runtime import DeviceMatrix, get_context, lookup_resident
-
-
-def _shape(read_hap_mat):
-    if isinstance(read_hap_mat, DeviceMatrix):
-        return read_hap_mat.shape
-    shape = numpy.shape(read_hap_mat)
-    if len(shape) != 2:
-        raise ValueError("read_hap_mat must be 2-dimensional")
-    return shape
+from .bootstrap import _deal_tasks, start_from_props
+from .consumers import _collective, _shard_mark
+from .runtime import OnDevice, get_context, matrix_shape
 
 
 def _weights(weights, n_rows):
@@ -84,18 +75,18 @@ def log_likelihood(read_hap_mat, weights, props, sharded=False):
     a resident ndarray or a ``DeviceMatrix``.  On a row shard (``sharded=True``, or a
     ``DeviceMatrix`` with ``row_shard``) each rank passes its rows and weights, and every rank
     returns the total of the whole matrix."""
-    n, h = _shape(read_hap_mat)
+    n, h = matrix_shape(read_hap_mat)
     lnp, single = _lnprops(props, h)
     mark, ctx = _shard_mark(read_hap_mat, sharded)
     if mark is None:
         w = _weights(weights, n)
-        with _OnDevice(read_hap_mat) as dev:
+        with OnDevice(read_hap_mat) as dev:
             out = _loglik(dev, w, lnp)
     else:
         out, err = numpy.zeros(lnp.shape[0]), None
         try:
             w = _weights(weights, n)
-            with _OnDevice(read_hap_mat, ctx) as dev:
+            with OnDevice(read_hap_mat, ctx) as dev:
                 out = _loglik(dev, w, lnp)
         except Exception as exc:      # local failure: reported through the sum
             err = exc
@@ -200,7 +191,7 @@ def contributor_lrt(read_hap_mat, weights, args, props, columns, tolerance=None)
     if shard == "rows":
         raise ValueError("a row-sharded likelihood-ratio test is not supported; use "
                          "b200_shard='restarts'")
-    n, h = _shape(read_hap_mat)
+    n, h = matrix_shape(read_hap_mat)
     w = _weights(weights, n)
     p = numpy.asarray(props, dtype=numpy.float64).reshape(-1)
     if (p < 0).any() or numpy.isinf(p).any():
@@ -212,29 +203,10 @@ def contributor_lrt(read_hap_mat, weights, args, props, columns, tolerance=None)
     n_fits = len(starts)
 
     ctx = get_context()
-    fan_out = False
-    if shard == "restarts":
-        ctx.init_comm_from_torch()
-        fan_out = ctx.world > 1
-    dev = read_hap_mat if isinstance(read_hap_mat, DeviceMatrix) else \
-        (lookup_resident(read_hap_mat) if isinstance(read_hap_mat, numpy.ndarray) else None)
-    owned = dev is None
-    if owned:
-        dev = DeviceMatrix.from_host(ctx, _lib.as_f64(read_hap_mat))
-    try:
-        if fan_out:
-            mine = sharding.restart_shard(n_fits, ctx.rank, ctx.world)
-            k0 = mine[0] if mine else 0
-            lnp, iters, conv, slots = _refit(dev, w, starts[k0:k0 + len(mine)], args.max_iter,
-                                             tol)
-            lnp, iters, conv = sharding.merge_bootstrap(lnp, iters, conv, k0, n_fits,
-                                                        ctx.allreduce_host)
-        else:
-            lnp, iters, conv, slots = _refit(dev, w, starts, args.max_iter, tol)
+    with OnDevice(read_hap_mat, ctx) as dev:
+        lnp, iters, conv, slots = _deal_tasks(
+            ctx, shard, n_fits, lambda k0, k: _refit(dev, w, starts[k0:k0 + k], args.max_iter, tol))
         loglik = _loglik(dev, w, lnp)
-    finally:
-        if owned:
-            dev.free()
     if getattr(args, "verbose", False):
         sys.stderr.write("LRT: %d columns, %d refits per launch, iterations mean %.1f, %d of %d "
                          "converged\n" % (len(cols), slots, iters.mean(), int(conv.sum()),

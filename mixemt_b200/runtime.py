@@ -205,3 +205,41 @@ def lookup_resident(host_arr):
         return None
     dev = ent[1]
     return dev if dev.handle and dev.shape == host_arr.shape else None
+
+
+def matrix_shape(read_hap_mat):
+    """``(n_rows, n_cols)`` of a matrix argument (``DeviceMatrix``, ndarray or nested
+    sequence), without moving it; ``ValueError`` unless it is 2-dimensional."""
+    if isinstance(read_hap_mat, DeviceMatrix):
+        return read_hap_mat.shape
+    shape = np.shape(read_hap_mat)
+    if len(shape) != 2:
+        raise ValueError("read_hap_mat must be 2-dimensional")
+    return shape
+
+
+class OnDevice(object):
+    """Context manager: a DeviceMatrix view of ``mat`` (the matrix itself, the HBM copy of a
+    resident ndarray, or an upload to ``ctx``, default ``get_context()``), freed on exit if it
+    was uploaded just for this call."""
+
+    def __init__(self, mat, ctx=None):
+        self.owned = False
+        if isinstance(mat, DeviceMatrix):
+            self.dev = mat
+            return
+        dev = lookup_resident(mat) if isinstance(mat, np.ndarray) else None
+        if dev is None:
+            arr = _lib.as_f64(mat)
+            if arr.ndim != 2:
+                raise ValueError("expected a 2-dimensional matrix")
+            dev = DeviceMatrix.from_host(ctx or get_context(), arr)
+            self.owned = True
+        self.dev = dev
+
+    def __enter__(self):
+        return self.dev
+
+    def __exit__(self, *exc):
+        if self.owned:
+            self.dev.free()

@@ -13,9 +13,13 @@ and 1; the split tail (MXB_EM_SPLIT_TAIL=1) and the general path (MXB_EM_FORCE_G
 sessions driven by mxb_em_iterate (mxb_em_get_lnprops and mxb_em_read_mix read back), by
 mxb_em_iterate_fixed (20 iterations) and by mxb_em_profile (launch count only: its times are
 not compared); em_step on the toy and the noise matrix; bootstraps on the Build-17 tiles with
-fewer replicates than slots and with more (refilled slots), over fp64 rows, and from a start
-whose row likelihoods underflow.  The second form compares two such directories: every array
-and every launch count must be equal; launch counts are printed side by side.
+fewer replicates than slots and with more (refilled slots), over fp64 rows, from a start whose
+row likelihoods underflow, at max_iter 0, and on the toy matrix with more replicates than one
+output window (4096); constrained refits (mxb_em_refit) on the Build-17 tiles with one start and
+with more starts than slots, over fp64 rows, from the underflowing starts, from starts with a
+-inf column (likelihood.null_start) and at max_iter 0.  The second form compares two such
+directories: every array and every launch count must be equal; launch counts are printed side
+by side.
 """
 import argparse
 import glob
@@ -119,6 +123,14 @@ def _cases():
     c.append(("b17_boot40", "b17", 40, 400, 1e-5, {}, "boot"))
     c.append(("b17_rows_boot5", "b17", 5, 400, 1e-5, {"MXB_EM_NO_PACK": "1"}, "boot"))
     c.append(("under_tiles_boot3", "under_tiles", 3, 60, 1e-6, {}, "boot"))
+    c.append(("b17_boot5_iter0", "b17", 5, 0, 1e-5, {}, "boot"))
+    c.append(("toy_boot4100", "toy", 4100, 30, 1e-4, {}, "boot"))
+    c.append(("b17_refit1", "b17", 1, 400, 1e-5, {}, "refit"))
+    c.append(("b17_refit40", "b17", 40, 400, 1e-5, {}, "refit"))
+    c.append(("b17_rows_refit5", "b17", 5, 400, 1e-5, {"MXB_EM_NO_PACK": "1"}, "refit"))
+    c.append(("under_tiles_refit3", "under_tiles", 3, 60, 1e-6, {}, "refit"))
+    c.append(("b17_refit_null4", "b17", 4, 400, 1e-5, {}, "refit_null"))
+    c.append(("b17_refit5_iter0", "b17", 5, 0, 1e-5, {}, "refit"))
     c.append(("toy_em_step", "toy", 1, 1, 0.0, {}, "step"))
     c.append(("noise_em_step", "noise", 1, 1, 0.0, {}, "step"))
     return c
@@ -191,6 +203,34 @@ def _boot(ctx, m, w, start, n_boot, max_iter, tol):
     return lnp, np.array([slots]), iters, conv, launches
 
 
+def _refit_starts(m, inits, k, null):
+    """The first k starts of a refit case: the case's inits, more Dirichlet draws past 5, or
+    (null) the normalised first init and likelihood.null_start of it for k - 1 columns."""
+    from mixemt_b200 import likelihood
+    h = m.shape[1]
+    if null:
+        p = np.exp(inits[0])
+        cols = [0, 5, h // 2, h - 1][:k - 1]
+        return np.array([np.log(p / p.sum())] + [likelihood.null_start(p, c) for c in cols])
+    if k <= len(inits):
+        return inits[:k]
+    return np.log(np.random.RandomState(h + 1).dirichlet([1.0] * h, size=k))
+
+
+def _refit(ctx, m, w, starts, max_iter, tol):
+    """mxb_em_refit from `starts`: their final log-proportions, iterations and converged flags;
+    the slot count goes with the read matrix."""
+    from mixemt_b200 import likelihood
+    from mixemt_b200.runtime import DeviceMatrix
+    dev = DeviceMatrix.from_host(ctx, m)
+    l0 = ctx.launch_count
+    lnp, iters, conv, slots = likelihood._refit(dev, w, np.ascontiguousarray(starts), max_iter,
+                                                tol)
+    launches = ctx.launch_count - l0
+    dev.free()
+    return lnp, np.array([slots]), iters, conv, launches
+
+
 def run(out_dir):
     from mixemt_b200 import em
     from mixemt_b200.runtime import DeviceMatrix, get_context
@@ -209,6 +249,9 @@ def run(out_dir):
                                                            kind == "profile")
             elif kind == "boot":
                 props, mix, iters, conv, launches = _boot(ctx, m, w, inits[0], k, it, tol)
+            elif kind in ("refit", "refit_null"):
+                starts = _refit_starts(m, inits, k, kind == "refit_null")
+                props, mix, iters, conv, launches = _refit(ctx, m, w, starts, it, tol)
             elif kind == "step":
                 mix = np.empty_like(m)
                 l0 = ctx.launch_count

@@ -1,4 +1,4 @@
-"""The bootstrap on the GPU (csrc/bootstrap.cu, csrc/em.cu: run_bootstrap): the draws equal the
+"""The bootstrap on the GPU (csrc/bootstrap.cu, csrc/em.cu: mxb_em_bootstrap): the draws equal the
 numpy restatement bit for bit, every replicate is the run_em restart on its counts from the
 bootstrapped fit (class tiles: within 1e-13 of run_em_device, fp64 rows: bit-identical), a
 replicate does not depend on how many are asked for or on the slot it ran in, uneven runs

@@ -1,4 +1,4 @@
-"""The EM driver (csrc/em.cu: em_poll_loop and run_restarts) takes the same decisions for one
+"""The EM driver (csrc/em.cu: em_poll_loop and run_tasks) takes the same decisions for one
 restart slot and for two: restarts combined on the device equal independent runs combined in
 restart order, max_iter 0 and 1 give the reference's results, a session iterated with
 mxb_em_iterate hands back what run_em computes, and em_step launches no more kernels than one

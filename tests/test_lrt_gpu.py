@@ -1,4 +1,4 @@
-"""The contributor likelihood-ratio test on the GPU (csrc/em.cu: mxb_em_refit through run_slots,
+"""The contributor likelihood-ratio test on the GPU (csrc/em.cu: mxb_em_refit through run_tasks,
 mixemt_b200.likelihood.contributor_lrt): every refit equals a one-restart run_em from its start
 (class tiles: within 1e-13, fp64 rows: bit-identical), the dropped column stays exactly 0, a
 refit does not depend on which other columns are tested, uneven refits refill their slots and a

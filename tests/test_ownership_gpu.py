@@ -283,6 +283,31 @@ def case_bootstrap_rows(ctx, inp):
     return _bootstrap(ctx, inp["noise"], inp["w_noise"])
 
 
+def _refit(ctx, a, w):
+    hs = _Handles()
+    try:
+        m = _upload(ctx, hs, a)
+        h, k = a.shape[1], 5
+        starts = _inits(h, k)
+        starts[1:, 0] = -np.inf          # constrained refits: column 0 held at 0
+        lnp = np.empty((k, h))
+        iters, conv = np.empty(k, np.int64), np.empty(k, np.int32)
+        slots = c_i32()
+        check(lib.mxb_em_refit(ctx.handle, m, ptr(w), ptr(starts), k, 30, 1e-6, ptr(lnp),
+                               ptr(iters), ptr(conv), ctypes.byref(slots)))
+        return lnp, iters, conv
+    finally:
+        hs.close()
+
+
+def case_refit_tiles(ctx, inp):
+    return _refit(ctx, inp["build17"], inp["w_mix"])
+
+
+def case_refit_rows(ctx, inp):
+    return _refit(ctx, inp["noise"], inp["w_noise"])
+
+
 def case_boot_counts(ctx, inp):
     w = inp["w_noise"]
     out = np.empty((3, w.shape[0]), np.uint32)
