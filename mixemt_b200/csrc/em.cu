@@ -42,8 +42,7 @@
 #include "bootstrap.cuh"
 #include "common.cuh"
 #include "em_kernels.cuh"
-#include "em_tiles.cuh"
-#include "tile_plan.h"
+#include "em_tiles.h"
 
 
 using namespace mxb;
@@ -59,6 +58,19 @@ enum class EmTail { kFused, kPeer, kSplit };
 // session of constrained refits (the slots share one weight vector) or of bootstrap replicates
 // (every slot iterates on its own resampled counts).
 enum class EmKind { kRestarts, kRefit, kBootstrap };
+
+// The fp64-row form: L and the launch geometry of its passes (row_form).  The streaming pass
+// (em_pass_fast_kernel, em_pass_pair_kernel) runs when the rows fit its ring (n_stages > 0);
+// otherwise the general path (em_rowdot_kernel, em_colacc_kernel).
+struct RowForm {
+    DevBlock lin;              // [n_rows][ld] doubles; not allocated over class tiles
+    double *coef = nullptr;    // [n_rows] (general path)
+    int nc = 0;                // double2 column chunks per thread of the streaming pass
+    int n_stages = 0;
+    size_t smem_bytes = 0;
+    int grid = 0;
+    int row_blocks = 0, col_blocks = 0;   // general path
+};
 }  // namespace mxb
 
 struct mxb_em {
@@ -66,9 +78,7 @@ struct mxb_em {
     const mxb_matrix *mat = nullptr;
     int64_t n_rows = 0, n_cols = 0, ld = 0;
     bool sharded = false;
-    DevBlock lin;                 // [n_rows][ld] doubles
     double *weights = nullptr;    // [n_rows]
-    double *coef = nullptr;       // [n_rows] (general path)
     double *lnp[2] = {nullptr, nullptr};
     double *pi[2] = {nullptr, nullptr};
     double *partials = nullptr;   // [n_part][ld]
@@ -85,40 +95,16 @@ struct mxb_em {
     // of L, a slotted session R restarts per iteration.  Slot s lives at lnp[b] + s*ld,
     // pi[b] + s*ld, partials + s*n_part*ld, state + s (slot_block).
     int n_slots = 1;
-    // streaming pass (n_stages > 0 when the rows fit its ring)
-    int nc = 0;
-    int n_stages = 0;
-    size_t smem_bytes = 0;
-    int grid_fast = 0;
-    // general path
-    int row_blocks = 0, col_blocks = 0;
-    // Class tiles (em_tiles.cuh): form kTiles reads `tile_v` instead of `lin`.
-    int n_batches = 0, tile_hs = 0, tile_grid = 0;   // (the gather's blocks: n_part)
-    DevBlock tile_block;   // [perm][cmap][cword][desc]
-    DevBlock tile_vecs;    // [pi_cls][u_sum][ctas][segs][gather entries]
-    unsigned short *tile_perm = nullptr, *tile_cmap = nullptr;
-    unsigned int *tile_cword = nullptr;
-    TileDesc *tile_desc = nullptr;
-    TileCta *tile_ctas = nullptr;           // plan of the pass (em_tiles.cuh)
-    TileSeg *tile_segs = nullptr;
-    int *tile_ent_batch = nullptr;          // gather entries: batch and offset of every U vector
-    int64_t *tile_ent_off = nullptr;
-    int tile_n_ent = 0, tile_n_slots = 0;
-    uint32_t tile_slot_bytes = 0;
-    double *tile_pi = nullptr, *tile_usum = nullptr;
-    DevBlock tile_v;                       // the tiles (doubles)
-    int64_t tile_cells = 0;                // doubles in tile_v
-    int64_t tile_bytes_per_pass = 0;
+    RowForm rows;     // the fp64 rows (geometry set for every session)
+    TileForm tiles;   // form kTiles: class tiles (em_tiles.h) instead of rows.lin
     DevBlock small;   // one device block behind weights ... props_in (fewer driver calls)
     DevBlock slots;   // the slot block (slot_block)
     bool zero_iter = false;  // last iterate() ran no iteration
     // Slotted session (EmKind::kRefit, kBootstrap): n_slots restarts per launch, side by side
     // over class tiles.  A bootstrap session gives every slot its own weight vector (own_weights:
-    // slot_w, the resampled counts); the slots of a refit session share `weights`.  Over class
-    // tiles the slots' Pi and U vectors lie tile_pi_stride and tile_u_stride doubles apart.
+    // slot_w, the resampled counts); the slots of a refit session share `weights`.
     bool slotted = false, own_weights = false;
     double *slot_w = nullptr;
-    int64_t tile_pi_stride = 0, tile_u_stride = 0;
 };
 
 namespace mxb {
@@ -150,100 +136,10 @@ static decltype(&em_pass_pair_kernel<1>) pick_pair(int nc) {
 constexpr int kMaxPairNC = 6;   // 2 restarts x (pi + T) x NC double2 must fit 128 registers
 constexpr int kMaxSlots = kBootMaxSlots;
 
-// Launch with the programmatic-stream-serialization attribute (see pdl_wait): the kernel may
-// be scheduled before its predecessor in the stream has finished.  MXB_EM_NO_PDL=1 turns the
-// attribute off (plain stream order).
-// (set before a call to launch that kernel in plain stream order)
-static thread_local bool g_plain_launch = false;
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem,
-                              cudaStream_t s, Args... args) {
-    static const bool pdl_on = getenv("MXB_EM_NO_PDL") == nullptr;
-    const bool use_pdl = pdl_on && !g_plain_launch;
-    g_plain_launch = false;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = use_pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
-}
-
 // The weights slot `slot` iterates on: its resampled counts in a bootstrap session.
 static double *slot_weights(mxb_em *em, int slot) {
     return em->own_weights ? em->slot_w + slot * em->n_rows : em->weights;
 }
-
-// The class-sum kernel of a tiled iteration for `per` = ceil(H / kTileThreads) columns a thread.
-template <bool kSlots>
-static auto pick_tile_pi(int64_t n_cols) {
-    const int per = (int)ceil_div(n_cols, kTileThreads);
-    return per <= 4 ? tile_pi_kernel<4, kSlots> : per <= 8 ? tile_pi_kernel<8, kSlots>
-           : per <= 12 ? tile_pi_kernel<12, kSlots> : tile_pi_kernel<16, kSlots>;
-}
-
-// The pass of a tiled iteration: class sums, pass and gather.  kSlots: the R slots of a slotted
-// session side by side (weights n_rows apart, or shared), the slot in blockIdx.y (z for the
-// gather), all on one plan of num_sms / R CTAs; a slot whose control block says done costs
-// nothing.
-template <bool kSlots>
-static int enqueue_tile_pass(mxb_em *em, unsigned R, cudaEvent_t *marks) {
-    mxb_ctx *ctx = em->ctx;
-    cudaStream_t s = ctx->stream;
-    const int64_t pi_stride = kSlots ? em->tile_pi_stride : 0;
-    const int64_t u_stride = kSlots ? em->tile_u_stride : 0;
-    MXB_CUDA(launch_pdl(pick_tile_pi<kSlots>(em->n_cols),
-                        dim3(std::min(em->n_batches, std::max(1, 2 * ctx->num_sms / (int)R)), R),
-                        dim3(kTileThreads), (size_t)em->ld * sizeof(double), s,
-                        (const unsigned short *)em->tile_perm, (const unsigned int *)em->tile_cword,
-                        em->tile_hs, (int)em->n_cols, (const TileDesc *)em->tile_desc,
-                        em->n_batches, (const double *)em->pi[0], (const double *)em->pi[1],
-                        (const EmState *)em->state, em->tile_pi, kSlots ? em->ld : (int64_t)0,
-                        pi_stride));
-    if (marks) MXB_CUDA(cudaEventRecord(marks[0], s));
-    MXB_CUDA(launch_pdl(tile_pass_kernel<kSlots>, dim3(em->tile_grid, R), dim3(kTilePassThreads),
-                        kSlots ? kTilePassSlotSmem : kTilePassSmem, s, (const TileCta *)em->tile_ctas,
-                        (const TileSeg *)em->tile_segs, em->tile_v.get<const double>(),
-                        (const double *)em->tile_pi, em->state, em->tile_usum,
-                        em->tile_slot_bytes, em->tile_n_slots,
-                        (const double *)(kSlots ? slot_weights(em, 0) : nullptr),
-                        em->own_weights ? em->n_rows : (int64_t)0, pi_stride, u_stride));
-    if (marks) MXB_CUDA(cudaEventRecord(marks[1], s));
-    // The gather waits in plain stream order: launched early it would sit on the SMs the
-    // first CTAs of the pass leave and keep them from nothing, but measured it costs 27 us
-    // per iteration (B200, config 2), while the other three launches gain from the overlap.
-    g_plain_launch = true;
-    MXB_CUDA(launch_pdl(tile_gather_kernel<kSlots>,
-                        dim3((unsigned)ceil_div(em->ld, kGatherThreads), em->n_part, R),
-                        dim3(kGatherThreads), 0, s, (const unsigned short *)em->tile_cmap,
-                        em->tile_hs, (int)em->n_cols, em->ld, (const int *)em->tile_ent_batch,
-                        (const int64_t *)em->tile_ent_off, em->tile_n_ent,
-                        (const double *)em->tile_usum, (const EmState *)em->state, em->partials,
-                        u_stride));
-    if (marks) MXB_CUDA(cudaEventRecord(marks[2], s));
-    ctx->launches += 3;
-    return MXB_OK;
-}
-
-// Shared memory of the pass and of the class sums, set once per session.
-template <bool kSlots>
-static cudaError_t tile_pass_attrs(int64_t n_cols) {
-    cudaError_t e = cudaFuncSetAttribute((const void *)tile_pass_kernel<kSlots>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)(kSlots ? kTilePassSlotSmem : kTilePassSmem));
-    if (e != cudaSuccess) return e;
-    return cudaFuncSetAttribute((const void *)pick_tile_pi<kSlots>(n_cols),
-                                cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)(kTileMaxCols * sizeof(double)));
-}
-
-// Blocks of the gather over n_ent U vectors: the partial column sums the tail adds (n_part).
-static int tile_gather_parts(int n_ent) { return std::max(1, std::min(32, n_ent / 8)); }
 
 // The tail of an iteration of R slots (em->tail): column sums, M-step, control block.
 static int enqueue_tail(mxb_em *em, unsigned R) {
@@ -268,62 +164,66 @@ static int enqueue_tail(mxb_em *em, unsigned R) {
         pa.rank = ctx->rank;
         for (int r = 0; r < ctx->world; ++r) pa.block[r] = ctx->p2p_block[r];
     }
-    MXB_CUDA(launch_pdl(em->tail == EmTail::kPeer ? em_finish_kernel<true> : em_finish_kernel<false>,
-                        dim3(kFinCtas, R), dim3(kFinThreads), 0, s, em->partials, em->n_part,
-                        em->n_cols, em->ld, em->lnp[0], em->lnp[1], em->pi[0], em->pi[1],
-                        em->state, pa));
+    MXB_CUDA(launch_kernel(true, em->tail == EmTail::kPeer ? em_finish_kernel<true>
+                                                           : em_finish_kernel<false>,
+                           dim3(kFinCtas, R), dim3(kFinThreads), 0, s, em->partials, em->n_part,
+                           em->n_cols, em->ld, em->lnp[0], em->lnp[1], em->pi[0], em->pi[1],
+                           em->state, pa));
     ctx->launches += 1;
     return MXB_OK;
 }
 
 // One EM iteration on em->ctx->stream (no host sync): the pass of the session's form, then its
-// tail.  `marks` (optional, 3 events) are recorded after the class sums, after the pass and
-// after the gather of a tiled iteration (after the pass only for fp64 rows): per-kernel
-// attribution.
-static int enqueue_iteration(mxb_em *em, cudaEvent_t pass_begin = nullptr,
-                             cudaEvent_t pass_end = nullptr, cudaEvent_t *marks = nullptr) {
+// tail.  `marks` (optional, kMarks events) are recorded before the pass, after the class sums,
+// after the pass and after the gather of a tiled iteration (the three coincide after the pass
+// of fp64 rows), and after the tail: per-kernel attribution.
+constexpr int kMarks = 5;
+static int enqueue_iteration(mxb_em *em, const cudaEvent_t *marks = nullptr) {
     mxb_ctx *ctx = em->ctx;
     cudaStream_t s = ctx->stream;
     const unsigned R = (unsigned)em->n_slots;
+    const RowForm &rf = em->rows;
     // fp64 rows of a slotted session: one restart at a time, with the slot's weights
     const double *weights = slot_weights(em, 0);
-    if (pass_begin) MXB_CUDA(cudaEventRecord(pass_begin, s));
+    if (marks) MXB_CUDA(cudaEventRecord(marks[0], s));
     switch (em->form) {
     case EmForm::kTiles:
-        MXB_TRY(em->slotted ? enqueue_tile_pass<true>(em, R, marks)
-                         : enqueue_tile_pass<false>(em, R, marks));
+        MXB_TRY(tile_pass(ctx, em->tiles, R, em->n_cols, em->ld, em->pi, em->state, em->partials,
+                          weights, em->own_weights ? em->n_rows : (int64_t)0,
+                          marks ? marks + 1 : nullptr));
         break;
     case EmForm::kRowPairs:
-        MXB_CUDA(launch_pdl(pick_pair(em->nc), dim3(em->grid_fast), dim3(kPassThreads),
-                            em->smem_bytes, s, em->lin.get<const double>(), em->ld, em->n_rows, em->weights,
-                            em->pi[0], em->pi[1], em->pi[0] + em->ld, em->pi[1] + em->ld,
-                            em->state, em->partials,
-                            em->partials + (size_t)em->n_part * em->ld, em->n_stages));
+        MXB_CUDA(launch_kernel(true, pick_pair(rf.nc), dim3(rf.grid), dim3(kPassThreads),
+                               rf.smem_bytes, s, rf.lin.get<const double>(), em->ld, em->n_rows,
+                               em->weights, em->pi[0], em->pi[1], em->pi[0] + em->ld,
+                               em->pi[1] + em->ld, em->state, em->partials,
+                               em->partials + (size_t)em->n_part * em->ld, rf.n_stages));
         ctx->launches += 1;
         break;
     case EmForm::kRows:
-        MXB_CUDA(launch_pdl(pick_pass(em->nc), dim3(em->grid_fast), dim3(kPassThreads),
-                            em->smem_bytes, s, em->lin.get<const unsigned char>(),
-                            (uint32_t)(em->ld * sizeof(double)), em->ld, em->n_rows, weights,
-                            em->pi[0], em->pi[1], em->state, em->partials, em->n_stages));
+        MXB_CUDA(launch_kernel(true, pick_pass(rf.nc), dim3(rf.grid), dim3(kPassThreads),
+                               rf.smem_bytes, s, rf.lin.get<const unsigned char>(),
+                               (uint32_t)(em->ld * sizeof(double)), em->ld, em->n_rows, weights,
+                               em->pi[0], em->pi[1], em->state, em->partials, rf.n_stages));
         ctx->launches += 1;
         break;
     case EmForm::kGeneral: {
         const int rd_blocks = (int)std::max<int64_t>(
             1, std::min<int64_t>(ceil_div(em->n_rows, 8), (int64_t)ctx->num_sms * 8));
-        em_rowdot_kernel<<<rd_blocks, 256, 0, s>>>(em->lin.get<double>(), em->ld, em->n_rows, weights,
-                                                   em->pi[0], em->pi[1], em->state, em->coef);
-        dim3 grid(em->row_blocks, em->col_blocks);
-        em_colacc_kernel<<<grid, 256, 0, s>>>(em->lin.get<double>(), em->ld, em->n_rows, em->coef, em->state,
+        em_rowdot_kernel<<<rd_blocks, 256, 0, s>>>(rf.lin.get<double>(), em->ld, em->n_rows, weights,
+                                                   em->pi[0], em->pi[1], em->state, rf.coef);
+        dim3 grid(rf.row_blocks, rf.col_blocks);
+        em_colacc_kernel<<<grid, 256, 0, s>>>(rf.lin.get<double>(), em->ld, em->n_rows, rf.coef, em->state,
                                               em->partials);
         ctx->launches += 2;
         break;
     }
     }
-    if (pass_end) MXB_CUDA(cudaEventRecord(pass_end, s));
     if (marks && em->form != EmForm::kTiles)
-        for (int i = 0; i < 3; ++i) MXB_CUDA(cudaEventRecord(marks[i], s));
-    return enqueue_tail(em, R);
+        for (int i = 1; i < 4; ++i) MXB_CUDA(cudaEventRecord(marks[i], s));
+    MXB_TRY(enqueue_tail(em, R));
+    if (marks) MXB_CUDA(cudaEventRecord(marks[4], s));
+    return MXB_OK;
 }
 
 // Wall-clock stage times of the one-call entry points: collected into g_stage_ms when
@@ -399,45 +299,14 @@ static void slot_block(mxb_em *em, int R, int n_part, Carve &c) {
     em->state = c.part<EmState>(ns);
 }
 
-// Layout of the batches and ring of the pass for the class counts of n rows (tile_plan.h).
-struct TileShape {
-    std::vector<TileDesc> desc;
-    int64_t v_cells = 0, p_cells = 0;
-    uint32_t ring_bytes = 0;   // ring slots of the pass and their count (tile_ring)
-    int ring_slots = 0;
-    bool ring_ok = false;      // false: rows too long for the ring
-};
-static void tile_shape(const int32_t *n_cls, int nb, int64_t n, TileShape &t) {
-    int max_r_pad = 4;
-    tile_layout(n_cls, nb, n, t.desc, t.v_cells, t.p_cells, max_r_pad);
-    t.ring_ok = tile_ring(max_r_pad, t.ring_bytes, t.ring_slots);
-}
-// The same for class counts handed in from outside (mxb_tile_plan, mxb_boot_slots), checked
-// first; an error names the entry point `who`.
-static int tile_shape_checked(const char *who, const int32_t *n_cls, int64_t n_batches,
-                              int64_t n_rows, int32_t num_sms, TileShape &t) {
-    const char *bad = nullptr;
-    if (!(n_cls != nullptr && n_batches > 0 && n_rows > (n_batches - 1) * kTileRows &&
-          n_rows <= n_batches * kTileRows && num_sms > 0))
-        bad = "bad arguments";
-    for (int64_t b = 0; !bad && b < n_batches; ++b)
-        if (n_cls[b] < 1 || n_cls[b] > kTileMaxCols) bad = "class counts must be in 1..8192";
-    if (bad) {
-        set_error("%s: %s", who, bad);
-        return MXB_ERR_ARG;
-    }
-    tile_shape(n_cls, (int)n_batches, n_rows, t);
-    return MXB_OK;
-}
-
 // The session's form, slot count and tail (EmForm, EmTail, n_slots): decided here and nowhere
-// else.  `tiles`: the session iterates over class tiles (em_pack_tiles, once their class counts
+// else.  `tiles`: the session iterates over class tiles (tile_classify, once their class counts
 // are known; `plan` is their plan on all SMs).  A session whose tiles do not pay off is decided
 // again without them.
 static void decide_form(mxb_em *em, int want_slots, const TileShape *tiles = nullptr,
                         const TilePlanOut *plan = nullptr) {
     mxb_ctx *ctx = em->ctx;
-    const bool streams = em->n_stages > 0;
+    const bool streams = em->rows.n_stages > 0;
     const bool across = em->sharded && ctx->world > 1;
     const bool fused = streams && em->ld <= (int64_t)kFinCtas * kFinThreads &&
                        (!across || ctx->p2p_ready) && getenv("MXB_EM_SPLIT_TAIL") == nullptr;
@@ -460,7 +329,7 @@ static void decide_form(mxb_em *em, int want_slots, const TileShape *tiles = nul
                                  (double)free_b);
     } else if (!streams) {
         em->form = EmForm::kGeneral;
-    } else if (want_slots == 2 && fused && em->nc <= kMaxPairNC && !em->sharded) {
+    } else if (want_slots == 2 && fused && em->rows.nc <= kMaxPairNC && !em->sharded) {
         em->form = EmForm::kRowPairs;
         em->n_slots = 2;
     } else {
@@ -468,222 +337,28 @@ static void decide_form(mxb_em *em, int want_slots, const TileShape *tiles = nul
     }
 }
 
-template <int ITEMS>
-static cudaError_t launch_tile_class(mxb_ctx *ctx, int grid, const unsigned long long *hash, int hs,
-                                     int n_cols, int n_batches, unsigned short *perm,
-                                     unsigned int *cword, unsigned short *cmap,
-                                     unsigned short *rep, int *n_cls) {
-    using Sort = cub::BlockRadixSort<unsigned long long, kTileThreads, ITEMS, unsigned short>;
-    using Scan = cub::BlockScan<int, kTileThreads>;
-    const size_t smem = std::max(sizeof(typename Sort::TempStorage), sizeof(typename Scan::TempStorage));
-    cudaError_t e = cudaFuncSetAttribute((const void *)tile_class_kernel<ITEMS>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    tile_class_kernel<ITEMS><<<grid, kTileThreads, smem, ctx->stream>>>(hash, hs, n_cols, n_batches,
-                                                                        perm, cword, cmap, rep, n_cls);
-    return cudaGetLastError();
-}
-// The class kernel for `items` = ceil(H / kTileThreads) columns a thread.
-static auto pick_tile_class(int64_t n_cols) {
-    const int items = (int)ceil_div(n_cols, kTileThreads);
-    return items <= 4 ? launch_tile_class<4> : items <= 8 ? launch_tile_class<8>
-           : items <= 12 ? launch_tile_class<12> : launch_tile_class<16>;
-}
-
-// Class tiles of the session's matrix (em_tiles.cuh), built straight from M: no N x ld copy of
-// L is ever allocated when this succeeds (`built`).  The session's form is decided once the
-// class counts are known (decide_form).  Falls through (MXB_OK, built == false) when the matrix
-// does not compress to less than half of its fp64 rows, when memory is short, or when a batch
-// fails the exact class check; the caller then decides the form without tiles and sets up the
-// fp64 rows.  MXB_EM_NO_PACK=1 keeps the fp64 rows (cross-check).
-static int em_pack_tiles(mxb_em *em, int want_slots, bool &built) {
-    mxb_ctx *ctx = em->ctx;
-    built = false;
-    if (em->n_stages == 0 || em->n_rows == 0 || em->n_cols > kTileMaxCols ||
-        getenv("MXB_EM_NO_PACK"))
-        return MXB_OK;
-    const int64_t n = em->n_rows, h = em->n_cols;
-    const int nb = (int)ceil_div(n, kTileRows);
-    const int hs = (int)round_up(h, 8);
-    const bool verbose = getenv("MXB_TIMING") != nullptr;
-    auto give_up = [&](const char *what) {
-        if (verbose) fprintf(stderr, "[mxb tiles] not used: %s\n", what);
-        return MXB_OK;
-    };
-    auto fail = [&](const char *what, cudaError_t e) {
-        cudaGetLastError();
-        set_error("em_pack_tiles (%s): %s", what, cudaGetErrorString(e));
-        return e == cudaErrorMemoryAllocation ? MXB_ERR_NOMEM : MXB_ERR_CUDA;
-    };
-    // scratch: [hash][rep][n_cls][bad]
-    DevBlock scratch;
-    unsigned long long *hash = nullptr;
-    unsigned short *rep = nullptr;
-    int *d_ncls = nullptr, *d_bad = nullptr;
-    if (scratch.alloc_parts(ctx, __func__, [&](Carve &c) {
-            hash = c.part<unsigned long long>((size_t)nb * hs);
-            rep = c.part<unsigned short>((size_t)nb * hs);
-            d_ncls = c.part<int>(nb);
-            d_bad = c.part<int>(nb);
-        }) != MXB_OK)
-        return give_up("scratch");
-    // persistent: [perm][cmap][cword][desc]; the class vectors and the plan of the pass follow in
-    // a second block once the class counts are known
-    DevBlock maps;
-    unsigned short *perm = nullptr, *cmap = nullptr;
-    unsigned int *cword = nullptr;
-    TileDesc *d_desc = nullptr;
-    if (maps.alloc_parts(ctx, __func__, [&](Carve &c) {
-            perm = c.part<unsigned short>((size_t)nb * hs);
-            cmap = c.part<unsigned short>((size_t)nb * hs);
-            cword = c.part<unsigned int>((size_t)nb * kTileThreads);
-            d_desc = c.part<TileDesc>(nb);
-        }) != MXB_OK)
-        return give_up("maps");
-
-    const int grid = std::min(nb, ctx->num_sms * 2);
-    tile_hash_kernel<<<std::min(nb, ctx->num_sms * 4), kTileThreads, 0, ctx->stream>>>(
-        em->mat->data, n, h, nb, hash, hs);
-    cudaError_t e = cudaGetLastError();
-    if (e == cudaSuccess)
-        e = pick_tile_class(h)(ctx, grid, hash, hs, (int)h, nb, perm, cword, cmap, rep, d_ncls);
-    ctx->launches += 2;
-    std::vector<int> ncls((size_t)nb);
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(ncls.data(), d_ncls, (size_t)nb * sizeof(int), cudaMemcpyDeviceToHost,
-                            ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) return fail("classes", e);
-
-    // layout of the batches, ring geometry and plan of the pass (tile_plan.h)
-    TileShape shape;
-    tile_shape(ncls.data(), nb, n, shape);
-    if (!shape.ring_ok) return give_up("rows too long for the ring");
-    const std::vector<TileDesc> &desc = shape.desc;
-    const int64_t v_cells = shape.v_cells, p_cells = shape.p_cells;
-    const uint32_t slot_bytes = shape.ring_bytes;
-    const int n_slots = shape.ring_slots;
-    TilePlanOut plan;
-    tile_plan(desc, n, ctx->num_sms, slot_bytes, p_cells, plan);
-    decide_form(em, want_slots, &shape, &plan);
-    const int n_rep = em->n_slots;   // the slots of a slotted session
-    if (n_rep > 1) {
-        plan = TilePlanOut();
-        tile_plan(desc, n, ctx->num_sms / n_rep, slot_bytes, p_cells, plan);
-    }
-    const std::vector<TileCta> &ctas = plan.ctas;
-    const std::vector<TileSeg> &segs = plan.segs;
-    const std::vector<int> &ent_batch = plan.ent_batch;
-    const std::vector<int64_t> &ent_off = plan.ent_off;
-    const int64_t extra_cells = plan.extra_cells;
-    const int n_copy = plan.n_copy;
-    const int n_cta = (int)ctas.size(), n_seg = (int)segs.size();
-    const int n_ent = (int)ent_batch.size();
-    const int64_t u_cells = p_cells + extra_cells;
-    const double tile_bytes = (double)v_cells * 8 + 3.0 * (double)nb * hs * 2 +
-                              ((double)p_cells + (double)u_cells) * 8 * 2;
-    const double fp64_bytes = (double)n * (double)em->ld * 8;
-    if (verbose) {
-        fprintf(stderr, "[mxb tiles] plan check: %d errors\n", tile_plan_check(desc, plan));
-        int64_t c_sum = 0, c_max = 0, wide = 0;
-        for (int b = 0; b < nb; ++b) {
-            c_sum += desc[(size_t)b].n_cls;
-            c_max = std::max<int64_t>(c_max, desc[(size_t)b].n_cls);
-            wide += desc[(size_t)b].lg > 5;
+// Launch geometry of the fp64-row passes of an n_rows x ld session: the streaming pass when a
+// ring of at least kPassGroup + 1 rows fits the shared memory (and MXB_EM_FORCE_GENERAL is not
+// set), else the general path.  Returns the blocks of column-sum partials of the pass (n_part).
+static int row_form(const mxb_ctx *ctx, int64_t n_rows, int64_t ld, RowForm &r) {
+    const size_t row_bytes = (size_t)ld * sizeof(double);
+    const size_t fixed = 2 * kPassWarps * kPassGroup * sizeof(double) + 8 * sizeof(uint64_t) + 128;
+    const bool force_general = getenv("MXB_EM_FORCE_GENERAL") != nullptr;
+    r.nc = (int)ceil_div(ld / 2, kPassThreads);
+    if (!force_general && ld >= 1024 && r.nc <= kMaxNC && ctx->smem_optin > fixed) {
+        int stages = (int)std::min<size_t>(8, (ctx->smem_optin - fixed) / row_bytes);
+        if (stages >= kPassGroup + 1) {
+            r.n_stages = stages;
+            r.smem_bytes = (size_t)stages * row_bytes + fixed;
+            r.grid = (int)std::max<int64_t>(1, std::min<int64_t>(ctx->num_sms, n_rows));
+            return r.grid;
         }
-        {
-            double mx = 0, mn = 1e30; int smx = 0, cmx = 0;
-            for (const TileCta &c : ctas) {
-                double by = 0;
-                for (int q = 0; q < c.n_segs; ++q) by += (double)segs[(size_t)(c.seg0 + q)].n_rows * segs[(size_t)(c.seg0 + q)].r_pad * 8;
-                mx = std::max(mx, by); mn = std::min(mn, by); smx = std::max(smx, c.n_segs); cmx = std::max(cmx, c.n_copies);
-            }
-            fprintf(stderr, "[mxb tiles] per CTA: bytes min %.0f max %.0f, segments max %d, copies max %d\n", mn, mx, smx, cmx);
-        }
-        fprintf(stderr, "[mxb tiles] %d batches of %d rows: classes mean %.1f max %lld, %lld wide "
-                "batches, tiles %.3f GB (+ maps and vectors: %.3f GB) vs fp64 rows %.3f GB; %d CTAs, "
-                "%d segments, %d copies, %d slots of %u B\n",
-                nb, kTileRows, (double)c_sum / nb, (long long)c_max, (long long)wide,
-                (double)v_cells * 8 / 1e9, tile_bytes / 1e9, fp64_bytes / 1e9, n_cta, n_seg, n_copy,
-                n_slots, slot_bytes);
     }
-    if (tile_bytes > 0.5 * fp64_bytes) return give_up("not worth it");
-
-    // [Pi x n_rep][U x n_rep][plan]
-    DevBlock v, vecs;
-    double *pi_cls = nullptr, *u_sum = nullptr;
-    TileCta *d_ctas = nullptr;
-    TileSeg *d_segs = nullptr;
-    int *d_entb = nullptr;
-    int64_t *d_ento = nullptr;
-    int64_t pi_stride = 0, u_stride = 0;
-    size_t b_vecs = 0;
-    if (v.alloc(ctx, (size_t)v_cells * sizeof(double), __func__) != MXB_OK ||
-        vecs.alloc_parts(ctx, __func__, [&](Carve &c) {
-            pi_cls = c.parts<double>(p_cells, n_rep, &pi_stride);
-            u_sum = c.parts<double>(u_cells, n_rep, &u_stride);
-            b_vecs = c.bytes();
-            d_ctas = c.part<TileCta>(n_cta);
-            d_segs = c.part<TileSeg>(n_seg);
-            d_entb = c.part<int>(n_ent);
-            d_ento = c.part<int64_t>(n_ent);
-        }) != MXB_OK)
-        return give_up("tiles");
-    e = cudaMemcpyAsync(d_desc, desc.data(), (size_t)nb * sizeof(TileDesc), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(d_ctas, ctas.data(), (size_t)n_cta * sizeof(TileCta), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(d_segs, segs.data(), (size_t)n_seg * sizeof(TileSeg), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(d_entb, ent_batch.data(), (size_t)n_ent * sizeof(int), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(d_ento, ent_off.data(), (size_t)n_ent * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(pi_cls, 0, b_vecs, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(d_bad, 0, (size_t)nb * sizeof(int), ctx->stream);
-    if (e == cudaSuccess) {
-        tile_fill_kernel<<<std::min(nb, ctx->num_sms * 4), kTileThreads, 0, ctx->stream>>>(
-            em->mat->data, h, d_desc, nb, cmap, rep, hs, (const double *)em->weights,
-            v.get<double>(), d_bad);
-        ctx->launches += 1;
-        e = cudaGetLastError();
-    }
-    std::vector<int> bad((size_t)nb);
-    if (e == cudaSuccess)
-        e = cudaMemcpyAsync(bad.data(), d_bad, (size_t)nb * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e == cudaSuccess) e = em->slotted ? tile_pass_attrs<true>(h) : tile_pass_attrs<false>(h);
-    if (e != cudaSuccess) return fail("fill", e);
-    for (int b = 0; b < nb; ++b)
-        if (bad[(size_t)b] != 0) return give_up("hash collision");
-
-    built = true;
-    em->n_batches = nb;
-    em->tile_hs = hs;
-    em->tile_block = std::move(maps);
-    em->tile_vecs = std::move(vecs);
-    em->tile_v = std::move(v);
-    em->tile_perm = perm;
-    em->tile_cmap = cmap;
-    em->tile_cword = cword;
-    em->tile_desc = d_desc;
-    em->tile_ctas = d_ctas;
-    em->tile_segs = d_segs;
-    em->tile_ent_batch = d_entb;
-    em->tile_ent_off = d_ento;
-    em->tile_n_ent = n_ent;
-    em->tile_slot_bytes = slot_bytes;
-    em->tile_n_slots = n_slots;
-    em->tile_usum = u_sum;
-    em->tile_pi = pi_cls;
-    em->tile_cells = v_cells;
-    em->tile_grid = n_cta;
-    em->n_part = tile_gather_parts(n_ent);
-    em->tile_pi_stride = pi_stride;
-    em->tile_u_stride = u_stride;
-    // what an iteration reads and writes: the tiles, perm + cmap (Pi), cmap (gather), the class
-    // vectors (Pi written and read, U written and read)
-    em->tile_bytes_per_pass = v_cells * 8 + 3 * (int64_t)nb * hs * 2 + 2 * (p_cells + u_cells) * 8;
-    return MXB_OK;
+    r.col_blocks = (int)ceil_div(ld / 2, 256);
+    int64_t rb = std::max<int64_t>(1, (int64_t)ctx->num_sms * 4 / r.col_blocks);
+    rb = std::min<int64_t>(rb, ceil_div(n_rows, 16));
+    r.row_blocks = (int)std::max<int64_t>(1, rb);
+    return r.row_blocks;
 }
 
 static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weights, int sharded,
@@ -705,28 +380,9 @@ static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weigh
     em->slotted = kind != EmKind::kRestarts;
     em->own_weights = kind == EmKind::kBootstrap;
 
-    // launch geometry
-    const size_t row_bytes = (size_t)em->ld * sizeof(double);
-    const size_t fixed = 2 * kPassWarps * kPassGroup * sizeof(double) + 8 * sizeof(uint64_t) + 128;
-    const bool force_general = getenv("MXB_EM_FORCE_GENERAL") != nullptr;
-    em->nc = (int)ceil_div(em->ld / 2, kPassThreads);
-    if (!force_general && em->ld >= 1024 && em->nc <= kMaxNC && ctx->smem_optin > fixed) {
-        int stages = (int)std::min<size_t>(8, (ctx->smem_optin - fixed) / row_bytes);
-        if (stages >= kPassGroup + 1) {
-            em->n_stages = stages;
-            em->smem_bytes = (size_t)stages * row_bytes + fixed;
-            em->grid_fast = (int)std::max<int64_t>(1, std::min<int64_t>(ctx->num_sms, em->n_rows));
-            em->n_part = em->grid_fast;
-        }
-    }
-    const bool streams = em->n_stages > 0;
-    if (!streams) {
-        em->col_blocks = (int)ceil_div(em->ld / 2, 256);
-        int64_t rb = std::max<int64_t>(1, (int64_t)ctx->num_sms * 4 / em->col_blocks);
-        rb = std::min<int64_t>(rb, ceil_div(em->n_rows, 16));
-        em->row_blocks = (int)std::max<int64_t>(1, rb);
-        em->n_part = em->row_blocks;
-    }
+    em->n_part = row_form(ctx, em->n_rows, em->ld, em->rows);
+    RowForm &rf = em->rows;
+    const bool streams = rf.n_stages > 0;
 
     // both blocks >= kCacheMinBlock: reused from the pool's cache, no cudaMalloc/cudaFree per session
     const char *who = "mxb_em_create";
@@ -734,7 +390,7 @@ static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weigh
     // flag][props_in]
     MXB_TRY(em->small.alloc_parts(ctx, who, [&](Carve &c) {
         em->weights = c.part<double>(em->n_rows);
-        if (!streams) em->coef = c.part<double>(em->n_rows);
+        if (!streams) rf.coef = c.part<double>(em->n_rows);
         em->tsum = c.part<double>(em->ld + 1);
         em->props_in = c.part<double>(em->n_cols);
     }, kCacheMinBlock));
@@ -745,30 +401,43 @@ static int em_create_impl(mxb_ctx *ctx, const mxb_matrix *m, const double *weigh
         set_error("%s: cannot pin %zu bytes of host memory", who, kPinnedScratchBytes);
         return MXB_ERR_NOMEM;
     }
-    if (em->n_rows > 0)   // (tile_fill_kernel reads them)
+    if (em->n_rows > 0)   // (tile_fill reads them)
         MXB_CUDA(cudaMemcpyAsync(em->weights, weights, em->n_rows * sizeof(double),
                                  cudaMemcpyHostToDevice, ctx->stream));
     MXB_CUDA(cudaStreamSynchronize(ctx->stream));
-    // class tiles straight from M; only a matrix that does not compress gets fp64 rows of L
+    // class tiles straight from M in a session whose rows stream (not the general path); only a
+    // matrix that does not compress gets fp64 rows of L
     bool tiled = false;
-    MXB_TRY(em_pack_tiles(em.get(), want_slots, tiled));
+    {
+        TileClasses classes;
+        if (streams) MXB_TRY(tile_classify(ctx, m, classes, tiled));
+        if (tiled) {
+            decide_form(em.get(), want_slots, &classes.shape, &classes.plan);
+            MXB_TRY(tile_fill(ctx, m, em->weights, em->ld, em->n_slots, em->slotted, classes,
+                              tiled));
+        }
+        if (tiled) {
+            em->tiles = std::move(classes.form);
+            em->n_part = tile_gather_parts(em->tiles.n_ent);
+        }
+    }
     if (!tiled) decide_form(em.get(), want_slots);
     if (streams)
-        MXB_CUDA(cudaFuncSetAttribute((const void *)pick_pass(em->nc),
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)em->smem_bytes));
+        MXB_CUDA(cudaFuncSetAttribute((const void *)pick_pass(rf.nc),
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rf.smem_bytes));
     if (em->form == EmForm::kRowPairs)
-        MXB_CUDA(cudaFuncSetAttribute((const void *)pick_pair(em->nc),
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)em->smem_bytes));
+        MXB_CUDA(cudaFuncSetAttribute((const void *)pick_pair(rf.nc),
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rf.smem_bytes));
     MXB_TRY(em->slots.alloc_parts(ctx, who, [&](Carve &c) {
         slot_block(em.get(), em->n_slots, em->n_part, c);
     }, kCacheMinBlock));
     MXB_CUDA(cudaMemsetAsync(em->state, 0, em->n_slots * sizeof(EmState), ctx->stream));
     if (!tiled) {
-        MXB_TRY(em->lin.alloc(ctx, (size_t)em->n_rows * row_bytes, who));
+        MXB_TRY(rf.lin.alloc(ctx, (size_t)em->n_rows * em->ld * sizeof(double), who));
         if (em->n_rows > 0) {
             const int grid = (int)std::min<int64_t>(em->n_rows, (int64_t)ctx->num_sms * 8);
             to_linear_kernel<<<grid, 256, 0, ctx->stream>>>(m->data, em->n_rows, em->n_cols, em->ld,
-                                                            em->lin.get<double>());
+                                                            rf.lin.get<double>());
             ctx->launches++;
             MXB_CUDA(cudaGetLastError());
         }
@@ -793,7 +462,7 @@ int mxb_em_pass_bytes(const mxb_em *em, int64_t *bytes_per_pass, int64_t *n_dens
     MXB_REQUIRE(em != nullptr, "NULL argument");
     const int64_t row_bytes = em->ld * (int64_t)sizeof(double);
     if (bytes_per_pass && em->form == EmForm::kTiles) {
-        *bytes_per_pass = em->tile_bytes_per_pass;
+        *bytes_per_pass = em->tiles.bytes_per_pass;
         if (n_dense_rows) *n_dense_rows = 0;
         return MXB_OK;
     }
@@ -976,6 +645,32 @@ static int launch_read_mix(mxb_em *em, const double *lnp, mxb_matrix *dst, int m
     return MXB_OK;
 }
 
+// The timed runs of mxb_em_iterate_fixed and mxb_em_profile: n_iter iterations from the
+// session's proportions that never converge, enqueued without a host sync.  `evs` (created
+// here; event errors name `who`) gets the start and the end of the run, then with `marked` the
+// kMarks marks of every iteration (enqueue_iteration).
+static int enqueue_fixed(mxb_em *em, int64_t n_iter, bool marked, Events &evs, const char *who) {
+    cudaStream_t s = em->ctx->stream;
+    em->zero_iter = false;
+    MXB_TRY(reset_state(em, (long long)1 << 60, -1.0));
+    MXB_TRY(evs.create(2 + (marked ? kMarks * (size_t)n_iter : 0), cudaEventDefault, who));
+    MXB_CUDA(cudaEventRecord(evs[0], s));
+    for (int64_t i = 0; i < n_iter; ++i)
+        MXB_TRY(enqueue_iteration(em, marked ? evs.data() + 2 + kMarks * i : nullptr));
+    MXB_CUDA(cudaEventRecord(evs[1], s));
+    return MXB_OK;
+}
+// Milliseconds from mark a to mark b of every iteration of enqueue_fixed, summed.
+static int marks_ms(Events &evs, int64_t n_iter, int a, int b, double &total) {
+    total = 0.0;
+    for (int64_t i = 0; i < n_iter; ++i) {
+        float ms = 0.f;
+        MXB_CUDA(cudaEventElapsedTime(&ms, evs[2 + kMarks * i + a], evs[2 + kMarks * i + b]));
+        total += ms;
+    }
+    return MXB_OK;
+}
+
 }  // namespace mxb
 
 extern "C" {
@@ -1018,17 +713,8 @@ int mxb_em_iterate_fixed(mxb_em *em, int64_t n_iter, float *elapsed_ms, float *p
     MXB_REQUIRE(em != nullptr && n_iter >= 1 && n_iter <= 100000, "bad argument");
     mxb_ctx *ctx = em->ctx;
     MXB_CUDA(cudaSetDevice(ctx->device));
-    em->zero_iter = false;
-    MXB_TRY(reset_state(em, (long long)1 << 60, -1.0));
-    // [start][end] of the run, then [begin][end] of every pass (pass_ms)
     Events evs;
-    MXB_TRY(evs.create(2 + (pass_ms ? 2 * (size_t)n_iter : 0), cudaEventDefault, __func__));
-    MXB_CUDA(cudaEventRecord(evs[0], ctx->stream));
-    for (int64_t i = 0; i < n_iter; ++i) {
-        if (pass_ms) MXB_TRY(enqueue_iteration(em, evs[2 + 2 * i], evs[3 + 2 * i]));
-        else MXB_TRY(enqueue_iteration(em));
-    }
-    MXB_CUDA(cudaEventRecord(evs[1], ctx->stream));
+    MXB_TRY(enqueue_fixed(em, n_iter, pass_ms != nullptr, evs, __func__));
     MXB_CUDA(cudaMemcpyAsync(&em->host_state[0], em->state, sizeof(EmState),
                              cudaMemcpyDeviceToHost, ctx->stream));
     MXB_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -1048,54 +734,8 @@ int mxb_em_iterate_fixed(mxb_em *em, int64_t n_iter, float *elapsed_ms, float *p
     if (elapsed_ms) MXB_CUDA(cudaEventElapsedTime(elapsed_ms, evs[0], evs[1]));
     if (pass_ms) {
         double total = 0.0;
-        for (int64_t i = 0; i < n_iter; ++i) {
-            float ms = 0.f;
-            MXB_CUDA(cudaEventElapsedTime(&ms, evs[2 + 2 * i], evs[3 + 2 * i]));
-            total += ms;
-        }
+        MXB_TRY(marks_ms(evs, n_iter, 0, 3, total));   // the pass: before it to after the gather
         *pass_ms = (float)total;
-    }
-    return MXB_OK;
-}
-
-#ifdef MXB_TILE_TRACE
-extern "C" int mxb_debug_tile_trace(unsigned long long *out, size_t n_words) {
-    cudaDeviceSynchronize();
-    return (int)cudaMemcpyFromSymbol(out, mxb::g_tile_trace, std::min(n_words * 8, sizeof(mxb::g_tile_trace)));
-}
-#endif
-
-int mxb_tile_plan(const int32_t *n_cls, int64_t n_batches, int64_t n_rows, int32_t num_sms,
-                  int32_t *seg_out, int64_t seg_cap, int32_t *n_cta, int32_t *n_seg,
-                  int32_t *n_slots_out, int32_t *slot_bytes_out, int32_t *errors) {
-    TileShape t;
-    MXB_TRY(tile_shape_checked(__func__, n_cls, n_batches, n_rows, num_sms, t));
-    const std::vector<TileDesc> &desc = t.desc;
-    if (n_slots_out) *n_slots_out = t.ring_slots;
-    if (slot_bytes_out) *slot_bytes_out = (int32_t)t.ring_bytes;
-    MXB_REQUIRE(t.ring_ok, "rows too long for the ring");
-    TilePlanOut plan;
-    tile_plan(desc, n_rows, num_sms, t.ring_bytes, t.p_cells, plan);
-    if (n_cta) *n_cta = (int32_t)plan.ctas.size();
-    if (n_seg) *n_seg = (int32_t)plan.segs.size();
-    if (errors) *errors = tile_plan_check(desc, plan);
-    if (seg_out) {
-        int64_t k = 0;
-        for (size_t c = 0; c < plan.ctas.size(); ++c) {
-            for (int q = 0; q < plan.ctas[c].n_segs && k < seg_cap; ++q, ++k) {
-                const TileSeg &g = plan.segs[(size_t)(plan.ctas[c].seg0 + q)];
-                const TileDesc &d = desc[(size_t)g.batch];
-                int32_t *o = seg_out + 8 * k;
-                o[0] = (int32_t)c;
-                o[1] = g.batch;
-                o[2] = (int32_t)((g.v_off - d.v_off) / d.r_pad);     // first row inside the batch
-                o[3] = g.n_rows;
-                o[4] = g.fit;
-                o[5] = g.n_copies;
-                o[6] = g.lg;
-                o[7] = g.r_pad;
-            }
-        }
     }
     return MXB_OK;
 }
@@ -1105,24 +745,11 @@ int mxb_em_profile(mxb_em *em, int64_t n_iter, float *ms_out) {
     MXB_REQUIRE(em->n_slots == 1, "single-restart sessions only");
     mxb_ctx *ctx = em->ctx;
     MXB_CUDA(cudaSetDevice(ctx->device));
-    em->zero_iter = false;
-    MXB_TRY(reset_state(em, (long long)1 << 60, -1.0));
     Events evs;
-    MXB_TRY(evs.create((size_t)n_iter * 5, cudaEventDefault, __func__));
-    for (int64_t i = 0; i < n_iter; ++i) {
-        cudaEvent_t *e = evs.data() + (size_t)i * 5;
-        MXB_TRY(enqueue_iteration(em, e[0], nullptr, e + 1));
-        MXB_CUDA(cudaEventRecord(e[4], ctx->stream));
-    }
+    MXB_TRY(enqueue_fixed(em, n_iter, true, evs, __func__));
     MXB_CUDA(cudaStreamSynchronize(ctx->stream));
-    double tot[4] = {0, 0, 0, 0};
-    for (int64_t i = 0; i < n_iter; ++i) {
-        for (int k = 0; k < 4; ++k) {
-            float ms = 0.f;
-            MXB_CUDA(cudaEventElapsedTime(&ms, evs[(size_t)i * 5 + k], evs[(size_t)i * 5 + k + 1]));
-            tot[k] += ms;
-        }
-    }
+    double tot[4] = {0, 0, 0, 0};   // class sums, pass, gather, tail
+    for (int k = 0; k < 4; ++k) MXB_TRY(marks_ms(evs, n_iter, k, k + 1, tot[k]));
     // fp64 rows: the three marks coincide after the pass, so [0] holds the pass
     if (em->form != EmForm::kTiles) { tot[1] = tot[0]; tot[0] = 0.0; }
     for (int k = 0; k < 4; ++k) ms_out[k] = (float)(tot[k] / (double)n_iter);
@@ -1213,7 +840,7 @@ constexpr int64_t kOutRows = 4096;
 // lnprops_out (host; downloaded one window of kOutRows tasks at a time), and finish(k, result)
 // is called.  With max_iter <= 0 em.py:126's loop body never runs: every task hands back its
 // start (em.py:141-143) and nothing is launched on the slots.  Over class tiles the slots of a
-// slotted session iterate side by side (enqueue_tile_pass<true>), over fp64 rows one at a time;
+// slotted session iterate side by side (tile_pass), over fp64 rows one at a time;
 // the two slots of a run_em session iterate two restarts per read of L.
 template <typename SetUp, typename Finish>
 static int run_tasks(mxb_em *em, int64_t n_tasks, int64_t max_iter, double tol,
@@ -1409,17 +1036,6 @@ static int run_slotted(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
 }  // namespace mxb
 
 extern "C" {
-
-int mxb_boot_slots(const int32_t *n_cls, int64_t n_batches, int64_t n_rows, int32_t num_sms,
-                   double bytes_per_slot, double free_bytes, int32_t *slots_out) {
-    MXB_REQUIRE(slots_out != nullptr, "bad arguments");
-    TileShape t;
-    MXB_TRY(tile_shape_checked(__func__, n_cls, n_batches, n_rows, num_sms, t));
-    MXB_REQUIRE(t.ring_ok, "rows too long for the ring");
-    *slots_out = boot_slots(t.desc, n_rows, num_sms, t.ring_bytes, t.p_cells, bytes_per_slot,
-                            free_bytes);
-    return MXB_OK;
-}
 
 int mxb_em_bootstrap(mxb_ctx *ctx, const mxb_matrix *m, const double *weights,
                      const double *start_lnprops, int64_t boot0, int64_t n_boot, uint64_t seed,

@@ -1,4 +1,4 @@
-// Class tiles: the EM pass over column classes instead of columns (csrc/em.cu: em_pack_tiles).
+// Class tiles: the EM pass over column classes instead of columns (host side: em_tiles.cu).
 //
 // A fragment covers ~78 of the 4070 variant positions, so over a batch of neighbouring
 // signature rows (the rows arrive string-sorted, preprocess.py:219: neighbours start at the
@@ -34,26 +34,17 @@
 #include <cub/block/block_radix_sort.cuh>
 #include <cub/block/block_scan.cuh>
 
-#include "em_kernels.cuh"
+#include "block_reduce.cuh"
+#include "em_common.cuh"
+#include "row_likelihood.cuh"
+#include "tile_plan.h"
 
 namespace mxb {
 
-constexpr int kTileRows = 128;       // signature rows per batch
 constexpr int kTileThreads = 512;
 constexpr int kTileWarps = kTileThreads / 32;
 constexpr int kTileMaxNK = 8;        // double2 per thread and row
 constexpr int kTileMaxCols = 8192;   // widest matrix (the fast path's limit on ld)
-
-struct TileDesc {           // one batch
-    int32_t row0, n_rows;
-    int32_t n_cls;          // classes
-    int32_t r_pad;          // row stride of its tile = length of its class vectors in doubles:
-                            // n_cls + 1 (the row's weight) rounded up to 4 (32-byte sectors)
-    int32_t lg;             // log2 of the threads that handle a row in the pass
-    int32_t pad0, pad1, pad2;
-    int64_t v_off;          // tile offset in V (doubles)
-    int64_t p_off;          // offset of the batch's class vectors Pi_b and U_b (doubles)
-};
 
 __device__ __forceinline__ uint64_t tile_mix(uint64_t h, uint64_t v) {
     h = (h ^ v) * 0xFF51AFD7ED558CCDull;
@@ -325,7 +316,7 @@ tile_pi_kernel(const unsigned short *__restrict__ perm, const unsigned int *__re
 
 // ---- the pass ------------------------------------------------------------------------------
 // Every CTA owns one contiguous range of rows (ranges of equal cost, fixed when the tiles are
-// built: em.cu) and streams it through a CTA-wide shared-memory ring of 1-D bulk async copies
+// built: em_tiles.cu) and streams it through a CTA-wide shared-memory ring of 1-D bulk async copies
 // (cp.async.bulk + mbarrier complete_tx) of whole rows, up to a slot per copy, in row order;
 // the warp that is the last to finish with a slot issues the copy that takes it next from a
 // cursor every warp keeps.  The 16 warps work on the rows of one batch (segment) at a time.
@@ -343,10 +334,7 @@ tile_pi_kernel(const unsigned short *__restrict__ perm, const unsigned int *__re
 // kernel adds them like two batches.
 constexpr int kTileConsumers = kTileWarps;
 constexpr int kTilePassThreads = kTileThreads;
-constexpr int kTileRingBytes = 160 * 1024;
-constexpr int kTileSlotBytes = 52 * 1024;                        // default slot: three per ring
 constexpr int kTileScratchBytes = 64 * 1024;                     // [row slices][class vector]
-constexpr int kTileMaxSlots = 6;                                 // named barriers 10..15
 constexpr int kTileSlotBarrier0 = 10;
 constexpr size_t kTilePassSmem = kTileRingBytes + kTileScratchBytes +
                                  2 * kTileMaxSlots * sizeof(uint64_t) +
@@ -357,25 +345,6 @@ constexpr size_t kTileWeightsOff = kTileRingBytes + kTileScratchBytes +
                                    2 * kTileMaxSlots * sizeof(uint64_t) +
                                    2 * kTileWarps * sizeof(double);
 constexpr size_t kTilePassSlotSmem = kTilePassSmem + 2 * kTileRows * sizeof(double);
-
-struct TileSeg {           // the rows of one batch inside one CTA's range
-    int64_t v_off;         // its first row in V (doubles)
-    int64_t p_off;         // Pi_b (doubles)
-    int64_t u_dst;         // where the segment's column sums go (doubles in u_sum)
-    int32_t r_pad;         // row stride of the tile = length of the class vectors (doubles)
-    int32_t n_cls;         // classes; column n_cls of a row holds the row's weight
-    int32_t lg;            // log2 of the threads per row: 3, 4, 5 (one warp), 6..9 (2..16 warps)
-    int32_t n_rows;
-    int32_t fit, n_copies; // rows per copy (the last one takes what is left), copies
-    int32_t batch;
-    int32_t row0;          // global index of its first row (the weight of a bootstrap slot)
-    int32_t pad[2];
-};
-static_assert(sizeof(TileSeg) == 64, "one record per 64-byte line");
-
-struct TileCta {           // one per CTA: its segments
-    int32_t seg0, n_segs, n_copies, pad;
-};
 
 struct TileCursor {        // the copy that takes a freed slot: n_slots copies ahead of the warps
     int64_t v_off;

@@ -1,5 +1,5 @@
-// Host side of the class tiles (em_tiles.cuh): layout of the batches and plan of the pass.
-// Plain C++ over the records the kernels read; em.cu calls it from em_pack_tiles, and
+// Host side of the class tiles (em_tiles.cuh): the records the kernels read, layout of the
+// batches and plan of the pass.  Plain C++; em_tiles.cu builds a session's tiles with it, and
 // mxb_tile_plan (include/mixemt_b200.h) exposes it to the CPU tests.
 #pragma once
 
@@ -7,9 +7,45 @@
 #include <cstring>
 #include <vector>
 
-#include "em_tiles.cuh"
+#include "common.cuh"
 
 namespace mxb {
+
+constexpr int kTileRows = 128;       // signature rows per batch
+// the ring of the pass (tile_ring)
+constexpr int kTileRingBytes = 160 * 1024;
+constexpr int kTileSlotBytes = 52 * 1024;                        // default slot: three per ring
+constexpr int kTileMaxSlots = 6;                                 // named barriers 10..15
+
+struct TileDesc {           // one batch
+    int32_t row0, n_rows;
+    int32_t n_cls;          // classes
+    int32_t r_pad;          // row stride of its tile = length of its class vectors in doubles:
+                            // n_cls + 1 (the row's weight) rounded up to 4 (32-byte sectors)
+    int32_t lg;             // log2 of the threads that handle a row in the pass
+    int32_t pad0, pad1, pad2;
+    int64_t v_off;          // tile offset in V (doubles)
+    int64_t p_off;          // offset of the batch's class vectors Pi_b and U_b (doubles)
+};
+
+struct TileSeg {           // the rows of one batch inside one CTA's range
+    int64_t v_off;         // its first row in V (doubles)
+    int64_t p_off;         // Pi_b (doubles)
+    int64_t u_dst;         // where the segment's column sums go (doubles in u_sum)
+    int32_t r_pad;         // row stride of the tile = length of the class vectors (doubles)
+    int32_t n_cls;         // classes; column n_cls of a row holds the row's weight
+    int32_t lg;            // log2 of the threads per row: 3, 4, 5 (one warp), 6..9 (2..16 warps)
+    int32_t n_rows;
+    int32_t fit, n_copies; // rows per copy (the last one takes what is left), copies
+    int32_t batch;
+    int32_t row0;          // global index of its first row (the weight of a bootstrap slot)
+    int32_t pad[2];
+};
+static_assert(sizeof(TileSeg) == 64, "one record per 64-byte line");
+
+struct TileCta {           // one per CTA: its segments
+    int32_t seg0, n_segs, n_copies, pad;
+};
 
 struct TilePlanOut {
     std::vector<TileCta> ctas;

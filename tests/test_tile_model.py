@@ -90,7 +90,7 @@ def test_tile_iteration_equals_reference_iteration(phylo17, num_sms):
 
 def test_rows_in_random_order_do_not_compress(phylo17):
     """The same rows shuffled: neighbouring rows no longer share column classes, which is why
-    such a session keeps fp64 rows (em.cu: tiles must save at least half of the bytes)."""
+    such a session keeps fp64 rows (em_tiles.cu: tiles must save at least half of the bytes)."""
     haps = sorted(phylo17.hap_var)
     mix = synth.make_mixture(phylo17, phylo17.refseq, [("H1", 0.6), ("L3e", 0.4)], 1500, seed=4)
     tables = HapVarBaseMatrix(phylo17.refseq, phylo17, haps).pack()

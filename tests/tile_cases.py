@@ -24,8 +24,8 @@ _SEED = 0x243F6A8885A308D3
 
 
 def per_of(h):
-    """Entries of the sorted columns one thread of tile_pi_kernel sums (em.cu: launch_tile_class
-    and the class-sum launch take ITEMS = 4, 8, 12 or 16 from ceil(H / 512))."""
+    """Entries of the sorted columns one thread of tile_pi_kernel sums (em_tiles.cu:
+    launch_tile_class and the class-sum launch take ITEMS = 4, 8, 12 or 16 from ceil(H / 512))."""
     items = -(-h // 512)
     return 4 if items <= 4 else 8 if items <= 8 else 12 if items <= 12 else 16
 
@@ -132,7 +132,7 @@ def class_matrix(ncls, h, n_rows, sizes, seed, dead=False, dying=False):
 
 
 def predicted_pass_bytes(ncls, n_rows, h, num_sms=NUM_SMS):
-    """What mxb_em_pass_bytes reports for a session over class tiles (em.cu: em_pack_tiles):
+    """What mxb_em_pass_bytes reports for a session over class tiles (em_tiles.cu: tile_pass_bytes):
     the tiles, perm + cmap for the class sums and cmap for the gather, and the class vectors Pi
     and U, each written and read.  A segment that starts inside its batch has a U vector of its
     own."""
